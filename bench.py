@@ -2,7 +2,7 @@
 """bench.py -- DLRM training samples/s on synthetic Criteo-shaped data (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload terabyte|kaggle|sweep] [--batch B] [--no-cpu-baseline]
+                    [--workload terabyte|kaggle|sweep] [--batch B] [--no-cpu-baseline] [--dump-outputs DIR]
 
 A "step" is one DLRM training step on one batch: embedding lookup -> bottom MLP -> dot
 interaction -> top MLP -> BCE -> backward (interaction pullback) -> dense SGD -> sparse
@@ -297,7 +297,7 @@ def run_reference(args):
         print(json.dumps({"impl": "reference", "unavailable": "the sweep workload has no CPU arm (run terabyte / kaggle)"}), flush=True)
         return
     wl = workload(args.workload, args.batch)
-    r = cpu_arm(wl, args.steps, args.warmup, args.cpu_rows_cap, budget_s=120.0)
+    r = cpu_arm(wl, args.steps, args.warmup, args.cpu_rows_cap, budget_s=float("inf"))   # exactly --steps timed steps
     line = {
         "impl": "reference", "metric": "dlrm_train_samples_per_sec", "value": r["value"], "unit": "samples/s",
         "n_gpus": args.gpus, "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -566,11 +566,13 @@ def run_ours(args):
     sampler.begin()
     e0.record()
     for i in range(K):
-        run_step(*devb[W + i])
+        last_loss_d = run_step(*devb[W + i])
     e1.record()
     barrier()
     sampler.end()
     launches = launch_count() - n0
+    if args.dump_outputs and rank == 0:     # now: the launch count and the timing passes below train further
+        dump_outputs(args.dump_outputs, last_loss_d, pflat, flat.flat, se, devb[W + K - 1][2])
     if graph is not None:   # replays do not pass through the host-side counter: count per captured step
         n1 = launch_count()
         train_step(*devb[0])
@@ -807,6 +809,33 @@ def run_ours(args):
     if world > 1:
         torch.cuda.synchronize()
         os._exit(0)
+
+
+DUMP_SAMPLES = 2048
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, loss, params, grads, se, idx):
+    """--dump-outputs: what the last timed step computed, as float32 .npy files: its loss, the MLP parameters
+    after its dense SGD, their gradients, and the embedding rows it looked up, read after its sparse SGD
+    ([tables of this rank][samples][D]; at most DUMP_SAMPLES of the batch's samples, a fixed seeded choice).
+    The batches and the initial weights are seeded, so two builds run with the same arguments can be
+    compared file for file."""
+    import torch
+    B = idx.shape[1]
+    pick = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_SAMPLES), replace=False))
+    sel = torch.from_numpy(pick).to(idx.device)
+    rows = torch.stack([se.tables.table(j)[idx[k, sel, 0].long()] for j, k in enumerate(se.local_ids)])
+    out = {"loss": loss.reshape(1), "dense_params": params, "dense_grads": grads, "embedding_rows": rows}
+    out = {n: t.detach().float().cpu().numpy() for n, t in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for n, a in out.items():
+        np.save(os.path.join(path, f"{n}.npy"), a)
+    print(f"[bench] outputs of the last timed step -> {path}: "
+          + ", ".join(f"{n}{list(a.shape)}" for n, a in out.items()), file=sys.stderr)
 
 
 OWN_KERNELS = {"lookup", "sort", "update", "update_fixup", "interaction_fwd", "interaction_bwd", "bce", "indices_scatter"}
@@ -1216,7 +1245,14 @@ def main():
     ap.add_argument("--no-host-leg", action="store_true", help="skip the e2e_host leg (hot path through the *_host entry points)")
     ap.add_argument("--opt", action="append", default=[],
                     help="library switch name=value (dlrmb_set_option) for A/B runs; recorded in config.library_options")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, MLP parameters and gradients, the embedding rows "
+                         "it looked up after the update) to DIR/<name>.npy, float32, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "sweep"):
+        ap.error("--dump-outputs applies to the GPU training step (--impl ours, terabyte or kaggle workload)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -158,16 +158,15 @@ def test_model_constants_match_reference():
 
 
 def test_hdf5_reader_and_natural_sort():
-    """The pure-Python HDF5 reader round-trips the committed goldens' source files when the
-    reference checkout is present, and layer names sort as the reference's NaturalSort does."""
+    """The pure-Python HDF5 reader reads every dataset of a file with the goldens' container shape
+    (tests/golden/hdf5_sample.h5), and layer names sort as the reference's NaturalSort does."""
+    from dlrm_jl_b200.hdf5_min import read_hdf5
     from dlrm_jl_b200.validation import _natural
+    from tests.helpers import hdf5_sample_arrays
     names = ["update_bot_10.weight", "update_bot_2.weight", "update_bot_0.weight"]
     assert sorted(names, key=_natural) == ["update_bot_0.weight", "update_bot_2.weight", "update_bot_10.weight"]
-    ref = "/root/reference/ref/pytorch_reference_single.hdf5"
-    if os.path.exists(ref):
-        from dlrm_jl_b200.hdf5_min import read_hdf5
-        d = read_hdf5(ref)
-        g = np.load(os.path.join(ROOT, "tests", "golden", "pytorch_reference_single.npz"))
-        assert sorted(d) == sorted(g.files) and len(d) == 58
-        for k in d:
-            assert np.array_equal(d[k], g[k]), k
+    d = read_hdf5(os.path.join(ROOT, "tests", "golden", "hdf5_sample.h5"))
+    want = hdf5_sample_arrays()
+    assert sorted(d) == sorted(want)
+    for k in d:
+        assert d[k].dtype == want[k].dtype and np.array_equal(d[k], want[k]), k

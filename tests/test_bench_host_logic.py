@@ -90,6 +90,28 @@ def test_hot_path_report_has_the_contract_keys():
     assert "back_to_back_us" not in rep2["kernels"]["update"] and rep2["kernels"]["update"]["in_step_us"] == 24.0
 
 
+def test_dump_outputs_writes_the_last_step_as_float32(tmp_path):
+    """--dump-outputs: loss, MLP parameters, gradients and the looked-up rows of this rank's tables, float32;
+    a batch larger than DUMP_SAMPLES is sampled the same way every run."""
+    gen = torch.Generator().manual_seed(0)
+    tables = [torch.randn(50, 8, generator=gen), torch.randn(70, 8, generator=gen)]
+    se = types.SimpleNamespace(local_ids=[1], tables=types.SimpleNamespace(table=lambda j: tables[1 + j]))
+    B = bench.DUMP_SAMPLES + 100
+    idx = torch.stack([torch.randint(0, 50, (B, 1), generator=gen), torch.randint(0, 70, (B, 1), generator=gen)]).int()
+    params, grads = torch.randn(33, generator=gen), torch.randn(33, generator=gen)
+    bench.dump_outputs(str(tmp_path / "a"), torch.tensor(0.5), params, grads, se, idx)
+    out = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("loss", "dense_params", "dense_grads", "embedding_rows")}
+    assert all(a.dtype == np.float32 for a in out.values())
+    assert out["loss"].tolist() == [0.5] and np.array_equal(out["dense_params"], params.numpy())
+    assert np.array_equal(out["dense_grads"], grads.numpy())
+    rows = out["embedding_rows"]
+    assert rows.shape == (1, bench.DUMP_SAMPLES, 8)
+    pick = np.sort(np.random.default_rng(0).choice(B, size=bench.DUMP_SAMPLES, replace=False))
+    assert np.array_equal(rows[0], tables[1][idx[1, pick, 0].long()].numpy())
+    bench.dump_outputs(str(tmp_path / "b"), torch.tensor(0.5), params, grads, se, idx)
+    assert np.array_equal(np.load(tmp_path / "b" / "embedding_rows.npy"), rows)
+
+
 def test_cpu_arm_thread_count_ignores_the_launcher_omp_setting(monkeypatch):
     """torch.distributed.run exports OMP_NUM_THREADS=1; the CPU arm must still use the host's cores."""
     import os
