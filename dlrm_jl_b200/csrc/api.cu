@@ -177,6 +177,7 @@ int32_t dlrmb_tables_create_ex(int32_t device, int32_t ntab, const int64_t* rows
     t->cap = (max_lookups + 3) / 4 * 4;
     t->sm_count = device_sm_count(device);
     t->h_rows = (int64_t*)malloc(sizeof(int64_t) * ntab);
+    t->h_sorted_P = (int32_t*)malloc(sizeof(int32_t) * ntab);
     t->h_offsets = (int64_t*)malloc(sizeof(int64_t) * (ntab + 1));
     int64_t off = 0;
     for (int k = 0; k < ntab; ++k) {
@@ -244,6 +245,7 @@ int32_t dlrmb_tables_destroy(dlrmb_tables* t) {
     cudaFree(t->stage_d);
     if (t->own_stream) cudaStreamDestroy(t->own_stream);
     free(t->h_rows);
+    free(t->h_sorted_P);
     free(t->h_offsets);
     delete t;
     return DLRMB_OK;
@@ -366,6 +368,7 @@ int32_t dlrmb_embedding_fwd_sort(dlrmb_tables* t, const void* idx, int32_t idx_b
     rc = launch_lookup_sort(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, (cudaStream_t)stream);
     if (rc) return rc;
     t->sorted_valid = true;
+    t->sorted_mp = false;
     t->sorted_B = B;
     t->sorted_P = P;
     return DLRMB_OK;
@@ -453,6 +456,7 @@ int32_t dlrmb_embedding_sort(dlrmb_tables* t, const void* idx, int32_t idx_bytes
     rc = launch_sort(t, idx, idx_bytes, idx_base, B, P, (cudaStream_t)stream);
     if (rc) return rc;
     t->sorted_valid = true;
+    t->sorted_mp = false;
     t->sorted_B = B;
     t->sorted_P = P;
     return DLRMB_OK;
@@ -491,7 +495,7 @@ int32_t dlrmb_sort_dedup_export(dlrmb_tables* t, int32_t k, int64_t* uniq, int32
     DLRMB_CUDA(cudaDeviceSynchronize());
     int rc = launch_dedup_export(t, k, t->own_stream);
     if (rc) return rc;
-    int64_t L = (int64_t)t->sorted_B * t->sorted_P;
+    int64_t L = sorted_lookups(t, k);
     int32_t n = 0;
     DLRMB_CUDA(cudaMemcpyAsync(&n, t->d_nuniq, sizeof(int32_t), cudaMemcpyDeviceToHost, t->own_stream));
     DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
@@ -640,8 +644,170 @@ int32_t dlrmb_embedding_bwd_sgd_host(dlrmb_tables* t, const void* idx, int32_t i
     t->sorted_valid = false;
     if ((rc = launch_sort(t, t->stage_idx, idx_bytes, idx_base, B, P, t->own_stream))) return rc;
     t->sorted_valid = true;
+    t->sorted_mp = false;
     t->sorted_B = B;
     t->sorted_P = P;
+    if ((rc = launch_update(t, t->stage_a, slots, slot0, lr, t->own_stream))) return rc;
+    DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
+    return DLRMB_OK;
+}
+
+// ---- per-table pooling factors (`_mp`) -----------------------------------------------------------
+static int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, const int32_t* P,
+                         MpGeom* g) {
+    DLRMB_REQUIRE(idx != nullptr, "idx is null");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(idx_base == 0 || idx_base == 1, "idx_base must be 0 or 1 (got %d)", idx_base);
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    DLRMB_REQUIRE(t->ntab <= kMpMaxTables, "per-table pooling factors support up to %d tables (handle has %d)",
+                  kMpMaxTables, t->ntab);
+    DLRMB_REQUIRE(B > 0, "B must be positive (got %d)", B);
+    int64_t off = 0;
+    int32_t maxP = 0;
+    for (int k = 0; k < t->ntab; ++k) {
+        DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+        maxP = P[k] > maxP ? P[k] : maxP;
+        g->P[k] = (uint32_t)P[k];
+        g->off[k] = off;
+        off += (int64_t)B * P[k];
+    }
+    DLRMB_REQUIRE((int64_t)B * maxP <= t->max_lookups, "B*max(P) = %lld exceeds max_lookups = %lld",
+                  (long long)B * maxP, (long long)t->max_lookups);
+    g->ntab = t->ntab;
+    g->B = (uint32_t)B;
+    g->nlist = 0;
+    return DLRMB_OK;
+}
+
+static int64_t mp_index_count(const MpGeom& g) { return (int64_t)g.off[g.ntab - 1] + (int64_t)g.B * g.P[g.ntab - 1]; }
+
+static void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g) {
+    t->sorted_valid = true;
+    t->sorted_mp = true;
+    t->sorted_B = (int)g.B;
+    t->sorted_P = 0;
+    for (int k = 0; k < g.ntab; ++k) t->h_sorted_P[k] = (int32_t)g.P[k];
+}
+
+int32_t dlrmb_mp_max_tables(void) { return kMpMaxTables; }
+
+int32_t dlrmb_embedding_fwd_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                               const int32_t* P, float* out, int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(out != nullptr, "out is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
+                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
+    return launch_lookup_mp(t, idx, idx_bytes, idx_base, g, out, slots, slot0, (cudaStream_t)stream);
+}
+
+int32_t dlrmb_embedding_fwd_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                    const int32_t* P, float* out, int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(out != nullptr, "out is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
+                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
+    t->sorted_valid = false;
+    rc = launch_lookup_sort_mp(t, idx, idx_bytes, idx_base, g, out, slots, slot0, (cudaStream_t)stream);
+    if (rc) return rc;
+    mark_sorted_mp(t, g);
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_embedding_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                const int32_t* P, dlrmb_stream stream) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    t->sorted_valid = false;
+    rc = launch_sort_mp(t, idx, idx_bytes, idx_base, g, 0, sort_mp_final_half(t, g), (cudaStream_t)stream);
+    if (rc) return rc;
+    mark_sorted_mp(t, g);
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_embedding_bwd_sgd_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                   const int32_t* P, const float* dT, int32_t slots, int32_t slot0, float lr,
+                                   dlrmb_stream stream) {
+    int rc = dlrmb_embedding_sort_mp(t, idx, idx_bytes, idx_base, B, P, stream);
+    if (rc) return rc;
+    return dlrmb_embedding_update_sorted(t, dT, slots, slot0, lr, stream);
+}
+
+int32_t dlrmb_check_indices_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                               const int32_t* P, int32_t idx_on_host) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    const void* d_idx = idx;
+    size_t bytes = (size_t)mp_index_count(g) * idx_bytes;
+    if (idx_on_host) {
+        rc = grow(&t->stage_idx, &t->stage_idx_bytes, bytes);
+        if (rc) return rc;
+        DLRMB_CUDA(cudaMemcpyAsync(t->stage_idx, idx, bytes, cudaMemcpyHostToDevice, t->own_stream));
+        d_idx = t->stage_idx;
+    } else {
+        DLRMB_CUDA(cudaDeviceSynchronize());
+    }
+    long long bt = -1, bp = -1, bv = 0;
+    rc = launch_check_indices_mp(t, d_idx, idx_bytes, idx_base, g, t->own_stream, &bt, &bp, &bv);
+    if (rc) return rc;
+    if (bt >= 0) {
+        set_error("index out of range: table %lld, flat position %lld, value %lld not in [%d, %lld]",
+                  bt, bp, bv, idx_base, (long long)t->h_rows[bt] - 1 + idx_base);
+        return DLRMB_EOOB;
+    }
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_embedding_fwd_mp_host(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                    const int32_t* P, float* out, int32_t slots, int32_t slot0) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(out != nullptr, "out is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab, "slots too small");
+    size_t ibytes = (size_t)mp_index_count(g) * idx_bytes;
+    size_t obytes = sizeof(float) * (size_t)B * slots * t->D;
+    if ((rc = grow(&t->stage_idx, &t->stage_idx_bytes, ibytes))) return rc;
+    DLRMB_CUDA(cudaMemcpyAsync(t->stage_idx, idx, ibytes, cudaMemcpyHostToDevice, t->own_stream));
+    if ((rc = grow((void**)&t->stage_a, &t->stage_a_bytes, obytes))) return rc;
+    if (slot0 > 0)  // reserved slots are the caller's (x); keep whatever the host buffer holds
+        DLRMB_CUDA(cudaMemcpyAsync(t->stage_a, out, obytes, cudaMemcpyHostToDevice, t->own_stream));
+    rc = launch_lookup_mp(t, t->stage_idx, idx_bytes, idx_base, g, t->stage_a, slots, slot0, t->own_stream);
+    if (rc) return rc;
+    DLRMB_CUDA(cudaMemcpyAsync(out, t->stage_a, obytes, cudaMemcpyDeviceToHost, t->own_stream));
+    DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_embedding_bwd_sgd_mp_host(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                        int32_t B, const int32_t* P, const float* dT, int32_t slots, int32_t slot0,
+                                        float lr) {
+    GUARD(t);
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B, P, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(dT != nullptr, "dT is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab, "slots too small");
+    size_t ibytes = (size_t)mp_index_count(g) * idx_bytes;
+    size_t gb = sizeof(float) * (size_t)B * slots * t->D;
+    if ((rc = grow(&t->stage_idx, &t->stage_idx_bytes, ibytes))) return rc;
+    DLRMB_CUDA(cudaMemcpyAsync(t->stage_idx, idx, ibytes, cudaMemcpyHostToDevice, t->own_stream));
+    if ((rc = grow((void**)&t->stage_a, &t->stage_a_bytes, gb))) return rc;
+    DLRMB_CUDA(cudaMemcpyAsync(t->stage_a, dT, gb, cudaMemcpyHostToDevice, t->own_stream));
+    t->sorted_valid = false;
+    if ((rc = launch_sort_mp(t, t->stage_idx, idx_bytes, idx_base, g, 0, sort_mp_final_half(t, g), t->own_stream)))
+        return rc;
+    mark_sorted_mp(t, g);
     if ((rc = launch_update(t, t->stage_a, slots, slot0, lr, t->own_stream))) return rc;
     DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
     return DLRMB_OK;

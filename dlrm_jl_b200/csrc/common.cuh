@@ -132,6 +132,35 @@ constexpr int kSmemSortMax = 16384;
 // Largest per-table lookup count whose sort rides in the lookup launch (256-thread sort CTAs).
 constexpr int kFusedSortMax = 4096;
 
+// Per-table pooling factors (the `_mp` entry points).  Table k's indices are the [B][P_k] block at
+// element off[k] = B * (P_0 + .. + P_{k-1}).  The geometry reaches the kernels by value as one
+// kernel-parameter struct (about 7 KB at kMpMaxTables; sm_100 accepts up to 32 KB), so a call needs no
+// device copy and stays graph-capturable.  `pre` is a prefix over tables of the CTAs (lookup) or chunks
+// (update) each table owns; a CTA finds its table by binary search in it.  `list` names the tables of
+// one sort launch, `units` counts per-table radix tiles or update tiles.
+constexpr int kMpMaxTables = 256;
+struct MpGeom {
+    int ntab;
+    uint32_t B;
+    int nlist;                          // entries of `list` used by this launch
+    uint32_t P[kMpMaxTables];
+    int64_t off[kMpMaxTables];
+    uint32_t pre[kMpMaxTables + 1];
+    uint16_t list[kMpMaxTables];
+    uint32_t units[kMpMaxTables];
+};
+
+// the table k whose range [pre[k], pre[k+1]) holds x (pre strictly increasing, pre[0] = 0)
+__device__ __forceinline__ int mp_find(const uint32_t* pre, int ntab, uint32_t x) {
+    int lo = 0, hi = ntab - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (pre[mid] <= x) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
 // Process-wide tuning / test switches (dlrmb_set_option); read by the launchers, never from the
 // environment.
 struct Options {
@@ -188,6 +217,8 @@ struct dlrmb_tables {
     // state of the last sort
     bool sorted_valid = false;
     int sorted_B = 0, sorted_P = 0;
+    bool sorted_mp = false;                   // the last sort was a `_mp` one: h_sorted_P holds P_k
+    int32_t* h_sorted_P = nullptr;            // [ntab], host
 
     // host-entry-point staging (device side), grown on demand
     void* stage_idx = nullptr;  size_t stage_idx_bytes = 0;
@@ -229,6 +260,22 @@ int launch_dense_fwd_bias_act(float* z, const float* bias, int B, int N, int rel
 int64_t dense_bwd_scratch_floats(int N);
 int launch_dense_bwd_act_bias(const float* dy, const float* y, int B, int N, float* dz, float* db,
                               float* scratch, cudaStream_t s);
+// `_mp` forms: `g` carries ntab, B, P and off filled in; the launchers fill the rest of their copy
+int launch_lookup_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                     float* out, int slots, int slot0, cudaStream_t s);
+int launch_lookup_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                          float* out, int slots, int slot0, cudaStream_t s);
+// sort of every table with L_k > skip_max (0 = all tables); keys[] / pos[] half `half` receives the result
+int launch_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g, int64_t skip_max,
+                   int half, cudaStream_t s);
+int sort_mp_final_half(const dlrmb_tables* t, const MpGeom& g);
+int launch_update_mp(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s);
+int launch_check_indices_mp(dlrmb_tables* t, const void* d_idx, int idx_bytes, int idx_base, const MpGeom& g,
+                            cudaStream_t s, long long* bad_table, long long* bad_pos, long long* bad_val);
+// lookups of table k in the last sort
+static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) {
+    return (int64_t)t->sorted_B * (t->sorted_mp ? t->h_sorted_P[k] : t->sorted_P);
+}
 int device_sm_count(int device);
 int64_t update_tiles_cap(int ntab, int D, int64_t max_lookups, int sm_count);
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per (kernel, device)

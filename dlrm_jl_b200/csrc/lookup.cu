@@ -283,6 +283,173 @@ int launch_lookup_sort(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_
               : launch_lookup_sort_t<int64_t, float>(t, p, idx_base, B, P, out, slots, slot0, s);
 }
 
+// ---- per-table pooling factors -----------------------------------------------------------------
+// One flat grid of gather CTAs; table k owns CTAs [g.pre[k], g.pre[k+1]), handed out in proportion to its
+// work B * P_k * C (lookup_grid_mp), so a hotness-100 table does not form the tail behind one-hot tables
+// holding the same number of CTAs.  The bodies are the uniform path's, pointed at table k (desc + k, its
+// index block, its output slot): P_k == 1 takes the U-chain gather, every other table the pooling loop.
+template <typename IdxT, int VEC, int U, typename RowT>
+__device__ __forceinline__ void lookup_mp_cta(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx,
+                                              int idx_base, const MpGeom& g, uint32_t C, int cshift,
+                                              float* __restrict__ out, int slots, int slot0, uint32_t lin) {
+    const int k = mp_find(g.pre, g.ntab, lin);
+    const uint32_t cx = lin - g.pre[k], nx = g.pre[k + 1] - g.pre[k];
+    const IdxT* ik = idx + g.off[k];
+    if (g.P[k] == 1)
+        lookup_gather_body<IdxT, VEC, U, RowT>(desc + k, ik, idx_base, g.B, C, cshift, out, slots, slot0 + k, 0, cx, nx);
+    else
+        lookup_pool_body<IdxT, VEC, RowT>(desc + k, ik, idx_base, g.B, g.P[k], C, cshift, out, slots, slot0 + k, 0, cx, nx);
+}
+
+template <typename IdxT, int VEC, int U, typename RowT>
+__global__ void __launch_bounds__(256)
+lookup_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
+                 const __grid_constant__ MpGeom g, uint32_t C, int cshift, float* __restrict__ out, int slots,
+                 int slot0, unsigned long long* clk) {
+    clock_in(clk, blockIdx.x);
+    lookup_mp_cta<IdxT, VEC, U, RowT>(desc, idx, idx_base, g, C, cshift, out, slots, slot0, blockIdx.x);
+    clock_out(clk, blockIdx.x);
+}
+
+// Training-step form: the first g.nlist CTAs sort the tables g.list[] (L_k <= kFusedSortMax) in shared
+// memory, as lookup_sort_kernel does for a uniform batch; the rest gather.
+template <typename IdxT, int U, typename RowT, int ITEMS>
+__global__ void __launch_bounds__(256, 5)
+lookup_sort_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
+                      const __grid_constant__ MpGeom g, uint32_t C, int cshift, float* __restrict__ out, int slots,
+                      int slot0, uint32_t* __restrict__ keys_out, uint32_t* __restrict__ pos_out, int64_t cap,
+                      unsigned long long* clk) {
+    extern __shared__ uint32_t sort_smem[];
+    clock_in(clk, blockIdx.x);
+    if ((int)blockIdx.x < g.nlist) {
+        const int k = g.list[blockIdx.x];
+        sort_small_body<IdxT, ITEMS, 256>(idx + g.off[k], idx_base, (int)(g.B * g.P[k]), desc[k].rows,
+                                          keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, sort_smem);
+        clock_out(clk, blockIdx.x);
+        return;
+    }
+    lookup_mp_cta<IdxT, 4, U, RowT>(desc, idx, idx_base, g, C, cshift, out, slots, slot0, blockIdx.x - g.nlist);
+    clock_out(clk, blockIdx.x);
+}
+
+// Gather CTAs per table: the uniform path's launch budget (32 CTAs per SM) split in proportion to B * P_k * C,
+// at least one per table and no more than the table has work items for.  Returns the total.
+static int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift) {
+    constexpr int U = 4;
+    int64_t sumP = 0;
+    for (int k = 0; k < g.ntab; ++k) sumP += g.P[k];
+    const int64_t budget = (int64_t)t->sm_count * 32;
+    const int64_t n = (int64_t)g.B * C;
+    int64_t total = 0;
+    for (int k = 0; k < g.ntab; ++k) {
+        const int64_t most = ceil_div64(n, 256 * (g.P[k] == 1 ? U : 1));
+        int64_t c = ceil_div64(budget * g.P[k], sumP);
+        if (c > most) c = most;
+        if (c < 1) c = 1;
+        g.pre[k] = (uint32_t)total;
+        total += c;
+    }
+    g.pre[g.ntab] = (uint32_t)total;
+    *cshift = -1;
+    if ((C & (C - 1)) == 0) {
+        int sh = 0;
+        while ((1u << sh) < C) ++sh;
+        *cshift = sh;
+    }
+    return total;
+}
+
+template <typename IdxT, int VEC, typename RowT>
+static int launch_lookup_mp_t(dlrmb_tables* t, const IdxT* idx, int idx_base, const MpGeom& g0, float* out,
+                              int slots, int slot0, cudaStream_t s) {
+    const uint32_t C = t->D / VEC;
+    DLRMB_REQUIRE((int64_t)g0.B * C < (1ll << 30), "B * D too large for one lookup launch");
+    MpGeom g = g0;
+    g.nlist = 0;
+    int cshift;
+    const int64_t ctas = lookup_grid_mp(t, g, C, &cshift);
+    lookup_mp_kernel<IdxT, VEC, 4, RowT><<<(unsigned)ctas, 256, 0, s>>>(t->d_desc, idx, idx_base, g, C, cshift, out, slots,
+                                                                       slot0, clock_slot(CLK_LOOKUP));
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename RowT>
+static int launch_lookup_mp_r(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                              float* out, int slots, int slot0, cudaStream_t s) {
+    const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    if (idx_bytes == 4) {
+        const uint32_t* p = static_cast<const uint32_t*>(idx);
+        return vec4 ? launch_lookup_mp_t<uint32_t, 4, RowT>(t, p, idx_base, g, out, slots, slot0, s)
+                    : launch_lookup_mp_t<uint32_t, 1, RowT>(t, p, idx_base, g, out, slots, slot0, s);
+    }
+    const int64_t* p = static_cast<const int64_t*>(idx);
+    return vec4 ? launch_lookup_mp_t<int64_t, 4, RowT>(t, p, idx_base, g, out, slots, slot0, s)
+                : launch_lookup_mp_t<int64_t, 1, RowT>(t, p, idx_base, g, out, slots, slot0, s);
+}
+
+int launch_lookup_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                     float* out, int slots, int slot0, cudaStream_t s) {
+    if (t->elem_bytes == 2)
+        return launch_lookup_mp_r<__nv_bfloat16>(t, idx, idx_bytes, idx_base, g, out, slots, slot0, s);
+    return launch_lookup_mp_r<float>(t, idx, idx_bytes, idx_base, g, out, slots, slot0, s);
+}
+
+template <typename IdxT, typename RowT, int ITEMS>
+static int launch_lookup_sort_mp_i(dlrmb_tables* t, const IdxT* idx, int idx_base, const MpGeom& g, float* out,
+                                   int slots, int slot0, int half, cudaStream_t s) {
+    const uint32_t C = t->D / 4;
+    int cshift;
+    MpGeom gg = g;
+    const int64_t ctas = lookup_grid_mp(t, gg, C, &cshift) + g.nlist;
+    constexpr size_t smem = SmallSortGeom<ITEMS, 256>::smem_bytes();
+    static unsigned long long attr_done = 0;
+    int rc = ensure_smem_attr((const void*)lookup_sort_mp_kernel<IdxT, 4, RowT, ITEMS>, (int)smem, &attr_done);
+    if (rc) return rc;
+    lookup_sort_mp_kernel<IdxT, 4, RowT, ITEMS><<<(unsigned)ctas, 256, smem, s>>>(
+        t->d_desc, idx, idx_base, gg, C, cshift, out, slots, slot0, t->keys[half], t->pos[half], t->cap,
+        clock_slot(CLK_LOOKUP));
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+// lookup + sort for the next update.  Tables with L_k <= kFusedSortMax are sorted by extra CTAs of the
+// lookup launch, the others by the stand-alone sort launches that follow (one shared-memory launch for
+// L_k <= kSmemSortMax, radix passes above); every table's sorted stream ends in the same ping-pong half.
+int launch_lookup_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                          float* out, int slots, int slot0, cudaStream_t s) {
+    DLRMB_REQUIRE((int64_t)g.B * (t->D / 4) < (1ll << 30), "B * D too large for one lookup launch");
+    const int half = sort_mp_final_half(t, g);
+    const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    MpGeom gs = g;
+    gs.nlist = 0;
+    int64_t fused_max = 0;
+    if (vec4)
+        for (int k = 0; k < g.ntab; ++k) {
+            const int64_t L = (int64_t)g.B * g.P[k];
+            if (L <= kFusedSortMax) {
+                gs.list[gs.nlist++] = (uint16_t)k;
+                if (L > fused_max) fused_max = L;
+            }
+        }
+    int rc;
+    if (gs.nlist == 0) {
+        rc = launch_lookup_mp(t, idx, idx_bytes, idx_base, g, out, slots, slot0, s);
+        if (rc) return rc;
+        return launch_sort_mp(t, idx, idx_bytes, idx_base, g, 0, half, s);
+    }
+    const bool bf = t->elem_bytes == 2;
+    const bool small = fused_max <= 2048;
+#define DLRMB_LSMP(IdxT, RowT)                                                                                      \
+    (small ? launch_lookup_sort_mp_i<IdxT, RowT, 8>(t, static_cast<const IdxT*>(idx), idx_base, gs, out, slots, slot0, half, s) \
+           : launch_lookup_sort_mp_i<IdxT, RowT, 16>(t, static_cast<const IdxT*>(idx), idx_base, gs, out, slots, slot0, half, s))
+    if (idx_bytes == 4) rc = bf ? DLRMB_LSMP(uint32_t, __nv_bfloat16) : DLRMB_LSMP(uint32_t, float);
+    else rc = bf ? DLRMB_LSMP(int64_t, __nv_bfloat16) : DLRMB_LSMP(int64_t, float);
+#undef DLRMB_LSMP
+    if (rc) return rc;
+    return launch_sort_mp(t, idx, idx_bytes, idx_base, g, kFusedSortMax, half, s);
+}
+
 // ---- ScaledUniform init (src/model/model.jl:61-65): U(-1/sqrt(rows), 1/sqrt(rows)) ------------
 __device__ __forceinline__ uint64_t mix64(uint64_t z) {
     z += 0x9E3779B97F4A7C15ull;
@@ -385,6 +552,58 @@ int launch_check_indices(dlrmb_tables* t, const void* d_idx, int idx_bytes, int 
     *bad_table = (long long)(h[0] >> 40);
     *bad_pos = (long long)(h[0] & ((1ull << 40) - 1));
     const char* src = (const char*)d_idx + ((size_t)*bad_table * L + (size_t)*bad_pos) * idx_bytes;
+    int64_t v64 = 0;
+    uint32_t v32 = 0;
+    if (idx_bytes == 4) {
+        DLRMB_CUDA(cudaMemcpy(&v32, src, 4, cudaMemcpyDeviceToHost));
+        v64 = v32;
+    } else {
+        DLRMB_CUDA(cudaMemcpy(&v64, src, 8, cudaMemcpyDeviceToHost));
+    }
+    *bad_val = (long long)v64;
+    return DLRMB_OK;
+}
+
+template <typename IdxT>
+__global__ void __launch_bounds__(256)
+check_indices_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
+                        const __grid_constant__ MpGeom g, unsigned long long* __restrict__ bad) {
+    const int k = blockIdx.y;
+    const int64_t rows = desc[k].rows;
+    const int64_t L = (int64_t)g.B * g.P[k];
+    const IdxT* ik = idx + g.off[k];
+    const int64_t step = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < L; i += step) {
+        int64_t r = (int64_t)ik[i] - idx_base;
+        if (r < 0 || r >= rows) atomicMin(&bad[0], ((unsigned long long)k << 40) | (unsigned long long)i);
+    }
+}
+
+int launch_check_indices_mp(dlrmb_tables* t, const void* d_idx, int idx_bytes, int idx_base, const MpGeom& g,
+                            cudaStream_t s, long long* bad_table, long long* bad_pos, long long* bad_val) {
+    unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(t->d_uniq);  // scratch reuse
+    unsigned long long init[2] = {~0ull, 0ull};
+    DLRMB_CUDA(cudaMemcpyAsync(d_bad, init, sizeof(init), cudaMemcpyHostToDevice, s));
+    uint32_t maxP = 0;
+    for (int k = 0; k < g.ntab; ++k) maxP = g.P[k] > maxP ? g.P[k] : maxP;
+    int64_t bx = ceil_div64((int64_t)g.B * maxP, 256 * 4);
+    if (bx > t->sm_count * 8) bx = t->sm_count * 8;
+    dim3 grid((unsigned)bx, (unsigned)g.ntab);
+    if (idx_bytes == 4)
+        check_indices_mp_kernel<uint32_t><<<grid, 256, 0, s>>>(t->d_desc, (const uint32_t*)d_idx, idx_base, g, d_bad);
+    else
+        check_indices_mp_kernel<int64_t><<<grid, 256, 0, s>>>(t->d_desc, (const int64_t*)d_idx, idx_base, g, d_bad);
+    DLRMB_LAUNCH_CHECK();
+    unsigned long long h[2];
+    DLRMB_CUDA(cudaMemcpyAsync(h, d_bad, sizeof(h), cudaMemcpyDeviceToHost, s));
+    DLRMB_CUDA(cudaStreamSynchronize(s));
+    if (h[0] == ~0ull) {
+        *bad_table = -1;
+        return DLRMB_OK;
+    }
+    *bad_table = (long long)(h[0] >> 40);
+    *bad_pos = (long long)(h[0] & ((1ull << 40) - 1));
+    const char* src = (const char*)d_idx + ((size_t)g.off[*bad_table] + (size_t)*bad_pos) * idx_bytes;
     int64_t v64 = 0;
     uint32_t v32 = 0;
     if (idx_bytes == 4) {

@@ -152,6 +152,7 @@ static int launch_p2p_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int Bg, 
             DLRMB_LAUNCH_CHECK();
             t->sorted_buf = 0;
             t->sorted_valid = true;
+            t->sorted_mp = false;
             t->sorted_B = Bg;
             t->sorted_P = P;
             return DLRMB_OK;
@@ -165,6 +166,7 @@ static int launch_p2p_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int Bg, 
         int rc = launch_sort(t, idx, (int)sizeof(IdxT), idx_base, Bg, P, s);
         if (rc) return rc;
         t->sorted_valid = true;
+        t->sorted_mp = false;
         t->sorted_B = Bg;
         t->sorted_P = P;
     }

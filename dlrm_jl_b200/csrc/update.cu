@@ -98,12 +98,11 @@ struct UpdateGeom {
 // depends only on the geometry, so the result is bit-reproducible (the work list's order is not,
 // but no arithmetic depends on it).  Scratch written by other CTAs of the same launch is read with
 // L1-bypassing loads.
+// The run that leaves head chunk g of table k (gm: that table's geometry).
 template <int VEC, int NCH, int THREADS, typename RowT>
-__device__ __forceinline__ void fixup_runs(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
-                                           float lr, const float* partial, const uint8_t* flags,
-                                           const uint32_t* head_list, uint32_t n_heads, uint32_t first,
-                                           uint32_t stride, const UpdateGeom& gm,
-                                           typename UV<VEC>::type* red, int* s_first) {
+__device__ __forceinline__ void fixup_one_run(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                                              float lr, const float* partial, const uint8_t* flags, int k, int g,
+                                              const UpdateGeom& gm, typename UV<VEC>::type* red, int* s_first) {
     using V = typename UV<VEC>::type;
     const int lpr = 1 << gm.lpr_log2;
     const int tid = threadIdx.x;
@@ -112,11 +111,7 @@ __device__ __forceinline__ void fixup_runs(const TableDesc* __restrict__ desc, c
     const int nsub = THREADS >> gm.lpr_log2;
     const size_t D = (size_t)gm.C * VEC;
     const int chunk_entries = gm.G * gm.tile;
-
-    for (uint32_t h = first; h < n_heads; h += stride) {
-        const int gid = (int)__ldcg(head_list + h);
-        const int k = gid / gm.chunks;
-        const int g = gid - k * gm.chunks;
+    {
         const uint8_t* fk = flags + (size_t)k * gm.pcap;
         const float* pk = partial + (size_t)k * gm.pcap * 2 * D;
         // where the run ends: the first later chunk whose carried run stops inside it (the table's
@@ -170,6 +165,20 @@ __device__ __forceinline__ void fixup_runs(const TableDesc* __restrict__ desc, c
             }
         }
         __syncthreads();
+    }
+}
+
+template <int VEC, int NCH, int THREADS, typename RowT>
+__device__ __forceinline__ void fixup_runs(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                                           float lr, const float* partial, const uint8_t* flags,
+                                           const uint32_t* head_list, uint32_t n_heads, uint32_t first,
+                                           uint32_t stride, const UpdateGeom& gm,
+                                           typename UV<VEC>::type* red, int* s_first) {
+    for (uint32_t h = first; h < n_heads; h += stride) {
+        const int gid = (int)__ldcg(head_list + h);
+        const int k = gid / gm.chunks;
+        const int g = gid - k * gm.chunks;
+        fixup_one_run<VEC, NCH, THREADS, RowT>(desc, keys, lr, partial, flags, k, g, gm, red, s_first);
     }
 }
 
@@ -293,16 +302,17 @@ __device__ __forceinline__ void fixup_runs_smem(const TableDesc* __restrict__ de
 
 // head_count: [0] = listed head chunks (two-launch path), [1 + k] = CTAs of table k that are done
 // (INLINE path; zero between launches).
+// Chunk `cta` of table k (gm: that table's geometry).  `gid` names the chunk in the two-launch head list,
+// `ndone` is the table's chunk count (the INLINE done-counter target), `clk_cta` its stamp slot.
 template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE>
-__global__ void __launch_bounds__(THREADS, (NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1))
-update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
-                    const uint32_t* __restrict__ pos, const float* __restrict__ dT, float lr,
-                    float* __restrict__ partial, uint8_t* __restrict__ flags,
-                    uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count, UpdateGeom gm,
-                    unsigned long long* clk) {
+__device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                                                  const uint32_t* __restrict__ pos, const float* __restrict__ dT, float lr,
+                                                  float* __restrict__ partial, uint8_t* __restrict__ flags,
+                                                  uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count,
+                                                  const UpdateGeom& gm, int k, int cta, uint32_t gid, uint32_t ndone,
+                                                  unsigned long long* clk, unsigned clk_cta) {
     using V = typename UV<VEC>::type;
     constexpr int U = 4;
-    const unsigned clk_cta = blockIdx.y * gridDim.x + blockIdx.x;
     clock_in(clk, clk_cta);
     __shared__ V s_carry[THREADS * NCH];   // per group: partial of the run carried in from the previous tile
     __shared__ V s_head[THREADS * NCH];    // per group: partial of the run that continues into the next tile
@@ -316,8 +326,6 @@ update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restri
     const int tid = threadIdx.x;
     const int grp = tid >> gm.lpr_log2;
     const int sl = tid & (lpr - 1);
-    const int k = blockIdx.y;
-    const int cta = blockIdx.x;
     const int g = cta * G + grp;              // tile index inside table k
     const bool active = g < gm.tiles;
     const size_t D = (size_t)gm.C * VEC;
@@ -481,7 +489,7 @@ update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restri
         if (tid == 0) {
             if (s_cta_head) {
                 cta_flag |= FLAG_HEAD;
-                head_list[atomicAdd(head_count, 1u)] = (uint32_t)(k * gm.chunks + cta);
+                head_list[atomicAdd(head_count, 1u)] = gid;
             }
             flags[(size_t)k * gm.pcap + cta] = cta_flag;
         }
@@ -496,8 +504,8 @@ update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restri
         *reinterpret_cast<volatile uint8_t*>(flags + (size_t)k * gm.pcap + cta) = cta_flag;
         __threadfence();
         const uint32_t done = atomicAdd(head_count + 1 + k, 1u) + 1u;
-        s_first = (done == gridDim.x) ? 1 : 0;
-        if (done == gridDim.x) head_count[1 + k] = 0;   // re-arm for the next launch (every CTA of the table has counted)
+        s_first = (done == ndone) ? 1 : 0;
+        if (done == ndone) head_count[1 + k] = 0;   // re-arm for the next launch (every CTA of the table has counted)
         s_nheads = 0;
     }
     __syncthreads();
@@ -546,6 +554,19 @@ update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restri
     clock_out(clk, clk_cta);
 }
 
+template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE>
+__global__ void __launch_bounds__(THREADS, (NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1))
+update_tiles_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                    const uint32_t* __restrict__ pos, const float* __restrict__ dT, float lr,
+                    float* __restrict__ partial, uint8_t* __restrict__ flags,
+                    uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count, UpdateGeom gm,
+                    unsigned long long* clk) {
+    const int k = blockIdx.y, cta = blockIdx.x;
+    update_tiles_body<VEC, NCH, THREADS, RowT, INLINE>(desc, keys, pos, dT, lr, partial, flags, head_list, head_count, gm,
+                                                       k, cta, (uint32_t)(k * gm.chunks + cta), gridDim.x, clk,
+                                                       blockIdx.y * gridDim.x + blockIdx.x);
+}
+
 template <int VEC, int NCH, typename RowT>
 __global__ void __launch_bounds__(256)
 update_fixup_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys, float lr,
@@ -558,6 +579,53 @@ update_fixup_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restri
     clock_in(clk, blockIdx.x);
     fixup_runs<VEC, NCH, 256, RowT>(desc, keys, lr, partial, flags, head_list, *head_count, blockIdx.x,
                                     gridDim.x, gm, red, &s_first);
+    clock_out(clk, blockIdx.x);
+}
+
+// ---- per-table pooling factors: one flat grid of sum_k chunks_k CTAs; g.pre maps a CTA to (table, chunk),
+// g.P / g.units give each table its P_k and tile count, so every table has its own L_k, tiles and chunks while
+// the tile length is the batch's (chosen from the total entry count, as for a uniform batch).  The two-launch
+// head list names chunks by their flat CTA id.
+__device__ __forceinline__ UpdateGeom update_geom_mp(const UpdateGeom& gm0, const MpGeom& g, int k) {
+    UpdateGeom gm = gm0;
+    gm.P = (int)g.P[k];
+    gm.L = (int)(g.B * g.P[k]);
+    gm.tiles = (int)g.units[k];
+    gm.chunks = (int)(g.pre[k + 1] - g.pre[k]);
+    return gm;
+}
+
+template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE>
+__global__ void __launch_bounds__(THREADS, (NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1))
+update_tiles_mp_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                       const uint32_t* __restrict__ pos, const float* __restrict__ dT, float lr,
+                       float* __restrict__ partial, uint8_t* __restrict__ flags,
+                       uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count, UpdateGeom gm0,
+                       const __grid_constant__ MpGeom g, unsigned long long* clk) {
+    const uint32_t lin = blockIdx.x;
+    const int k = mp_find(g.pre, g.ntab, lin);
+    const UpdateGeom gm = update_geom_mp(gm0, g, k);
+    update_tiles_body<VEC, NCH, THREADS, RowT, INLINE>(desc, keys, pos, dT, lr, partial, flags, head_list, head_count, gm,
+                                                       k, (int)(lin - g.pre[k]), lin, (uint32_t)gm.chunks, clk, lin);
+}
+
+template <int VEC, int NCH, typename RowT>
+__global__ void __launch_bounds__(256)
+update_fixup_mp_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys, float lr,
+                       const float* __restrict__ partial, const uint8_t* __restrict__ flags,
+                       const uint32_t* __restrict__ head_list, const uint32_t* __restrict__ head_count,
+                       UpdateGeom gm0, const __grid_constant__ MpGeom g, unsigned long long* clk) {
+    using V = typename UV<VEC>::type;
+    __shared__ V red[256 * NCH];
+    __shared__ int s_first;
+    clock_in(clk, blockIdx.x);
+    const uint32_t n_heads = *head_count;
+    for (uint32_t h = blockIdx.x; h < n_heads; h += gridDim.x) {
+        const uint32_t gid = __ldcg(head_list + h);
+        const int k = mp_find(g.pre, g.ntab, gid);
+        const UpdateGeom gm = update_geom_mp(gm0, g, k);
+        fixup_one_run<VEC, NCH, 256, RowT>(desc, keys, lr, partial, flags, k, (int)(gid - g.pre[k]), gm, red, &s_first);
+    }
     clock_out(clk, blockIdx.x);
 }
 
@@ -646,7 +714,74 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
     return DLRMB_OK;
 }
 
-template <typename RowT>
+template <int VEC, int NCH, typename RowT>
+static int launch_update_mp_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
+    UpdateGeom gm;
+    MpGeom g;
+    g.ntab = t->ntab;
+    g.B = (uint32_t)t->sorted_B;
+    g.nlist = 0;
+    int64_t total = 0, maxL = 0;
+    for (int k = 0; k < t->ntab; ++k) {
+        g.P[k] = (uint32_t)t->h_sorted_P[k];
+        g.off[k] = 0;   // unused by the update
+        const int64_t L = (int64_t)g.B * g.P[k];
+        total += L;
+        maxL = L > maxL ? L : maxL;
+    }
+    gm.L = (int)maxL;
+    gm.P = 1;
+    gm.C = t->D / VEC;
+    gm.lpr_log2 = lanes_per_row_log2(gm.C);
+    const int lpr = 1 << gm.lpr_log2;
+    constexpr int THREADS = (NCH > 4) ? 128 : 256;
+    const int G = THREADS / lpr;
+    gm.G = G;
+    gm.tile = choose_update_tile(total, lpr, t->sm_count, THREADS * ((NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1)));
+    {
+        const int v = g_opt.update_tile.load(std::memory_order_relaxed);
+        if (v >= 4 && v <= 32 && v % 4 == 0) gm.tile = v;
+    }
+    gm.slots = slots;
+    gm.slot0 = slot0;
+    gm.cap = t->cap;
+    gm.pcap = t->partial_tiles_cap;
+    int64_t chunks_total = 0;
+    for (int k = 0; k < t->ntab; ++k) {
+        const int64_t tiles = ceil_div64((int64_t)g.B * g.P[k], gm.tile);
+        const int64_t chunks = ceil_div64(tiles, G);
+        DLRMB_REQUIRE(chunks <= gm.pcap, "internal: update chunk capacity exceeded (%lld > %lld)", (long long)chunks,
+                      (long long)gm.pcap);
+        g.units[k] = (uint32_t)tiles;
+        g.pre[k] = (uint32_t)chunks_total;
+        chunks_total += chunks;
+    }
+    g.pre[t->ntab] = (uint32_t)chunks_total;
+    gm.tiles = 0;
+    gm.chunks = 0;
+    DLRMB_REQUIRE(chunks_total < (1ll << 31), "batch too large for one update launch");
+    const uint32_t* keys = t->keys[t->sorted_buf];
+    const uint32_t* pos = t->pos[t->sorted_buf];
+    const bool inline_fixup = total <= kUpdateInlineMaxEntries &&
+                              g_opt.update_two_launches.load(std::memory_order_relaxed) == 0;
+    if (inline_fixup) {
+        update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, true><<<(unsigned)chunks_total, THREADS, 0, s>>>(
+            t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g, clock_slot(CLK_UPDATE));
+        DLRMB_LAUNCH_CHECK();
+        return DLRMB_OK;
+    }
+    DLRMB_CUDA(cudaMemsetAsync(t->head_count, 0, sizeof(uint32_t), s));
+    update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, false><<<(unsigned)chunks_total, THREADS, 0, s>>>(
+        t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g, clock_slot(CLK_UPDATE));
+    DLRMB_LAUNCH_CHECK();
+    unsigned fgrid = (unsigned)(chunks_total < (int64_t)t->sm_count * 8 ? chunks_total : (int64_t)t->sm_count * 8);
+    update_fixup_mp_kernel<VEC, NCH, RowT><<<fgrid, 256, 0, s>>>(t->d_desc, keys, lr, t->partial, t->tile_flags,
+                                                                t->head_list, t->head_count, gm, g, clock_slot(CLK_FIXUP));
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename RowT, bool MP>
 static int launch_update_r(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
     const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(dT) & 15) == 0);
     if (t->D % 4 == 0 && !vec4) {
@@ -657,23 +792,35 @@ static int launch_update_r(dlrmb_tables* t, const float* dT, int slots, int slot
     const int lpr = 1 << lanes_per_row_log2(C);
     const int nch = (C + lpr - 1) / lpr;
     if (vec4) {
-        if (nch == 1) return launch_update_t<4, 1, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch == 2) return launch_update_t<4, 2, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 4) return launch_update_t<4, 4, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 8) return launch_update_t<4, 8, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 1) return MP ? launch_update_mp_t<4, 1, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<4, 1, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 2) return MP ? launch_update_mp_t<4, 2, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<4, 2, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 4) return MP ? launch_update_mp_t<4, 4, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<4, 4, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 8) return MP ? launch_update_mp_t<4, 8, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<4, 8, RowT>(t, dT, slots, slot0, lr, s);
     } else {
-        if (nch == 1) return launch_update_t<1, 1, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch == 2) return launch_update_t<1, 2, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 4) return launch_update_t<1, 4, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 8) return launch_update_t<1, 8, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 1) return MP ? launch_update_mp_t<1, 1, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<1, 1, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 2) return MP ? launch_update_mp_t<1, 2, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<1, 2, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 4) return MP ? launch_update_mp_t<1, 4, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<1, 4, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 8) return MP ? launch_update_mp_t<1, 8, RowT>(t, dT, slots, slot0, lr, s)
+                             : launch_update_t<1, 8, RowT>(t, dT, slots, slot0, lr, s);
     }
     set_error("embedding dim %d unsupported by the update kernel", t->D);
     return DLRMB_EINVAL;
 }
 
+// consumes whichever sort ran last: uniform, or per-table pooling factors (t->sorted_mp)
 int launch_update(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
-    if (t->elem_bytes == 2) return launch_update_r<__nv_bfloat16>(t, dT, slots, slot0, lr, s);
-    return launch_update_r<float>(t, dT, slots, slot0, lr, s);
+    if (t->sorted_mp)
+        return t->elem_bytes == 2 ? launch_update_r<__nv_bfloat16, true>(t, dT, slots, slot0, lr, s)
+                                  : launch_update_r<float, true>(t, dT, slots, slot0, lr, s);
+    if (t->elem_bytes == 2) return launch_update_r<__nv_bfloat16, false>(t, dT, slots, slot0, lr, s);
+    return launch_update_r<float, false>(t, dT, slots, slot0, lr, s);
 }
 
 }  // namespace dlrmb

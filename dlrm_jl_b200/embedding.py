@@ -25,7 +25,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import List, Optional, Sequence, Union
+from typing import List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -37,17 +37,40 @@ def _stream_ptr(device: torch.device) -> int:
     return int(torch.cuda.current_stream(device).cuda_stream)
 
 
-def _as_index_tensor(sparse, ntab: int, device: torch.device) -> torch.Tensor:
-    """Normalise the index containers DLRM.jl accepts (vector of vectors, vector of P x B
-    matrices given here as [B][P], or one [ntab][B] / [ntab][B][P] array) to a contiguous
-    table-major device tensor [ntab][B][P] of int32 or int64."""
-    if isinstance(sparse, torch.Tensor):
-        t = sparse
-    elif isinstance(sparse, np.ndarray):
-        t = torch.from_numpy(np.ascontiguousarray(sparse))
-    else:
-        parts = [torch.as_tensor(np.asarray(s) if not isinstance(s, torch.Tensor) else s) for s in sparse]
-        t = torch.stack([p.reshape(p.shape[0], -1) for p in parts], dim=0)
+@dataclass(frozen=True, eq=False)
+class PackedIndices:
+    """Indices of a batch whose tables have different pooling factors (multi-hot with mixed hotness):
+    table k's [B][P_k] block starts at element B * (P_0 + .. + P_{k-1}) of the flat int32 / int64
+    tensor ``flat`` (Julia: ``reduce(vcat, vec.(sparse))``).  ``pack[k]`` is table k's [B][P_k] view."""
+    flat: torch.Tensor
+    P: Tuple[int, ...]
+    B: int
+
+    def __len__(self) -> int:
+        return len(self.P)
+
+    def __getitem__(self, k: int) -> torch.Tensor:
+        o = self.B * sum(self.P[:k])
+        return self.flat[o:o + self.B * self.P[k]].view(self.B, self.P[k])
+
+    def P_array(self):
+        return (C.c_int32 * len(self.P))(*self.P)
+
+    def element_size(self) -> int:
+        return self.flat.element_size()
+
+    def data_ptr(self) -> int:
+        return self.flat.data_ptr()
+
+    @property
+    def is_cuda(self) -> bool:
+        return self.flat.is_cuda
+
+    def to(self, device, non_blocking: bool = False) -> "PackedIndices":
+        return PackedIndices(self.flat.to(device, non_blocking=non_blocking).contiguous(), self.P, self.B)
+
+
+def _index_dtype(t: torch.Tensor) -> torch.Tensor:
     if t.dtype in (torch.uint8, torch.int8, torch.int16):
         t = t.to(torch.int32)
     if t.dtype not in (torch.int32, torch.int64):
@@ -55,11 +78,52 @@ def _as_index_tensor(sparse, ntab: int, device: torch.device) -> torch.Tensor:
             t = t.view(torch.int32)
         else:
             raise TypeError(f"index dtype {t.dtype} not supported (int32/uint32/int64)")
+    return t
+
+
+def _pack_mixed(parts: List[torch.Tensor], ntab: int, device: torch.device) -> PackedIndices:
+    """Per-table [B][P_k] arrays of different widths -> PackedIndices (int64 if any table is int64)."""
+    if len(parts) != ntab:
+        raise ValueError(f"indices must hold one array per table: {ntab} tables, got {len(parts)}")
+    Bs = {p.shape[0] for p in parts}
+    if len(Bs) != 1:
+        raise ValueError(f"every table's indices must cover the same batch, got B = {[p.shape[0] for p in parts]}")
+    parts = [_index_dtype(p) for p in parts]
+    dtype = torch.int64 if any(p.dtype == torch.int64 for p in parts) else torch.int32
+    flat = torch.cat([p.reshape(-1).to(dtype) for p in parts])
+    return PackedIndices(flat.to(device, non_blocking=True).contiguous(), tuple(int(p.shape[1]) for p in parts),
+                         int(parts[0].shape[0]))
+
+
+def _as_index_tensor(sparse, ntab: int, device: torch.device):
+    """Normalise the index containers DLRM.jl accepts (vector of vectors, vector of P x B
+    matrices given here as [B][P], or one [ntab][B] / [ntab][B][P] array) to a contiguous
+    table-major device tensor [ntab][B][P] of int32 or int64.  A vector whose tables have different
+    widths (the reference's load_inputs with per-table P = length / B) becomes :class:`PackedIndices`."""
+    if isinstance(sparse, PackedIndices):
+        if len(sparse) != ntab:
+            raise ValueError(f"indices must hold one array per table: {ntab} tables, got {len(sparse)}")
+        return sparse.to(device, non_blocking=True)
+    if isinstance(sparse, torch.Tensor):
+        t = sparse
+    elif isinstance(sparse, np.ndarray):
+        t = torch.from_numpy(np.ascontiguousarray(sparse))
+    else:
+        parts = [torch.as_tensor(np.asarray(s) if not isinstance(s, torch.Tensor) else s) for s in sparse]
+        parts = [p.reshape(p.shape[0], -1) for p in parts]
+        if len({p.shape[1] for p in parts}) > 1:
+            return _pack_mixed(parts, ntab, device)
+        t = torch.stack(parts, dim=0)
+    t = _index_dtype(t)
     if t.dim() == 2:
         t = t.unsqueeze(-1)
     if t.dim() != 3 or t.shape[0] != ntab:
         raise ValueError(f"indices must be [ntab={ntab}][B] or [ntab][B][P], got {tuple(t.shape)}")
     return t.to(device, non_blocking=True).contiguous()
+
+
+def _batch(idx) -> int:
+    return idx.B if isinstance(idx, PackedIndices) else idx.shape[1]
 
 
 class _DevicePtrView:
@@ -159,10 +223,14 @@ class EmbeddingTables:
         """Gather + sum-pool into ``out``.  ``sort=True`` is the training-step form: the same launch also
         sorts / dedups the indices for the sparse update of this batch (dlrmb_embedding_fwd_sort), so
         :meth:`update_sorted` can follow the backward pass without a sort launch."""
-        ntab, B, P = idx.shape
         slots = out.shape[1]
+        if isinstance(idx, PackedIndices):   # per-table pooling factors
+            B, P = idx.B, idx.P_array()
+            fn = self._lib.dlrmb_embedding_fwd_sort_mp if sort else self._lib.dlrmb_embedding_fwd_mp
+        else:
+            ntab, B, P = idx.shape
+            fn = self._lib.dlrmb_embedding_fwd_sort if sort else self._lib.dlrmb_embedding_fwd
         assert out.is_contiguous() and out.dtype == torch.float32 and out.shape == (B, slots, self.D)
-        fn = self._lib.dlrmb_embedding_fwd_sort if sort else self._lib.dlrmb_embedding_fwd
         with _prof.range("lookup"):
             _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P, out.data_ptr(), slots, slot0,
                           _stream_ptr(self.device)))
@@ -195,7 +263,10 @@ class EmbeddingTables:
     def sort(self, idx: torch.Tensor, idx_base: int = 0, side_stream: bool = False) -> None:
         """Index sort/dedup for the next update.  With ``side_stream`` it is issued on a second
         stream (it depends on the indices only) so it overlaps the forward/backward pass."""
-        ntab, B, P = idx.shape
+        if isinstance(idx, PackedIndices):
+            B, P, fn, rec = idx.B, idx.P_array(), self._lib.dlrmb_embedding_sort_mp, idx.flat
+        else:
+            (ntab, B, P), fn, rec = idx.shape, self._lib.dlrmb_embedding_sort, idx
         if side_stream:
             if self._side_stream is None:
                 self._side_stream = torch.cuda.Stream(self.device)
@@ -203,16 +274,15 @@ class EmbeddingTables:
             self._side_stream.wait_stream(torch.cuda.current_stream(self.device))
             with torch.cuda.stream(self._side_stream):
                 with _prof.range("sort"):
-                    _lib.check(self._lib.dlrmb_embedding_sort(
-                        self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P, self._side_stream.cuda_stream))
+                    _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P,
+                                  self._side_stream.cuda_stream))
                 if not torch.cuda.is_current_stream_capturing():
-                    idx.record_stream(self._side_stream)
+                    rec.record_stream(self._side_stream)
                 self._sorted_event.record(self._side_stream)
             self._pending_side = True
         else:
             with _prof.range("sort"):
-                _lib.check(self._lib.dlrmb_embedding_sort(
-                    self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P, _stream_ptr(self.device)))
+                _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P, _stream_ptr(self.device)))
             self._pending_side = False
 
     def update_sorted(self, dT: torch.Tensor, slot0: int, lr: float) -> None:
@@ -230,7 +300,8 @@ class EmbeddingTables:
         self.update_sorted(dT, slot0, lr)
 
     def sort_dedup_export(self, k: int, L: int):
-        """(uniq, seg_offsets, perm) of the last sort for table k, as numpy arrays."""
+        """(uniq, seg_offsets, perm) of the last sort for table k, as numpy arrays.  ``L`` = B * P_k, the
+        table's lookups in that sort."""
         uniq = np.empty(L, dtype=np.int64)
         seg = np.empty(L + 1, dtype=np.int32)
         perm = np.empty(L, dtype=np.int32)
@@ -241,8 +312,12 @@ class EmbeddingTables:
         return uniq[:n.value].copy(), seg[:n.value + 1].copy(), perm
 
     def check_indices(self, idx: torch.Tensor, idx_base: int = 0) -> None:
-        ntab, B, P = idx.shape
         on_host = 0 if idx.is_cuda else 1
+        if isinstance(idx, PackedIndices):
+            _lib.check(self._lib.dlrmb_check_indices_mp(
+                self._h, idx.data_ptr(), idx.element_size(), idx_base, idx.B, idx.P_array(), on_host))
+            return
+        ntab, B, P = idx.shape
         _lib.check(self._lib.dlrmb_check_indices(
             self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P, on_host))
 
@@ -282,7 +357,7 @@ def maplookup(strategy, tables: EmbeddingTables, sparse, idx_base: int = 0, requ
         raise TypeError(f"unknown lookup strategy {strategy!r}")
     if check:
         tables.check_indices(idx, idx_base)
-    B = idx.shape[1]
+    B = _batch(idx)
     alloc = torch.zeros if slot0 > 0 else torch.empty
     T = alloc((B, slot0 + tables.ntab, tables.D), dtype=torch.float32, device=tables.device)
     tables.lookup(idx, T, slot0, idx_base, sort=requires_grad)
@@ -313,9 +388,10 @@ class SparseEmbeddingUpdate:
 
 
 def sparse_updates(dT: torch.Tensor, indices: torch.Tensor, slot0: int, idx_base: int = 0) -> List[SparseEmbeddingUpdate]:
-    """The lookup pullback: slice dT per table, no arithmetic (test/model/embedding_update.jl:36-40)."""
+    """The lookup pullback: slice dT per table, no arithmetic (test/model/embedding_update.jl:36-40).
+    ``indices`` is the [ntab][B][P] tensor or :class:`PackedIndices`."""
     return [SparseEmbeddingUpdate(dT[:, slot0 + k, :], indices[k], dT, slot0 + k, idx_base)
-            for k in range(indices.shape[0])]
+            for k in range(len(indices))]
 
 
 def uncompress(update: SparseEmbeddingUpdate, nrows: int) -> torch.Tensor:
@@ -351,6 +427,6 @@ def update_(opt: Descent, tables: EmbeddingTables, grads: Sequence[SparseEmbeddi
         dT = torch.stack([g.delta for g in grads], dim=1).contiguous()
         slot0 = 0
     if not presorted:
-        idx = torch.stack([g.indices.reshape(g.delta.shape[0], -1) for g in grads], dim=0).contiguous()
+        idx = _as_index_tensor([g.indices.reshape(g.delta.shape[0], -1) for g in grads], tables.ntab, tables.device)
         tables.sort(idx, grads[0].idx_base)
     tables.update_sorted(dT, slot0, opt.eta)

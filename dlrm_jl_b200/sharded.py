@@ -20,6 +20,7 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Callable, List, Optional, Sequence
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -77,9 +78,21 @@ def _a2a(out: torch.Tensor, inp: torch.Tensor, out_splits, in_splits, group) -> 
     dist.all_to_all_single(out, inp, output_split_sizes=out_splits, input_split_sizes=in_splits, group=group)
 
 
+def _require_uniform_pooling(idx) -> None:
+    """The table-sharded path takes one pooling factor for all tables."""
+    from .embedding import PackedIndices
+    mixed = isinstance(idx, PackedIndices) or (
+        isinstance(idx, (list, tuple)) and len({int(np.asarray(s).reshape(np.asarray(s).shape[0], -1).shape[1])
+                                                for s in idx}) > 1)
+    if mixed:
+        raise ValueError("per-table pooling factors (mixed multi-hot widths) are not supported by the "
+                         "table-sharded path; give every table the same P or use EmbeddingTables")
+
+
 def exchange_indices(idx_local: torch.Tensor, sh: TableSharding, rank: int, group=None) -> torch.Tensor:
     """idx_local [ntab][B_local][P] (this rank's samples, all tables) ->
     [t_mine][B_global][P] (all samples, this rank's tables; sample order = rank-major)."""
+    _require_uniform_pooling(idx_local)
     ntab, Bl, P = idx_local.shape
     W = sh.world
     if W == 1:
@@ -447,6 +460,7 @@ class ShardedEmbedding:
     def lookup_fused(self, idx_local: torch.Tensor) -> torch.Tensor:
         """Forward of the fully fused path: no autograd node (the gradient never comes back through
         T; it is scattered to the owners by the interaction backward)."""
+        _require_uniform_pooling(idx_local)
         with torch.no_grad():
             idx_owned = self._exchange_indices(idx_local)
             self.idx_owned = idx_owned
@@ -519,6 +533,7 @@ class ShardedEmbedding:
     def lookup(self, idx_local: torch.Tensor, anchor: torch.Tensor) -> torch.Tensor:
         """idx_local [ntab][B_local][P] -> T [B_local][1 + ntab][D] (requires grad through `anchor`,
         any tensor that requires grad, so autograd calls the gradient exchange)."""
+        _require_uniform_pooling(idx_local)
         return _ShardedLookupFn.apply(anchor, self, idx_local)
 
     def sort_async(self) -> None:

@@ -173,6 +173,39 @@ int32_t dlrmb_sort_dedup_export(dlrmb_tables* t, int32_t k, int64_t* uniq, int32
 int32_t dlrmb_check_indices(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
                             int32_t B, int32_t P, int32_t idx_on_host);
 
+/* ---- per-table pooling factors (multi-hot with mixed hotness): the index container of the reference's
+ * load_inputs, "a vector mixing per-table vectors and P x B matrices" with each table's P = length / B
+ * (src/data/criteo.jl:551-557).  `P` is a host array [ntab] of pooling factors, each >= 1; table k's
+ * indices are the [B][P_k] block starting at element B * (P_0 + .. + P_{k-1}) of `idx` (Julia:
+ * reduce(vcat, vec.(sparse))).  Per table the semantics are those of the uniform entry points above
+ * (pooling in ascending p, dedup ties by flat position b*P_k + p, Flux.Descent with duplicates summed),
+ * and with every P_k equal the results are bit-identical to them.  Limits: B * max_k P_k <= max_lookups
+ * (grow with dlrmb_tables_reserve) and ntab <= dlrmb_mp_max_tables() (256: the per-table geometry reaches
+ * the kernels as one kernel-parameter struct); anything else returns DLRMB_EINVAL.  Device-pointer calls
+ * do not allocate, synchronise or copy from host memory, so they can be captured into a CUDA graph.
+ * dlrmb_embedding_update_sorted and dlrmb_sort_dedup_export consume the last sort, uniform or _mp: after
+ * an _mp sort, the export of table k returns its B * P_k entries.  The table-sharded multi-GPU entry
+ * points take one P only. */
+int32_t dlrmb_mp_max_tables(void);
+int32_t dlrmb_embedding_fwd_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                               const int32_t* P, float* out, int32_t slots, int32_t slot0, dlrmb_stream stream);
+/* lookup + the sort for the coming update (tables with B * P_k <= 4096 sort inside the lookup launch) */
+int32_t dlrmb_embedding_fwd_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                    const int32_t* P, float* out, int32_t slots, int32_t slot0, dlrmb_stream stream);
+int32_t dlrmb_embedding_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                const int32_t* P, dlrmb_stream stream);
+int32_t dlrmb_embedding_bwd_sgd_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                   const int32_t* P, const float* dT, int32_t slots, int32_t slot0, float lr,
+                                   dlrmb_stream stream);
+int32_t dlrmb_check_indices_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                               const int32_t* P, int32_t idx_on_host);
+/* host-buffer forms (every pointer host memory), as dlrmb_embedding_fwd_host / dlrmb_embedding_bwd_sgd_host */
+int32_t dlrmb_embedding_fwd_mp_host(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                    const int32_t* P, float* out, int32_t slots, int32_t slot0);
+int32_t dlrmb_embedding_bwd_sgd_mp_host(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                        int32_t B, const int32_t* P, const float* dT, int32_t slots, int32_t slot0,
+                                        float lr);
+
 /* ---- loss: the top MLP's final sigmoid (src/model/model.jl:87-90) fused with bce_loss and its
  * pullback (src/train/train.jl:33-41, 45-71).  logits/labels [B] device f32.  Writes the mean loss
  * (one float), d(loss)/d(logit) [B] (sensitivity 1 folded in) and, if `prob` is non-NULL, the

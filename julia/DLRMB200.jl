@@ -167,12 +167,17 @@ Base.isapprox(a::B200Embedding, b::B200Embedding; kw...) = isapprox(Array(a), Ar
 
 # `sparse` is DACLoader's B x ntab UInt32 matrix (src/data/criteo.jl:320-326) or a vector of per-table
 # index vectors / P x B matrices (src/data/criteo.jl:551-557).  Both are already the table-major layout
-# the library wants once concatenated; indices stay 1-based (idx_base = 1).
+# the library wants once concatenated; indices stay 1-based (idx_base = 1).  When the tables' widths
+# differ (multi-hot with per-table hotness) the result is the flat reduce(vcat, vec.(sparse)) and the
+# vector of pooling factors, for the `_mp` entry points.
 _pack(sparse::AbstractMatrix{<:Integer}) = (Matrix(sparse), 1)                        # B x ntab, P = 1
 function _pack(sparse::AbstractVector)
-    P = ndims(first(sparse)) == 1 ? 1 : size(first(sparse), 1)
-    return (reduce(hcat, [vec(s) for s in sparse]), P)                                # (P*B) x ntab
+    Ps = [ndims(s) == 1 ? 1 : size(s, 1) for s in sparse]
+    all(==(first(Ps)), Ps) && return (reduce(hcat, [vec(s) for s in sparse]), first(Ps))   # (P*B) x ntab
+    return (reduce(vcat, [vec(s) for s in sparse]), Int32.(Ps))                       # sum(P)*B, P per table
 end
+_batch(idx, P::Integer) = div(size(idx, 1), P)
+_batch(idx, P::AbstractVector) = div(length(idx), sum(P))
 _table_indices(sparse::AbstractMatrix{<:Integer}, k) = view(sparse, :, k)
 _table_indices(sparse::AbstractVector, k) = sparse[k]
 _idxbytes(::AbstractArray{T}) where {T} = Int32(sizeof(T))
@@ -184,16 +189,22 @@ _prepend(s::PreallocationStrategy) = s.prependrows                              
 
 function _lookup(tables::AbstractVector{<:B200Embedding}, sparse, prependrows::Integer)
     idx, P = _pack(sparse)
-    B = div(size(idx, 1), P)
-    slab = materialize!(tables, B * P)
+    B = _batch(idx, P)
+    slab = materialize!(tables, B * maximum(P))
     D = slab.featuresize
     @assert iszero(mod(prependrows, D))
     slot0 = div(prependrows, D)
     slots = slot0 + length(tables)
     out = zeros(Float32, slots * D, B)                                                # == C [B][slots][D]
-    check(ccall((:dlrmb_embedding_fwd_host, libdlrm_b200), Int32,
-                (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Int32, Ptr{Float32}, Int32, Int32),
-                slab.handle, idx, _idxbytes(idx), 1, B, P, out, slots, slot0))
+    if P isa Integer
+        check(ccall((:dlrmb_embedding_fwd_host, libdlrm_b200), Int32,
+                    (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Int32, Ptr{Float32}, Int32, Int32),
+                    slab.handle, idx, _idxbytes(idx), 1, B, P, out, slots, slot0))
+    else
+        check(ccall((:dlrmb_embedding_fwd_mp_host, libdlrm_b200), Int32,
+                    (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Ptr{Int32}, Ptr{Float32}, Int32, Int32),
+                    slab.handle, idx, _idxbytes(idx), 1, B, P, out, slots, slot0))
+    end
     return out, slot0
 end
 
@@ -264,8 +275,8 @@ function EmbeddingTables.update!(opt::Flux.Descent, tables::AbstractVector{<:B20
     @assert length(tables) == length(grads)
     D = first(tables).slab.featuresize
     idx, P = _pack([g.indices for g in grads])
-    B = div(size(idx, 1), P)
-    slab = materialize!(tables, B * P)
+    B = _batch(idx, P)
+    slab = materialize!(tables, B * maximum(P))
     shared = _shared_parent(grads, D)
     if shared === nothing      # updates built one by one: pack into one (ntab*D) x B matrix
         delta, slot0 = reduce(vcat, [Matrix{Float32}(g.delta) for g in grads]), 0
@@ -275,9 +286,15 @@ function EmbeddingTables.update!(opt::Flux.Descent, tables::AbstractVector{<:B20
     slots = div(size(delta, 1), D)
     # `indexers`, `num_splits`, `nthreads` steer the reference's CPU dedup / threading; here the dedup is
     # the device-side sort and the whole update is one launch, so they are accepted and ignored
-    check(ccall((:dlrmb_embedding_bwd_sgd_host, libdlrm_b200), Int32,
-                (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Int32, Ptr{Float32}, Int32, Int32, Float32),
-                slab.handle, idx, _idxbytes(idx), 1, B, P, delta, slots, slot0, Float32(opt.eta)))
+    if P isa Integer
+        check(ccall((:dlrmb_embedding_bwd_sgd_host, libdlrm_b200), Int32,
+                    (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Int32, Ptr{Float32}, Int32, Int32, Float32),
+                    slab.handle, idx, _idxbytes(idx), 1, B, P, delta, slots, slot0, Float32(opt.eta)))
+    else
+        check(ccall((:dlrmb_embedding_bwd_sgd_mp_host, libdlrm_b200), Int32,
+                    (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int32, Int32, Ptr{Int32}, Ptr{Float32}, Int32, Int32, Float32),
+                    slab.handle, idx, _idxbytes(idx), 1, B, P, delta, slots, slot0, Float32(opt.eta)))
+    end
     return nothing
 end
 
