@@ -256,7 +256,8 @@ __device__ __forceinline__ void fixup_runs_smem(const TableDesc* __restrict__ de
     const int nsub = 256 >> gm.lpr_log2;                 // lane groups of update_fixup_kernel
     const size_t D = (size_t)gm.C * VEC;
     const unsigned gshift = (threadIdx.x & 31) & ~(lpr - 1);
-    const unsigned gmask = (lpr >= 32) ? 0xffffffffu : (((1u << lpr) - 1u) << gshift);
+    const unsigned gbits = (lpr >= 32) ? 0xffffffffu : ((1u << lpr) - 1u);
+    const unsigned gmask = gbits << gshift;
     const float* pk = partial + (size_t)k * gm.pcap * 2 * D;
     float* tbase = desc[k].base;
     for (uint32_t h = grp; h < n_heads; h += G) {
@@ -266,7 +267,9 @@ __device__ __forceinline__ void fixup_runs_smem(const TableDesc* __restrict__ de
         for (int base = g + 1; base < gm.chunks; base += lpr) {
             const int u = base + sl;
             const bool ends = (u >= gm.chunks) || (s_fl[u] & FLAG_CARRY_ENDS);
-            const unsigned b = __ballot_sync(gmask, ends) >> gshift;
+            // the ballot also carries the flags of other lane groups of the warp that vote at the same time
+            // (the mask names who must take part, not whose bits come back): keep this group's own
+            const unsigned b = (__ballot_sync(gmask, ends) >> gshift) & gbits;
             if (b != 0) {
                 u_last = min(gm.chunks - 1, base + __ffs((int)b) - 1);
                 break;
