@@ -66,11 +66,14 @@ SIGNATURES = {
     "dlrmb_tables_set_slot_map": (_i32, [_vp, C.POINTER(_i32)]),
     "dlrmb_embedding_fwd_p2p": (_i32, [_vp, *_idx_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
     "dlrmb_embedding_fwd_p2p_sort": (_i32, [_vp, *_idx_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
+    "dlrmb_embedding_fwd_p2p_mp": (_i32, [_vp, *_idx_mp_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
+    "dlrmb_embedding_fwd_p2p_sort_mp": (_i32, [_vp, *_idx_mp_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
     "dlrmb_peer_barrier": (_i32, [_i32, C.POINTER(_vp), _i32, _i32, _i32, _vp, _vp]),
     "dlrmb_peer_barrier_flag_bytes": (_i64, []),
     "dlrmb_peer_barrier_state_bytes": (_i64, []),
     "dlrmb_peer_allreduce_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), _i32, _i32, _i32, _vp, _vp, _i64, _vp]),
     "dlrmb_indices_scatter_p2p": (_i32, [_i32, _vp, _i32, _i32, _i32, _i32, _vp, _i32, _vp]),
+    "dlrmb_indices_scatter_p2p_mp": (_i32, [_i32, _vp, _i32, _i32, _i32, C.POINTER(_i32), _vp, _i32, _vp]),
     "dlrmb_interaction_has_warp_path": (_i32, [_i32, _i32]),
     "dlrmb_dense_fwd_bias_act": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _vp]),
     "dlrmb_dense_bwd_scratch_floats": (_i64, [_i32]),
@@ -79,11 +82,13 @@ SIGNATURES = {
     "dlrmb_interaction_bwd_dx": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp]),
     "dlrmb_dac_unpack": (_i32, [_i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "dlrmb_shard_plan": (_i32, [_i32, C.POINTER(_i64), _i32, C.POINTER(_i32)]),
+    "dlrmb_shard_plan_mp": (_i32, [_i32, C.POINTER(_i64), C.POINTER(_i32), _i32, C.POINTER(_i32)]),
     "dlrmb_comm_unique_id": (_i32, [_vp]),
     "dlrmb_comm_create": (_i32, [_i32, _vp, _i32, _i32, C.POINTER(_vp)]),
     "dlrmb_comm_destroy": (_i32, [_vp]),
     "dlrmb_comm_info": (_i32, [_vp, C.POINTER(_i32), C.POINTER(_i32)]),
     "dlrmb_comm_a2a_indices": (_i32, [_vp, C.POINTER(_i32), _i32, _vp, _i32, _i32, _i32, _vp, _vp]),
+    "dlrmb_comm_a2a_indices_mp": (_i32, [_vp, C.POINTER(_i32), _i32, _vp, _i32, _i32, C.POINTER(_i32), _vp, _vp]),
     "dlrmb_comm_a2a_fwd": (_i32, [_vp, C.POINTER(_i32), _i32, _vp, _i32, _i32, _vp, _vp]),
     "dlrmb_comm_a2a_bwd": (_i32, [_vp, C.POINTER(_i32), _i32, _vp, _i32, _i32, _vp, _vp]),
     "dlrmb_comm_allreduce_f32": (_i32, [_vp, _vp, _i64, _vp]),

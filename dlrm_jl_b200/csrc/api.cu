@@ -652,9 +652,13 @@ int32_t dlrmb_embedding_bwd_sgd_host(dlrmb_tables* t, const void* idx, int32_t i
     return DLRMB_OK;
 }
 
+}  // extern "C"
+
 // ---- per-table pooling factors (`_mp`) -----------------------------------------------------------
-static int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, const int32_t* P,
-                         MpGeom* g) {
+namespace dlrmb {
+
+int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, const int32_t* P,
+                  MpGeom* g) {
     DLRMB_REQUIRE(idx != nullptr, "idx is null");
     DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
     DLRMB_REQUIRE(idx_base == 0 || idx_base == 1, "idx_base must be 0 or 1 (got %d)", idx_base);
@@ -681,13 +685,17 @@ static int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, 
 
 static int64_t mp_index_count(const MpGeom& g) { return (int64_t)g.off[g.ntab - 1] + (int64_t)g.B * g.P[g.ntab - 1]; }
 
-static void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g) {
+void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g) {
     t->sorted_valid = true;
     t->sorted_mp = true;
     t->sorted_B = (int)g.B;
     t->sorted_P = 0;
     for (int k = 0; k < g.ntab; ++k) t->h_sorted_P[k] = (int32_t)g.P[k];
 }
+
+}  // namespace dlrmb
+
+extern "C" {
 
 int32_t dlrmb_mp_max_tables(void) { return kMpMaxTables; }
 

@@ -8,7 +8,9 @@
 // same order on every rank.
 //
 //   dlrmb_shard_plan          which rank owns which table (lookup count first, bytes second)
+//   dlrmb_shard_plan_mp       the same with per-table pooling factors (weighted by P_k when they differ)
 //   dlrmb_comm_a2a_indices    idx_local [ntab][B_local][P] -> idx_owned [t_mine][B_global][P]
+//   dlrmb_comm_a2a_indices_mp the `_mp` layout at B_local -> this rank's tables' `_mp` layout at B_global
 //   dlrmb_comm_a2a_fwd        pooled [B_global][t_mine][D] (owner) -> T [B_local][1 + ntab][D]
 //   dlrmb_comm_a2a_bwd        dT [B_local][1 + ntab][D] -> grads [B_global][t_mine][D] (owner)
 //   dlrmb_comm_allreduce_f32  data-parallel dense gradients (sum, in place)
@@ -169,6 +171,38 @@ int32_t dlrmb_shard_plan(int32_t ntab, const int64_t* rows, int32_t world, int32
     return DLRMB_OK;
 }
 
+int32_t dlrmb_shard_plan_mp(int32_t ntab, const int64_t* rows, const int32_t* P, int32_t world, int32_t* owner) {
+    DLRMB_REQUIRE(ntab > 0, "ntab must be positive (got %d)", ntab);
+    DLRMB_REQUIRE(world > 0, "world must be positive (got %d)", world);
+    DLRMB_REQUIRE(rows && owner, "null argument");
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    bool uniform = true;
+    for (int k = 0; k < ntab; ++k) {
+        DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+        uniform = uniform && P[k] == P[0];
+    }
+    if (uniform) return dlrmb_shard_plan(ntab, rows, world, owner);
+    // table k receives B_global * P_k lookups per step: deal the tables longest first (descending P_k, then
+    // rows, then id), each to the rank with the fewest lookups so far (ties: fewer rows, then lower rank)
+    std::vector<int> order(ntab);
+    for (int k = 0; k < ntab; ++k) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](int a, int b) {
+        if (P[a] != P[b]) return P[a] > P[b];
+        if (rows[a] != rows[b]) return rows[a] > rows[b];
+        return a < b;
+    });
+    std::vector<int64_t> load(world, 0), bytes(world, 0);
+    for (int k : order) {
+        int best = 0;
+        for (int r = 1; r < world; ++r)
+            if (load[r] < load[best] || (load[r] == load[best] && bytes[r] < bytes[best])) best = r;
+        owner[k] = best;
+        load[best] += P[k];
+        bytes[best] += rows[k];
+    }
+    return DLRMB_OK;
+}
+
 int32_t dlrmb_comm_unique_id(uint8_t* id128) {
     DLRMB_REQUIRE(id128 != nullptr, "id buffer is null");
     if (!nccl().ok) {
@@ -242,6 +276,41 @@ int32_t dlrmb_comm_a2a_indices(dlrmb_comm* c, const int32_t* owner, int32_t ntab
     for (int h = 0; h < c->world; ++h)                              // rank h's samples of my table j
         for (size_t j = 0; j < mine.size(); ++j)
             DLRMB_NCCL(nccl().Recv(dst + ((size_t)j * c->world + h) * msg, msg, ncclInt8, h, c->comm, s));
+    DLRMB_NCCL(nccl().GroupEnd());
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_comm_a2a_indices_mp(dlrmb_comm* c, const int32_t* owner, int32_t ntab, const void* idx_local,
+                                  int32_t idx_bytes, int32_t B_local, const int32_t* P, void* idx_owned,
+                                  dlrmb_stream stream) {
+    DLRMB_REQUIRE(c && idx_local && idx_owned, "null argument");
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(B_local > 0, "B_local must be positive");
+    for (int k = 0; k < ntab; ++k) DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+    DeviceGuard guard(c->device);
+    int rc = comm_prepare(c, owner, ntab, 0);
+    if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const char* src = static_cast<const char*>(idx_local);
+    char* dst = static_cast<char*>(idx_owned);
+    const std::vector<int>& mine = c->local[c->rank];
+    const size_t Bg = (size_t)B_local * c->world;
+    DLRMB_NCCL(nccl().GroupStart());
+    size_t off = 0;                                                 // elements: table k's block of my samples
+    for (int k = 0; k < ntab; ++k) {
+        const size_t n = (size_t)B_local * P[k];
+        DLRMB_NCCL(nccl().Send(src + off * idx_bytes, n * idx_bytes, ncclInt8, owner[k], c->comm, s));
+        off += n;
+    }
+    for (int h = 0; h < c->world; ++h) {                            // rank h's samples of my table j: rows
+        size_t base = 0;                                            // [h * B_local, (h + 1) * B_local) of its block
+        for (int k : mine) {
+            const size_t n = (size_t)B_local * P[k];
+            DLRMB_NCCL(nccl().Recv(dst + (base + (size_t)h * n) * idx_bytes, n * idx_bytes, ncclInt8, h, c->comm, s));
+            base += Bg * P[k];
+        }
+    }
     DLRMB_NCCL(nccl().GroupEnd());
     return DLRMB_OK;
 }

@@ -272,6 +272,13 @@ int sort_mp_final_half(const dlrmb_tables* t, const MpGeom& g);
 int launch_update_mp(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s);
 int launch_check_indices_mp(dlrmb_tables* t, const void* d_idx, int idx_bytes, int idx_base, const MpGeom& g,
                             cudaStream_t s, long long* bad_table, long long* bad_pos, long long* bad_val);
+// argument checks of the `_mp` entry points at batch B; fills ntab, B, P and off of `g`
+int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, const int32_t* P,
+                  MpGeom* g);
+// record that the last sort was an `_mp` one of geometry g (dlrmb_embedding_update_sorted reads it)
+void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g);
+// gather CTAs per table of an `_mp` lookup (fills g.pre); returns the total
+int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift);
 // lookups of table k in the last sort
 static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) {
     return (int64_t)t->sorted_B * (t->sorted_mp ? t->h_sorted_P[k] : t->sorted_P);

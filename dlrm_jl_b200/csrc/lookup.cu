@@ -334,7 +334,7 @@ lookup_sort_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict
 
 // Gather CTAs per table: the uniform path's launch budget (32 CTAs per SM) split in proportion to B * P_k * C,
 // at least one per table and no more than the table has work items for.  Returns the total.
-static int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift) {
+int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift) {
     constexpr int U = 4;
     int64_t sumP = 0;
     for (int k = 0; k < g.ntab; ++k) sumP += g.P[k];

@@ -173,6 +173,173 @@ static int launch_p2p_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int Bg, 
     return DLRMB_OK;
 }
 
+// ---- per-table pooling factors ------------------------------------------------------------------
+// The `_mp` lookup's geometry (one flat grid, table k owns CTAs [g.pre[k], g.pre[k+1]) in proportion to
+// B_global * P_k * C, lookup_grid_mp of lookup.cu) with the peer-store epilogue above: P_k == 1 takes the
+// U-chain gather, every other table the 4-deep pooling loop in ascending p (the `_mp` lookup's order, so
+// the pooled rows are bit-identical to dlrmb_embedding_fwd_mp).  With SORT_ITEMS > 0 the first g.nlist
+// CTAs sort the tables g.list[] (B_global * P_k <= kFusedSortMax) in shared memory, as
+// lookup_sort_mp_kernel does.  Both parameter structs go by value (__grid_constant__: peers.p[h] is read
+// with a run-time h straight from the parameter bank), so the launch needs no device copy.
+__device__ __forceinline__ float4 p2p_add(float4 a, float4 b) {
+    return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+}
+__device__ __forceinline__ float p2p_add(float a, float b) { return __fadd_rn(a, b); }
+
+template <typename IdxT, int VEC, int U, typename RowT>
+__device__ __forceinline__ void lookup_p2p_mp_cta(const TableDesc* __restrict__ desc, const int32_t* __restrict__ slotmap,
+                                                  const IdxT* __restrict__ idx, int idx_base, const MpGeom& g,
+                                                  uint32_t C, int cshift, uint32_t B_local, const PeerPtrs& peers,
+                                                  int slots, uint32_t lin) {
+    using V = typename std::conditional<VEC == 4, float4, float>::type;
+    const int k = mp_find(g.pre, g.ntab, lin);
+    const uint32_t cx = lin - g.pre[k], nctas = g.pre[k + 1] - g.pre[k];
+    const float* __restrict__ tb = desc[k].base;
+    const IdxT* __restrict__ ik = idx + g.off[k];
+    const uint32_t P = g.P[k];
+    const uint32_t n = g.B * C;
+    const uint32_t step = nctas * blockDim.x;
+    const size_t D = (size_t)C * VEC;
+    const size_t slot_off = (size_t)slotmap[k] * D;
+    const size_t ostride = (size_t)slots * D;
+
+    if (P == 1) {
+        for (uint32_t t = cx * blockDim.x + threadIdx.x; t < n; t += step * U) {
+            int64_t row[U];
+            uint32_t b[U], c[U];
+            bool ok[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                const uint32_t tt = t + (uint32_t)u * step;
+                ok[u] = tt < n;
+                b[u] = cshift >= 0 ? (tt >> cshift) : (tt / C);
+                c[u] = tt - b[u] * C;
+                row[u] = ok[u] ? (int64_t)__ldg(ik + b[u]) - idx_base : 0;
+            }
+            V v[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                if (ok[u]) v[u] = p2p_ldrow<VEC, RowT>(tb, (size_t)row[u], D, c[u]);
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                if (!ok[u]) continue;
+                const uint32_t h = b[u] / B_local;
+                const uint32_t bl = b[u] - h * B_local;
+                reinterpret_cast<V*>(peers.p[h] + (size_t)bl * ostride + slot_off)[c[u]] = v[u];
+            }
+        }
+        return;
+    }
+    for (uint32_t t = cx * blockDim.x + threadIdx.x; t < n; t += step) {
+        const uint32_t b = cshift >= 0 ? (t >> cshift) : (t / C);
+        const uint32_t c = t - b * C;
+        const IdxT* __restrict__ ip = ik + (size_t)b * P;
+        V acc;
+        if constexpr (VEC == 4) acc = make_float4(0.f, 0.f, 0.f, 0.f);
+        else acc = 0.f;
+        uint32_t p = 0;
+        for (; p + 4 <= P; p += 4) {
+            const int64_t r0 = (int64_t)__ldg(ip + p) - idx_base;
+            const int64_t r1 = (int64_t)__ldg(ip + p + 1) - idx_base;
+            const int64_t r2 = (int64_t)__ldg(ip + p + 2) - idx_base;
+            const int64_t r3 = (int64_t)__ldg(ip + p + 3) - idx_base;
+            const V v0 = p2p_ldrow<VEC, RowT>(tb, (size_t)r0, D, c);
+            const V v1 = p2p_ldrow<VEC, RowT>(tb, (size_t)r1, D, c);
+            const V v2 = p2p_ldrow<VEC, RowT>(tb, (size_t)r2, D, c);
+            const V v3 = p2p_ldrow<VEC, RowT>(tb, (size_t)r3, D, c);
+            acc = p2p_add(acc, v0);
+            acc = p2p_add(acc, v1);
+            acc = p2p_add(acc, v2);
+            acc = p2p_add(acc, v3);
+        }
+        for (; p < P; ++p)
+            acc = p2p_add(acc, p2p_ldrow<VEC, RowT>(tb, (size_t)((int64_t)__ldg(ip + p) - idx_base), D, c));
+        const uint32_t h = b / B_local;
+        const uint32_t bl = b - h * B_local;
+        reinterpret_cast<V*>(peers.p[h] + (size_t)bl * ostride + slot_off)[c] = acc;
+    }
+}
+
+template <typename IdxT, int VEC, int U, typename RowT, int SORT_ITEMS>
+__global__ void __launch_bounds__(256, (SORT_ITEMS > 0) ? 4 : 1)
+lookup_p2p_mp_kernel(const TableDesc* __restrict__ desc, const int32_t* __restrict__ slotmap, const IdxT* __restrict__ idx,
+                     int idx_base, const __grid_constant__ MpGeom g, uint32_t C, int cshift, uint32_t B_local,
+                     const __grid_constant__ PeerPtrs peers, int slots, uint32_t* __restrict__ keys_out,
+                     uint32_t* __restrict__ pos_out, int64_t cap, unsigned long long* clk) {
+    clock_in(clk, blockIdx.x);
+    uint32_t lin = blockIdx.x;
+    if constexpr (SORT_ITEMS > 0) {
+        extern __shared__ uint32_t sort_smem[];
+        if ((int)blockIdx.x < g.nlist) {
+            const int k = g.list[blockIdx.x];
+            sort_small_body<IdxT, SORT_ITEMS, 256>(idx + g.off[k], idx_base, (int)(g.B * g.P[k]), desc[k].rows,
+                                                   keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, sort_smem);
+            clock_out(clk, blockIdx.x);
+            return;
+        }
+        lin -= (uint32_t)g.nlist;
+    }
+    lookup_p2p_mp_cta<IdxT, VEC, U, RowT>(desc, slotmap, idx, idx_base, g, C, cshift, B_local, peers, slots, lin);
+    clock_out(clk, blockIdx.x);
+}
+
+// `g` carries ntab, B (= B_global), P and off; gs.nlist > 0 (VEC 4 only) adds the fused sort CTAs of gs.list
+template <typename IdxT, int VEC, typename RowT, int SORT_ITEMS>
+static int launch_p2p_mp_t(dlrmb_tables* t, const IdxT* idx, int idx_base, const MpGeom& g0, const PeerPtrs& peers,
+                           int B_local, int slots, int half, cudaStream_t s) {
+    constexpr int U = 4;
+    const uint32_t C = t->D / VEC;
+    DLRMB_REQUIRE((int64_t)g0.B * C < (1ll << 30), "B * D too large for one lookup launch");
+    MpGeom g = g0;
+    int cshift;
+    const int64_t ctas = lookup_grid_mp(t, g, C, &cshift) + (SORT_ITEMS > 0 ? g.nlist : 0);
+    size_t smem = 0;
+    if constexpr (SORT_ITEMS > 0) {
+        smem = SmallSortGeom<SORT_ITEMS, 256>::smem_bytes();
+        static unsigned long long done = 0;
+        int rc = ensure_smem_attr((const void*)lookup_p2p_mp_kernel<IdxT, VEC, U, RowT, SORT_ITEMS>, (int)smem, &done);
+        if (rc) return rc;
+    }
+    lookup_p2p_mp_kernel<IdxT, VEC, U, RowT, SORT_ITEMS><<<(unsigned)ctas, 256, smem, s>>>(
+        t->d_desc, t->d_slotmap, idx, idx_base, g, C, cshift, (uint32_t)B_local, peers, slots,
+        SORT_ITEMS > 0 ? t->keys[half] : nullptr, SORT_ITEMS > 0 ? t->pos[half] : nullptr, t->cap, clock_slot(CLK_LOOKUP));
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename IdxT, typename RowT>
+static int launch_p2p_mp_i(dlrmb_tables* t, const IdxT* idx, int idx_base, const MpGeom& g, const PeerPtrs& peers,
+                           int B_local, int slots, bool vec4, bool with_sort, cudaStream_t s) {
+    if (!with_sort)
+        return vec4 ? launch_p2p_mp_t<IdxT, 4, RowT, 0>(t, idx, idx_base, g, peers, B_local, slots, 0, s)
+                    : launch_p2p_mp_t<IdxT, 1, RowT, 0>(t, idx, idx_base, g, peers, B_local, slots, 0, s);
+    // the sort of the coming update, as launch_lookup_sort_mp: tables with L_k <= kFusedSortMax in CTAs of
+    // the lookup launch (VEC 4 only), the rest by launch_sort_mp behind it; every table ends in `half`
+    const int half = sort_mp_final_half(t, g);
+    MpGeom gs = g;
+    gs.nlist = 0;
+    int64_t fused_max = 0;
+    if (vec4)
+        for (int k = 0; k < g.ntab; ++k) {
+            const int64_t L = (int64_t)g.B * g.P[k];
+            if (L <= kFusedSortMax) {
+                gs.list[gs.nlist++] = (uint16_t)k;
+                if (L > fused_max) fused_max = L;
+            }
+        }
+    int rc;
+    if (gs.nlist == 0) {
+        rc = vec4 ? launch_p2p_mp_t<IdxT, 4, RowT, 0>(t, idx, idx_base, g, peers, B_local, slots, 0, s)
+                  : launch_p2p_mp_t<IdxT, 1, RowT, 0>(t, idx, idx_base, g, peers, B_local, slots, 0, s);
+        if (rc) return rc;
+        return launch_sort_mp(t, idx, (int)sizeof(IdxT), idx_base, g, 0, half, s);
+    }
+    rc = fused_max <= 2048 ? launch_p2p_mp_t<IdxT, 4, RowT, 8>(t, idx, idx_base, gs, peers, B_local, slots, half, s)
+                           : launch_p2p_mp_t<IdxT, 4, RowT, 16>(t, idx, idx_base, gs, peers, B_local, slots, half, s);
+    if (rc) return rc;
+    return launch_sort_mp(t, idx, (int)sizeof(IdxT), idx_base, g, kFusedSortMax, half, s);
+}
+
 }  // namespace dlrmb
 
 using namespace dlrmb;
@@ -316,6 +483,64 @@ int32_t dlrmb_embedding_fwd_p2p_sort(dlrmb_tables* t, const void* idx, int32_t i
     return embedding_fwd_p2p_impl(t, idx, idx_bytes, idx_base, B_global, P, peer_T, world, B_local, slots, true, stream);
 }
 
+static int32_t embedding_fwd_p2p_mp_impl(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                         int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
+                                         int32_t B_local, int32_t slots, bool with_sort, dlrmb_stream stream) {
+    DLRMB_REQUIRE(t != nullptr && peer_T != nullptr, "null argument");
+    MpGeom g;
+    int rc = check_mp_args(t, idx, idx_bytes, idx_base, B_global, P, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(world >= 1 && world <= kMaxPeers, "world must be in 1..%d (got %d)", kMaxPeers, world);
+    DLRMB_REQUIRE(B_local > 0 && (int64_t)B_global == (int64_t)B_local * world,
+                  "B_global (%d) must equal B_local (%d) * world (%d)", B_global, B_local, world);
+    if (!t->d_slotmap) {
+        set_error("dlrmb_embedding_fwd_p2p_mp needs dlrmb_tables_set_slot_map first");
+        return DLRMB_ESTATE;
+    }
+    DLRMB_REQUIRE(slots > t->slotmap_max, "slots = %d does not cover the slot map (largest slot %d)", slots,
+                  t->slotmap_max);
+    DeviceGuard guard(t->device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", t->device);
+    PeerPtrs peers;
+    bool vec4 = (t->D % 4 == 0);
+    for (int r = 0; r < kMaxPeers; ++r) {
+        peers.p[r] = r < world ? peer_T[r] : nullptr;
+        if (r < world) {
+            DLRMB_REQUIRE(peer_T[r] != nullptr, "peer_T[%d] is null", r);
+            vec4 = vec4 && ((reinterpret_cast<uintptr_t>(peer_T[r]) & 15) == 0);
+        }
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool bf = t->elem_bytes == 2;
+    if (idx_bytes == 4) {
+        const uint32_t* ip = (const uint32_t*)idx;
+        rc = bf ? launch_p2p_mp_i<uint32_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
+                : launch_p2p_mp_i<uint32_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
+    } else {
+        const int64_t* ip = (const int64_t*)idx;
+        rc = bf ? launch_p2p_mp_i<int64_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
+                : launch_p2p_mp_i<int64_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
+    }
+    if (rc) return rc;
+    if (with_sort) mark_sorted_mp(t, g);
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_embedding_fwd_p2p_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                   int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
+                                   int32_t B_local, int32_t slots, dlrmb_stream stream) {
+    return embedding_fwd_p2p_mp_impl(t, idx, idx_bytes, idx_base, B_global, P, peer_T, world, B_local, slots, false,
+                                     stream);
+}
+
+int32_t dlrmb_embedding_fwd_p2p_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                        int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
+                                        int32_t B_local, int32_t slots, dlrmb_stream stream) {
+    if (t) t->sorted_valid = false;
+    return embedding_fwd_p2p_mp_impl(t, idx, idx_bytes, idx_base, B_global, P, peer_T, world, B_local, slots, true,
+                                     stream);
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------
@@ -391,6 +616,27 @@ indices_scatter_kernel(const IdxT* __restrict__ idx_local, const IdxDest* __rest
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
+// Per-table pooling factors: idx_local is the `_mp` layout at B_local (table k's [B_local][P_k] block at
+// element src_off[k]); table k's block lands at dests[k] + rank * B_local * P_k, i.e. rows
+// [rank * B_local, (rank + 1) * B_local) of the owner's [B_global][P_k] block.  The geometry goes by value.
+struct IdxScatterMpGeom {
+    int ntab;
+    int B_local;
+    uint32_t P[kMpMaxTables];
+    int64_t src_off[kMpMaxTables];
+};
+
+template <typename IdxT>
+__global__ void __launch_bounds__(256)
+indices_scatter_mp_kernel(const IdxT* __restrict__ idx_local, const IdxDest* __restrict__ dests,
+                          const __grid_constant__ IdxScatterMpGeom g, int rank) {
+    const int k = blockIdx.y;
+    const int n = g.B_local * (int)g.P[k];
+    const IdxT* src = idx_local + g.src_off[k];
+    IdxT* dst = static_cast<IdxT*>(dests[k].base) + (size_t)rank * n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = src[i];
+}
+
 }  // namespace dlrmb
 
 extern "C" {
@@ -432,6 +678,41 @@ int32_t dlrmb_indices_scatter_p2p(int32_t device, const void* idx_local, int32_t
         indices_scatter_kernel<uint32_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)idx_local, d, ntab, B_local, P, rank);
     else
         indices_scatter_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const int64_t*)idx_local, d, ntab, B_local, P, rank);
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_indices_scatter_p2p_mp(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
+                                     int32_t B_local, const int32_t* P, const void* const* dests_dev, int32_t rank,
+                                     dlrmb_stream stream) {
+    DLRMB_REQUIRE(idx_local && dests_dev, "null argument");
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(ntab > 0 && ntab <= kMpMaxTables, "ntab must be in 1..%d (got %d)", kMpMaxTables, ntab);
+    DLRMB_REQUIRE(B_local > 0 && rank >= 0, "bad index scatter geometry");
+    IdxScatterMpGeom g;
+    g.ntab = ntab;
+    g.B_local = B_local;
+    int64_t off = 0;
+    int32_t maxP = 0;
+    for (int k = 0; k < ntab; ++k) {
+        DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+        DLRMB_REQUIRE((int64_t)B_local * P[k] < (1ll << 30), "B_local * P[%d] too large", k);
+        g.P[k] = (uint32_t)P[k];
+        g.src_off[k] = off;
+        off += (int64_t)B_local * P[k];
+        maxP = P[k] > maxP ? P[k] : maxP;
+    }
+    DeviceGuard guard(device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", device);
+    int bx = (int)((B_local * (int64_t)maxP + 255) / 256);
+    if (bx > 64) bx = 64;
+    dim3 grid((unsigned)bx, (unsigned)ntab);
+    const IdxDest* d = reinterpret_cast<const IdxDest*>(dests_dev);
+    if (idx_bytes == 4)
+        indices_scatter_mp_kernel<uint32_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)idx_local, d, g, rank);
+    else
+        indices_scatter_mp_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const int64_t*)idx_local, d, g, rank);
     DLRMB_LAUNCH_CHECK();
     return DLRMB_OK;
 }

@@ -66,6 +66,10 @@ class PackedIndices:
     def is_cuda(self) -> bool:
         return self.flat.is_cuda
 
+    @property
+    def device(self) -> torch.device:
+        return self.flat.device
+
     def to(self, device, non_blocking: bool = False) -> "PackedIndices":
         return PackedIndices(self.flat.to(device, non_blocking=non_blocking).contiguous(), self.P, self.B)
 
@@ -249,11 +253,16 @@ class EmbeddingTables:
         """Pool this rank's tables for the global batch and store every pooled row directly into
         the owning rank's interaction buffer (NVLink peer stores): lookup + forward exchange fused.
         ``sort=True`` also sorts / dedups the indices for this batch's sparse update in the same launch
-        (dlrmb_embedding_fwd_p2p_sort)."""
-        ntab, Bg, P = idx.shape
+        (dlrmb_embedding_fwd_p2p_sort).  ``idx`` may be :class:`PackedIndices` at B_global (per-table
+        pooling factors, dlrmb_embedding_fwd_p2p_mp / _sort_mp)."""
+        if isinstance(idx, PackedIndices):
+            Bg, P = idx.B, idx.P_array()
+            fn = self._lib.dlrmb_embedding_fwd_p2p_sort_mp if sort else self._lib.dlrmb_embedding_fwd_p2p_mp
+        else:
+            ntab, Bg, P = idx.shape
+            fn = self._lib.dlrmb_embedding_fwd_p2p_sort if sort else self._lib.dlrmb_embedding_fwd_p2p
         world = len(peer_ptrs)
         arr = (C.c_void_p * world)(*[int(p) for p in peer_ptrs])
-        fn = self._lib.dlrmb_embedding_fwd_p2p_sort if sort else self._lib.dlrmb_embedding_fwd_p2p
         with _prof.range("lookup"):
             _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, Bg, P, arr, world, B_local, slots,
                           _stream_ptr(self.device)))

@@ -18,7 +18,7 @@ CUDA library.
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import Callable, List, Optional, Sequence
+from typing import Callable, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -29,12 +29,17 @@ import torch.distributed as dist
 class TableSharding:
     """Which rank owns which table, balanced by LOOKUP COUNT first (every table receives
     B_global * P lookups per step whatever its size), then by bytes: tables are dealt in
-    descending row count, snake order, so the big tables land on different ranks."""
+    descending row count, snake order, so the big tables land on different ranks.
+
+    With per-table pooling factors P_k (not all equal) table k receives B_global * P_k lookups, so the
+    tables are dealt longest first instead: descending P_k, then rows, then id, each to the rank with the
+    smallest sum of P_k so far (ties: fewer rows, then the lower rank).  Equal P_k give the snake plan."""
     rows: List[int]
     world: int
     owner: List[int]
     local: List[List[int]]      # local[r] = global table ids owned by rank r, ascending
     _slot_cache: Optional[dict] = None
+    P: Optional[Tuple[int, ...]] = None     # per-table pooling factors the plan was built for (None: one P)
 
     def slot_index(self, r: int, device) -> torch.Tensor:
         """Device tensor of the interaction slots (1 + table id) of rank r's tables (cached: no
@@ -57,15 +62,36 @@ class TableSharding:
         return self._slot_cache[key]
 
     @classmethod
-    def build(cls, rows: Sequence[int], world: int) -> "TableSharding":
+    def build(cls, rows: Sequence[int], world: int, P: Optional[Sequence[int]] = None) -> "TableSharding":
+        """The same rule as dlrmb_shard_plan (``P`` None or all equal) / dlrmb_shard_plan_mp."""
         rows = [int(r) for r in rows]
-        order = sorted(range(len(rows)), key=lambda k: (-rows[k], k))
+        Pt = None
+        if P is not None:
+            if world < 1 or not rows:
+                raise ValueError(f"a shard plan needs world >= 1 and a table (world {world}, {len(rows)} tables)")
+            Pt = tuple(int(p) for p in P)
+            if len(Pt) != len(rows) or min(Pt) < 1:
+                raise ValueError(f"P must hold one pooling factor >= 1 per table ({len(rows)} tables), got {list(Pt)}")
         owner = [0] * len(rows)
-        for i, k in enumerate(order):
-            rnd, pos = divmod(i, world)
-            owner[k] = pos if rnd % 2 == 0 else world - 1 - pos
+        if Pt is None or len(set(Pt)) == 1:
+            order = sorted(range(len(rows)), key=lambda k: (-rows[k], k))
+            for i, k in enumerate(order):
+                rnd, pos = divmod(i, world)
+                owner[k] = pos if rnd % 2 == 0 else world - 1 - pos
+        else:
+            load, size = [0] * world, [0] * world
+            for k in sorted(range(len(rows)), key=lambda k: (-Pt[k], -rows[k], k)):
+                r = min(range(world), key=lambda r: (load[r], size[r], r))
+                owner[k] = r
+                load[r] += Pt[k]
+                size[r] += rows[k]
         local = [[k for k in range(len(rows)) if owner[k] == r] for r in range(world)]
-        return cls(rows, world, owner, local)
+        return cls(rows, world, owner, local, P=Pt)
+
+    def lookups_per_rank(self) -> List[int]:
+        """Sum of P_k over each rank's tables (per sample of the global batch)."""
+        P = self.P or (1,) * len(self.rows)
+        return [sum(P[k] for k in l) for l in self.local]
 
     def counts(self) -> List[int]:
         return [len(l) for l in self.local]
@@ -105,6 +131,35 @@ def exchange_indices(idx_local: torch.Tensor, sh: TableSharding, rank: int, grou
     _a2a(recv.view(-1), send.view(-1), out_splits, in_splits, group)
     # [W][t][Bl][P] -> [t][W*Bl][P]
     return recv.permute(1, 0, 2, 3).reshape(t_mine, W * Bl, P).contiguous()
+
+
+def exchange_indices_mp(packed, sh: TableSharding, rank: int, group=None):
+    """Per-table pooling factors: ``packed`` (:class:`~dlrm_jl_b200.embedding.PackedIndices` of this rank's
+    B_local samples, every table) -> this rank's tables in the owner layout: a PackedIndices at B_global of
+    the owned tables in ascending id (table j's [B_global][P_j] block after the blocks of the owned tables
+    before it, rank h's samples in its rows [h * B_local, (h + 1) * B_local)), which the `_mp` lookup, sort
+    and update read as is."""
+    from .embedding import PackedIndices
+    W = sh.world
+    if W == 1:
+        return packed
+    P, Bl, flat = packed.P, packed.B, packed.flat
+    mine = sh.local[rank]
+    offs = np.concatenate([[0], np.cumsum([Bl * p for p in P])]).tolist()
+    order = [k for r in range(W) for k in sh.local[r]]                                  # grouped by owner
+    send = torch.cat([flat[offs[k]:offs[k + 1]] for k in order]) if order else flat[:0]
+    in_splits = [Bl * sum(P[k] for k in sh.local[r]) for r in range(W)]
+    per_rank = Bl * sum(P[k] for k in mine)
+    recv = torch.empty((W * per_rank,), dtype=flat.dtype, device=flat.device)
+    _a2a(recv, send.contiguous(), [per_rank] * W, in_splits, group)
+    # [h][j][B_local][P_j] -> [j][h][B_local][P_j]
+    parts, o = [], 0
+    for k in mine:
+        n = Bl * P[k]
+        parts.extend(recv[h * per_rank + o:h * per_rank + o + n] for h in range(W))
+        o += n
+    owned = torch.cat(parts) if parts else recv[:0]
+    return PackedIndices(owned.contiguous(), tuple(P[k] for k in mine), Bl * W)
 
 
 def exchange_pooled(pooled: torch.Tensor, T: torch.Tensor, sh: TableSharding, rank: int, group=None) -> None:
@@ -203,10 +258,16 @@ class PeerExchange:
             torch.cuda.synchronize(self.device)
             dist.barrier(group=group)           # every rank's flag array exists and is zero before anyone signals
 
-    def enable_index_exchange(self, sharding: "TableSharding", B_local: int, P: int, idx_bytes: int = 4):
+    def enable_index_exchange(self, sharding: "TableSharding", B_local: int, P: Union[int, Sequence[int]],
+                              idx_bytes: int = 4):
         """Index exchange by peer stores: an index buffer [t_mine][B_global][P] on every rank, mapped
-        everywhere; each rank stores its samples' index columns straight into the owners' buffers."""
+        everywhere; each rank stores its samples' index columns straight into the owners' buffers.
+        ``P`` a sequence (one pooling factor per table): the buffer holds the owner layout of
+        :func:`exchange_indices_mp` (sum over the owned tables of B_global * P_k indices) and ``idx_owned``
+        is a :class:`~dlrm_jl_b200.embedding.PackedIndices`."""
         from .embedding import _DevicePtrView
+        if not isinstance(P, (int, np.integer)):
+            return self._enable_index_exchange_mp(sharding, B_local, tuple(int(p) for p in P), idx_bytes)
         counts = sharding.counts()
         t_mine = counts[self.rank]
         Bg = B_local * self.world
@@ -219,6 +280,27 @@ class PeerExchange:
                  for k in range(len(sharding.rows))]
         self._idx_dests = torch.tensor(dests, dtype=torch.int64, device=self.device)
         self._idx_geom = (len(sharding.rows), B_local, P, idx_bytes)
+
+    def _enable_index_exchange_mp(self, sharding: "TableSharding", B_local: int, P: Tuple[int, ...], idx_bytes: int):
+        import ctypes as C
+
+        from .embedding import PackedIndices, _DevicePtrView
+        if len(P) != len(sharding.rows) or min(P) < 1:
+            raise ValueError(f"P must hold one pooling factor >= 1 per table ({len(sharding.rows)} tables), got {list(P)}")
+        Bg = B_local * self.world
+        mine = sharding.local[self.rank]
+        n_owned = sum(Bg * P[k] for k in mine)
+        self._ibuf, own, peer_idx = self._share(max(1, n_owned) * idx_bytes)
+        ts = "<i4" if idx_bytes == 4 else "<i8"
+        flat = torch.as_tensor(_DevicePtrView(own, (max(1, n_owned),), self, ts), device=self.device)
+        self.idx_owned = PackedIndices(flat[:n_owned], tuple(P[k] for k in mine), Bg)
+        dests = []
+        for k in range(len(sharding.rows)):        # owner's block of table k: after its owned tables below k
+            o = sharding.owner[k]
+            dests.append(peer_idx[o] + sum(Bg * P[i] for i in sharding.local[o] if i < k) * idx_bytes)
+        self._idx_dests = torch.tensor(dests, dtype=torch.int64, device=self.device)
+        self._idx_geom = (len(sharding.rows), B_local, P, idx_bytes)
+        self._idx_P = (C.c_int32 * len(P))(*P)
 
     def enable_small_allreduce(self, n: int) -> None:
         """Exchange buffer [2][world][n] floats for `allreduce_small` (dlrmb_peer_allreduce_f32)."""
@@ -240,9 +322,19 @@ class PeerExchange:
 
     def scatter_indices(self, idx_local: torch.Tensor) -> torch.Tensor:
         """idx_local [ntab][B_local][P] -> the owners' buffers (peer stores) + barrier; returns this rank's
-        idx_owned [t_mine][B_global][P]."""
+        idx_owned [t_mine][B_global][P] (PackedIndices in, PackedIndices in the owner layout out when the
+        exchange was enabled with per-table pooling factors)."""
         from . import _lib
         ntab, Bl, P, ib = self._idx_geom
+        if isinstance(P, tuple):
+            from . import _prof
+            assert tuple(idx_local.P) == P and idx_local.B == Bl and idx_local.element_size() == ib
+            with _prof.range("indices_scatter"):
+                _lib.check(self.lib.dlrmb_indices_scatter_p2p_mp(
+                    self.device.index or 0, idx_local.data_ptr(), ib, ntab, Bl, self._idx_P, self._idx_dests.data_ptr(),
+                    self.rank, int(torch.cuda.current_stream(self.device).cuda_stream)))
+            self.barrier(0)
+            return self.idx_owned
         assert tuple(idx_local.shape) == (ntab, Bl, P) and idx_local.element_size() == ib and idx_local.is_contiguous()
         from . import _prof
         with _prof.range("indices_scatter"):
@@ -348,9 +440,10 @@ class _ShardedLookupFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, anchor: torch.Tensor, se: "ShardedEmbedding", idx_local: torch.Tensor):
+        from .embedding import _batch
         ctx.se = se
         D = se.D
-        Bl = idx_local.shape[1]
+        Bl = _batch(idx_local)
         if se.world == 1:
             # no exchange: pool straight into the interaction input (slot 0 is filled with x by
             # the interaction kernel's fused fast_vcat); the same launch sorts the indices for the update
@@ -362,12 +455,12 @@ class _ShardedLookupFn(torch.autograd.Function):
         idx_owned = se._exchange_indices(idx_local)
         se.idx_owned = idx_owned
         se.presorted = False
-        Bg = idx_owned.shape[1]
+        Bg = _batch(idx_owned)
         if se.peer is not None:
             # fused path: pooled rows go straight into the owners' T over NVLink; the barrier
             # orders every rank's stores before anyone reads its own T
             if len(se.local_ids):
-                fuse = idx_owned.shape[1] * idx_owned.shape[2] <= se.tables.FUSED_SORT_MAX
+                fuse = se._fuse_sort(idx_owned)
                 se.tables.lookup_p2p(idx_owned, se.peer.peer_ptrs, Bl, 1 + se.ntab, se.idx_base, sort=fuse)
                 se.presorted = fuse
             se.peer.barrier(1)
@@ -404,11 +497,16 @@ class ShardedEmbedding:
 
     def __init__(self, rows: Sequence[int], D: int, rank: int, world: int, lookup_fn: Callable,
                  update_fn: Callable, group=None, sort_fn: Optional[Callable] = None, idx_base: int = 0,
-                 lookup_sorts: bool = False):
+                 lookup_sorts: bool = False, P: Optional[Sequence[int]] = None):
         """``idx_base``: 1 for reference-format (1-based) ids, 0 for PyTorch-style ids; it is handed to
         every kernel that reads the indices.  ``lookup_sorts``: `lookup_fn` also prepares the sort /
-        dedup of the step's update (the fused launch), so `sort_async` has nothing left to do."""
-        self.sharding = TableSharding.build(rows, world)
+        dedup of the step's update (the fused launch), so `sort_async` has nothing left to do.
+        ``P``: per-table pooling factors (one per table).  Then the tables are placed by
+        ``TableSharding.build(rows, world, P)``, batches are :class:`~dlrm_jl_b200.embedding.PackedIndices`
+        (or anything ``_as_index_tensor`` turns into one) and the owners receive theirs in the owner layout
+        of :func:`exchange_indices_mp`.  Without it every table has the same P and mixed widths are refused."""
+        self.P = None if P is None else tuple(int(p) for p in P)
+        self.sharding = TableSharding.build(rows, world, self.P)
         self.rank, self.world, self.group = rank, world, group
         self.idx_base = int(idx_base)
         self.lookup_sorts = bool(lookup_sorts)
@@ -460,23 +558,59 @@ class ShardedEmbedding:
     def lookup_fused(self, idx_local: torch.Tensor) -> torch.Tensor:
         """Forward of the fully fused path: no autograd node (the gradient never comes back through
         T; it is scattered to the owners by the interaction backward)."""
-        _require_uniform_pooling(idx_local)
+        from .embedding import _batch
+        idx_local = self._indices(idx_local)
         with torch.no_grad():
             idx_owned = self._exchange_indices(idx_local)
             self.idx_owned = idx_owned
             self.presorted = False
             if len(self.local_ids):
                 # up to 4096 lookups per table the sort of the coming update rides in the lookup launch
-                fuse = idx_owned.shape[1] * idx_owned.shape[2] <= self.tables.FUSED_SORT_MAX
-                self.tables.lookup_p2p(idx_owned, self.peer.peer_ptrs, idx_local.shape[1], 1 + self.ntab, self.idx_base,
+                fuse = self._fuse_sort(idx_owned)
+                self.tables.lookup_p2p(idx_owned, self.peer.peer_ptrs, _batch(idx_local), 1 + self.ntab, self.idx_base,
                                        sort=fuse)
                 self.presorted = fuse
             self.peer.barrier(1)
             return self.peer.T.detach()
 
+    def _fuse_sort(self, idx_owned) -> bool:
+        """Whether every owned table's sort fits the lookup launch (B_global * P_k <= FUSED_SORT_MAX); otherwise
+        the large sorts go to the side stream (`sort_async`), off the critical path."""
+        from .embedding import PackedIndices
+        if isinstance(idx_owned, PackedIndices):
+            return max(idx_owned.P) * idx_owned.B <= self.tables.FUSED_SORT_MAX
+        return idx_owned.shape[1] * idx_owned.shape[2] <= self.tables.FUSED_SORT_MAX
+
+    def _indices(self, idx_local):
+        """A handle with one P refuses mixed widths; one with per-table P takes PackedIndices or anything
+        `_as_index_tensor` normalises (the reference's mixed list, or a [ntab][B][P] tensor when every P_k
+        is equal) and checks the widths against its P."""
+        if self.P is None:
+            _require_uniform_pooling(idx_local)
+            return idx_local
+        from .embedding import PackedIndices, _as_index_tensor
+        tables = getattr(self, "tables", None)
+        if tables is not None:
+            device = tables.device
+        else:
+            device = idx_local.flat.device if isinstance(idx_local, PackedIndices) else (
+                idx_local.device if isinstance(idx_local, torch.Tensor) else torch.device("cpu"))
+        idx = _as_index_tensor(idx_local, self.ntab, device)
+        if not isinstance(idx, PackedIndices):
+            if tuple(int(idx.shape[2]) for _ in range(self.ntab)) != self.P:
+                raise ValueError(f"batch widths {[int(idx.shape[2])] * self.ntab} differ from the handle's P {list(self.P)}")
+            idx = PackedIndices(idx.reshape(-1), self.P, int(idx.shape[1]))
+        if tuple(idx.P) != self.P:
+            raise ValueError(f"batch widths {list(idx.P)} differ from the handle's P {list(self.P)}")
+        return idx
+
     def _exchange_indices(self, idx_local: torch.Tensor) -> torch.Tensor:
         """Index columns to the tables' owners: peer stores + flag barrier when the index buffers are
         mapped (`enable_index_exchange`), NCCL all-to-all otherwise."""
+        if self.P is not None:
+            if self.peer is not None and self.peer._idx_dests is not None:
+                return self.peer.scatter_indices(idx_local)
+            return exchange_indices_mp(idx_local, self.sharding, self.rank, self.group)
         if self.peer is not None and self.peer._idx_dests is not None:
             owned = self.peer.scatter_indices(idx_local)
             return owned[:len(self.local_ids)] if len(self.local_ids) else owned[:0]
@@ -497,11 +631,14 @@ class ShardedEmbedding:
         self.owned_grad = self.peer.G
 
     def enable_peer_exchange(self, B_local: int, barrier: Optional[Callable] = None, flag_barrier: bool = True,
-                             P: Optional[int] = None, idx_bytes: int = 4) -> None:
+                             P: Optional[Union[int, Sequence[int]]] = None, idx_bytes: int = 4) -> None:
         """Switch the forward exchange to the fused lookup + NVLink peer-store kernel.  Safe with
         one buffer per rank when every step also runs the backward exchange (a barrier all ranks
-        reach only after they have finished reading T).  With ``P`` (lookups per sample) given, the
-        index exchange also goes over peer stores instead of an NCCL all-to-all."""
+        reach only after they have finished reading T).  With ``P`` (lookups per sample, or the handle's
+        per-table pooling factors) given, the index exchange also goes over peer stores instead of an NCCL
+        all-to-all."""
+        if self.P is not None and P is not None and tuple(int(p) for p in P) != self.P:
+            raise ValueError(f"P {list(P)} differs from the handle's per-table P {list(self.P)}")
         if self.world == 1:
             return
         self.tables.set_slot_map([1 + k for k in self.local_ids] or [1])
@@ -511,13 +648,17 @@ class ShardedEmbedding:
             self.peer.enable_index_exchange(self.sharding, B_local, P, idx_bytes)
 
     @classmethod
-    def create(cls, rows: Sequence[int], D: int, B_local: int, P: int, rank: int, world: int, device,
-               group=None, seed: int = 51234, idx_base: int = 0, dtype=None) -> "ShardedEmbedding":
+    def create(cls, rows: Sequence[int], D: int, B_local: int, P: Union[int, Sequence[int]], rank: int, world: int,
+               device, group=None, seed: int = 51234, idx_base: int = 0, dtype=None) -> "ShardedEmbedding":
+        """``P``: lookups per sample of every table, or a sequence of one pooling factor per table (mixed
+        multi-hot; the plan then weighs each table by its P_k, see :class:`TableSharding`)."""
         from .embedding import EmbeddingTables
-        sh = TableSharding.build(rows, world)
+        Pseq = None if isinstance(P, (int, np.integer)) else tuple(int(p) for p in P)
+        sh = TableSharding.build(rows, world, Pseq)
         mine = sh.local[rank]
         kw = {} if dtype is None else {"dtype": dtype}
-        tables = EmbeddingTables([rows[k] for k in mine] or [1], D, B_local * world * P, device, **kw)
+        max_lookups = B_local * world * (P if Pseq is None else max([Pseq[k] for k in mine] or [1]))
+        tables = EmbeddingTables([rows[k] for k in mine] or [1], D, max_lookups, device, **kw)
         tables.init_uniform(seed + 7919 * rank)
         fused_sort = world == 1      # single GPU: the sort rides in the lookup launch
         se = cls(rows, D, rank, world,
@@ -526,15 +667,15 @@ class ShardedEmbedding:
                      tables.update_sorted(g, slot0, lr) if presorted else tables.bwd_sgd(idx, g, slot0, lr, idx_base)),
                  group=group,
                  sort_fn=lambda idx: tables.sort(idx, idx_base, side_stream=True),
-                 idx_base=idx_base, lookup_sorts=fused_sort)
+                 idx_base=idx_base, lookup_sorts=fused_sort, P=Pseq)
         se.tables = tables
         return se
 
     def lookup(self, idx_local: torch.Tensor, anchor: torch.Tensor) -> torch.Tensor:
         """idx_local [ntab][B_local][P] -> T [B_local][1 + ntab][D] (requires grad through `anchor`,
-        any tensor that requires grad, so autograd calls the gradient exchange)."""
-        _require_uniform_pooling(idx_local)
-        return _ShardedLookupFn.apply(anchor, self, idx_local)
+        any tensor that requires grad, so autograd calls the gradient exchange).  A handle with per-table
+        pooling factors takes PackedIndices (or the reference's mixed list) instead."""
+        return _ShardedLookupFn.apply(anchor, self, self._indices(idx_local))
 
     def sort_async(self) -> None:
         """Start the index sort/dedup for this step's update on the side stream (nothing to do when

@@ -185,7 +185,8 @@ int32_t dlrmb_check_indices(dlrmb_tables* t, const void* idx, int32_t idx_bytes,
  * do not allocate, synchronise or copy from host memory, so they can be captured into a CUDA graph.
  * dlrmb_embedding_update_sorted and dlrmb_sort_dedup_export consume the last sort, uniform or _mp: after
  * an _mp sort, the export of table k returns its B * P_k entries.  The table-sharded multi-GPU entry
- * points take one P only. */
+ * points have `_mp` forms too (dlrmb_shard_plan_mp, dlrmb_comm_a2a_indices_mp, dlrmb_indices_scatter_p2p_mp,
+ * dlrmb_embedding_fwd_p2p_mp / _sort_mp below). */
 int32_t dlrmb_mp_max_tables(void);
 int32_t dlrmb_embedding_fwd_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base, int32_t B,
                                const int32_t* P, float* out, int32_t slots, int32_t slot0, dlrmb_stream stream);
@@ -263,6 +264,20 @@ int32_t dlrmb_embedding_fwd_p2p(dlrmb_tables* t, const void* idx, int32_t idx_by
 int32_t dlrmb_embedding_fwd_p2p_sort(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
                                      int32_t B_global, int32_t P, float* const* peer_T, int32_t world,
                                      int32_t B_local, int32_t slots, dlrmb_stream stream);
+/* Per-table pooling factors: `P` is a host array of the handle's ntab pooling factors and `idx` the `_mp`
+ * layout at B = B_global (table k's [B_global][P_k] block at element B_global * (P_0 + .. + P_{k-1}), the
+ * owner layout that dlrmb_comm_a2a_indices_mp / dlrmb_indices_scatter_p2p_mp fill).  The pooled rows are
+ * bit-identical to dlrmb_embedding_fwd_mp's.  The _sort_mp form sorts every table for the coming
+ * dlrmb_embedding_update_sorted as dlrmb_embedding_fwd_sort_mp does (B_global * P_k <= 4096 inside the
+ * lookup launch, larger tables by the stand-alone sorts on the same stream).  Arguments are checked as for
+ * the `_mp` and p2p entry points (B_global * max P_k <= max_lookups; DLRMB_ESTATE without a slot map).
+ * No allocation, synchronisation or host copy: graph-capturable. */
+int32_t dlrmb_embedding_fwd_p2p_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                   int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
+                                   int32_t B_local, int32_t slots, dlrmb_stream stream);
+int32_t dlrmb_embedding_fwd_p2p_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
+                                        int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
+                                        int32_t B_local, int32_t slots, dlrmb_stream stream);
 
 /* Ordering point of the fused exchanges without NCCL: a flag barrier over IPC-mapped memory, one tiny
  * kernel per call.  Every rank allocates a zero-initialised dlrmb_xbuf of dlrmb_peer_barrier_flag_bytes()
@@ -294,6 +309,13 @@ int32_t dlrmb_peer_allreduce_f32(int32_t device, float* const* peer_bufs, uint32
 int32_t dlrmb_indices_scatter_p2p(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
                                   int32_t B_local, int32_t P, const void* const* dests_dev, int32_t rank,
                                   dlrmb_stream stream);
+/* Per-table pooling factors: idx_local is the `_mp` layout at B_local (table k's [B_local][P_k] block at
+ * element B_local * (P_0 + .. + P_{k-1})), `P` a host array [ntab] (ntab <= dlrmb_mp_max_tables()), and
+ * dests_dev[k] the owner's [B_global][P_k] block of global table k; this rank fills rows
+ * [rank * B_local, (rank + 1) * B_local) of it.  No allocation; graph-capturable. */
+int32_t dlrmb_indices_scatter_p2p_mp(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
+                                     int32_t B_local, const int32_t* P, const void* const* dests_dev, int32_t rank,
+                                     dlrmb_stream stream);
 
 /* Interaction backward fused with the gradient exchange: as dlrmb_interaction_bwd, but the gradient
  * row of feature slot f >= 1 of local sample b is stored at
@@ -328,15 +350,28 @@ int32_t dlrmb_interaction_bwd_scatter(int32_t device, const float* dOut, const f
  *   dlrmb_comm_allgather     nbytes per rank, device buffers (e.g. the 64-byte dlrmb_xbuf IPC handles that
  *                            set up the fused peer-store exchanges above)
  * The first a2a call sizes a staging buffer (cudaMalloc); later calls with the same geometry do not
- * allocate and can be captured into a CUDA graph. */
+ * allocate and can be captured into a CUDA graph.
+ * Per-table pooling factors (`P` = host array [ntab] of P_k >= 1):
+ *   dlrmb_shard_plan_mp      equal P_k: exactly dlrmb_shard_plan.  Mixed: tables dealt longest first
+ *                            (descending P_k, then rows, then id), each to the rank with the smallest sum
+ *                            of P_k so far (ties: fewer rows, then the lower rank)
+ *   dlrmb_comm_a2a_indices_mp  idx_local (`_mp` layout at B_local) -> idx_owned, the `_mp` layout of this
+ *                            rank's tables (ascending global id) at B_global: table j's [B_global][P_j] block
+ *                            starts at B_global * (sum of P_i of the owned tables before it), rank h's samples
+ *                            are its rows [h * B_local, (h + 1) * B_local).  dlrmb_embedding_fwd_mp /
+ *                            _sort_mp / _bwd_sgd_mp read it with the owned tables' P as is. */
 typedef struct dlrmb_comm dlrmb_comm;
 int32_t dlrmb_shard_plan(int32_t ntab, const int64_t* rows, int32_t world, int32_t* owner);
+int32_t dlrmb_shard_plan_mp(int32_t ntab, const int64_t* rows, const int32_t* P, int32_t world, int32_t* owner);
 int32_t dlrmb_comm_unique_id(uint8_t* id128);
 int32_t dlrmb_comm_create(int32_t device, const uint8_t* id128, int32_t rank, int32_t world, dlrmb_comm** out);
 int32_t dlrmb_comm_destroy(dlrmb_comm* c);
 int32_t dlrmb_comm_info(const dlrmb_comm* c, int32_t* rank, int32_t* world);
 int32_t dlrmb_comm_a2a_indices(dlrmb_comm* c, const int32_t* owner, int32_t ntab, const void* idx_local,
                                int32_t idx_bytes, int32_t B_local, int32_t P, void* idx_owned, dlrmb_stream stream);
+int32_t dlrmb_comm_a2a_indices_mp(dlrmb_comm* c, const int32_t* owner, int32_t ntab, const void* idx_local,
+                                  int32_t idx_bytes, int32_t B_local, const int32_t* P, void* idx_owned,
+                                  dlrmb_stream stream);
 int32_t dlrmb_comm_a2a_fwd(dlrmb_comm* c, const int32_t* owner, int32_t ntab, const float* pooled, int32_t B_local,
                            int32_t D, float* T, dlrmb_stream stream);
 int32_t dlrmb_comm_a2a_bwd(dlrmb_comm* c, const int32_t* owner, int32_t ntab, const float* dT, int32_t B_local,

@@ -394,6 +394,15 @@ function shard_plan(rows::Vector{Int64}, world::Integer)
     return owner
 end
 
+"""Per-table pooling factors `P[k]`: equal P gives `shard_plan(rows, world)`; mixed P deals the tables longest
+first (descending P, rows, id), each to the rank with the smallest sum of P so far (ties: fewer rows, lower rank)."""
+function shard_plan(rows::Vector{Int64}, world::Integer, P::Vector{Int32})
+    owner = Vector{Int32}(undef, length(rows))
+    check(ccall((:dlrmb_shard_plan_mp, libdlrm_b200), Int32, (Int32, Ptr{Int64}, Ptr{Int32}, Int32, Ptr{Int32}),
+                length(rows), rows, P, world, owner))
+    return owner
+end
+
 "Rank 0: the 128-byte NCCL id to hand to the other ranks (file, socket, MPI.bcast ...)."
 function comm_unique_id()
     id = Vector{UInt8}(undef, 128)
