@@ -16,7 +16,7 @@ for i in 1 2; do
   (cd $PARENT && python benchmarks/hotpath.py --workload kaggle --no-interaction) >> $O/hotpath_parent_kaggle.jsonl
   python benchmarks/hotpath.py --workload kaggle --no-interaction >> $O/hotpath_pr_kaggle.jsonl
 done
-timeout 1200 python benchmarks/multihot.py --mode ab full overhead step --out $O/multihot.jsonl > $O/multihot.log 2>&1
+timeout 1200 python benchmarks/multihot.py --mode ab full step --out $O/multihot.jsonl > $O/multihot.log 2>&1
 timeout 1500 python -m pytest tests -q -m gpu > $O/pytest_gpu_all.log 2>&1
 python -c "import __graft_entry__ as g; g.smoke()" > $O/smoke.log 2>&1
 python bench.py --gpus 1 --steps 50 --warmup 10 > $O/bench.json

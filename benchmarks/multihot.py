@@ -8,7 +8,6 @@ with CUDA events; one JSON line per mode, with the GPU name and power limit read
 
     python benchmarks/multihot.py --mode ab --rows-cap 20000000     # mixed vs one handle per hotness group
     python benchmarks/multihot.py --mode full                        # mixed only, rows capped at 40M
-    python benchmarks/multihot.py --mode overhead                    # every P_k = 1: _mp vs uniform entry points
     python benchmarks/multihot.py --mode step                        # DLRMModel training step, samples/s
 """
 from __future__ import annotations
@@ -180,33 +179,6 @@ def mode_ab(a, rows, P, dev, info):
     return r
 
 
-def mode_overhead(a, rows, dev, info):
-    D, B = a.D, a.batch
-    t = EmbeddingTables(rows, D, B, dev)
-    t.init_uniform(1)
-    rng = np.random.default_rng(1234)
-    P = [1] * len(rows)
-    batches = make_batches(rng, rows, P, B, a.nb, a.zipf, dev)
-    uni = [b.flat.view(len(rows), B, 1) for b in batches]
-    T = torch.empty((B, 1 + len(rows), D), device=dev)
-    dT = torch.randn((B, 1 + len(rows), D), device=dev) * 0.01
-
-    def chain(idx):
-        def f(i):
-            t.lookup(idx[i], T, 1, sort=True)
-            t.update_sorted(dT, 1, 0.01)
-        return f
-    res = {"uniform": {"lookup": [], "chain": []}, "mp": {"lookup": [], "chain": []}}
-    for _ in range(a.repeats):
-        for name, idx in (("uniform", uni), ("mp", batches)):
-            res[name]["lookup"].append(timed(lambda i: t.lookup(idx[i], T, 1), a.nb, a.iters))
-            res[name]["chain"].append(timed(chain(idx), a.nb, a.iters))
-    t.close()
-    summary = {n: {k: {"median": float(np.median(v)), "min": min(v), "max": max(v)} for k, v in d.items()}
-               for n, d in res.items()}
-    return dict(info, mode="overhead", rows_cap=a.rows_cap, D=D, B=B, hotness=P, us=summary, raw_us=res)
-
-
 def mode_step(a, rows, P, dev, info):
     from dlrm_jl_b200.embedding import Descent
     from dlrm_jl_b200.model import dlrm
@@ -236,7 +208,7 @@ def mode_step(a, rows, P, dev, info):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--mode", choices=["ab", "full", "overhead", "step"], nargs="+", default=["full"])
+    ap.add_argument("--mode", choices=["ab", "full", "step"], nargs="+", default=["full"])
     ap.add_argument("--hotness", default=MLPERF_HOTNESS)
     ap.add_argument("--zipf", type=float, default=0.0)
     ap.add_argument("--batch", type=int, default=2048)
@@ -263,8 +235,6 @@ def main():
             r = mode_full(a, rows, P, dev, info)
         elif mode == "ab":
             r = mode_ab(a, rows, P, dev, info)
-        elif mode == "overhead":
-            r = mode_overhead(a, rows, dev, info)
         else:
             r = mode_step(a, rows, P, dev, info)
         torch.cuda.empty_cache()

@@ -352,7 +352,9 @@ int32_t dlrmb_embedding_fwd(dlrmb_tables* t, const void* idx, int32_t idx_bytes,
     DLRMB_REQUIRE(out != nullptr, "out is null");
     DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
                   "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
-    return launch_lookup(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, (cudaStream_t)stream);
+    return run_uniform(t, idx, idx_bytes, B, P, slot0, false, [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int gslot0) {
+        return launch_lookup_mp(v, gidx, idx_bytes, idx_base, g, out, slots, gslot0, (cudaStream_t)stream);
+    });
 }
 
 int32_t dlrmb_embedding_fwd_sort(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
@@ -365,13 +367,9 @@ int32_t dlrmb_embedding_fwd_sort(dlrmb_tables* t, const void* idx, int32_t idx_b
     DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
                   "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
     t->sorted_valid = false;
-    rc = launch_lookup_sort(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, (cudaStream_t)stream);
-    if (rc) return rc;
-    t->sorted_valid = true;
-    t->sorted_mp = false;
-    t->sorted_B = B;
-    t->sorted_P = P;
-    return DLRMB_OK;
+    return run_uniform(t, idx, idx_bytes, B, P, slot0, true, [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int gslot0) {
+        return launch_lookup_sort_mp(v, gidx, idx_bytes, idx_base, g, out, slots, gslot0, (cudaStream_t)stream);
+    });
 }
 
 static int check_interaction_args(int B, int F, int d, int pad_to_mul) {
@@ -453,13 +451,9 @@ int32_t dlrmb_embedding_sort(dlrmb_tables* t, const void* idx, int32_t idx_bytes
     int rc = check_idx_args(t, idx, idx_bytes, idx_base, B, P);
     if (rc) return rc;
     t->sorted_valid = false;
-    rc = launch_sort(t, idx, idx_bytes, idx_base, B, P, (cudaStream_t)stream);
-    if (rc) return rc;
-    t->sorted_valid = true;
-    t->sorted_mp = false;
-    t->sorted_B = B;
-    t->sorted_P = P;
-    return DLRMB_OK;
+    return run_uniform(t, idx, idx_bytes, B, P, 0, true, [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int) {
+        return launch_sort_mp(v, gidx, idx_bytes, idx_base, g, 0, sort_mp_final_half(v, g), (cudaStream_t)stream);
+    });
 }
 
 int32_t dlrmb_embedding_update_sorted(dlrmb_tables* t, const float* dT, int32_t slots,
@@ -566,7 +560,9 @@ int32_t dlrmb_embedding_fwd_host(dlrmb_tables* t, const void* idx, int32_t idx_b
     if ((rc = grow((void**)&t->stage_a, &t->stage_a_bytes, obytes))) return rc;
     if (slot0 > 0)  // reserved slots are the caller's (x); keep whatever the host buffer holds
         DLRMB_CUDA(cudaMemcpyAsync(t->stage_a, out, obytes, cudaMemcpyHostToDevice, t->own_stream));
-    rc = launch_lookup(t, t->stage_idx, idx_bytes, idx_base, B, P, t->stage_a, slots, slot0, t->own_stream);
+    rc = run_uniform(t, t->stage_idx, idx_bytes, B, P, slot0, false, [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int gslot0) {
+        return launch_lookup_mp(v, gidx, idx_bytes, idx_base, g, t->stage_a, slots, gslot0, t->own_stream);
+    });
     if (rc) return rc;
     DLRMB_CUDA(cudaMemcpyAsync(out, t->stage_a, obytes, cudaMemcpyDeviceToHost, t->own_stream));
     DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
@@ -642,11 +638,10 @@ int32_t dlrmb_embedding_bwd_sgd_host(dlrmb_tables* t, const void* idx, int32_t i
     if ((rc = grow((void**)&t->stage_a, &t->stage_a_bytes, gb))) return rc;
     DLRMB_CUDA(cudaMemcpyAsync(t->stage_a, dT, gb, cudaMemcpyHostToDevice, t->own_stream));
     t->sorted_valid = false;
-    if ((rc = launch_sort(t, t->stage_idx, idx_bytes, idx_base, B, P, t->own_stream))) return rc;
-    t->sorted_valid = true;
-    t->sorted_mp = false;
-    t->sorted_B = B;
-    t->sorted_P = P;
+    rc = run_uniform(t, t->stage_idx, idx_bytes, B, P, 0, true, [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int) {
+        return launch_sort_mp(v, gidx, idx_bytes, idx_base, g, 0, sort_mp_final_half(v, g), t->own_stream);
+    });
+    if (rc) return rc;
     if ((rc = launch_update(t, t->stage_a, slots, slot0, lr, t->own_stream))) return rc;
     DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
     return DLRMB_OK;
@@ -685,12 +680,24 @@ int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx
 
 static int64_t mp_index_count(const MpGeom& g) { return (int64_t)g.off[g.ntab - 1] + (int64_t)g.B * g.P[g.ntab - 1]; }
 
-void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g) {
-    t->sorted_valid = true;
-    t->sorted_mp = true;
+void mark_sorted(dlrmb_tables* t, const MpGeom& g, int k0) {
     t->sorted_B = (int)g.B;
-    t->sorted_P = 0;
-    for (int k = 0; k < g.ntab; ++k) t->h_sorted_P[k] = (int32_t)g.P[k];
+    for (int k = 0; k < g.ntab; ++k) t->h_sorted_P[k0 + k] = (int32_t)g.P[k];
+    t->sorted_valid = k0 + g.ntab == t->ntab;
+}
+
+dlrmb_tables table_group(const dlrmb_tables& t, int k0, int n) {
+    dlrmb_tables v = t;
+    v.ntab = n;
+    v.d_desc += k0;
+    if (v.d_slotmap) v.d_slotmap += k0;
+    for (int i = 0; i < 2; ++i) {
+        v.keys[i] += (size_t)k0 * t.cap;
+        v.pos[i] += (size_t)k0 * t.cap;
+    }
+    v.tile_hist += (size_t)k0 * 512 * t.radix_tiles_cap;
+    v.digit_total += (size_t)k0 * 512;
+    return v;
 }
 
 }  // namespace dlrmb
@@ -723,7 +730,7 @@ int32_t dlrmb_embedding_fwd_sort_mp(dlrmb_tables* t, const void* idx, int32_t id
     t->sorted_valid = false;
     rc = launch_lookup_sort_mp(t, idx, idx_bytes, idx_base, g, out, slots, slot0, (cudaStream_t)stream);
     if (rc) return rc;
-    mark_sorted_mp(t, g);
+    mark_sorted(t, g, 0);
     return DLRMB_OK;
 }
 
@@ -736,7 +743,7 @@ int32_t dlrmb_embedding_sort_mp(dlrmb_tables* t, const void* idx, int32_t idx_by
     t->sorted_valid = false;
     rc = launch_sort_mp(t, idx, idx_bytes, idx_base, g, 0, sort_mp_final_half(t, g), (cudaStream_t)stream);
     if (rc) return rc;
-    mark_sorted_mp(t, g);
+    mark_sorted(t, g, 0);
     return DLRMB_OK;
 }
 
@@ -815,7 +822,7 @@ int32_t dlrmb_embedding_bwd_sgd_mp_host(dlrmb_tables* t, const void* idx, int32_
     t->sorted_valid = false;
     if ((rc = launch_sort_mp(t, t->stage_idx, idx_bytes, idx_base, g, 0, sort_mp_final_half(t, g), t->own_stream)))
         return rc;
-    mark_sorted_mp(t, g);
+    mark_sorted(t, g, 0);
     if ((rc = launch_update(t, t->stage_a, slots, slot0, lr, t->own_stream))) return rc;
     DLRMB_CUDA(cudaStreamSynchronize(t->own_stream));
     return DLRMB_OK;

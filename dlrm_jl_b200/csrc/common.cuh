@@ -216,9 +216,8 @@ struct dlrmb_tables {
 
     // state of the last sort
     bool sorted_valid = false;
-    int sorted_B = 0, sorted_P = 0;
-    bool sorted_mp = false;                   // the last sort was a `_mp` one: h_sorted_P holds P_k
-    int32_t* h_sorted_P = nullptr;            // [ntab], host
+    int sorted_B = 0;
+    int32_t* h_sorted_P = nullptr;            // [ntab], host: P_k of every table
 
     // host-entry-point staging (device side), grown on demand
     void* stage_idx = nullptr;  size_t stage_idx_bytes = 0;
@@ -231,8 +230,6 @@ struct dlrmb_tables {
 namespace dlrmb {
 
 // kernels' host-side launchers (each returns a dlrmb_status)
-int launch_lookup(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                  float* out, int slots, int slot0, cudaStream_t s);
 int launch_interaction_fwd(float* T, const float* x, int B, int F, int d, int pad_to_mul,
                            float* out, int sm_count, cudaStream_t s);
 int launch_interaction_bwd(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
@@ -243,10 +240,6 @@ int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, i
 int launch_interaction_bwd_dx(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul, float* dx,
                               int sm_count, cudaStream_t s);
 bool interaction_has_warp_path(int F, int d);
-int launch_sort(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                cudaStream_t s);
-int launch_lookup_sort(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                       float* out, int slots, int slot0, cudaStream_t s);
 int launch_update(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s);
 int launch_dedup_export(dlrmb_tables* t, int k, cudaStream_t s);
 int launch_init_uniform(dlrmb_tables* t, uint64_t seed, cudaStream_t s);
@@ -260,7 +253,7 @@ int launch_dense_fwd_bias_act(float* z, const float* bias, int B, int N, int rel
 int64_t dense_bwd_scratch_floats(int N);
 int launch_dense_bwd_act_bias(const float* dy, const float* y, int B, int N, float* dz, float* db,
                               float* scratch, cudaStream_t s);
-// `_mp` forms: `g` carries ntab, B, P and off filled in; the launchers fill the rest of their copy
+// lookup / sort launchers: `g` carries ntab, B, P and off filled in; the launchers fill the rest of their copy
 int launch_lookup_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
                      float* out, int slots, int slot0, cudaStream_t s);
 int launch_lookup_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
@@ -275,13 +268,41 @@ int launch_check_indices_mp(dlrmb_tables* t, const void* d_idx, int idx_bytes, i
 // argument checks of the `_mp` entry points at batch B; fills ntab, B, P and off of `g`
 int check_mp_args(const dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, const int32_t* P,
                   MpGeom* g);
-// record that the last sort was an `_mp` one of geometry g (dlrmb_embedding_update_sorted reads it)
-void mark_sorted_mp(dlrmb_tables* t, const MpGeom& g);
+// record tables [k0, k0 + g.ntab) of the sort that just ran (dlrmb_embedding_update_sorted and the dedup export
+// read it); the sort is valid once its last table is recorded
+void mark_sorted(dlrmb_tables* t, const MpGeom& g, int k0);
+// tables [k0, k0 + n) of `t` as a handle of their own: the same tables and workspaces from table k0 on.
+// max_rows stays the handle's, so the radix sort of every group ends in the same ping-pong half.
+dlrmb_tables table_group(const dlrmb_tables& t, int k0, int n);
 // gather CTAs per table of an `_mp` lookup (fills g.pre); returns the total
 int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift);
 // lookups of table k in the last sort
-static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) {
-    return (int64_t)t->sorted_B * (t->sorted_mp ? t->h_sorted_P[k] : t->sorted_P);
+static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) { return (int64_t)t->sorted_B * t->h_sorted_P[k]; }
+
+// A batch with one pooling factor P for every table, through the launchers above (MpGeom holds kMpMaxTables
+// tables): launch(v, idx, g, slot0) runs once per group of at most kMpMaxTables consecutive tables, where v is
+// table_group of the group, idx and slot0 are moved to its first table and g has P_k = P.  With `sorts` the
+// launches sort the indices, and the batch is recorded as the last sort.
+template <typename Launch>
+int run_uniform(dlrmb_tables* t, const void* idx, int idx_bytes, int B, int P, int slot0, bool sorts, Launch&& launch) {
+    MpGeom g;
+    g.B = (uint32_t)B;
+    g.nlist = 0;
+    for (int k = 0; k < kMpMaxTables; ++k) {
+        g.P[k] = (uint32_t)P;
+        g.off[k] = (int64_t)k * B * P;
+    }
+    for (int k0 = 0; k0 < t->ntab; k0 += kMpMaxTables) {
+        g.ntab = t->ntab - k0 < kMpMaxTables ? t->ntab - k0 : kMpMaxTables;
+        dlrmb_tables v = table_group(*t, k0, g.ntab);
+        int rc = launch(&v, static_cast<const char*>(idx) + (size_t)k0 * B * P * idx_bytes, g, slot0 + k0);
+        if (rc) return rc;
+        if (sorts) {
+            t->sorted_buf = v.sorted_buf;
+            mark_sorted(t, g, k0);
+        }
+    }
+    return DLRMB_OK;
 }
 int device_sm_count(int device);
 int64_t update_tiles_cap(int ntab, int D, int64_t max_lookups, int sm_count);

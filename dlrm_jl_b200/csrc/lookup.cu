@@ -4,9 +4,11 @@
 // semantics pinned by test/model/model.jl:265-271 and the `concatenated_result` golden).
 //
 // HBM-bound: per (table, sample) one D*4-byte row read per pooled index and one D*4-byte
-// write.  Mapping: grid.y = table, and inside a table one thread per 16-byte chunk of an
-// output row (chunk index fastest), so a row is read and written by D/4 consecutive lanes as
-// whole 128-byte lines; the index of a row is fetched once per lane group through L1.
+// write.  Mapping: one flat grid in which every table owns a range of CTAs, and inside a table
+// one thread per 16-byte chunk of an output row (chunk index fastest), so a row is read and
+// written by D/4 consecutive lanes as whole 128-byte lines; the index of a row is fetched once
+// per lane group through L1.  Every table has its own pooling factor P_k; a uniform batch is
+// the case of equal P_k.
 // Memory-level parallelism comes from U independent (index -> row) chains per thread when
 // P == 1 and from a 4-deep unrolled pooling loop when P > 1.  The pooled sum runs in ascending
 // p, so results are bit-identical to the CPU restatement.
@@ -118,176 +120,10 @@ __device__ __forceinline__ void lookup_pool_body(const TableDesc* __restrict__ d
     }
 }
 
-template <typename IdxT, int VEC, int U, typename RowT>
-__global__ void __launch_bounds__(256)
-lookup_gather_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
-                     uint32_t B, uint32_t C, int cshift, float* __restrict__ out, int slots, int slot0,
-                     unsigned long long* clk) {
-    const unsigned lin = blockIdx.y * gridDim.x + blockIdx.x;
-    clock_in(clk, lin);
-    lookup_gather_body<IdxT, VEC, U, RowT>(desc, idx, idx_base, B, C, cshift, out, slots, slot0, blockIdx.y,
-                                           blockIdx.x, gridDim.x);
-    clock_out(clk, lin);
-}
-
-template <typename IdxT, int VEC, typename RowT>
-__global__ void __launch_bounds__(256)
-lookup_pool_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
-                   uint32_t B, uint32_t P, uint32_t C, int cshift, float* __restrict__ out, int slots, int slot0,
-                   unsigned long long* clk) {
-    const unsigned lin = blockIdx.y * gridDim.x + blockIdx.x;
-    clock_in(clk, lin);
-    lookup_pool_body<IdxT, VEC, RowT>(desc, idx, idx_base, B, P, C, cshift, out, slots, slot0, blockIdx.y,
-                                      blockIdx.x, gridDim.x);
-    clock_out(clk, lin);
-}
-
-// Training-step form: the lookup and the index sort / dedup of the NEXT sparse update in one launch.
-// The sort needs the indices only, and one CTA per table sorts that table's B*P keys in shared
-// memory (sort_small.cuh) in less time than the gather takes, so the first `ntab` CTAs of the grid
-// are sort CTAs and the rest gather: the sort costs no launch of its own and no time on the stream.
-// (Measured and not kept: the gather CTAs as ONE persistent wave over all tables, every thread walking its CTA's
-// share 5 rows at a time with the next round's indices prefetched -- 10.6 vs 12.3 us with L2 flushed before the
-// launch, but 10.2 vs 9.6 us back to back and no change in the training step, profiles/r02_lookup_flat.txt.)
-template <typename IdxT, int U, typename RowT, int ITEMS, bool POOL>
-__global__ void __launch_bounds__(256, 5)
-lookup_sort_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base, uint32_t B,
-                   uint32_t P, uint32_t C, int cshift, float* __restrict__ out, int slots, int slot0, int ntab,
-                   uint32_t bx, uint32_t* __restrict__ keys_out, uint32_t* __restrict__ pos_out, int64_t cap,
-                   unsigned long long* clk) {
-    extern __shared__ uint32_t sort_smem[];
-    clock_in(clk, blockIdx.x);
-    if ((int)blockIdx.x < ntab) {
-        const int k = blockIdx.x;
-        const int L = (int)(B * P);
-        sort_small_body<IdxT, ITEMS, 256>(idx + (size_t)k * L, idx_base, L, desc[k].rows,
-                                          keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, sort_smem);
-        clock_out(clk, blockIdx.x);
-        return;
-    }
-    const uint32_t lin = blockIdx.x - ntab;
-    const int k = (int)(lin / bx);
-    const uint32_t cx = lin - (uint32_t)k * bx;
-    if (POOL) lookup_pool_body<IdxT, 4, RowT>(desc, idx, idx_base, B, P, C, cshift, out, slots, slot0, k, cx, bx);
-    else lookup_gather_body<IdxT, 4, U, RowT>(desc, idx, idx_base, B, C, cshift, out, slots, slot0, k, cx, bx);
-    clock_out(clk, blockIdx.x);
-}
-
-static void lookup_grid(const dlrmb_tables* t, int64_t n, int P, int64_t* bx, int* cshift, uint32_t C) {
-    constexpr int U = 4;
-    const int per_block = 256 * (P == 1 ? U : 1);
-    int64_t b = ceil_div64(n, per_block);
-    const int64_t cap = (int64_t)t->sm_count * 32;
-    if (b * t->ntab > cap) b = cap / t->ntab > 0 ? cap / t->ntab : 1;
-    *bx = b;
-    *cshift = -1;
-    if ((C & (C - 1)) == 0) {
-        int sh = 0;
-        while ((1u << sh) < C) ++sh;
-        *cshift = sh;
-    }
-}
-
-template <typename IdxT, int VEC, typename RowT>
-static int launch_lookup_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int B, int P, float* out,
-                           int slots, int slot0, cudaStream_t s) {
-    const uint32_t C = t->D / VEC;
-    const int64_t n = (int64_t)B * C;
-    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
-    constexpr int U = 4;
-    int64_t bx;
-    int cshift;
-    lookup_grid(t, n, P, &bx, &cshift, C);
-    dim3 grid((unsigned)bx, (unsigned)t->ntab);
-    if (P == 1)
-        lookup_gather_kernel<IdxT, VEC, U, RowT><<<grid, 256, 0, s>>>(t->d_desc, idx, idx_base, B, C, cshift, out, slots, slot0, clock_slot(CLK_LOOKUP));
-    else
-        lookup_pool_kernel<IdxT, VEC, RowT><<<grid, 256, 0, s>>>(t->d_desc, idx, idx_base, B, P, C, cshift, out, slots, slot0, clock_slot(CLK_LOOKUP));
-    DLRMB_LAUNCH_CHECK();
-    return DLRMB_OK;
-}
-
-template <typename RowT>
-static int launch_lookup_r(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                           float* out, int slots, int slot0, cudaStream_t s) {
-    const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
-    if (idx_bytes == 4) {
-        const uint32_t* p = static_cast<const uint32_t*>(idx);
-        return vec4 ? launch_lookup_t<uint32_t, 4, RowT>(t, p, idx_base, B, P, out, slots, slot0, s)
-                    : launch_lookup_t<uint32_t, 1, RowT>(t, p, idx_base, B, P, out, slots, slot0, s);
-    }
-    const int64_t* p = static_cast<const int64_t*>(idx);
-    return vec4 ? launch_lookup_t<int64_t, 4, RowT>(t, p, idx_base, B, P, out, slots, slot0, s)
-                : launch_lookup_t<int64_t, 1, RowT>(t, p, idx_base, B, P, out, slots, slot0, s);
-}
-
-int launch_lookup(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                  float* out, int slots, int slot0, cudaStream_t s) {
-    if (t->elem_bytes == 2)
-        return launch_lookup_r<__nv_bfloat16>(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, s);
-    return launch_lookup_r<float>(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, s);
-}
-
-template <typename IdxT, typename RowT, int ITEMS, bool POOL>
-static int launch_lookup_sort_i(dlrmb_tables* t, const IdxT* idx, int idx_base, int B, int P, float* out,
-                                int slots, int slot0, cudaStream_t s) {
-    const uint32_t C = t->D / 4;
-    const int64_t n = (int64_t)B * C;
-    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
-    constexpr int U = 4;
-    int64_t bx;
-    int cshift;
-    lookup_grid(t, n, P, &bx, &cshift, C);
-    constexpr size_t smem = SmallSortGeom<ITEMS, 256>::smem_bytes();
-    static unsigned long long attr_done = 0;
-    int rc = ensure_smem_attr((const void*)lookup_sort_kernel<IdxT, U, RowT, ITEMS, POOL>, (int)smem, &attr_done);
-    if (rc) return rc;
-    const unsigned grid = (unsigned)(t->ntab + bx * t->ntab);
-    lookup_sort_kernel<IdxT, U, RowT, ITEMS, POOL><<<grid, 256, smem, s>>>(
-        t->d_desc, idx, idx_base, B, P, C, cshift, out, slots, slot0, t->ntab, (uint32_t)bx, t->keys[0], t->pos[0], t->cap,
-        clock_slot(CLK_LOOKUP));
-    DLRMB_LAUNCH_CHECK();
-    t->sorted_buf = 0;
-    return DLRMB_OK;
-}
-
-template <typename IdxT, typename RowT>
-static int launch_lookup_sort_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int B, int P, float* out,
-                                int slots, int slot0, cudaStream_t s) {
-    const int64_t L = (int64_t)B * P;
-    if (L <= 2048)
-        return P == 1 ? launch_lookup_sort_i<IdxT, RowT, 8, false>(t, idx, idx_base, B, P, out, slots, slot0, s)
-                      : launch_lookup_sort_i<IdxT, RowT, 8, true>(t, idx, idx_base, B, P, out, slots, slot0, s);
-    return P == 1 ? launch_lookup_sort_i<IdxT, RowT, 16, false>(t, idx, idx_base, B, P, out, slots, slot0, s)
-                  : launch_lookup_sort_i<IdxT, RowT, 16, true>(t, idx, idx_base, B, P, out, slots, slot0, s);
-}
-
-// lookup + sort for the next update: fused into one launch when the sort fits the 256-thread
-// shared-memory path and the rows are 16-byte vectorisable; two launches otherwise.
-int launch_lookup_sort(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                       float* out, int slots, int slot0, cudaStream_t s) {
-    const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
-    if (!vec4 || (int64_t)B * P > kFusedSortMax) {
-        int rc = launch_lookup(t, idx, idx_bytes, idx_base, B, P, out, slots, slot0, s);
-        if (rc) return rc;
-        return launch_sort(t, idx, idx_bytes, idx_base, B, P, s);
-    }
-    const bool bf = t->elem_bytes == 2;
-    if (idx_bytes == 4) {
-        const uint32_t* p = static_cast<const uint32_t*>(idx);
-        return bf ? launch_lookup_sort_t<uint32_t, __nv_bfloat16>(t, p, idx_base, B, P, out, slots, slot0, s)
-                  : launch_lookup_sort_t<uint32_t, float>(t, p, idx_base, B, P, out, slots, slot0, s);
-    }
-    const int64_t* p = static_cast<const int64_t*>(idx);
-    return bf ? launch_lookup_sort_t<int64_t, __nv_bfloat16>(t, p, idx_base, B, P, out, slots, slot0, s)
-              : launch_lookup_sort_t<int64_t, float>(t, p, idx_base, B, P, out, slots, slot0, s);
-}
-
-// ---- per-table pooling factors -----------------------------------------------------------------
 // One flat grid of gather CTAs; table k owns CTAs [g.pre[k], g.pre[k+1]), handed out in proportion to its
 // work B * P_k * C (lookup_grid_mp), so a hotness-100 table does not form the tail behind one-hot tables
-// holding the same number of CTAs.  The bodies are the uniform path's, pointed at table k (desc + k, its
-// index block, its output slot): P_k == 1 takes the U-chain gather, every other table the pooling loop.
+// holding the same number of CTAs.  The bodies above are pointed at table k (desc + k, its index block, its
+// output slot): P_k == 1 takes the U-chain gather, every other table the pooling loop.
 template <typename IdxT, int VEC, int U, typename RowT>
 __device__ __forceinline__ void lookup_mp_cta(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx,
                                               int idx_base, const MpGeom& g, uint32_t C, int cshift,
@@ -311,8 +147,13 @@ lookup_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ id
     clock_out(clk, blockIdx.x);
 }
 
-// Training-step form: the first g.nlist CTAs sort the tables g.list[] (L_k <= kFusedSortMax) in shared
-// memory, as lookup_sort_kernel does for a uniform batch; the rest gather.
+// Training-step form: the lookup and the index sort / dedup of the NEXT sparse update in one launch.
+// The sort needs the indices only, and one CTA per table sorts that table's B*P_k keys in shared memory
+// (sort_small.cuh) in less time than the gather takes, so the first g.nlist CTAs sort the tables g.list[]
+// (L_k <= kFusedSortMax) and the rest gather: the sort costs no launch of its own and no time on the stream.
+// (Measured and not kept: the gather CTAs as ONE persistent wave over all tables, every thread walking its CTA's
+// share 5 rows at a time with the next round's indices prefetched -- 10.6 vs 12.3 us with L2 flushed before the
+// launch, but 10.2 vs 9.6 us back to back and no change in the training step, profiles/r02_lookup_flat.txt.)
 template <typename IdxT, int U, typename RowT, int ITEMS>
 __global__ void __launch_bounds__(256, 5)
 lookup_sort_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ idx, int idx_base,
@@ -332,7 +173,7 @@ lookup_sort_mp_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict
     clock_out(clk, blockIdx.x);
 }
 
-// Gather CTAs per table: the uniform path's launch budget (32 CTAs per SM) split in proportion to B * P_k * C,
+// Gather CTAs per table: a launch budget of 32 CTAs per SM split in proportion to B * P_k * C,
 // at least one per table and no more than the table has work items for.  Returns the total.
 int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift) {
     constexpr int U = 4;
@@ -363,7 +204,8 @@ template <typename IdxT, int VEC, typename RowT>
 static int launch_lookup_mp_t(dlrmb_tables* t, const IdxT* idx, int idx_base, const MpGeom& g0, float* out,
                               int slots, int slot0, cudaStream_t s) {
     const uint32_t C = t->D / VEC;
-    DLRMB_REQUIRE((int64_t)g0.B * C < (1ll << 30), "B * D too large for one lookup launch");
+    const int64_t n = (int64_t)g0.B * C;
+    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
     MpGeom g = g0;
     g.nlist = 0;
     int cshift;
@@ -418,7 +260,8 @@ static int launch_lookup_sort_mp_i(dlrmb_tables* t, const IdxT* idx, int idx_bas
 // L_k <= kSmemSortMax, radix passes above); every table's sorted stream ends in the same ping-pong half.
 int launch_lookup_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
                           float* out, int slots, int slot0, cudaStream_t s) {
-    DLRMB_REQUIRE((int64_t)g.B * (t->D / 4) < (1ll << 30), "B * D too large for one lookup launch");
+    const int64_t n = (int64_t)g.B * (t->D / 4);
+    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
     const int half = sort_mp_final_half(t, g);
     const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
     MpGeom gs = g;

@@ -22,8 +22,6 @@ struct PeerPtrs {
     float* p[kMaxPeers];
 };
 
-// Same mapping as lookup_gather_kernel (one thread per 16-byte chunk, 4 independent index -> row
-// chains), but sample b lives on rank b / B_local and table k lands in slot slotmap[k].
 template <int VEC, typename RowT>
 __device__ __forceinline__ typename std::conditional<VEC == 4, float4, float>::type
 p2p_ldrow(const float* base, size_t r, size_t D, int c) {
@@ -31,155 +29,14 @@ p2p_ldrow(const float* base, size_t r, size_t D, int c) {
     else return RowIO<RowT>::ldg1(RowIO<RowT>::row(base, r, D), c);
 }
 
-// SORT_ITEMS > 0: the first `ntab` CTAs of the (then one-dimensional) grid sort the tables' index lists for
-// the coming sparse update in shared memory (sort_small.cuh), as in lookup_sort_kernel of lookup.cu.
-template <typename IdxT, int VEC, int U, typename RowT, int SORT_ITEMS>
-__global__ void __launch_bounds__(256, (SORT_ITEMS > 0) ? 4 : 1)
-lookup_p2p_kernel(const TableDesc* __restrict__ desc, const int32_t* __restrict__ slotmap,
-                  const IdxT* __restrict__ idx, int idx_base, uint32_t Bg, uint32_t B_local, uint32_t P,
-                  uint32_t C, PeerPtrs peers, int slots, int ntab, uint32_t bx, uint32_t* __restrict__ keys_out,
-                  uint32_t* __restrict__ pos_out, int64_t cap, unsigned long long* clk) {
-    using V = typename std::conditional<VEC == 4, float4, float>::type;
-    int k;
-    uint32_t cx, nctas;
-    const unsigned clk_cta = blockIdx.y * gridDim.x + blockIdx.x;
-    clock_in(clk, clk_cta);
-    if constexpr (SORT_ITEMS > 0) {
-        extern __shared__ uint32_t sort_smem[];
-        if ((int)blockIdx.x < ntab) {
-            k = blockIdx.x;
-            const int L = (int)(Bg * P);
-            sort_small_body<IdxT, (SORT_ITEMS > 0 ? SORT_ITEMS : 4), 256>(idx + (size_t)k * L, idx_base, L, desc[k].rows,
-                                                                          keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, sort_smem);
-            clock_out(clk, clk_cta);
-            return;
-        }
-        const uint32_t lin = blockIdx.x - ntab;
-        k = (int)(lin / bx);
-        cx = lin - (uint32_t)k * bx;
-        nctas = bx;
-    } else {
-        k = blockIdx.y;
-        cx = blockIdx.x;
-        nctas = gridDim.x;
-    }
-    const float* __restrict__ tb = desc[k].base;
-    const IdxT* __restrict__ ik = idx + (size_t)k * Bg * P;
-    const uint32_t n = Bg * C;
-    const uint32_t step = nctas * blockDim.x;
-    const size_t D = (size_t)C * VEC;
-    const size_t slot_off = (size_t)slotmap[k] * D;
-    const size_t ostride = (size_t)slots * D;
-
-    for (uint32_t t = cx * blockDim.x + threadIdx.x; t < n; t += step * U) {
-        uint32_t b[U], c[U];
-        bool ok[U];
-        V acc[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const uint32_t tt = t + (uint32_t)u * step;
-            ok[u] = tt < n;
-            b[u] = tt / C;
-            c[u] = tt - b[u] * C;
-        }
-        if (P == 1) {
-            int64_t row[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) row[u] = ok[u] ? (int64_t)__ldg(ik + b[u]) - idx_base : 0;
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (ok[u]) acc[u] = p2p_ldrow<VEC, RowT>(tb, (size_t)row[u], D, c[u]);
-        } else {
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                if (!ok[u]) continue;
-                const IdxT* ip = ik + (size_t)b[u] * P;
-                V a = p2p_ldrow<VEC, RowT>(tb, (size_t)((int64_t)__ldg(ip) - idx_base), D, c[u]);
-                for (uint32_t p = 1; p < P; ++p) {
-                    V v = p2p_ldrow<VEC, RowT>(tb, (size_t)((int64_t)__ldg(ip + p) - idx_base), D, c[u]);
-                    if constexpr (VEC == 4) {
-                        a = make_float4(__fadd_rn(a.x, v.x), __fadd_rn(a.y, v.y), __fadd_rn(a.z, v.z), __fadd_rn(a.w, v.w));
-                    } else {
-                        a = __fadd_rn(a, v);
-                    }
-                }
-                acc[u] = a;
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            if (!ok[u]) continue;
-            const uint32_t h = b[u] / B_local;
-            const uint32_t bl = b[u] - h * B_local;
-            float* dst = peers.p[h] + (size_t)bl * ostride + slot_off;
-            reinterpret_cast<V*>(dst)[c[u]] = acc[u];
-        }
-    }
-    clock_out(clk, clk_cta);
-}
-
 int ensure_smem_attr(const void* func, int bytes, unsigned long long* done_mask);
 
-template <typename IdxT, int VEC, typename RowT>
-static int launch_p2p_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int Bg, int P, const PeerPtrs& peers,
-                        int B_local, int slots, bool with_sort, cudaStream_t s) {
-    const uint32_t C = t->D / VEC;
-    const int64_t n = (int64_t)Bg * C;
-    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
-    constexpr int U = 4;
-    int64_t bx = ceil_div64(n, 256 * U);
-    const int64_t cap = (int64_t)t->sm_count * 32;
-    if (bx * t->ntab > cap) bx = cap / t->ntab > 0 ? cap / t->ntab : 1;
-    const int64_t L = (int64_t)Bg * P;
-    if constexpr (VEC == 4) {
-        if (with_sort && L <= kFusedSortMax) {   // the sort of the coming update rides in the same launch
-            const unsigned grid1 = (unsigned)(t->ntab + bx * t->ntab);
-            if (L <= 2048) {
-                constexpr size_t smem = SmallSortGeom<8, 256>::smem_bytes();
-                static unsigned long long done = 0;
-                int rc = ensure_smem_attr((const void*)lookup_p2p_kernel<IdxT, 4, U, RowT, 8>, (int)smem, &done);
-                if (rc) return rc;
-                lookup_p2p_kernel<IdxT, 4, U, RowT, 8><<<grid1, 256, smem, s>>>(t->d_desc, t->d_slotmap, idx, idx_base, Bg, B_local, P, C,
-                                                                             peers, slots, t->ntab, (uint32_t)bx, t->keys[0], t->pos[0], t->cap, clock_slot(CLK_LOOKUP));
-            } else {
-                constexpr size_t smem = SmallSortGeom<16, 256>::smem_bytes();
-                static unsigned long long done = 0;
-                int rc = ensure_smem_attr((const void*)lookup_p2p_kernel<IdxT, 4, U, RowT, 16>, (int)smem, &done);
-                if (rc) return rc;
-                lookup_p2p_kernel<IdxT, 4, U, RowT, 16><<<grid1, 256, smem, s>>>(t->d_desc, t->d_slotmap, idx, idx_base, Bg, B_local, P, C,
-                                                                              peers, slots, t->ntab, (uint32_t)bx, t->keys[0], t->pos[0], t->cap, clock_slot(CLK_LOOKUP));
-            }
-            DLRMB_LAUNCH_CHECK();
-            t->sorted_buf = 0;
-            t->sorted_valid = true;
-            t->sorted_mp = false;
-            t->sorted_B = Bg;
-            t->sorted_P = P;
-            return DLRMB_OK;
-        }
-    }
-    dim3 grid((unsigned)bx, (unsigned)t->ntab);
-    lookup_p2p_kernel<IdxT, VEC, U, RowT, 0><<<grid, 256, 0, s>>>(t->d_desc, t->d_slotmap, idx, idx_base, Bg, B_local, P, C,
-                                                            peers, slots, t->ntab, (uint32_t)bx, nullptr, nullptr, 0, clock_slot(CLK_LOOKUP));
-    DLRMB_LAUNCH_CHECK();
-    if (with_sort) {   // too many keys for the 256-thread sort CTAs: the stand-alone sort, same stream
-        int rc = launch_sort(t, idx, (int)sizeof(IdxT), idx_base, Bg, P, s);
-        if (rc) return rc;
-        t->sorted_valid = true;
-        t->sorted_mp = false;
-        t->sorted_B = Bg;
-        t->sorted_P = P;
-    }
-    return DLRMB_OK;
-}
-
-// ---- per-table pooling factors ------------------------------------------------------------------
-// The `_mp` lookup's geometry (one flat grid, table k owns CTAs [g.pre[k], g.pre[k+1]) in proportion to
-// B_global * P_k * C, lookup_grid_mp of lookup.cu) with the peer-store epilogue above: P_k == 1 takes the
-// U-chain gather, every other table the 4-deep pooling loop in ascending p (the `_mp` lookup's order, so
-// the pooled rows are bit-identical to dlrmb_embedding_fwd_mp).  With SORT_ITEMS > 0 the first g.nlist
-// CTAs sort the tables g.list[] (B_global * P_k <= kFusedSortMax) in shared memory, as
-// lookup_sort_mp_kernel does.  Both parameter structs go by value (__grid_constant__: peers.p[h] is read
+// The lookup's geometry (one flat grid, table k owns CTAs [g.pre[k], g.pre[k+1]) in proportion to
+// B_global * P_k * C, lookup_grid_mp of lookup.cu) with a peer-store epilogue: sample b lives on rank
+// b / B_local and table k lands in slot slotmap[k].  P_k == 1 takes the U-chain gather, every other table
+// the 4-deep pooling loop in ascending p (the lookup's order, so the pooled rows are bit-identical to
+// dlrmb_embedding_fwd).  With SORT_ITEMS > 0 the first g.nlist CTAs sort the tables g.list[]
+// (B_global * P_k <= kFusedSortMax) in shared memory, as lookup_sort_mp_kernel does.  Both parameter structs go by value (__grid_constant__: peers.p[h] is read
 // with a run-time h straight from the parameter bank), so the launch needs no device copy.
 __device__ __forceinline__ float4 p2p_add(float4 a, float4 b) {
     return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
@@ -289,7 +146,8 @@ static int launch_p2p_mp_t(dlrmb_tables* t, const IdxT* idx, int idx_base, const
                            int B_local, int slots, int half, cudaStream_t s) {
     constexpr int U = 4;
     const uint32_t C = t->D / VEC;
-    DLRMB_REQUIRE((int64_t)g0.B * C < (1ll << 30), "B * D too large for one lookup launch");
+    const int64_t n = (int64_t)g0.B * C;
+    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
     MpGeom g = g0;
     int cshift;
     const int64_t ctas = lookup_grid_mp(t, g, C, &cshift) + (SORT_ITEMS > 0 ? g.nlist : 0);
@@ -422,6 +280,32 @@ int32_t dlrmb_tables_set_slot_map(dlrmb_tables* t, const int32_t* slots) {
     return DLRMB_OK;
 }
 
+// the peer pointers of `world` ranks; vec4: D % 4 == 0 and every pointer 16-byte aligned
+static int peer_ptrs(const dlrmb_tables* t, float* const* peer_T, int world, PeerPtrs* peers, bool* vec4) {
+    *vec4 = (t->D % 4 == 0);
+    for (int r = 0; r < kMaxPeers; ++r) {
+        peers->p[r] = r < world ? peer_T[r] : nullptr;
+        if (r < world) {
+            DLRMB_REQUIRE(peer_T[r] != nullptr, "peer_T[%d] is null", r);
+            *vec4 = *vec4 && ((reinterpret_cast<uintptr_t>(peer_T[r]) & 15) == 0);
+        }
+    }
+    return DLRMB_OK;
+}
+
+static int launch_p2p(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, const MpGeom& g,
+                      const PeerPtrs& peers, int B_local, int slots, bool vec4, bool with_sort, cudaStream_t s) {
+    const bool bf = t->elem_bytes == 2;
+    if (idx_bytes == 4) {
+        const uint32_t* ip = (const uint32_t*)idx;
+        return bf ? launch_p2p_mp_i<uint32_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
+                  : launch_p2p_mp_i<uint32_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
+    }
+    const int64_t* ip = (const int64_t*)idx;
+    return bf ? launch_p2p_mp_i<int64_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
+              : launch_p2p_mp_i<int64_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
+}
+
 static int32_t embedding_fwd_p2p_impl(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
                                       int32_t B_global, int32_t P, float* const* peer_T, int32_t world,
                                       int32_t B_local, int32_t slots, bool with_sort, dlrmb_stream stream) {
@@ -443,31 +327,14 @@ static int32_t embedding_fwd_p2p_impl(dlrmb_tables* t, const void* idx, int32_t 
     DeviceGuard guard(t->device);
     DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", t->device);
     PeerPtrs peers;
-    bool aligned = (t->D % 4 == 0);
-    for (int r = 0; r < kMaxPeers; ++r) {
-        peers.p[r] = r < world ? peer_T[r] : nullptr;
-        if (r < world) {
-            DLRMB_REQUIRE(peer_T[r] != nullptr, "peer_T[%d] is null", r);
-            aligned = aligned && ((reinterpret_cast<uintptr_t>(peer_T[r]) & 15) == 0);
-        }
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    int rc;
-    const bool bf = t->elem_bytes == 2;
-    if (idx_bytes == 4) {
-        const uint32_t* ip = (const uint32_t*)idx;
-        if (aligned) rc = bf ? launch_p2p_t<uint32_t, 4, __nv_bfloat16>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s)
-                             : launch_p2p_t<uint32_t, 4, float>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s);
-        else rc = bf ? launch_p2p_t<uint32_t, 1, __nv_bfloat16>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s)
-                     : launch_p2p_t<uint32_t, 1, float>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s);
-    } else {
-        const int64_t* ip = (const int64_t*)idx;
-        if (aligned) rc = bf ? launch_p2p_t<int64_t, 4, __nv_bfloat16>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s)
-                             : launch_p2p_t<int64_t, 4, float>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s);
-        else rc = bf ? launch_p2p_t<int64_t, 1, __nv_bfloat16>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s)
-                     : launch_p2p_t<int64_t, 1, float>(t, ip, idx_base, B_global, P, peers, B_local, slots, with_sort, s);
-    }
-    return rc;
+    bool vec4;
+    int rc = peer_ptrs(t, peer_T, world, &peers, &vec4);
+    if (rc) return rc;
+    return run_uniform(t, idx, idx_bytes, B_global, P, 0, with_sort,
+                       [&](dlrmb_tables* v, const void* gidx, const MpGeom& g, int) {
+                           return launch_p2p(v, gidx, idx_bytes, idx_base, g, peers, B_local, slots, vec4, with_sort,
+                                             (cudaStream_t)stream);
+                       });
 }
 
 int32_t dlrmb_embedding_fwd_p2p(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
@@ -502,27 +369,12 @@ static int32_t embedding_fwd_p2p_mp_impl(dlrmb_tables* t, const void* idx, int32
     DeviceGuard guard(t->device);
     DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", t->device);
     PeerPtrs peers;
-    bool vec4 = (t->D % 4 == 0);
-    for (int r = 0; r < kMaxPeers; ++r) {
-        peers.p[r] = r < world ? peer_T[r] : nullptr;
-        if (r < world) {
-            DLRMB_REQUIRE(peer_T[r] != nullptr, "peer_T[%d] is null", r);
-            vec4 = vec4 && ((reinterpret_cast<uintptr_t>(peer_T[r]) & 15) == 0);
-        }
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    const bool bf = t->elem_bytes == 2;
-    if (idx_bytes == 4) {
-        const uint32_t* ip = (const uint32_t*)idx;
-        rc = bf ? launch_p2p_mp_i<uint32_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
-                : launch_p2p_mp_i<uint32_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
-    } else {
-        const int64_t* ip = (const int64_t*)idx;
-        rc = bf ? launch_p2p_mp_i<int64_t, __nv_bfloat16>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s)
-                : launch_p2p_mp_i<int64_t, float>(t, ip, idx_base, g, peers, B_local, slots, vec4, with_sort, s);
-    }
+    bool vec4;
+    rc = peer_ptrs(t, peer_T, world, &peers, &vec4);
     if (rc) return rc;
-    if (with_sort) mark_sorted_mp(t, g);
+    rc = launch_p2p(t, idx, idx_bytes, idx_base, g, peers, B_local, slots, vec4, with_sort, (cudaStream_t)stream);
+    if (rc) return rc;
+    if (with_sort) mark_sorted(t, g, 0);
     return DLRMB_OK;
 }
 

@@ -6,13 +6,13 @@
 // table, which makes duplicates adjacent and fixes their accumulation order (ascending flat
 // position) so the update is deterministic without floating-point atomics.
 //
-// Two paths, chosen per call from L = B*P:
-//   * L <= kSmemSortMax: one CTA per table runs the whole LSD radix sort in shared memory
+// Two paths, chosen per table from L_k = B*P_k (one batch can use both):
+//   * L_k <= kSmemSortMax: one CTA per table runs the whole LSD radix sort in shared memory
 //     (digits of up to 9 bits, as many passes as that table's row count needs); a single launch
-//     covers all tables.  Training steps do not even pay that launch: dlrmb_embedding_fwd_sort runs
+//     covers all such tables.  Training steps do not even pay that launch: dlrmb_embedding_fwd_sort runs
 //     the same sort in extra CTAs of the lookup launch (lookup.cu), hidden behind the gather.
-//   * larger L: least-significant-digit radix sort, digits of up to 9 bits, tiles of 4096 keys, all tables
-//     batched through grid.y.  Per pass: per-tile digit histogram -> exclusive scan over
+//   * larger L_k: least-significant-digit radix sort, digits of up to 9 bits, tiles of 4096 keys, all such
+//     tables batched through grid.y.  Per pass: per-tile digit histogram -> exclusive scan over
 //     (digit, tile), one CTA per digit -> stable scatter whose in-tile ranks come from warp match_any + per-warp
 //     digit counters in shared memory and whose keys are reordered in shared memory first, so each
 //     digit's keys leave the CTA as one contiguous run.  The sort arrays of a whole batch fit L2 (126 MB), so the
@@ -25,36 +25,7 @@
 namespace dlrmb {
 
 // ---------------------------------------------------------------------------------------------
-// small path: LSD radix sort held in shared memory, one CTA per table, one launch for all tables
-// (body in sort_small.cuh; the fused lookup + sort launch of lookup.cu runs the same body)
-// ---------------------------------------------------------------------------------------------
-template <typename IdxT, int ITEMS, int THREADS>
-__global__ void __launch_bounds__(THREADS)
-sort_small_kernel(const IdxT* __restrict__ idx, int idx_base, int L, const TableDesc* __restrict__ desc,
-                  uint32_t* __restrict__ keys_out, uint32_t* __restrict__ pos_out, int64_t cap,
-                  unsigned long long* clk) {
-    extern __shared__ uint32_t sort_smem[];
-    const int k = blockIdx.x;
-    clock_in(clk, blockIdx.x);
-    sort_small_body<IdxT, ITEMS, THREADS>(idx + (size_t)k * L, idx_base, L, desc[k].rows,
-                                          keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, sort_smem);
-    clock_out(clk, blockIdx.x);
-}
-
-template <typename IdxT, int ITEMS, int THREADS>
-static int launch_sort_small(dlrmb_tables* t, const IdxT* idx, int idx_base, int L, cudaStream_t s) {
-    constexpr size_t smem = SmallSortGeom<ITEMS, THREADS>::smem_bytes();
-    static unsigned long long attr_done = 0;
-    int rc = ensure_smem_attr((const void*)sort_small_kernel<IdxT, ITEMS, THREADS>, (int)smem, &attr_done);
-    if (rc) return rc;
-    sort_small_kernel<IdxT, ITEMS, THREADS><<<t->ntab, THREADS, smem, s>>>(idx, idx_base, L, t->d_desc, t->keys[0],
-                                                                          t->pos[0], t->cap, clock_slot(CLK_SORT));
-    DLRMB_LAUNCH_CHECK();
-    return DLRMB_OK;
-}
-
-// ---------------------------------------------------------------------------------------------
-// large path: LSD radix sort over global memory, all tables batched through grid.y
+// large path: LSD radix sort over global memory (device bodies; the kernels are below)
 // ---------------------------------------------------------------------------------------------
 constexpr int RT = 256;        // threads per CTA
 constexpr int RI = 16;         // keys per thread
@@ -119,15 +90,6 @@ __device__ __forceinline__ void radix_hist_body(const IdxT* __restrict__ ik, int
     for (uint32_t d = tid; d <= mask; d += RT) hist[(size_t)d * tiles + tile] = h[d];
 }
 
-template <typename IdxT, bool FIRST>
-__global__ void __launch_bounds__(RT)
-radix_hist_kernel(const IdxT* __restrict__ idx, int idx_base, const uint32_t* __restrict__ keys, int64_t cap,
-                  int L, int shift, uint32_t mask, uint32_t* __restrict__ tile_hist, int tiles) {
-    const int k = blockIdx.y;
-    radix_hist_body<IdxT, FIRST>(idx + (size_t)k * L, idx_base, keys + (size_t)k * cap, L, shift, mask,
-                                 tile_hist + (size_t)k * NB * tiles, tiles, blockIdx.x);
-}
-
 // One CTA per (digit, table): exclusive scan over that digit's per-tile counts (contiguous, so
 // the loads coalesce), in place, plus the digit's total.
 __device__ __forceinline__ void radix_scan_body(uint32_t* __restrict__ h, uint32_t* __restrict__ total, int tiles) {
@@ -142,12 +104,6 @@ __device__ __forceinline__ void radix_scan_body(uint32_t* __restrict__ h, uint32
         running += tot;
     }
     if (threadIdx.x == 0) *total = running;
-}
-
-__global__ void __launch_bounds__(RT)
-radix_scan_kernel(uint32_t* __restrict__ tile_hist, uint32_t* __restrict__ digit_total, int tiles) {
-    const int d = blockIdx.x, k = blockIdx.y;
-    radix_scan_body(tile_hist + ((size_t)k * NB + d) * tiles, digit_total + k * NB + d, tiles);
 }
 
 // Scatter with a shared-memory reorder: the tile's keys are first placed in digit order in shared
@@ -248,86 +204,20 @@ __device__ __forceinline__ void radix_scatter_body(const IdxT* __restrict__ ik, 
     }
 }
 
-template <typename IdxT, bool FIRST>
-__global__ void __launch_bounds__(RT)
-radix_scatter_kernel(const IdxT* __restrict__ idx, int idx_base, const uint32_t* __restrict__ keys_in,
-                     const uint32_t* __restrict__ pos_in, uint32_t* __restrict__ keys_out,
-                     uint32_t* __restrict__ pos_out, int64_t cap, int L, int shift, uint32_t mask,
-                     const uint32_t* __restrict__ tile_hist, const uint32_t* __restrict__ digit_total, int tiles) {
-    const int k = blockIdx.y;
-    radix_scatter_body<IdxT, FIRST>(idx + (size_t)k * L, idx_base, keys_in + (size_t)k * cap, pos_in + (size_t)k * cap,
-                                    keys_out + (size_t)k * cap, pos_out + (size_t)k * cap, L, shift, mask,
-                                    tile_hist + (size_t)k * NB * tiles, digit_total + k * NB, tiles, blockIdx.x);
-}
-
 static int key_bits(int64_t max_rows) {
     int bits = 1;
     while (bits < 32 && (1ll << bits) < max_rows) ++bits;
     return bits;
 }
 
-template <typename IdxT>
-static int launch_sort_t(dlrmb_tables* t, const IdxT* idx, int idx_base, int B, int P, cudaStream_t s) {
-    const int64_t L64 = (int64_t)B * P;
-    const int L = (int)L64;
-    const int64_t cap = t->cap;
-    if (L <= kSmemSortMax) {
-        int rc;
-        if (L <= 1024) rc = launch_sort_small<IdxT, 4, 256>(t, idx, idx_base, L, s);
-        else if (L <= 2048) rc = launch_sort_small<IdxT, 8, 256>(t, idx, idx_base, L, s);
-        else if (L <= 4096) rc = launch_sort_small<IdxT, 16, 256>(t, idx, idx_base, L, s);
-        else if (L <= 8192) rc = launch_sort_small<IdxT, 8, 1024>(t, idx, idx_base, L, s);
-        else rc = launch_sort_small<IdxT, 16, 1024>(t, idx, idx_base, L, s);
-        if (rc) return rc;
-        t->sorted_buf = 0;
-        return DLRMB_OK;
-    }
-    const int tiles = (int)ceil_div64(L, RTILE);
-    DLRMB_REQUIRE(tiles <= t->radix_tiles_cap, "internal: radix tile capacity exceeded");
-    const int bits = key_bits(t->max_rows);
-    const int passes = (bits + 8) / 9;
-    const int per_pass = (bits + passes - 1) / passes;     // <= 9
-    int cur = 0;
-    dim3 grid((unsigned)tiles, (unsigned)t->ntab);
-    int shift = 0;
-    for (int p = 0; p < passes; ++p) {
-        const int nb = (bits - shift) < per_pass ? (bits - shift) : per_pass;
-        const uint32_t mask = (1u << nb) - 1u;
-        dim3 sgrid(mask + 1u, (unsigned)t->ntab);
-        if (p == 0)
-            radix_hist_kernel<IdxT, true><<<grid, RT, 0, s>>>(idx, idx_base, t->keys[cur], cap, L, shift, mask, t->tile_hist, tiles);
-        else
-            radix_hist_kernel<IdxT, false><<<grid, RT, 0, s>>>(idx, idx_base, t->keys[cur], cap, L, shift, mask, t->tile_hist, tiles);
-        DLRMB_LAUNCH_CHECK();
-        radix_scan_kernel<<<sgrid, RT, 0, s>>>(t->tile_hist, t->digit_total, tiles);
-        DLRMB_LAUNCH_CHECK();
-        if (p == 0)
-            radix_scatter_kernel<IdxT, true><<<grid, RT, 0, s>>>(idx, idx_base, t->keys[cur], t->pos[cur], t->keys[cur ^ 1],
-                                                                t->pos[cur ^ 1], cap, L, shift, mask, t->tile_hist, t->digit_total, tiles);
-        else
-            radix_scatter_kernel<IdxT, false><<<grid, RT, 0, s>>>(idx, idx_base, t->keys[cur], t->pos[cur], t->keys[cur ^ 1],
-                                                                 t->pos[cur ^ 1], cap, L, shift, mask, t->tile_hist, t->digit_total, tiles);
-        DLRMB_LAUNCH_CHECK();
-        cur ^= 1;
-        shift += nb;
-    }
-    t->sorted_buf = cur;
-    return DLRMB_OK;
-}
-
-int launch_sort(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base, int B, int P,
-                cudaStream_t s) {
-    if (idx_bytes == 4) return launch_sort_t<uint32_t>(t, static_cast<const uint32_t*>(idx), idx_base, B, P, s);
-    return launch_sort_t<int64_t>(t, static_cast<const int64_t*>(idx), idx_base, B, P, s);
-}
-
 // ---------------------------------------------------------------------------------------------
-// per-table pooling factors: every regime in one batch.  Table k has L_k = B * P_k keys at g.off[k].
-//   L_k <= kSmemSortMax: one shared-memory launch, one CTA per listed table (sized for the longest list)
+// Every regime in one batch.  Table k has L_k = B * P_k keys at g.off[k].
+//   L_k <= kSmemSortMax: one shared-memory launch, one CTA per listed table (sized for the longest list;
+//                        body in sort_small.cuh, which the fused lookup + sort launches also run)
 //   larger L_k:          the radix passes above, grid.y over the listed tables, grid.x over the largest
 //                        table's tiles (CTAs past their own table's tile count return at once)
-// The radix pass count follows the largest table of the handle, as for a uniform batch, so the radix
-// tables finish in half passes % 2; the shared-memory sorts write there directly.
+// The radix pass count follows the largest table of the handle, so the radix tables finish in half
+// passes % 2; the shared-memory sorts write there directly.
 // ---------------------------------------------------------------------------------------------
 template <typename IdxT, int ITEMS, int THREADS>
 __global__ void __launch_bounds__(THREADS)

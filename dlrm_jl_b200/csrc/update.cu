@@ -666,91 +666,81 @@ int64_t update_tiles_cap(int ntab, int D, int64_t max_lookups, int sm_count) {
     return ceil_div64(ceil_div64(max_lookups, 4), G) + 2;   // smallest tile (4) gives the most chunks
 }
 
+// Consumes the last sort (B and every table's P_k).  With equal P_k the tables share one geometry and the grid
+// is two-dimensional (grid.y = table); otherwise one flat grid of sum_k chunks_k CTAs, g.pre mapping a CTA to
+// (table, chunk).  The tile is chosen from the total entry count either way, so equal P_k take the same tiles
+// and chunks on both grids, hence the same bits.
 template <int VEC, int NCH, typename RowT>
-static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr,
-                           cudaStream_t s) {
+static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
+    constexpr int THREADS = (NCH > 4) ? 128 : 256;   // keeps the two partial arrays within 48 KB
+    const int32_t* P = t->h_sorted_P;
+    bool equal = true;
+    int64_t total = 0, maxL = 0;
+    for (int k = 0; k < t->ntab; ++k) {
+        const int64_t L = (int64_t)t->sorted_B * P[k];
+        total += L;
+        maxL = L > maxL ? L : maxL;
+        equal = equal && P[k] == P[0];
+    }
     UpdateGeom gm;
-    gm.L = t->sorted_B * t->sorted_P;
-    gm.P = t->sorted_P;
     gm.C = t->D / VEC;
     gm.lpr_log2 = lanes_per_row_log2(gm.C);
     const int lpr = 1 << gm.lpr_log2;
-    constexpr int THREADS = (NCH > 4) ? 128 : 256;   // keeps the two partial arrays within 48 KB
     const int G = THREADS / lpr;
     gm.G = G;
-    gm.tile = choose_update_tile((int64_t)t->ntab * gm.L, lpr, t->sm_count,
-                                 THREADS * ((NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1)));
+    gm.tile = choose_update_tile(total, lpr, t->sm_count, THREADS * ((NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1)));
     {   // tuning aid (dlrmb_set_option("update_tile", v)): 4, 8, 16 or 32 entries per lane group
         const int v = g_opt.update_tile.load(std::memory_order_relaxed);
         if (v >= 4 && v <= 32 && v % 4 == 0) gm.tile = v;
     }
-    gm.tiles = (gm.L + gm.tile - 1) / gm.tile;
-    gm.chunks = (gm.tiles + G - 1) / G;
     gm.slots = slots;
     gm.slot0 = slot0;
     gm.cap = t->cap;
     gm.pcap = t->partial_tiles_cap;
-    DLRMB_REQUIRE(gm.chunks <= gm.pcap, "internal: update chunk capacity exceeded (%d > %lld)",
-                  gm.chunks, (long long)gm.pcap);
-    DLRMB_REQUIRE((int64_t)t->ntab * gm.chunks < (1ll << 31), "batch too large for one update launch");
     const uint32_t* keys = t->keys[t->sorted_buf];
     const uint32_t* pos = t->pos[t->sorted_buf];
-    dim3 grid((unsigned)gm.chunks, (unsigned)t->ntab);
-    const int64_t total_chunks = (int64_t)t->ntab * gm.chunks;
     // DLRM-sized batches: level 3 runs inside the same launch (see the header comment)
-    const bool inline_fixup = (int64_t)t->ntab * gm.L <= kUpdateInlineMaxEntries &&
+    const bool inline_fixup = total <= kUpdateInlineMaxEntries &&
                               g_opt.update_two_launches.load(std::memory_order_relaxed) == 0;
-    if (inline_fixup) {
-        update_tiles_kernel<VEC, NCH, THREADS, RowT, true><<<grid, THREADS, 0, s>>>(
+    if (equal) {
+        gm.L = (int)maxL;
+        gm.P = P[0];
+        gm.tiles = (gm.L + gm.tile - 1) / gm.tile;
+        gm.chunks = (gm.tiles + G - 1) / G;
+        DLRMB_REQUIRE(gm.chunks <= gm.pcap, "internal: update chunk capacity exceeded (%d > %lld)",
+                      gm.chunks, (long long)gm.pcap);
+        DLRMB_REQUIRE((int64_t)t->ntab * gm.chunks < (1ll << 31), "batch too large for one update launch");
+        dim3 grid((unsigned)gm.chunks, (unsigned)t->ntab);
+        const int64_t total_chunks = (int64_t)t->ntab * gm.chunks;
+        if (inline_fixup) {
+            update_tiles_kernel<VEC, NCH, THREADS, RowT, true><<<grid, THREADS, 0, s>>>(
+                t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, clock_slot(CLK_UPDATE));
+            DLRMB_LAUNCH_CHECK();
+            return DLRMB_OK;
+        }
+        DLRMB_CUDA(cudaMemsetAsync(t->head_count, 0, sizeof(uint32_t), s));
+        update_tiles_kernel<VEC, NCH, THREADS, RowT, false><<<grid, THREADS, 0, s>>>(
             t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, clock_slot(CLK_UPDATE));
+        DLRMB_LAUNCH_CHECK();
+        unsigned fgrid = (unsigned)(total_chunks < (int64_t)t->sm_count * 8 ? total_chunks : (int64_t)t->sm_count * 8);
+        update_fixup_kernel<VEC, NCH, RowT><<<fgrid, 256, 0, s>>>(t->d_desc, keys, lr, t->partial, t->tile_flags,
+                                                                 t->head_list, t->head_count, gm, clock_slot(CLK_FIXUP));
         DLRMB_LAUNCH_CHECK();
         return DLRMB_OK;
     }
-    DLRMB_CUDA(cudaMemsetAsync(t->head_count, 0, sizeof(uint32_t), s));
-    update_tiles_kernel<VEC, NCH, THREADS, RowT, false><<<grid, THREADS, 0, s>>>(
-        t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, clock_slot(CLK_UPDATE));
-    DLRMB_LAUNCH_CHECK();
-    unsigned fgrid = (unsigned)(total_chunks < (int64_t)t->sm_count * 8 ? total_chunks : (int64_t)t->sm_count * 8);
-    update_fixup_kernel<VEC, NCH, RowT><<<fgrid, 256, 0, s>>>(t->d_desc, keys, lr, t->partial, t->tile_flags,
-                                                        t->head_list, t->head_count, gm, clock_slot(CLK_FIXUP));
-    DLRMB_LAUNCH_CHECK();
-    return DLRMB_OK;
-}
-
-template <int VEC, int NCH, typename RowT>
-static int launch_update_mp_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
-    UpdateGeom gm;
+    // mixed P_k: only the `_mp` sorts, at most kMpMaxTables tables
     MpGeom g;
     g.ntab = t->ntab;
     g.B = (uint32_t)t->sorted_B;
     g.nlist = 0;
-    int64_t total = 0, maxL = 0;
-    for (int k = 0; k < t->ntab; ++k) {
-        g.P[k] = (uint32_t)t->h_sorted_P[k];
-        g.off[k] = 0;   // unused by the update
-        const int64_t L = (int64_t)g.B * g.P[k];
-        total += L;
-        maxL = L > maxL ? L : maxL;
-    }
     gm.L = (int)maxL;
     gm.P = 1;
-    gm.C = t->D / VEC;
-    gm.lpr_log2 = lanes_per_row_log2(gm.C);
-    const int lpr = 1 << gm.lpr_log2;
-    constexpr int THREADS = (NCH > 4) ? 128 : 256;
-    const int G = THREADS / lpr;
-    gm.G = G;
-    gm.tile = choose_update_tile(total, lpr, t->sm_count, THREADS * ((NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1)));
-    {
-        const int v = g_opt.update_tile.load(std::memory_order_relaxed);
-        if (v >= 4 && v <= 32 && v % 4 == 0) gm.tile = v;
-    }
-    gm.slots = slots;
-    gm.slot0 = slot0;
-    gm.cap = t->cap;
-    gm.pcap = t->partial_tiles_cap;
+    gm.tiles = 0;
+    gm.chunks = 0;
     int64_t chunks_total = 0;
     for (int k = 0; k < t->ntab; ++k) {
+        g.P[k] = (uint32_t)P[k];
+        g.off[k] = 0;   // unused by the update
         const int64_t tiles = ceil_div64((int64_t)g.B * g.P[k], gm.tile);
         const int64_t chunks = ceil_div64(tiles, G);
         DLRMB_REQUIRE(chunks <= gm.pcap, "internal: update chunk capacity exceeded (%lld > %lld)", (long long)chunks,
@@ -760,13 +750,7 @@ static int launch_update_mp_t(dlrmb_tables* t, const float* dT, int slots, int s
         chunks_total += chunks;
     }
     g.pre[t->ntab] = (uint32_t)chunks_total;
-    gm.tiles = 0;
-    gm.chunks = 0;
     DLRMB_REQUIRE(chunks_total < (1ll << 31), "batch too large for one update launch");
-    const uint32_t* keys = t->keys[t->sorted_buf];
-    const uint32_t* pos = t->pos[t->sorted_buf];
-    const bool inline_fixup = total <= kUpdateInlineMaxEntries &&
-                              g_opt.update_two_launches.load(std::memory_order_relaxed) == 0;
     if (inline_fixup) {
         update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, true><<<(unsigned)chunks_total, THREADS, 0, s>>>(
             t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g, clock_slot(CLK_UPDATE));
@@ -784,7 +768,7 @@ static int launch_update_mp_t(dlrmb_tables* t, const float* dT, int slots, int s
     return DLRMB_OK;
 }
 
-template <typename RowT, bool MP>
+template <typename RowT>
 static int launch_update_r(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
     const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(dT) & 15) == 0);
     if (t->D % 4 == 0 && !vec4) {
@@ -795,35 +779,23 @@ static int launch_update_r(dlrmb_tables* t, const float* dT, int slots, int slot
     const int lpr = 1 << lanes_per_row_log2(C);
     const int nch = (C + lpr - 1) / lpr;
     if (vec4) {
-        if (nch == 1) return MP ? launch_update_mp_t<4, 1, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<4, 1, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch == 2) return MP ? launch_update_mp_t<4, 2, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<4, 2, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 4) return MP ? launch_update_mp_t<4, 4, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<4, 4, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 8) return MP ? launch_update_mp_t<4, 8, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<4, 8, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 1) return launch_update_t<4, 1, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 2) return launch_update_t<4, 2, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 4) return launch_update_t<4, 4, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 8) return launch_update_t<4, 8, RowT>(t, dT, slots, slot0, lr, s);
     } else {
-        if (nch == 1) return MP ? launch_update_mp_t<1, 1, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<1, 1, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch == 2) return MP ? launch_update_mp_t<1, 2, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<1, 2, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 4) return MP ? launch_update_mp_t<1, 4, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<1, 4, RowT>(t, dT, slots, slot0, lr, s);
-        if (nch <= 8) return MP ? launch_update_mp_t<1, 8, RowT>(t, dT, slots, slot0, lr, s)
-                             : launch_update_t<1, 8, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 1) return launch_update_t<1, 1, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch == 2) return launch_update_t<1, 2, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 4) return launch_update_t<1, 4, RowT>(t, dT, slots, slot0, lr, s);
+        if (nch <= 8) return launch_update_t<1, 8, RowT>(t, dT, slots, slot0, lr, s);
     }
     set_error("embedding dim %d unsupported by the update kernel", t->D);
     return DLRMB_EINVAL;
 }
 
-// consumes whichever sort ran last: uniform, or per-table pooling factors (t->sorted_mp)
 int launch_update(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
-    if (t->sorted_mp)
-        return t->elem_bytes == 2 ? launch_update_r<__nv_bfloat16, true>(t, dT, slots, slot0, lr, s)
-                                  : launch_update_r<float, true>(t, dT, slots, slot0, lr, s);
-    if (t->elem_bytes == 2) return launch_update_r<__nv_bfloat16, false>(t, dT, slots, slot0, lr, s);
-    return launch_update_r<float, false>(t, dT, slots, slot0, lr, s);
+    if (t->elem_bytes == 2) return launch_update_r<__nv_bfloat16>(t, dT, slots, slot0, lr, s);
+    return launch_update_r<float>(t, dT, slots, slot0, lr, s);
 }
 
 }  // namespace dlrmb

@@ -93,6 +93,66 @@ def test_equal_pooling_factors_match_uniform_bitwise(P):
         assert np.array_equal(t_u.download(k), t_m.download(k))
 
 
+# A uniform batch on a handle with more tables than one per-table geometry holds (dlrmb_mp_max_tables):
+# the uniform entry points run the per-table launchers once per group of tables.  B = 256: lookup and
+# fused sort in one launch; B = 6000 with P = 3: separate lookup and radix sort.
+@pytest.mark.parametrize("P,B,dtype", [(1, 256, torch.float32), (3, 256, torch.float32),
+                                       (1, 256, torch.bfloat16), (3, 256, torch.bfloat16),
+                                       (3, 6000, torch.float32)])
+def test_uniform_more_tables_than_one_geometry(P, B, dtype):
+    from dlrm_jl_b200 import _lib
+    ntab, D, W, lr = 300, 16, 2, 0.05
+    assert ntab > _lib.load().dlrmb_mp_max_tables()
+    rng = np.random.default_rng(P + B)
+    rows = [int(r) for r in rng.integers(1, 200, size=ntab)]
+    t = _tables(_rand_tables(rng, rows, D), B * P, dtype)
+    idx = np.stack([rng.integers(0, r, size=(B, P)) for r in rows])
+    u_idx = torch.from_numpy(idx).to(_dev())
+    dT = torch.from_numpy(rng.standard_normal((B, 1 + ntab, D)).astype(np.float32)).to(_dev())
+    dTn = dT.cpu().numpy()
+
+    def check_dedup():
+        for k in range(ntab):
+            for a, b in zip(t.sort_dedup_export(k, B * P), O.sort_dedup(idx[k])):
+                assert np.array_equal(a, b), k
+
+    def check_update(stored):
+        for k in range(ntab):
+            ref, got = stored[k].copy(), t.download(k)
+            if dtype == torch.bfloat16:
+                O.sparse_sgd_update_bf16(ref, idx[k], np.ascontiguousarray(dTn[:, 1 + k]), lr)
+                assert O.rel_err(got, ref) < 2e-3, k
+            else:
+                O.sparse_sgd_update_fast(ref, idx[k], np.ascontiguousarray(dTn[:, 1 + k]), lr)
+                assert O.rel_err(got, ref) < SGD_RTOL, k
+
+    stored = [t.download(k) for k in range(ntab)]
+    ref = O.lookup(stored, idx, slot0=1)
+    for sort in (False, True):
+        T = torch.zeros((B, 1 + ntab, D), device=_dev())
+        t.lookup(u_idx, T, 1, sort=sort)
+        assert np.array_equal(T.cpu().numpy()[:, 1:], ref[:, 1:]), sort
+    t.update_sorted(dT, 1, lr)
+    check_update(stored)
+
+    t.sort(u_idx.to(torch.int32))
+    check_dedup()
+
+    stored = [t.download(k) for k in range(ntab)]
+    slotmap = [ntab - k for k in range(ntab)]          # reversed: a group must read its own part of the map
+    t.set_slot_map(slotmap)
+    bufs = [torch.full((B // W, 1 + ntab, D), float("nan"), device=_dev()) for _ in range(W)]
+    t.lookup_p2p(u_idx, [b.data_ptr() for b in bufs], B // W, 1 + ntab, 0, sort=True)
+    got = torch.cat(bufs).cpu().numpy()
+    want = O.lookup(stored, idx, slot0=0)
+    assert np.isnan(got[:, 0]).all()
+    assert np.array_equal(got[:, slotmap], want)
+    check_dedup()
+    t.update_sorted(dT, 1, lr)
+    check_update(stored)
+    t.close()
+
+
 def test_sort_dedup_all_three_regimes_in_one_batch():
     rng = np.random.default_rng(7)
     B = 2048
