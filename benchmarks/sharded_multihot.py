@@ -16,6 +16,11 @@ mode with the GPU name and power limit read in the same process.
     local dlrmb_embedding_fwd_sort_mp into one [B_global][t][D] buffer + update_sorted -- same bytes
   µs per step (median, min-max of --repeats), the fraction of the device-to-device copy bandwidth measured
   in the same process, and the busiest rank in µs under each plan.
+--plan column (with --mode owner): the column-wise plan (TableSharding.build(rows, W, P, D=D, max_col_shards=8))
+  beside the lookup-weighted one: every rank's owner-side µs -- for each of its width groups (one handle each),
+  dlrmb_embedding_fwd_p2p_sort_mp with the destination map + update_sorted, all groups in one timed step -- the
+  busiest rank under both plans, and, for the groups of split tables, the stand-alone sort of their indices
+  (every holder of a split table sorts its whole index stream; column sharding cannot shrink that part).
 --mode step: samples/s of the mixed-P sharded training step of the embeddings (NCCL index exchange,
   fused lookup + peer stores, gradient all-to-all, owner-side sparse SGD) under torchrun with >= 2 GPUs.
   With fewer GPUs it prints that nothing was measured.
@@ -26,6 +31,7 @@ import argparse
 import json
 import os
 import sys
+from fractions import Fraction
 
 import numpy as np
 import torch
@@ -93,6 +99,70 @@ def owner_rank(a, rows, P, sh, rank, dev, bw, with_local):
     del bufs, out, G, batches
     torch.cuda.empty_cache()
     return r
+
+
+def owner_rank_cw(a, rows, P, sh, rank, dev):
+    """One rank's units under a column-wise plan: one handle per width group, all groups in one timed step."""
+    W, Bl, D, ntab = sh.world, a.batch, a.D, len(rows)
+    Bg = Bl * W
+    groups = sh.groups(rank)
+    if not groups:
+        return {"rank": rank, "groups": [], "lookups_per_sample": 0, "p2p_us": None}
+    bufs = [torch.empty((Bl, 1 + ntab, D), device=dev) for _ in range(W)]
+    ptrs = [b.data_ptr() for b in bufs]
+    rng = np.random.default_rng(1234 + rank)
+    hs, bats, Gs = [], [], []
+    for c, ks in groups:
+        r_rows, r_P = [rows[k] for k in ks], [P[k] for k in ks]
+        t = EmbeddingTables(r_rows, D // c, Bg * max(r_P), dev)
+        t.init_uniform(1 + rank + 97 * c)
+        t.set_dest_map([1 + k for k in ks], [sh.slice_of(k, rank) * (D // c) for k in ks], D)
+        hs.append(t)
+        bats.append(make_batches(rng, r_rows, r_P, Bg, a.nb, 0.0, dev))
+        Gs.append(torch.randn((Bg, len(ks), D // c), device=dev) * 0.01)
+
+    def step(i):
+        for t, b, G in zip(hs, bats, Gs):
+            t.lookup_p2p(b[i], ptrs, Bl, 1 + ntab, 0, sort=True)
+            t.update_sorted(G, 0, 0.01)
+
+    res = [timed(step, a.nb, a.iters) for _ in range(a.repeats)]
+    r = {"rank": rank, "groups": [{"shards": c, "tables": ks, "slices": [sh.slice_of(k, rank) for k in ks]} for c, ks in groups],
+         "lookups_per_sample": float(sum(Fraction(P[k], c) for c, ks in groups for k in ks)), "p2p_us": _stats(res)}
+    split = [(t, b) for (c, _ks), t, b in zip(groups, hs, bats) if c > 1]
+    if split:
+        r["split_sort_us"] = _stats([timed(lambda i: [t.sort(b[i]) for t, b in split], a.nb, a.iters)
+                                     for _ in range(a.repeats)])
+    for t in hs:
+        t.close()
+    del bufs, bats, Gs
+    torch.cuda.empty_cache()
+    return r
+
+
+def mode_owner_column(a, rows, P, dev, info):
+    lines = []
+    for W in (2, 4, 8):
+        res = {}
+        for plan in ("lookup_weighted", "column"):
+            if plan == "column":
+                sh = TableSharding.build(rows, W, P, D=a.D, max_col_shards=8)
+                ranks = [owner_rank_cw(a, rows, P, sh, r, dev) for r in range(W)]
+            else:
+                sh = TableSharding.build(rows, W, P)
+                ranks = [owner_rank(a, rows, P, sh, r, dev, info["copy_gbs"], False) for r in range(W)]
+            busiest = max((x for x in ranks if x["p2p_us"]), key=lambda x: x["p2p_us"]["median"])
+            res[plan] = {"shards": list(sh.shards) if sh.split else None,
+                         "holders": sh.holders if sh.split else [[o] for o in sh.owner],
+                         "lookups_per_rank": [float(x) for x in sh.lookups_per_rank()],
+                         "ranks": ranks, "busiest_rank": busiest["rank"],
+                         "busiest_rank_p2p_us": busiest["p2p_us"]["median"]}
+        r = dict(info, mode="owner", plan="column", world=W, rows_cap=a.rows_cap, D=a.D, B_local=a.batch,
+                 B_global=W * a.batch, hotness=list(P), max_col_shards=8, nb=a.nb, iters=a.iters, repeats=a.repeats,
+                 **res, busiest_rank_us={p: res[p]["busiest_rank_p2p_us"] for p in res})
+        print(json.dumps(r), flush=True)
+        lines.append(r)
+    return lines
 
 
 def mode_owner(a, rows, P, dev, info):
@@ -166,6 +236,8 @@ def mode_step(a, rows, P):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--mode", default="owner", choices=["owner", "step"])
+    ap.add_argument("--plan", default="table", choices=["table", "column"],
+                    help="owner mode: table-wise plans (lookup-weighted and snake) or the column-wise plan")
     ap.add_argument("--hotness", default=MLPERF_HOTNESS)
     ap.add_argument("--rows-cap", type=int, default=20_000_000)
     ap.add_argument("--D", type=int, default=128)
@@ -185,7 +257,7 @@ def main():
         raise SystemExit("--mode owner measures on a GPU; none is visible (nothing measured)")
     dev = torch.device("cuda", 0)
     info = dict(gpu_info(), copy_gbs=copy_bandwidth_gbs(dev))
-    lines = mode_owner(a, rows, P, dev, info)
+    lines = (mode_owner_column if a.plan == "column" else mode_owner)(a, rows, P, dev, info)
     if a.out:
         with open(a.out, "a") as f:
             for r in lines:

@@ -64,6 +64,7 @@ SIGNATURES = {
     "dlrmb_xbuf_open": (_i32, [_i32, _vp, C.POINTER(_vp)]),
     "dlrmb_xbuf_close": (_i32, [_i32, _vp]),
     "dlrmb_tables_set_slot_map": (_i32, [_vp, C.POINTER(_i32)]),
+    "dlrmb_tables_set_dest_map": (_i32, [_vp, C.POINTER(_i32), C.POINTER(_i32), _i32]),
     "dlrmb_embedding_fwd_p2p": (_i32, [_vp, *_idx_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
     "dlrmb_embedding_fwd_p2p_sort": (_i32, [_vp, *_idx_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
     "dlrmb_embedding_fwd_p2p_mp": (_i32, [_vp, *_idx_mp_args, C.POINTER(_vp), _i32, _i32, _i32, _vp]),
@@ -74,15 +75,20 @@ SIGNATURES = {
     "dlrmb_peer_allreduce_f32": (_i32, [_i32, C.POINTER(_vp), C.POINTER(_vp), _i32, _i32, _i32, _vp, _vp, _i64, _vp]),
     "dlrmb_indices_scatter_p2p": (_i32, [_i32, _vp, _i32, _i32, _i32, _i32, _vp, _i32, _vp]),
     "dlrmb_indices_scatter_p2p_mp": (_i32, [_i32, _vp, _i32, _i32, _i32, C.POINTER(_i32), _vp, _i32, _vp]),
+    "dlrmb_indices_scatter_p2p_mp_list": (_i32, [_i32, _vp, _i32, _i32, _i32, C.POINTER(_i32), _i32, C.POINTER(_i32),
+                                                 _vp, _i32, _vp]),
     "dlrmb_interaction_has_warp_path": (_i32, [_i32, _i32]),
     "dlrmb_dense_fwd_bias_act": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _vp]),
     "dlrmb_dense_bwd_scratch_floats": (_i64, [_i32]),
     "dlrmb_dense_bwd_act_bias": (_i32, [_i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "dlrmb_interaction_bwd_scatter": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _i64, _vp, _vp]),
+    "dlrmb_interaction_bwd_scatter_cols": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _i32, _i64, _vp, _vp]),
     "dlrmb_interaction_bwd_dx": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp]),
     "dlrmb_dac_unpack": (_i32, [_i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "dlrmb_shard_plan": (_i32, [_i32, C.POINTER(_i64), _i32, C.POINTER(_i32)]),
     "dlrmb_shard_plan_mp": (_i32, [_i32, C.POINTER(_i64), C.POINTER(_i32), _i32, C.POINTER(_i32)]),
+    "dlrmb_shard_plan_cw": (_i32, [_i32, C.POINTER(_i64), C.POINTER(_i32), _i32, _i32, _i32, C.POINTER(_i32),
+                                   C.POINTER(_i32)]),
     "dlrmb_comm_unique_id": (_i32, [_vp]),
     "dlrmb_comm_create": (_i32, [_i32, _vp, _i32, _i32, C.POINTER(_vp)]),
     "dlrmb_comm_destroy": (_i32, [_vp]),

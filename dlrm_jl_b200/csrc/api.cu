@@ -432,7 +432,23 @@ int32_t dlrmb_interaction_bwd_scatter(int32_t device, const float* dOut, const f
     DeviceGuard guard(device);
     DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", device);
     return launch_interaction_bwd_ex(dOut, T, B, F, d, pad_to_mul, const_cast<float*>(T) /* unused */, dx, dests,
-                                     (long long)sample_offset, device_sm_count(device), (cudaStream_t)stream);
+                                     (long long)sample_offset, 0, device_sm_count(device), (cudaStream_t)stream);
+}
+
+int32_t dlrmb_interaction_bwd_scatter_cols(int32_t device, const float* dOut, const float* T, int32_t B,
+                                           int32_t F, int32_t d, int32_t pad_to_mul, const dlrmb_slot_dest* dests,
+                                           int32_t Q, int64_t sample_offset, float* dx, dlrmb_stream stream) {
+    int rc = check_interaction_args(B, F, d, pad_to_mul);
+    if (rc) return rc;
+    DLRMB_REQUIRE(dOut && T && dests && dx, "null buffer");
+    DLRMB_REQUIRE(Q >= 1 && Q <= 32 && (Q & (Q - 1)) == 0, "Q must be a power of two in 1..32 (got %d)", Q);
+    DLRMB_REQUIRE(d % Q == 0 && (d / Q) % 4 == 0, "d / Q must be a multiple of 4 (d = %d, Q = %d)", d, Q);
+    int qlog = 0;
+    while ((1 << qlog) < Q) ++qlog;
+    DeviceGuard guard(device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", device);
+    return launch_interaction_bwd_ex(dOut, T, B, F, d, pad_to_mul, const_cast<float*>(T) /* unused */, dx, dests,
+                                     (long long)sample_offset, qlog, device_sm_count(device), (cudaStream_t)stream);
 }
 
 int32_t dlrmb_interaction_bwd_dx(int32_t device, const float* dOut, const float* T, int32_t B, int32_t F, int32_t d,

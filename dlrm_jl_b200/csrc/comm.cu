@@ -203,6 +203,74 @@ int32_t dlrmb_shard_plan_mp(int32_t ntab, const int64_t* rows, const int32_t* P,
     return DLRMB_OK;
 }
 
+int32_t dlrmb_shard_plan_cw(int32_t ntab, const int64_t* rows, const int32_t* P, int32_t world, int32_t D, int32_t S,
+                            int32_t* shards, int32_t* owner) {
+    DLRMB_REQUIRE(ntab > 0, "ntab must be positive (got %d)", ntab);
+    DLRMB_REQUIRE(world > 0, "world must be positive (got %d)", world);
+    DLRMB_REQUIRE(rows && shards && owner, "null argument");
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    DLRMB_REQUIRE(S >= 1 && (S & (S - 1)) == 0, "max_col_shards must be a power of two (got %d)", S);
+    DLRMB_REQUIRE(D >= 1, "D must be positive (got %d)", D);
+    DLRMB_REQUIRE(S == 1 || (D % S == 0 && (D / S) % 4 == 0),
+                  "D / max_col_shards must be a multiple of 4 (D = %d, max_col_shards = %d)", D, S);
+    int64_t total = 0;
+    for (int k = 0; k < ntab; ++k) {
+        DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+        total += P[k];
+    }
+    // halve the hottest table's columns while its share P_k / c_k is above the even share sum(P) / world
+    std::vector<int64_t> c(ntab, 1);
+    const int64_t cmax = S < world ? S : world;
+    for (;;) {
+        int k = 0;
+        for (int i = 1; i < ntab; ++i) {   // largest P_i / c_i, then more rows, then the lower id
+            const int64_t lhs = (int64_t)P[i] * c[k], rhs = (int64_t)P[k] * c[i];
+            if (lhs > rhs || (lhs == rhs && rows[i] > rows[k])) k = i;
+        }
+        if ((int64_t)P[k] * world <= c[k] * total || 2 * c[k] > cmax) break;
+        c[k] *= 2;
+    }
+    int64_t M = 1;
+    for (int k = 0; k < ntab; ++k) M = c[k] > M ? c[k] : M;
+    for (int k = 0; k < ntab; ++k) {
+        shards[k] = (int32_t)c[k];
+        for (int j = 0; j < S; ++j) owner[(size_t)k * S + j] = -1;
+    }
+    if (M == 1) {   // nothing split: the table-wise plan
+        std::vector<int32_t> own(ntab);
+        int rc = dlrmb_shard_plan_mp(ntab, rows, P, world, own.data());
+        if (rc) return rc;
+        for (int k = 0; k < ntab; ++k) owner[(size_t)k * S] = own[k];
+        return DLRMB_OK;
+    }
+    // deal the units (k, j) longest first; loads and bytes in units of 1 / M (exact: every c_k divides M)
+    std::vector<std::pair<int, int>> units;
+    for (int k = 0; k < ntab; ++k)
+        for (int j = 0; j < c[k]; ++j) units.emplace_back(k, j);
+    std::sort(units.begin(), units.end(), [&](const std::pair<int, int>& a, const std::pair<int, int>& b) {
+        const int64_t lhs = (int64_t)P[a.first] * c[b.first], rhs = (int64_t)P[b.first] * c[a.first];
+        if (lhs != rhs) return lhs > rhs;
+        if (rows[a.first] != rows[b.first]) return rows[a.first] > rows[b.first];
+        if (a.first != b.first) return a.first < b.first;
+        return a.second < b.second;
+    });
+    std::vector<int64_t> load(world, 0), bytes(world, 0);
+    for (const auto& u : units) {
+        const int k = u.first;
+        int best = -1;
+        for (int r = 0; r < world; ++r) {
+            bool holds = false;
+            for (int j = 0; j < c[k]; ++j) holds = holds || owner[(size_t)k * S + j] == r;
+            if (holds) continue;
+            if (best < 0 || load[r] < load[best] || (load[r] == load[best] && bytes[r] < bytes[best])) best = r;
+        }
+        owner[(size_t)k * S + u.second] = best;
+        load[best] += (int64_t)P[k] * (M / c[k]);
+        bytes[best] += rows[k] * (M / c[k]);
+    }
+    return DLRMB_OK;
+}
+
 int32_t dlrmb_comm_unique_id(uint8_t* id128) {
     DLRMB_REQUIRE(id128 != nullptr, "id buffer is null");
     if (!nccl().ok) {

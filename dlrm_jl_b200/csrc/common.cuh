@@ -193,8 +193,11 @@ struct dlrmb_tables {
     int64_t* h_offsets = nullptr;    // element offsets of each table inside `slab`
     float* slab = nullptr;           // all tables, one allocation (f32 or bf16 elements)
     dlrmb::TableDesc* d_desc = nullptr;
-    int32_t* d_slotmap = nullptr;    // sharded use: interaction slot of each local table
-    int slotmap_max = -1;
+    int32_t* d_slotmap = nullptr;    // sharded use: element offset of each local table in a destination sample row
+                                     // (slot * dest_D + col0, dlrmb_tables_set_slot_map / _set_dest_map)
+    int slotmap_max = -1;            // largest slot of the map
+    int dest_D = 0;                  // floats per slot of the destination rows
+    bool dest_vec4 = false;          // dest_D and every col0 are multiples of 4 (16-byte peer stores possible)
     cudaStream_t own_stream = nullptr;
 
     // sort / update workspace (all [ntab][max_lookups] unless noted)
@@ -235,7 +238,7 @@ int launch_interaction_fwd(float* T, const float* x, int B, int F, int d, int pa
 int launch_interaction_bwd(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
                            float* dT, float* dx, int sm_count, cudaStream_t s);
 int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
-                              float* dT, float* dx, const void* dests, long long sample_offset,
+                              float* dT, float* dx, const void* dests, long long sample_offset, int qlog,
                               int sm_count, cudaStream_t s);
 int launch_interaction_bwd_dx(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul, float* dx,
                               int sm_count, cudaStream_t s);

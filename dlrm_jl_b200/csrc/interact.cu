@@ -306,7 +306,7 @@ static int launch_fwd_tb(float* T, const float* x, int B, int F, int d, int widt
 int try_interaction_fwd_warp(float* T, const float* x, int B, int F, int d, int width, float* out,
                              cudaStream_t s);
 int try_interaction_bwd_warp(const float* dOut, const float* T, int B, int F, int d, int width,
-                             float* dT, float* dx, const void* dests, long long sample_offset,
+                             float* dT, float* dx, const void* dests, long long sample_offset, int qlog,
                              cudaStream_t s);
 
 int launch_interaction_fwd(float* T, const float* x, int B, int F, int d, int pad_to_mul,
@@ -359,11 +359,13 @@ struct SlotDest {
     long long offset;          // floats: position of this table inside a destination sample
 };
 
-template <bool SCATTER>
-__global__ void __launch_bounds__(256)
-interaction_bwd_kernel(const float* __restrict__ dOut, const float* __restrict__ T, int B, int F,
-                       int d, int width, float* __restrict__ dT, float* __restrict__ dx, int NS,
-                       const SlotDest* __restrict__ dests, long long sample_offset) {
+// COLS: column pieces, dests[f * Q + q] for columns [q * d / Q, (q + 1) * d / Q) of slot f (Q = 1 << qlog, d / Q a
+// multiple of 4): chunk k goes to piece k / (d / 4Q) at chunk k % (d / 4Q) (column-wise sharded tables).
+template <bool SCATTER, bool COLS>
+__device__ __forceinline__ void
+interaction_bwd_body(const float* __restrict__ dOut, const float* __restrict__ T, int B, int F,
+                     int d, int width, float* __restrict__ dT, float* __restrict__ dx, int NS,
+                     const SlotDest* __restrict__ dests, long long sample_offset, int qlog) {
     extern __shared__ float4 smem4[];
     const int d4 = d >> 2;
     const int ldt4 = d4 + 1;
@@ -433,7 +435,20 @@ interaction_bwd_kernel(const float* __restrict__ dOut, const float* __restrict__
             a3.x = fmaf(sv.w, t.x, a3.x); a3.y = fmaf(sv.w, t.y, a3.y); a3.z = fmaf(sv.w, t.z, a3.z); a3.w = fmaf(sv.w, t.w, a3.w);
         }
         const int f0 = fb * 4;
-        if (SCATTER) {
+        if (SCATTER && COLS) {
+            const float4 av[4] = {a0, a1, a2, a3};
+            const int qw = d4 >> qlog;                 // chunks per piece
+            const int piece = k / qw, kc = k - piece * qw;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int f = f0 + q;
+                if (f >= 1 && f < F) {
+                    const SlotDest dd = dests[(f << qlog) + piece];
+                    float* row = dd.base + (sample_offset + s0 + s) * dd.sample_stride + dd.offset;
+                    reinterpret_cast<float4*>(row)[kc] = av[q];
+                }
+            }
+        } else if (SCATTER) {
             const float4 av[4] = {a0, a1, a2, a3};
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
@@ -457,6 +472,21 @@ interaction_bwd_kernel(const float* __restrict__ dOut, const float* __restrict__
             reinterpret_cast<float4*>(dx + (size_t)(s0 + s) * d)[k] = r;
         }
     }
+}
+
+template <bool SCATTER>
+__global__ void __launch_bounds__(256)
+interaction_bwd_kernel(const float* __restrict__ dOut, const float* __restrict__ T, int B, int F,
+                       int d, int width, float* __restrict__ dT, float* __restrict__ dx, int NS,
+                       const SlotDest* __restrict__ dests, long long sample_offset) {
+    interaction_bwd_body<SCATTER, false>(dOut, T, B, F, d, width, dT, dx, NS, dests, sample_offset, 0);
+}
+
+__global__ void __launch_bounds__(256)
+interaction_bwd_cols_kernel(const float* __restrict__ dOut, const float* __restrict__ T, int B, int F, int d, int width,
+                            float* __restrict__ dx, int NS, const SlotDest* __restrict__ dests, long long sample_offset,
+                            int qlog) {
+    interaction_bwd_body<true, true>(dOut, T, B, F, d, width, nullptr, dx, NS, dests, sample_offset, qlog);
 }
 
 __global__ void __launch_bounds__(256)
@@ -526,17 +556,13 @@ int launch_interaction_bwd_dx(const float* dOut, const float* T, int B, int F, i
     return DLRMB_OK;
 }
 
-int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
-                              float* dT, float* dx, const void* dests, long long sample_offset,
-                              int sm_count, cudaStream_t s);
-
 int launch_interaction_bwd(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
                            float* dT, float* dx, int sm_count, cudaStream_t s) {
-    return launch_interaction_bwd_ex(dOut, T, B, F, d, pad_to_mul, dT, dx, nullptr, 0, sm_count, s);
+    return launch_interaction_bwd_ex(dOut, T, B, F, d, pad_to_mul, dT, dx, nullptr, 0, 0, sm_count, s);
 }
 
 int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, int d, int pad_to_mul,
-                              float* dT, float* dx, const void* dests, long long sample_offset,
+                              float* dT, float* dx, const void* dests, long long sample_offset, int qlog,
                               int sm_count, cudaStream_t s) {
     const int width = interaction_width(F, d, pad_to_mul);
     const bool aligned = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(T) & 15) == 0) &&
@@ -554,7 +580,7 @@ int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, i
         return DLRMB_OK;
     }
     {
-        int rc = try_interaction_bwd_warp(dOut, T, B, F, d, width, dT, dx, dests, sample_offset, s);
+        int rc = try_interaction_bwd_warp(dOut, T, B, F, d, width, dT, dx, dests, sample_offset, qlog, s);
         if (rc >= 0) return rc;
     }
     const int d4 = d / 4;
@@ -564,11 +590,16 @@ int launch_interaction_bwd_ex(const float* dOut, const float* T, int B, int F, i
     DLRMB_REQUIRE(p.smem <= 200 * 1024, "interaction tile needs %zu bytes of shared memory", p.smem);
     static unsigned long long attr_done = 0;
     static unsigned long long attr_done2 = 0;
-    int rc = dests ? ensure_smem_attr((const void*)interaction_bwd_kernel<true>, 200 * 1024, &attr_done2)
-                   : ensure_smem_attr((const void*)interaction_bwd_kernel<false>, 200 * 1024, &attr_done);
+    static unsigned long long attr_done3 = 0;
+    int rc = (dests && qlog > 0) ? ensure_smem_attr((const void*)interaction_bwd_cols_kernel, 200 * 1024, &attr_done3)
+             : dests             ? ensure_smem_attr((const void*)interaction_bwd_kernel<true>, 200 * 1024, &attr_done2)
+                                 : ensure_smem_attr((const void*)interaction_bwd_kernel<false>, 200 * 1024, &attr_done);
     if (rc) return rc;
     int grid = (B + p.ns - 1) / p.ns;
-    if (dests)
+    if (dests && qlog > 0)
+        interaction_bwd_cols_kernel<<<grid, p.threads, p.smem, s>>>(dOut, T, B, F, d, width, dx, p.ns,
+                                                                     static_cast<const SlotDest*>(dests), sample_offset, qlog);
+    else if (dests)
         interaction_bwd_kernel<true><<<grid, p.threads, p.smem, s>>>(dOut, T, B, F, d, width, dT, dx, p.ns,
                                                                       static_cast<const SlotDest*>(dests), sample_offset);
     else

@@ -73,6 +73,7 @@ __device__ const PairTable kPairTable{};
 template <int F, int D, int VAR = 0>
 struct BwdGeom {
     static constexpr int LPS = D / 4;            // lanes per sample (one float4 of k each)
+    static constexpr int LPS_LOG2 = LPS >= 32 ? 5 : LPS >= 16 ? 4 : LPS >= 8 ? 3 : LPS >= 4 ? 2 : LPS >= 2 ? 1 : 0;
     static constexpr int SPW = 32 / LPS;         // samples per warp
     static constexpr int FP2 = (F + 1) & ~1;     // S row length, even
     static constexpr int NPAIR = F * (F - 1) / 2;
@@ -105,11 +106,15 @@ struct BwdGeom {
     static_assert(F <= 32, "pair table covers F <= 32");
 };
 
-template <int F, int D, bool SCATTER, int VAR>
+// COLS: the scatter destinations are column pieces, dests[f * Q + q] for columns [q * D / Q, (q + 1) * D / Q) of
+// slot f (Q = 1 << qlog, D / Q a multiple of 4): lane kl stores its float4 into piece kl / (LPS / Q) at chunk
+// kl % (LPS / Q) (column-wise sharded tables).
+template <int F, int D, bool SCATTER, int VAR, bool COLS = false>
 __global__ void __launch_bounds__(BwdGeom<F, D, VAR>::WARPS * 32) __maxnreg__((BwdGeom<F, D, VAR>::max_regs(SCATTER)))
 interaction_bwd_warp_kernel(const float* __restrict__ dOut, const float* __restrict__ T, int B, int width,
                             float* __restrict__ dT, float* __restrict__ dx,
-                            const SlotDestW* __restrict__ dests, long long sample_offset, unsigned long long* clk) {
+                            const SlotDestW* __restrict__ dests, long long sample_offset, unsigned long long* clk,
+                            int qlog = 0) {
     using G = BwdGeom<F, D, VAR>;
     extern __shared__ float4 smem4[];
     clock_in(clk, blockIdx.x);
@@ -237,7 +242,14 @@ interaction_bwd_warp_kernel(const float* __restrict__ dOut, const float* __restr
         for (int q = 0; q < G::NF; ++q) {
             const int f = f0 + q;
             const float4 r = make_float4(lo2[q].x, lo2[q].y, hi2[q].x, hi2[q].y);
-            if (SCATTER) {
+            if (SCATTER && COLS) {
+                if (f >= 1) {
+                    const int lqlog = G::LPS_LOG2 - qlog;     // lanes per piece: 1 << lqlog
+                    const SlotDestW dd = dests[(f << qlog) + (kl >> lqlog)];
+                    float* row = dd.base + (sample_offset + b) * dd.sample_stride + dd.offset;
+                    reinterpret_cast<float4*>(row)[kl & ((1 << lqlog) - 1)] = r;
+                }
+            } else if (SCATTER) {
                 if (f >= 1) {
                     const SlotDestW dd = dests[f];
                     float* row = dd.base + (sample_offset + b) * dd.sample_stride + dd.offset;
@@ -940,8 +952,21 @@ int launch_bwd_ring(const float* dOut, const float* T, int B, int width, float* 
 
 template <int F, int D>
 int launch_bwd_warp(const float* dOut, const float* T, int B, int width, float* dT, float* dx,
-                    const void* dests, long long sample_offset, cudaStream_t s) {
+                    const void* dests, long long sample_offset, int qlog, cudaStream_t s) {
     using G = BwdGeom<F, D>;
+    if (dests && qlog > 0) {   // column pieces: the peer-store kernel below with the piece-wise epilogue
+        constexpr int SV = (G::SPW == 1) ? 2 : 0;
+        static unsigned long long attr_done = 0;
+        const size_t smem = BwdGeom<F, D, SV>::smem_bytes();
+        const long long groups = ((long long)B + G::SPW - 1) / G::SPW;
+        const long long grid = (groups + G::WARPS - 1) / G::WARPS;
+        int rc = ensure_smem_attr((const void*)interaction_bwd_warp_kernel<F, D, true, SV, true>, (int)smem, &attr_done);
+        if (rc) return rc;
+        interaction_bwd_warp_kernel<F, D, true, SV, true><<<(unsigned)grid, G::WARPS * 32, smem, s>>>(
+            dOut, T, B, width, nullptr, dx, static_cast<const SlotDestW*>(dests), sample_offset, clock_slot(CLK_IBWD), qlog);
+        DLRMB_LAUNCH_CHECK();
+        return DLRMB_OK;
+    }
     if (dests) {   // peer-store epilogue: the resident kernel, with S stored once (VAR 2) for one sample per warp
         constexpr int SV = (G::SPW == 1) ? 2 : 0;
         static unsigned long long attr_done = 0;
@@ -1010,11 +1035,11 @@ int try_interaction_fwd_warp(float* T, const float* x, int B, int F, int d, int 
 }
 
 int try_interaction_bwd_warp(const float* dOut, const float* T, int B, int F, int d, int width,
-                             float* dT, float* dx, const void* dests, long long sample_offset,
+                             float* dT, float* dx, const void* dests, long long sample_offset, int qlog,
                              cudaStream_t s) {
     if (!warp_path_enabled()) return -1;
 #define X(FF, DD) \
-    if (F == FF && d == DD) return launch_bwd_warp<FF, DD>(dOut, T, B, width, dT, dx, dests, sample_offset, s);
+    if (F == FF && d == DD) return launch_bwd_warp<FF, DD>(dOut, T, B, width, dT, dx, dests, sample_offset, qlog, s);
     DLRMB_WARP_SHAPES(X)
 #undef X
     return -1;

@@ -9,6 +9,8 @@
 #include "common.cuh"
 #include "sort_small.cuh"
 
+#include <vector>
+
 struct dlrmb_xbuf {
     int device;
     void* ptr;
@@ -33,7 +35,8 @@ int ensure_smem_attr(const void* func, int bytes, unsigned long long* done_mask)
 
 // The lookup's geometry (one flat grid, table k owns CTAs [g.pre[k], g.pre[k+1]) in proportion to
 // B_global * P_k * C, lookup_grid_mp of lookup.cu) with a peer-store epilogue: sample b lives on rank
-// b / B_local and table k lands in slot slotmap[k].  P_k == 1 takes the U-chain gather, every other table
+// b / B_local and table k lands at element dstoff[k] of the sample's destination row (slot * D_dest + col0, the
+// dest map of dlrmb_tables_set_dest_map; rows are `ostride` floats apart).  P_k == 1 takes the U-chain gather, every other table
 // the 4-deep pooling loop in ascending p (the lookup's order, so the pooled rows are bit-identical to
 // dlrmb_embedding_fwd).  With SORT_ITEMS > 0 the first g.nlist CTAs sort the tables g.list[]
 // (B_global * P_k <= kFusedSortMax) in shared memory, as lookup_sort_mp_kernel does.  Both parameter structs go by value (__grid_constant__: peers.p[h] is read
@@ -44,10 +47,10 @@ __device__ __forceinline__ float4 p2p_add(float4 a, float4 b) {
 __device__ __forceinline__ float p2p_add(float a, float b) { return __fadd_rn(a, b); }
 
 template <typename IdxT, int VEC, int U, typename RowT>
-__device__ __forceinline__ void lookup_p2p_mp_cta(const TableDesc* __restrict__ desc, const int32_t* __restrict__ slotmap,
+__device__ __forceinline__ void lookup_p2p_mp_cta(const TableDesc* __restrict__ desc, const int32_t* __restrict__ dstoff,
                                                   const IdxT* __restrict__ idx, int idx_base, const MpGeom& g,
                                                   uint32_t C, int cshift, uint32_t B_local, const PeerPtrs& peers,
-                                                  int slots, uint32_t lin) {
+                                                  long long ostride, uint32_t lin) {
     using V = typename std::conditional<VEC == 4, float4, float>::type;
     const int k = mp_find(g.pre, g.ntab, lin);
     const uint32_t cx = lin - g.pre[k], nctas = g.pre[k + 1] - g.pre[k];
@@ -57,8 +60,7 @@ __device__ __forceinline__ void lookup_p2p_mp_cta(const TableDesc* __restrict__ 
     const uint32_t n = g.B * C;
     const uint32_t step = nctas * blockDim.x;
     const size_t D = (size_t)C * VEC;
-    const size_t slot_off = (size_t)slotmap[k] * D;
-    const size_t ostride = (size_t)slots * D;
+    const size_t slot_off = (size_t)dstoff[k];
 
     if (P == 1) {
         for (uint32_t t = cx * blockDim.x + threadIdx.x; t < n; t += step * U) {
@@ -119,9 +121,9 @@ __device__ __forceinline__ void lookup_p2p_mp_cta(const TableDesc* __restrict__ 
 
 template <typename IdxT, int VEC, int U, typename RowT, int SORT_ITEMS>
 __global__ void __launch_bounds__(256, (SORT_ITEMS > 0) ? 4 : 1)
-lookup_p2p_mp_kernel(const TableDesc* __restrict__ desc, const int32_t* __restrict__ slotmap, const IdxT* __restrict__ idx,
+lookup_p2p_mp_kernel(const TableDesc* __restrict__ desc, const int32_t* __restrict__ dstoff, const IdxT* __restrict__ idx,
                      int idx_base, const __grid_constant__ MpGeom g, uint32_t C, int cshift, uint32_t B_local,
-                     const __grid_constant__ PeerPtrs peers, int slots, uint32_t* __restrict__ keys_out,
+                     const __grid_constant__ PeerPtrs peers, long long ostride, uint32_t* __restrict__ keys_out,
                      uint32_t* __restrict__ pos_out, int64_t cap, unsigned long long* clk) {
     clock_in(clk, blockIdx.x);
     uint32_t lin = blockIdx.x;
@@ -136,7 +138,7 @@ lookup_p2p_mp_kernel(const TableDesc* __restrict__ desc, const int32_t* __restri
         }
         lin -= (uint32_t)g.nlist;
     }
-    lookup_p2p_mp_cta<IdxT, VEC, U, RowT>(desc, slotmap, idx, idx_base, g, C, cshift, B_local, peers, slots, lin);
+    lookup_p2p_mp_cta<IdxT, VEC, U, RowT>(desc, dstoff, idx, idx_base, g, C, cshift, B_local, peers, ostride, lin);
     clock_out(clk, blockIdx.x);
 }
 
@@ -159,7 +161,7 @@ static int launch_p2p_mp_t(dlrmb_tables* t, const IdxT* idx, int idx_base, const
         if (rc) return rc;
     }
     lookup_p2p_mp_kernel<IdxT, VEC, U, RowT, SORT_ITEMS><<<(unsigned)ctas, 256, smem, s>>>(
-        t->d_desc, t->d_slotmap, idx, idx_base, g, C, cshift, (uint32_t)B_local, peers, slots,
+        t->d_desc, t->d_slotmap, idx, idx_base, g, C, cshift, (uint32_t)B_local, peers, (long long)slots * t->dest_D,
         SORT_ITEMS > 0 ? t->keys[half] : nullptr, SORT_ITEMS > 0 ? t->pos[half] : nullptr, t->cap, clock_slot(CLK_LOOKUP));
     DLRMB_LAUNCH_CHECK();
     return DLRMB_OK;
@@ -265,24 +267,47 @@ int32_t dlrmb_xbuf_close(int32_t device, void* peer_ptr) {
     return DLRMB_OK;
 }
 
-int32_t dlrmb_tables_set_slot_map(dlrmb_tables* t, const int32_t* slots) {
+static int32_t set_dest_map(dlrmb_tables* t, const int32_t* slots, const int32_t* col0, int32_t D_dest) {
     DLRMB_REQUIRE(t && slots, "null argument");
+    DLRMB_REQUIRE(D_dest >= t->D, "D_dest = %d is narrower than the handle's D = %d", D_dest, t->D);
     DeviceGuard guard(t->device);
     DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", t->device);
     int max_slot = -1;
+    bool vec4 = D_dest % 4 == 0;
+    std::vector<int32_t> off(t->ntab);
     for (int k = 0; k < t->ntab; ++k) {
         DLRMB_REQUIRE(slots[k] >= 0, "slot_map[%d] = %d is negative", k, slots[k]);
+        const int32_t c0 = col0 ? col0[k] : 0;
+        DLRMB_REQUIRE(c0 >= 0 && (int64_t)c0 + t->D <= D_dest, "col0[%d] = %d: columns [%d, %d) leave the destination row of %d",
+                      k, c0, c0, c0 + t->D, D_dest);
+        DLRMB_REQUIRE(((int64_t)slots[k] + 1) * D_dest < (1ll << 31), "slot_map[%d] = %d: destination offset too large", k,
+                      slots[k]);
         if (slots[k] > max_slot) max_slot = slots[k];
+        vec4 = vec4 && c0 % 4 == 0;
+        off[k] = slots[k] * D_dest + c0;
     }
     if (!t->d_slotmap) DLRMB_CUDA(cudaMalloc((void**)&t->d_slotmap, sizeof(int32_t) * t->ntab));
-    DLRMB_CUDA(cudaMemcpy(t->d_slotmap, slots, sizeof(int32_t) * t->ntab, cudaMemcpyHostToDevice));
+    DLRMB_CUDA(cudaMemcpy(t->d_slotmap, off.data(), sizeof(int32_t) * t->ntab, cudaMemcpyHostToDevice));
     t->slotmap_max = max_slot;
+    t->dest_D = D_dest;
+    t->dest_vec4 = vec4;
     return DLRMB_OK;
 }
 
-// the peer pointers of `world` ranks; vec4: D % 4 == 0 and every pointer 16-byte aligned
+int32_t dlrmb_tables_set_slot_map(dlrmb_tables* t, const int32_t* slots) {
+    DLRMB_REQUIRE(t, "null argument");
+    return set_dest_map(t, slots, nullptr, t->D);
+}
+
+int32_t dlrmb_tables_set_dest_map(dlrmb_tables* t, const int32_t* slots, const int32_t* col0, int32_t D_dest) {
+    DLRMB_REQUIRE(t && slots && col0, "null argument");
+    return set_dest_map(t, slots, col0, D_dest);
+}
+
+// the peer pointers of `world` ranks; vec4: D % 4 == 0, a dest map of 16-byte column offsets and every pointer
+// 16-byte aligned
 static int peer_ptrs(const dlrmb_tables* t, float* const* peer_T, int world, PeerPtrs* peers, bool* vec4) {
-    *vec4 = (t->D % 4 == 0);
+    *vec4 = (t->D % 4 == 0) && t->dest_vec4;
     for (int r = 0; r < kMaxPeers; ++r) {
         peers->p[r] = r < world ? peer_T[r] : nullptr;
         if (r < world) {
@@ -489,6 +514,27 @@ indices_scatter_mp_kernel(const IdxT* __restrict__ idx_local, const IdxDest* __r
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
+// Column-wise sharding: a split table's block goes to every holder of one of its slices.  Destination i receives
+// table dest_table[i]'s block at dests[i] + rank * B_local * P_k, one launch for all destinations.
+constexpr int kMaxScatterDests = 1024;
+struct IdxScatterListGeom {
+    int B_local;
+    uint32_t P[kMpMaxTables];
+    int64_t src_off[kMpMaxTables];
+    uint16_t table[kMaxScatterDests];
+};
+
+template <typename IdxT>
+__global__ void __launch_bounds__(256)
+indices_scatter_list_kernel(const IdxT* __restrict__ idx_local, const IdxDest* __restrict__ dests,
+                            const __grid_constant__ IdxScatterListGeom g, int rank) {
+    const int k = g.table[blockIdx.y];
+    const int n = g.B_local * (int)g.P[k];
+    const IdxT* src = idx_local + g.src_off[k];
+    IdxT* dst = static_cast<IdxT*>(dests[blockIdx.y].base) + (size_t)rank * n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = src[i];
+}
+
 }  // namespace dlrmb
 
 extern "C" {
@@ -565,6 +611,46 @@ int32_t dlrmb_indices_scatter_p2p_mp(int32_t device, const void* idx_local, int3
         indices_scatter_mp_kernel<uint32_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)idx_local, d, g, rank);
     else
         indices_scatter_mp_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const int64_t*)idx_local, d, g, rank);
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_indices_scatter_p2p_mp_list(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
+                                          int32_t B_local, const int32_t* P, int32_t ndest, const int32_t* dest_table,
+                                          const void* const* dests_dev, int32_t rank, dlrmb_stream stream) {
+    DLRMB_REQUIRE(idx_local && dests_dev && dest_table, "null argument");
+    DLRMB_REQUIRE(P != nullptr, "P (per-table pooling factors) is null");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(ntab > 0 && ntab <= kMpMaxTables, "ntab must be in 1..%d (got %d)", kMpMaxTables, ntab);
+    DLRMB_REQUIRE(ndest > 0 && ndest <= kMaxScatterDests, "ndest must be in 1..%d (got %d)", kMaxScatterDests, ndest);
+    DLRMB_REQUIRE(B_local > 0 && rank >= 0, "bad index scatter geometry");
+    IdxScatterListGeom g;
+    g.B_local = B_local;
+    int64_t off = 0;
+    int32_t maxP = 0;
+    for (int k = 0; k < ntab; ++k) {
+        DLRMB_REQUIRE(P[k] >= 1, "P[%d] = %d: every pooling factor must be >= 1", k, P[k]);
+        DLRMB_REQUIRE((int64_t)B_local * P[k] < (1ll << 30), "B_local * P[%d] too large", k);
+        g.P[k] = (uint32_t)P[k];
+        g.src_off[k] = off;
+        off += (int64_t)B_local * P[k];
+        maxP = P[k] > maxP ? P[k] : maxP;
+    }
+    for (int i = 0; i < ndest; ++i) {
+        DLRMB_REQUIRE(dest_table[i] >= 0 && dest_table[i] < ntab, "dest_table[%d] = %d is not a table (ntab %d)", i,
+                      dest_table[i], ntab);
+        g.table[i] = (uint16_t)dest_table[i];
+    }
+    DeviceGuard guard(device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", device);
+    int bx = (int)((B_local * (int64_t)maxP + 255) / 256);
+    if (bx > 64) bx = 64;
+    dim3 grid((unsigned)bx, (unsigned)ndest);
+    const IdxDest* d = reinterpret_cast<const IdxDest*>(dests_dev);
+    if (idx_bytes == 4)
+        indices_scatter_list_kernel<uint32_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)idx_local, d, g, rank);
+    else
+        indices_scatter_list_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const int64_t*)idx_local, d, g, rank);
     DLRMB_LAUNCH_CHECK();
     return DLRMB_OK;
 }

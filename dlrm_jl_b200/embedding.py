@@ -246,7 +246,14 @@ class EmbeddingTables:
         arr = (C.c_int32 * self.ntab)(*[int(v) for v in slots])
         _lib.check(self._lib.dlrmb_tables_set_slot_map(self._h, arr))
 
-    FUSED_SORT_MAX = 4096     # kFusedSortMax of csrc/common.cuh: largest B*P whose sort rides in the lookup launch
+    def set_dest_map(self, slots: Sequence[int], col0: Sequence[int], D_dest: int) -> None:
+        """Column-wise sharded use: local table k's pooled rows land at columns [col0[k], col0[k] + D) of slot
+        slots[k] in destination rows of D_dest floats per slot (dlrmb_tables_set_dest_map)."""
+        arr = (C.c_int32 * self.ntab)(*[int(v) for v in slots])
+        cols = (C.c_int32 * self.ntab)(*[int(v) for v in col0])
+        _lib.check(self._lib.dlrmb_tables_set_dest_map(self._h, arr, cols, int(D_dest)))
+
+    FUSED_SORT_MAX = 4096    # kFusedSortMax of csrc/common.cuh: largest B*P whose sort rides in the lookup launch
 
     def lookup_p2p(self, idx: torch.Tensor, peer_ptrs: Sequence[int], B_local: int, slots: int, idx_base: int = 0,
                    sort: bool = False) -> None:

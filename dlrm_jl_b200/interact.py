@@ -84,20 +84,34 @@ class _DotInteractionFn(torch.autograd.Function):
 class ScatterPlan:
     """Where the interaction backward stores the gradient row of every feature slot when the
     embedding tables are sharded: `dests` is a device int64 tensor [F][3] laid out as the C struct
-    dlrmb_slot_dest {base pointer, floats per destination sample, float offset of the table}."""
+    dlrmb_slot_dest {base pointer, floats per destination sample, float offset of the table}.  With ``Q`` > 1
+    it is [F * Q][3]: entry f * Q + q receives columns [q d / Q, (q + 1) d / Q) of slot f (column-wise sharded
+    tables, dlrmb_interaction_bwd_scatter_cols)."""
 
-    def __init__(self, dests: torch.Tensor, sample_offset: int, stream: "torch.cuda.Stream" = None):
+    def __init__(self, dests: torch.Tensor, sample_offset: int, stream: "torch.cuda.Stream" = None, Q: int = 1):
         """``stream``: when given, the backward is split -- dx alone (dlrmb_interaction_bwd_dx) on the
         current stream, the full pullback with the peer stores on ``stream`` -- so whatever consumes dx
         (the bottom MLP's backward) overlaps the gradient exchange; wait for ``done`` before using the
         exchanged rows (ShardedEmbedding.finish_backward does)."""
         assert dests.dtype == torch.int64 and dests.dim() == 2 and dests.shape[1] == 3 and dests.is_contiguous()
         self.dests = dests
+        self.Q = int(Q)
         self.sample_offset = int(sample_offset)
         self.stream = stream
         self.done = torch.cuda.Event() if stream is not None else None
         self._keep = None
         self.on_launched = None      # callable run right after the scattering backward has been launched
+
+
+def _scatter(lib, T, dOut, B, F, d, pad_to_mul, plan: ScatterPlan, dx, stream) -> None:
+    if plan.Q == 1:
+        _lib.check(lib.dlrmb_interaction_bwd_scatter(
+            T.device.index or 0, dOut.data_ptr(), T.data_ptr(), B, F, d, pad_to_mul,
+            plan.dests.data_ptr(), plan.sample_offset, dx.data_ptr(), stream))
+    else:
+        _lib.check(lib.dlrmb_interaction_bwd_scatter_cols(
+            T.device.index or 0, dOut.data_ptr(), T.data_ptr(), B, F, d, pad_to_mul,
+            plan.dests.data_ptr(), plan.Q, plan.sample_offset, dx.data_ptr(), stream))
 
 
 class _DotInteractionScatterFn(torch.autograd.Function):
@@ -109,7 +123,7 @@ class _DotInteractionScatterFn(torch.autograd.Function):
     def forward(ctx, x: torch.Tensor, T: torch.Tensor, pad_to_mul: int, plan: ScatterPlan):
         _require_cuda(x, T)
         B, F, d = T.shape
-        assert T.is_contiguous() and T.dtype == torch.float32 and plan.dests.shape[0] == F
+        assert T.is_contiguous() and T.dtype == torch.float32 and plan.dests.shape[0] == F * plan.Q
         xc = x.contiguous()
         out = torch.empty((B, interaction_width(F, d, pad_to_mul)), dtype=torch.float32, device=T.device)
         lib = _lib.load()
@@ -137,18 +151,14 @@ class _DotInteractionScatterFn(torch.autograd.Function):
             dx_full = torch.empty_like(dx)
             with torch.cuda.stream(plan.stream):
                 with _prof.range("interaction_bwd"):
-                    _lib.check(lib.dlrmb_interaction_bwd_scatter(
-                        T.device.index or 0, dOut.data_ptr(), T.data_ptr(), B, F, d, ctx.pad_to_mul,
-                        plan.dests.data_ptr(), plan.sample_offset, dx_full.data_ptr(), plan.stream.cuda_stream))
+                    _scatter(lib, T, dOut, B, F, d, ctx.pad_to_mul, plan, dx_full, plan.stream.cuda_stream)
                 plan.done.record(plan.stream)
             plan._keep = (dOut, dx_full)      # alive until the exchange has been joined (finish_backward)
             if plan.on_launched is not None:
                 plan.on_launched()
             return dx, None, None, None
         with _prof.range("interaction_bwd"):
-            _lib.check(lib.dlrmb_interaction_bwd_scatter(
-                T.device.index or 0, dOut.data_ptr(), T.data_ptr(), B, F, d, ctx.pad_to_mul,
-                plan.dests.data_ptr(), plan.sample_offset, dx.data_ptr(), _stream(T)))
+            _scatter(lib, T, dOut, B, F, d, ctx.pad_to_mul, plan, dx, _stream(T))
         if plan.on_launched is not None:
             plan.on_launched()
         return dx, None, None, None

@@ -18,6 +18,7 @@ CUDA library.
 from __future__ import annotations
 
 from dataclasses import dataclass
+from fractions import Fraction
 from typing import Callable, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
@@ -33,13 +34,40 @@ class TableSharding:
 
     With per-table pooling factors P_k (not all equal) table k receives B_global * P_k lookups, so the
     tables are dealt longest first instead: descending P_k, then rows, then id, each to the rank with the
-    smallest sum of P_k so far (ties: fewer rows, then the lower rank).  Equal P_k give the snake plan."""
+    smallest sum of P_k so far (ties: fewer rows, then the lower rank).  Equal P_k give the snake plan.
+
+    With ``max_col_shards`` S > 1 a table hotter than the even share may be split by columns into c_k slices
+    (``shards``), slice j on rank ``holders[k][j]`` (columns [j D / c_k, (j + 1) D / c_k)); see :meth:`build`.
+    Then ``local[r]`` lists every table of which rank r holds a slice and ``owner[k]`` is the holder of slice 0."""
     rows: List[int]
     world: int
     owner: List[int]
     local: List[List[int]]      # local[r] = global table ids owned by rank r, ascending
     _slot_cache: Optional[dict] = None
     P: Optional[Tuple[int, ...]] = None     # per-table pooling factors the plan was built for (None: one P)
+    D: Optional[int] = None                 # embedding width of a column-wise plan
+    shards: Optional[Tuple[int, ...]] = None        # c_k of a plan that splits a table (None: every table whole)
+    holders: Optional[List[List[int]]] = None       # holders[k][j] = rank holding slice j of table k
+
+    @property
+    def split(self) -> bool:
+        """Whether the plan splits a table by columns."""
+        return self.shards is not None
+
+    def groups(self, r: int) -> List[Tuple[int, List[int]]]:
+        """Rank r's units grouped by width: [(c, tables ascending)] in ascending c, i.e. whole tables (width D)
+        first, then slices of width D / 2, D / 4, ...  One EmbeddingTables handle serves each group."""
+        if not self.split:
+            return [(1, list(self.local[r]))]
+        by_c = {}
+        for k in range(len(self.rows)):
+            if r in self.holders[k]:
+                by_c.setdefault(self.shards[k], []).append(k)
+        return sorted(by_c.items())
+
+    def slice_of(self, k: int, r: int) -> int:
+        """Index j of the slice of table k that rank r holds."""
+        return self.holders[k].index(r) if self.split else 0
 
     def slot_index(self, r: int, device) -> torch.Tensor:
         """Device tensor of the interaction slots (1 + table id) of rank r's tables (cached: no
@@ -62,9 +90,21 @@ class TableSharding:
         return self._slot_cache[key]
 
     @classmethod
-    def build(cls, rows: Sequence[int], world: int, P: Optional[Sequence[int]] = None) -> "TableSharding":
-        """The same rule as dlrmb_shard_plan (``P`` None or all equal) / dlrmb_shard_plan_mp."""
+    def build(cls, rows: Sequence[int], world: int, P: Optional[Sequence[int]] = None, *, D: Optional[int] = None,
+              max_col_shards: int = 1) -> "TableSharding":
+        """The same rule as dlrmb_shard_plan (``P`` None or all equal) / dlrmb_shard_plan_mp, and with
+        ``max_col_shards`` S > 1 as dlrmb_shard_plan_cw: while the table with the largest P_k / c_k (ties: more rows,
+        then the lower id) is above the even share (P_k * world > c_k * sum(P)) and 2 c_k <= min(S, world), its c_k
+        doubles.  Nothing split: the table-wise plan.  Otherwise the slices are dealt longest first (descending
+        P_k / c_k, then rows, then k, then j), each to the rank with the smallest sum of P_k / c_k among those
+        holding no slice of k (ties: fewer rows * D / c_k, then the lower rank).  ``P`` None counts one lookup per
+        table.  S must be a power of two and, when S > 1, D / S a multiple of 4."""
         rows = [int(r) for r in rows]
+        S = int(max_col_shards)
+        if S < 1 or S & (S - 1):
+            raise ValueError(f"max_col_shards must be a power of two, got {max_col_shards}")
+        if S > 1 and (D is None or int(D) < 1 or int(D) % S or (int(D) // S) % 4):
+            raise ValueError(f"D / max_col_shards must be a multiple of 4 (D = {D}, max_col_shards = {S})")
         Pt = None
         if P is not None:
             if world < 1 or not rows:
@@ -72,6 +112,10 @@ class TableSharding:
             Pt = tuple(int(p) for p in P)
             if len(Pt) != len(rows) or min(Pt) < 1:
                 raise ValueError(f"P must hold one pooling factor >= 1 per table ({len(rows)} tables), got {list(Pt)}")
+        if S > 1:
+            plan = cls._build_cw(rows, world, Pt or (1,) * len(rows), int(D), S, Pt)
+            if plan is not None:
+                return plan
         owner = [0] * len(rows)
         if Pt is None or len(set(Pt)) == 1:
             order = sorted(range(len(rows)), key=lambda k: (-rows[k], k))
@@ -86,18 +130,63 @@ class TableSharding:
                 load[r] += Pt[k]
                 size[r] += rows[k]
         local = [[k for k in range(len(rows)) if owner[k] == r] for r in range(world)]
-        return cls(rows, world, owner, local, P=Pt)
+        return cls(rows, world, owner, local, P=Pt, D=None if D is None else int(D))
 
-    def lookups_per_rank(self) -> List[int]:
-        """Sum of P_k over each rank's tables (per sample of the global batch)."""
+    @classmethod
+    def _build_cw(cls, rows, world, P, D, S, Pt) -> Optional["TableSharding"]:
+        """The column-wise plan, or None when it splits nothing (exact arithmetic: fractions as cross products)."""
+        n, total = len(rows), sum(P)
+        c = [1] * n
+        cmax = min(S, world)
+        while True:
+            k = 0
+            for i in range(1, n):
+                lhs, rhs = P[i] * c[k], P[k] * c[i]
+                if lhs > rhs or (lhs == rhs and rows[i] > rows[k]):
+                    k = i
+            if P[k] * world <= c[k] * total or 2 * c[k] > cmax:
+                break
+            c[k] *= 2
+        M = max(c)
+        if M == 1:
+            return None
+        units = sorted(((k, j) for k in range(n) for j in range(c[k])),
+                       key=lambda u: (Fraction(-P[u[0]], c[u[0]]), -rows[u[0]], u[0], u[1]))
+        load, size = [0] * world, [0] * world            # in units of 1 / M
+        holders = [[-1] * c[k] for k in range(n)]
+        for k, j in units:
+            r = min((r for r in range(world) if r not in holders[k]), key=lambda r: (load[r], size[r], r))
+            holders[k][j] = r
+            load[r] += P[k] * (M // c[k])
+            size[r] += rows[k] * (M // c[k])
+        local = [[k for k in range(n) if r in holders[k]] for r in range(world)]
+        return cls(rows, world, [h[0] for h in holders], local, P=Pt, D=D, shards=tuple(c), holders=holders)
+
+    def lookups_per_rank(self) -> List[Union[int, Fraction]]:
+        """Sum of P_k over each rank's tables (per sample of the global batch); a slice of a split table counts
+        P_k / c_k (exact fractions)."""
         P = self.P or (1,) * len(self.rows)
+        if self.split:
+            return [sum((Fraction(P[k], self.shards[k]) for k in l), Fraction(0)) for l in self.local]
         return [sum(P[k] for k in l) for l in self.local]
 
     def counts(self) -> List[int]:
         return [len(l) for l in self.local]
 
     def bytes_per_rank(self, D: int) -> List[int]:
+        if self.split:
+            return [sum(self.rows[k] * (D // self.shards[k]) for k in l) * 4 for l in self.local]
         return [sum(self.rows[k] for k in l) * D * 4 for l in self.local]
+
+    def _unit_index(self, r: int, c: int, ks: Sequence[int], device) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(slots, slice ids) of rank r's group of width D / c as device tensors (cached)."""
+        if self._slot_cache is None:
+            self._slot_cache = {}
+        key = ("units", r, c, str(device))
+        if key not in self._slot_cache:
+            self._slot_cache[key] = (torch.tensor([1 + k for k in ks], dtype=torch.int64, device=device),
+                                     torch.tensor([self.slice_of(k, r) for k in ks], dtype=torch.int64, device=device))
+        return self._slot_cache[key]
 
 
 def _a2a(out: torch.Tensor, inp: torch.Tensor, out_splits, in_splits, group) -> None:
@@ -201,6 +290,85 @@ def exchange_grads(dT: torch.Tensor, sh: TableSharding, rank: int, group=None) -
     return recv
 
 
+def exchange_indices_cw(packed, sh: TableSharding, rank: int, group=None) -> list:
+    """Column-wise plan: ``packed`` (PackedIndices of this rank's B_local samples, every table) -> one PackedIndices
+    per width group of this rank (:meth:`TableSharding.groups`), each the owner layout of its tables at B_global as
+    :func:`exchange_indices_mp` builds it.  A split table's block goes to every holder of one of its slices."""
+    from .embedding import PackedIndices
+    W = sh.world
+    P, Bl, flat = packed.P, packed.B, packed.flat
+    offs = np.concatenate([[0], np.cumsum([Bl * p for p in P])]).tolist()
+    order = [k for r in range(W) for _c, ks in sh.groups(r) for k in ks]          # grouped by holder
+    send = torch.cat([flat[offs[k]:offs[k + 1]] for k in order]) if order else flat[:0]
+    in_splits = [Bl * sum(P[k] for _c, ks in sh.groups(r) for k in ks) for r in range(W)]
+    groups = sh.groups(rank)
+    per_rank = Bl * sum(P[k] for _c, ks in groups for k in ks)
+    recv = torch.empty((W * per_rank,), dtype=flat.dtype, device=flat.device)
+    _a2a(recv, send.contiguous(), [per_rank] * W, in_splits, group)
+    # [h][unit][B_local][P_k] -> per group [unit][h][B_local][P_k]
+    rv = recv.view(W, per_rank)
+    out, o = [], 0
+    for _c, ks in groups:
+        parts = []
+        for k in ks:
+            n = Bl * P[k]
+            parts.append(rv[:, o:o + n].reshape(-1))
+            o += n
+        out.append(PackedIndices(torch.cat(parts).contiguous() if parts else recv[:0], tuple(P[k] for k in ks), Bl * W))
+    return out
+
+
+def exchange_pooled_cw(pooled: Sequence[torch.Tensor], T: torch.Tensor, sh: TableSharding, rank: int,
+                       group=None) -> None:
+    """Column-wise plan: pooled[g] [B_global][t_g][D / c_g] of this rank's width groups -> the column range of every
+    slice in T[:, 1 + k, :] on the rank that owns the samples.  T is [B_local][1 + ntab][D]."""
+    W = sh.world
+    Bl, F, D = T.shape
+    send = torch.cat([p[h * Bl:(h + 1) * Bl].reshape(-1) for h in range(W) for p in pooled]) if pooled else T.new_empty(0)
+    n_mine = Bl * sum(len(ks) * (D // c) for c, ks in sh.groups(rank))
+    out_splits = [Bl * sum(len(ks) * (D // c) for c, ks in sh.groups(r)) for r in range(W)]
+    recv = torch.empty((sum(out_splits),), dtype=T.dtype, device=T.device)
+    _a2a(recv, send, out_splits, [n_mine] * W, group)
+    off = 0
+    for r in range(W):
+        for c, ks in sh.groups(r):
+            if not ks:
+                continue
+            w = D // c
+            n = Bl * len(ks) * w
+            slots, js = sh._unit_index(r, c, ks, T.device)
+            T.view(Bl, F, c, w)[:, slots, js, :] = recv[off:off + n].view(Bl, len(ks), w)
+            off += n
+
+
+def exchange_grads_cw(dT: torch.Tensor, sh: TableSharding, rank: int, group=None) -> List[torch.Tensor]:
+    """Column-wise plan, mirror of :func:`exchange_pooled_cw`: dT [B_local][1 + ntab][D] -> one gradient
+    [B_global][t_g][D / c_g] per width group of this rank."""
+    W = sh.world
+    Bl, F, D = dT.shape
+    parts, in_splits = [], []
+    for r in range(W):
+        n = 0
+        for c, ks in sh.groups(r):
+            if not ks:
+                continue
+            slots, js = sh._unit_index(r, c, ks, dT.device)
+            parts.append(dT.view(Bl, F, c, D // c)[:, slots, js, :].reshape(-1))
+            n += Bl * len(ks) * (D // c)
+        in_splits.append(n)
+    groups = sh.groups(rank)
+    per_rank = Bl * sum(len(ks) * (D // c) for c, ks in groups)
+    recv = torch.empty((W * per_rank,), dtype=dT.dtype, device=dT.device)
+    _a2a(recv, torch.cat(parts) if parts else dT.new_empty(0), [per_rank] * W, in_splits, group)
+    rv = recv.view(W, per_rank)
+    out, o = [], 0
+    for c, ks in groups:
+        n = Bl * len(ks) * (D // c)
+        out.append(rv[:, o:o + n].reshape(W * Bl, len(ks), D // c))
+        o += n
+    return out
+
+
 class PeerExchange:
     """The interaction input buffer T [B_local][1 + ntab][D] of every rank, allocated by the
     library and mapped into every other rank's address space through CUDA IPC, so the owner of a
@@ -266,6 +434,9 @@ class PeerExchange:
         :func:`exchange_indices_mp` (sum over the owned tables of B_global * P_k indices) and ``idx_owned``
         is a :class:`~dlrm_jl_b200.embedding.PackedIndices`."""
         from .embedding import _DevicePtrView
+        if sharding.split:
+            Pt = (int(P),) * len(sharding.rows) if isinstance(P, (int, np.integer)) else tuple(int(p) for p in P)
+            return self._enable_index_exchange_cw(sharding, B_local, Pt, idx_bytes)
         if not isinstance(P, (int, np.integer)):
             return self._enable_index_exchange_mp(sharding, B_local, tuple(int(p) for p in P), idx_bytes)
         counts = sharding.counts()
@@ -302,6 +473,44 @@ class PeerExchange:
         self._idx_geom = (len(sharding.rows), B_local, P, idx_bytes)
         self._idx_P = (C.c_int32 * len(P))(*P)
 
+    def _enable_index_exchange_cw(self, sharding: "TableSharding", B_local: int, P: Tuple[int, ...], idx_bytes: int):
+        """Column-wise plan: the index buffer holds the owner layout of every width group of this rank, group after
+        group; ``idx_owned`` is a list of PackedIndices (one per group) and every holder of a slice of table k is a
+        destination of k's block (dlrmb_indices_scatter_p2p_mp_list)."""
+        import ctypes as C
+
+        from .embedding import PackedIndices, _DevicePtrView
+        if len(P) != len(sharding.rows) or min(P) < 1:
+            raise ValueError(f"P must hold one pooling factor >= 1 per table ({len(sharding.rows)} tables), got {list(P)}")
+        Bg = B_local * self.world
+
+        def layout(r):       # element offset of every table's block in rank r's buffer
+            off, o = {}, 0
+            for _c, ks in sharding.groups(r):
+                for k in ks:
+                    off[k] = o
+                    o += Bg * P[k]
+            return off, o
+        mine, n_owned = layout(self.rank)
+        self._ibuf, own, peer_idx = self._share(max(1, n_owned) * idx_bytes)
+        ts = "<i4" if idx_bytes == 4 else "<i8"
+        flat = torch.as_tensor(_DevicePtrView(own, (max(1, n_owned),), self, ts), device=self.device)
+        self.idx_owned = []
+        for _c, ks in sharding.groups(self.rank):
+            o = mine[ks[0]] if ks else 0
+            n = sum(Bg * P[k] for k in ks)
+            self.idx_owned.append(PackedIndices(flat[o:o + n], tuple(P[k] for k in ks), Bg))
+        dest_table, dests = [], []
+        for r in range(self.world):
+            off, _n = layout(r)
+            for k in sorted(off):
+                dest_table.append(k)
+                dests.append(peer_idx[r] + off[k] * idx_bytes)
+        self._idx_dests = torch.tensor(dests, dtype=torch.int64, device=self.device)
+        self._idx_list = (C.c_int32 * len(dest_table))(*dest_table)
+        self._idx_geom = (len(sharding.rows), B_local, P, idx_bytes)
+        self._idx_P = (C.c_int32 * len(P))(*P)
+
     def enable_small_allreduce(self, n: int) -> None:
         """Exchange buffer [2][world][n] floats for `allreduce_small` (dlrmb_peer_allreduce_f32)."""
         import ctypes as C
@@ -326,6 +535,16 @@ class PeerExchange:
         exchange was enabled with per-table pooling factors)."""
         from . import _lib
         ntab, Bl, P, ib = self._idx_geom
+        if isinstance(P, tuple) and getattr(self, "_idx_list", None) is not None:
+            from . import _prof
+            assert tuple(idx_local.P) == P and idx_local.B == Bl and idx_local.element_size() == ib
+            with _prof.range("indices_scatter"):
+                _lib.check(self.lib.dlrmb_indices_scatter_p2p_mp_list(
+                    self.device.index or 0, idx_local.data_ptr(), ib, ntab, Bl, self._idx_P, len(self._idx_list),
+                    self._idx_list, self._idx_dests.data_ptr(), self.rank,
+                    int(torch.cuda.current_stream(self.device).cuda_stream)))
+            self.barrier(0)
+            return self.idx_owned
         if isinstance(P, tuple):
             from . import _prof
             assert tuple(idx_local.P) == P and idx_local.B == Bl and idx_local.element_size() == ib
@@ -398,6 +617,8 @@ class PeerExchange:
         the per-slot destination table the scattered interaction backward reads."""
         from .embedding import _DevicePtrView
         from .interact import ScatterPlan
+        if sharding.split:
+            return self._enable_gradient_exchange_cw(sharding, B_local, D, split_dx)
         counts = sharding.counts()
         t_mine = counts[self.rank]
         Bg = B_local * self.world
@@ -409,6 +630,37 @@ class PeerExchange:
             rows.append([self.peer_G_ptrs[o], counts[o] * D, sharding.local[o].index(k) * D])
         dests = torch.tensor(rows, dtype=torch.int64, device=self.device)
         return ScatterPlan(dests, self.rank * B_local, torch.cuda.Stream(self.device) if split_dx else None)
+
+    def _enable_gradient_exchange_cw(self, sharding: "TableSharding", B_local: int, D: int, split_dx: bool):
+        """Column-wise plan: one gradient buffer G [B_global][tables of the group][D / c] per width group, mapped
+        everywhere (``self.G`` is the list of this rank's, in group order), and a scatter plan of Q = max c_k column
+        pieces per slot (dlrmb_interaction_bwd_scatter_cols)."""
+        from .embedding import _DevicePtrView
+        from .interact import ScatterPlan
+        Bg = B_local * self.world
+        widths = sorted(set(sharding.shards))
+        grp = [dict(sharding.groups(r)) for r in range(self.world)]       # rank -> {c: tables}
+        peer_G = {}
+        mine = dict(sharding.groups(self.rank))
+        G = {}
+        for c in widths:      # collective: every rank maps one buffer per width of the plan, in the same order
+            t = len(mine.get(c, []))
+            _h, own, peer_G[c] = self._share(Bg * max(1, t) * (D // c) * 4)
+            G[c] = torch.as_tensor(_DevicePtrView(own, (Bg, max(1, t), D // c), self), device=self.device)
+        self.G = [G[c] for c, _ks in sharding.groups(self.rank)]
+        self.peer_G_ptrs = peer_G
+        Q = max(sharding.shards)
+        pw = D // Q
+        rows = [[0, 0, 0]] * Q                                # slot 0 (x) has no destination
+        for k in range(len(sharding.rows)):
+            c = sharding.shards[k]
+            for q in range(Q):
+                j, sub = divmod(q, Q // c)
+                h = sharding.holders[k][j]
+                ks = grp[h][c]
+                rows.append([peer_G[c][h], len(ks) * (D // c), ks.index(k) * (D // c) + sub * pw])
+        dests = torch.tensor(rows, dtype=torch.int64, device=self.device)
+        return ScatterPlan(dests, self.rank * B_local, torch.cuda.Stream(self.device) if split_dx else None, Q=Q)
 
     def barrier(self, channel: int = 0) -> None:
         """Order this rank's earlier peer stores before every rank's later reads (stream-ordered).
@@ -452,6 +704,8 @@ class _ShardedLookupFn(torch.autograd.Function):
             se.lookup_fn(idx_local, T, 1)
             se.presorted = se.lookup_sorts
             return T
+        if se.split:
+            return se._forward_cw(idx_local, Bl)
         idx_owned = se._exchange_indices(idx_local)
         se.idx_owned = idx_owned
         se.presorted = False
@@ -480,6 +734,8 @@ class _ShardedLookupFn(torch.autograd.Function):
         se = ctx.se
         if se.world == 1:
             se.owned_grad = dT.contiguous()      # [B][1 + ntab][D], consumed with slot0 = 1
+        elif se.split:
+            se.owned_grad = exchange_grads_cw(dT.contiguous(), se.sharding, se.rank, se.group)
         else:
             se.owned_grad = exchange_grads(dT.contiguous(), se.sharding, se.rank, se.group)
         se._update_from_backward(fused=False)
@@ -493,20 +749,32 @@ class ShardedEmbedding:
     ``update_fn(idx_owned, grad [Bg][slot0 + t][D], lr, slot0, presorted)`` do the local compute;
     :meth:`create` wires them to an :class:`~dlrm_jl_b200.embedding.EmbeddingTables` holding this
     rank's tables.  ``slot0`` is 1 at world size 1 (the buffers ARE the interaction input) else 0.
+
+    When the plan splits a table by columns (``max_col_shards`` > 1), the rank's units form width groups
+    (:meth:`TableSharding.groups`, ``self.groups``) and the injected functions take the group's position as one
+    more argument: ``lookup_fn(idx_g, out [Bg][t_g][D / c_g], 0, g)``, ``update_fn(idx_g, grad_g, lr, 0, presorted,
+    g)``, ``sort_fn(idx_g, g)``; :meth:`create` gives each group an EmbeddingTables of its width.
     """
 
     def __init__(self, rows: Sequence[int], D: int, rank: int, world: int, lookup_fn: Callable,
                  update_fn: Callable, group=None, sort_fn: Optional[Callable] = None, idx_base: int = 0,
-                 lookup_sorts: bool = False, P: Optional[Sequence[int]] = None):
+                 lookup_sorts: bool = False, P: Optional[Sequence[int]] = None, max_col_shards: int = 1):
         """``idx_base``: 1 for reference-format (1-based) ids, 0 for PyTorch-style ids; it is handed to
         every kernel that reads the indices.  ``lookup_sorts``: `lookup_fn` also prepares the sort /
         dedup of the step's update (the fused launch), so `sort_async` has nothing left to do.
         ``P``: per-table pooling factors (one per table).  Then the tables are placed by
         ``TableSharding.build(rows, world, P)``, batches are :class:`~dlrm_jl_b200.embedding.PackedIndices`
         (or anything ``_as_index_tensor`` turns into one) and the owners receive theirs in the owner layout
-        of :func:`exchange_indices_mp`.  Without it every table has the same P and mixed widths are refused."""
+        of :func:`exchange_indices_mp`.  Without it every table has the same P and mixed widths are refused.
+        ``max_col_shards``: split hot tables by columns into up to that many slices (a power of two, D divisible into
+        slices of a multiple of 4 columns); see :meth:`TableSharding.build`."""
         self.P = None if P is None else tuple(int(p) for p in P)
-        self.sharding = TableSharding.build(rows, world, self.P)
+        if int(max_col_shards) == 1:
+            self.sharding = TableSharding.build(rows, world, self.P)
+        else:
+            self.sharding = TableSharding.build(rows, world, self.P, D=D, max_col_shards=max_col_shards)
+        self.split = self.sharding.split
+        self.groups = self.sharding.groups(rank)
         self.rank, self.world, self.group = rank, world, group
         self.idx_base = int(idx_base)
         self.lookup_sorts = bool(lookup_sorts)
@@ -521,6 +789,45 @@ class ShardedEmbedding:
         self.peer: Optional[PeerExchange] = None
         self.scatter_plan = None
         self._auto_update = None
+
+    # ---- column-wise plans: one handle / index block / gradient per width group -------------------------
+    def _forward_cw(self, idx_local, Bl: int) -> torch.Tensor:
+        idx_groups = self._exchange_indices(idx_local)
+        self.idx_owned = idx_groups
+        self.presorted = [False] * len(self.groups)
+        if self.peer is not None:
+            self._lookup_p2p_cw(idx_groups, Bl)
+            self.peer.barrier(1)
+            return self.peer.T.detach()
+        dev = idx_groups[0].flat.device if idx_groups else torch.device("cpu")
+        pooled = []
+        for g, (c, ks) in enumerate(self.groups):
+            out = torch.empty((Bl * self.world, len(ks), self.D // c), dtype=torch.float32, device=dev)
+            self.lookup_fn(idx_groups[g], out, 0, g)
+            pooled.append(out)
+        T = torch.empty((Bl, 1 + self.ntab, self.D), dtype=torch.float32, device=self._device(idx_local))
+        exchange_pooled_cw(pooled, T, self.sharding, self.rank, self.group)
+        return T
+
+    def _lookup_p2p_cw(self, idx_groups, Bl: int) -> None:
+        for g, tables in enumerate(self.group_tables):
+            fuse = self._fuse_sort(idx_groups[g])
+            tables.lookup_p2p(idx_groups[g], self.peer.peer_ptrs, Bl, 1 + self.ntab, self.idx_base, sort=fuse)
+            self.presorted[g] = fuse
+
+    @staticmethod
+    def _device(idx):
+        from .embedding import PackedIndices
+        return idx.flat.device if isinstance(idx, PackedIndices) else idx.device
+
+    def download(self, k: int) -> List[Tuple[int, np.ndarray]]:
+        """Read back what this rank holds of global table k: [(first column, [rows_k][width] array)] for every
+        slice (one entry, column 0, for a whole table; none when the rank holds nothing of k).  Needs :meth:`create`."""
+        out = []
+        for (c, ks), tables in zip(self.groups, self.group_tables):
+            if k in ks:
+                out.append((self.sharding.slice_of(k, self.rank) * (self.D // c), tables.download(ks.index(k))))
+        return out
 
     def update_inside_backward(self, lr: float, stream: "torch.cuda.Stream") -> None:
         """Launch the sparse update from INSIDE the backward pass, on ``stream``, as soon as the pooled-embedding
@@ -563,6 +870,11 @@ class ShardedEmbedding:
         with torch.no_grad():
             idx_owned = self._exchange_indices(idx_local)
             self.idx_owned = idx_owned
+            if self.split:
+                self.presorted = [False] * len(self.groups)
+                self._lookup_p2p_cw(idx_owned, _batch(idx_local))
+                self.peer.barrier(1)
+                return self.peer.T.detach()
             self.presorted = False
             if len(self.local_ids):
                 # up to 4096 lookups per table the sort of the coming update rides in the lookup launch
@@ -587,6 +899,10 @@ class ShardedEmbedding:
         is equal) and checks the widths against its P."""
         if self.P is None:
             _require_uniform_pooling(idx_local)
+            if self.split:       # column-wise plans exchange through the per-table-P machinery
+                from .embedding import PackedIndices
+                ntab, B, P = idx_local.shape
+                return PackedIndices(idx_local.contiguous().reshape(-1), (int(P),) * ntab, int(B))
             return idx_local
         from .embedding import PackedIndices, _as_index_tensor
         tables = getattr(self, "tables", None)
@@ -607,6 +923,10 @@ class ShardedEmbedding:
     def _exchange_indices(self, idx_local: torch.Tensor) -> torch.Tensor:
         """Index columns to the tables' owners: peer stores + flag barrier when the index buffers are
         mapped (`enable_index_exchange`), NCCL all-to-all otherwise."""
+        if self.split:
+            if self.peer is not None and self.peer._idx_dests is not None:
+                return self.peer.scatter_indices(idx_local)
+            return exchange_indices_cw(idx_local, self.sharding, self.rank, self.group)
         if self.P is not None:
             if self.peer is not None and self.peer._idx_dests is not None:
                 return self.peer.scatter_indices(idx_local)
@@ -620,9 +940,10 @@ class ShardedEmbedding:
         """After loss.backward() on the fused path: every rank's gradient rows have landed.  The index
         sort of this step (side stream) is joined first: once a rank passes this barrier its peers may
         start the next step and overwrite the index buffer the sort reads."""
-        if len(self.local_ids) and getattr(self.tables, "_pending_side", False):
-            torch.cuda.current_stream(self.tables.device).wait_event(self.tables._sorted_event)
-            self.tables._pending_side = False
+        for tables in (self.group_tables if self.split else [self.tables] if len(self.local_ids) else []):
+            if getattr(tables, "_pending_side", False):
+                torch.cuda.current_stream(tables.device).wait_event(tables._sorted_event)
+                tables._pending_side = False
         plan = self.scatter_plan
         if plan is not None and plan.stream is not None and plan._keep is not None:
             torch.cuda.current_stream(self.tables.device).wait_event(plan.done)     # this rank's peer stores are issued
@@ -641,7 +962,12 @@ class ShardedEmbedding:
             raise ValueError(f"P {list(P)} differs from the handle's per-table P {list(self.P)}")
         if self.world == 1:
             return
-        self.tables.set_slot_map([1 + k for k in self.local_ids] or [1])
+        if self.split:
+            for (c, ks), tables in zip(self.groups, self.group_tables):
+                tables.set_dest_map([1 + k for k in ks], [self.sharding.slice_of(k, self.rank) * (self.D // c) for k in ks],
+                                    self.D)
+        else:
+            self.tables.set_slot_map([1 + k for k in self.local_ids] or [1])
         self.peer = PeerExchange(B_local, self.ntab, self.D, self.rank, self.world, self.tables.device,
                                  self.group, barrier, flag_barrier)
         if P is not None:
@@ -649,11 +975,18 @@ class ShardedEmbedding:
 
     @classmethod
     def create(cls, rows: Sequence[int], D: int, B_local: int, P: Union[int, Sequence[int]], rank: int, world: int,
-               device, group=None, seed: int = 51234, idx_base: int = 0, dtype=None) -> "ShardedEmbedding":
+               device, group=None, seed: int = 51234, idx_base: int = 0, dtype=None,
+               max_col_shards: int = 1) -> "ShardedEmbedding":
         """``P``: lookups per sample of every table, or a sequence of one pooling factor per table (mixed
-        multi-hot; the plan then weighs each table by its P_k, see :class:`TableSharding`)."""
+        multi-hot; the plan then weighs each table by its P_k, see :class:`TableSharding`).  ``max_col_shards``:
+        split hot tables by columns (one EmbeddingTables per width group of this rank)."""
         from .embedding import EmbeddingTables
         Pseq = None if isinstance(P, (int, np.integer)) else tuple(int(p) for p in P)
+        if int(max_col_shards) != 1:
+            sh = TableSharding.build(rows, world, Pseq, D=D, max_col_shards=max_col_shards)
+            if sh.split:
+                return cls._create_cw(rows, D, B_local, P, Pseq, rank, world, device, group, seed, idx_base, dtype,
+                                      max_col_shards)
         sh = TableSharding.build(rows, world, Pseq)
         mine = sh.local[rank]
         kw = {} if dtype is None else {"dtype": dtype}
@@ -671,6 +1004,30 @@ class ShardedEmbedding:
         se.tables = tables
         return se
 
+    @classmethod
+    def _create_cw(cls, rows, D, B_local, P, Pseq, rank, world, device, group, seed, idx_base, dtype,
+                   max_col_shards) -> "ShardedEmbedding":
+        from .embedding import EmbeddingTables
+        sh = TableSharding.build(rows, world, Pseq, D=D, max_col_shards=max_col_shards)
+        kw = {} if dtype is None else {"dtype": dtype}
+        group_tables = []
+        for g, (c, ks) in enumerate(sh.groups(rank)):
+            max_lookups = B_local * world * (P if Pseq is None else max(Pseq[k] for k in ks))
+            tables = EmbeddingTables([rows[k] for k in ks], D // c, max_lookups, device, **kw)
+            tables.init_uniform(seed + 7919 * rank + 104729 * g)
+            group_tables.append(tables)
+        se = cls(rows, D, rank, world,
+                 lookup_fn=lambda idx, out, slot0, g: group_tables[g].lookup(idx, out, slot0, idx_base),
+                 update_fn=lambda idx, grad, lr, slot0, presorted, g: (
+                     group_tables[g].update_sorted(grad, slot0, lr) if presorted
+                     else group_tables[g].bwd_sgd(idx, grad, slot0, lr, idx_base)),
+                 group=group,
+                 sort_fn=lambda idx, g: group_tables[g].sort(idx, idx_base, side_stream=True),
+                 idx_base=idx_base, P=Pseq, max_col_shards=max_col_shards)
+        se.group_tables = group_tables
+        se.tables = group_tables[0] if group_tables else None
+        return se
+
     def lookup(self, idx_local: torch.Tensor, anchor: torch.Tensor) -> torch.Tensor:
         """idx_local [ntab][B_local][P] -> T [B_local][1 + ntab][D] (requires grad through `anchor`,
         any tensor that requires grad, so autograd calls the gradient exchange).  A handle with per-table
@@ -680,6 +1037,12 @@ class ShardedEmbedding:
     def sort_async(self) -> None:
         """Start the index sort/dedup for this step's update on the side stream (nothing to do when
         the lookup launch already produced it)."""
+        if self.split:
+            for g in range(len(self.groups)):
+                if not self.presorted[g] and self.sort_fn is not None:
+                    self.sort_fn(self.idx_owned[g], g)
+                    self.presorted[g] = True
+            return
         if self.presorted:
             return
         if self.sort_fn is not None and len(self.local_ids):
@@ -689,6 +1052,12 @@ class ShardedEmbedding:
     def update(self, lr: float, presorted: Optional[bool] = None) -> None:
         """Owner-side sparse SGD.  ``presorted`` defaults to whether this step's sort already ran
         (fused lookup launch or `sort_async`)."""
+        if self.split:
+            for g in range(len(self.groups)):
+                self.update_fn(self.idx_owned[g], self.owned_grad[g], lr, self.slot0,
+                               self.presorted[g] if presorted is None else presorted, g)
+            self.presorted = [False] * len(self.groups)
+            return
         if len(self.local_ids) == 0:
             return
         if presorted is None:

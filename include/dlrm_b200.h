@@ -254,6 +254,13 @@ int32_t dlrmb_xbuf_ipc_handle(dlrmb_xbuf* x, uint8_t* handle64);
 int32_t dlrmb_xbuf_open(int32_t device, const uint8_t* handle64, void** peer_ptr);
 int32_t dlrmb_xbuf_close(int32_t device, void* peer_ptr);
 int32_t dlrmb_tables_set_slot_map(dlrmb_tables* t, const int32_t* slots);
+/* Destination map of the p2p lookups for column-wise sharded tables (dlrmb_shard_plan_cw): local table k's pooled
+ * row of sample b lands at columns [col0[k], col0[k] + D) of slot slots[k] in destination rows of `D_dest` floats
+ * per slot, i.e. at peer_T[h] + b_local * slots_arg * D_dest + slots[k] * D_dest + col0[k] (slots_arg: the `slots`
+ * argument of the lookup call).  col0[k] + D <= D_dest.  dlrmb_tables_set_slot_map(t, s) is the map with col0 = 0
+ * and D_dest = D; a later call of either replaces the map.  The 16-byte store path needs D, D_dest and every
+ * col0 to be multiples of 4 (and 16-byte aligned peer_T); otherwise the lookups store one float at a time. */
+int32_t dlrmb_tables_set_dest_map(dlrmb_tables* t, const int32_t* slots, const int32_t* col0, int32_t D_dest);
 int32_t dlrmb_embedding_fwd_p2p(dlrmb_tables* t, const void* idx, int32_t idx_bytes, int32_t idx_base,
                                 int32_t B_global, int32_t P, float* const* peer_T, int32_t world,
                                 int32_t B_local, int32_t slots, dlrmb_stream stream);
@@ -316,6 +323,14 @@ int32_t dlrmb_indices_scatter_p2p(int32_t device, const void* idx_local, int32_t
 int32_t dlrmb_indices_scatter_p2p_mp(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
                                      int32_t B_local, const int32_t* P, const void* const* dests_dev, int32_t rank,
                                      dlrmb_stream stream);
+/* Column-wise sharding: a split table's block goes to every rank holding one of its slices.  Destination i
+ * (0 <= i < ndest <= 1024) receives global table dest_table[i]'s block (`dest_table` a host array) at
+ * dests_dev[i] + rank * B_local * P_k indices, i.e. rows [rank * B_local, (rank + 1) * B_local) of that holder's
+ * [B_global][P_k] block; idx_local and P as for dlrmb_indices_scatter_p2p_mp.  One launch for every destination;
+ * no allocation; graph-capturable. */
+int32_t dlrmb_indices_scatter_p2p_mp_list(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
+                                          int32_t B_local, const int32_t* P, int32_t ndest, const int32_t* dest_table,
+                                          const void* const* dests_dev, int32_t rank, dlrmb_stream stream);
 
 /* Interaction backward fused with the gradient exchange: as dlrmb_interaction_bwd, but the gradient
  * row of feature slot f >= 1 of local sample b is stored at
@@ -332,6 +347,15 @@ int32_t dlrmb_interaction_bwd_scatter(int32_t device, const float* dOut, const f
                                       int32_t F, int32_t d, int32_t pad_to_mul,
                                       const dlrmb_slot_dest* dests, int64_t sample_offset, float* dx,
                                       dlrmb_stream stream);
+/* Column pieces (column-wise sharded tables): `dests` is a DEVICE array [F][Q] and entry (f, q) receives columns
+ * [q * d / Q, (q + 1) * d / Q) of slot f's gradient row, at
+ *   dests[f * Q + q].base + (sample_offset + b) * dests[f * Q + q].sample_stride + dests[f * Q + q].offset
+ * (floats; the offset addresses the piece's first column).  A slot held whole gets Q entries pointing at
+ * consecutive column ranges of one row.  Q a power of two in 1..32, d / Q a multiple of 4; Q = 1 is
+ * dlrmb_interaction_bwd_scatter.  Same products in the same order: the pieces carry the bits of dT. */
+int32_t dlrmb_interaction_bwd_scatter_cols(int32_t device, const float* dOut, const float* T, int32_t B,
+                                           int32_t F, int32_t d, int32_t pad_to_mul, const dlrmb_slot_dest* dests,
+                                           int32_t Q, int64_t sample_offset, float* dx, dlrmb_stream stream);
 
 /* ---- collectives of the sharded path (new functionality; one process per GPU, NCCL over NVLink).
  * A non-Python host runs BASELINE config 4 with these: rank 0 calls dlrmb_comm_unique_id, carries the 128
@@ -359,10 +383,26 @@ int32_t dlrmb_interaction_bwd_scatter(int32_t device, const float* dOut, const f
  *                            rank's tables (ascending global id) at B_global: table j's [B_global][P_j] block
  *                            starts at B_global * (sum of P_i of the owned tables before it), rank h's samples
  *                            are its rows [h * B_local, (h + 1) * B_local).  dlrmb_embedding_fwd_mp /
- *                            _sort_mp / _bwd_sgd_mp read it with the owned tables' P as is. */
+ *                            _sort_mp / _bwd_sgd_mp read it with the owned tables' P as is.
+ * The a2a calls take one owner per table, so they serve table-wise plans only; a column-wise plan
+ * (dlrmb_shard_plan_cw below) goes through the peer-store exchanges.
+ * Column-wise sharding of hot tables (S = max_col_shards, a power of two; D / S a multiple of 4 when S > 1):
+ *   dlrmb_shard_plan_cw      shards[k] = c_k, the number of column slices of table k (a power of two <= min(S,
+ *                            world)); owner[k * S + j] = rank holding slice j, columns [j * D / c_k, (j + 1) * D / c_k),
+ *                            -1 for j >= c_k.  Rule: start with every c_k = 1; repeatedly take the table with the
+ *                            largest P_k / c_k (ties: more rows, then lower id) and double its c_k, until
+ *                            P_k * world <= c_k * sum(P) or 2 * c_k > min(S, world).  Nothing split: exactly
+ *                            dlrmb_shard_plan_mp's owners in owner[k * S].  Otherwise the slices are dealt longest
+ *                            first (descending P_k / c_k, then rows, then k, then j), each to the rank with the
+ *                            smallest sum of P_k / c_k so far among those holding no slice of k (ties: fewer
+ *                            rows * D / c_k, then the lower rank).  Column j of a pooled row is an ordered sum of
+ *                            column j of the rows it gathers, so a slice's holder produces exactly the columns the
+ *                            whole-table lookup would. */
 typedef struct dlrmb_comm dlrmb_comm;
 int32_t dlrmb_shard_plan(int32_t ntab, const int64_t* rows, int32_t world, int32_t* owner);
 int32_t dlrmb_shard_plan_mp(int32_t ntab, const int64_t* rows, const int32_t* P, int32_t world, int32_t* owner);
+int32_t dlrmb_shard_plan_cw(int32_t ntab, const int64_t* rows, const int32_t* P, int32_t world, int32_t D, int32_t S,
+                            int32_t* shards, int32_t* owner);
 int32_t dlrmb_comm_unique_id(uint8_t* id128);
 int32_t dlrmb_comm_create(int32_t device, const uint8_t* id128, int32_t rank, int32_t world, dlrmb_comm** out);
 int32_t dlrmb_comm_destroy(dlrmb_comm* c);
