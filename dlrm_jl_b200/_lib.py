@@ -25,6 +25,7 @@ class DLRMB200Error(RuntimeError):
 _i32, _i64, _f32, _vp = C.c_int32, C.c_int64, C.c_float, C.c_void_p
 _idx_args = [_vp, _i32, _i32, _i32, _i32]  # idx, idx_bytes, idx_base, B, P
 _idx_mp_args = [_vp, _i32, _i32, _i32, C.POINTER(_i32)]  # idx, idx_bytes, idx_base, B, P[ntab]
+_idx_jagged_args = [_vp, _vp, _i32, _i32, _i32, C.POINTER(_i64)]  # values, offsets, idx_bytes, idx_base, B, L[ntab]
 
 # name -> (restype, argtypes); every symbol include/dlrm_b200.h declares
 SIGNATURES = {
@@ -111,6 +112,10 @@ SIGNATURES = {
     "dlrmb_check_indices_mp": (_i32, [_vp, *_idx_mp_args, _i32]),
     "dlrmb_embedding_fwd_mp_host": (_i32, [_vp, *_idx_mp_args, _vp, _i32, _i32]),
     "dlrmb_embedding_bwd_sgd_mp_host": (_i32, [_vp, *_idx_mp_args, _vp, _i32, _i32, _f32]),
+    "dlrmb_embedding_fwd_jagged": (_i32, [_vp, *_idx_jagged_args, _i32, _vp, _i32, _i32, _vp]),
+    "dlrmb_embedding_fwd_sort_jagged": (_i32, [_vp, *_idx_jagged_args, _i32, _vp, _i32, _i32, _vp]),
+    "dlrmb_embedding_sort_jagged": (_i32, [_vp, *_idx_jagged_args, _i32, _vp]),
+    "dlrmb_check_indices_jagged": (_i32, [_vp, *_idx_jagged_args, _i32]),
 }
 
 _lib: Optional[C.CDLL] = None

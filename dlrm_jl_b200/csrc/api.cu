@@ -5,6 +5,7 @@
 #include <string.h>
 
 #include <mutex>
+#include <vector>
 
 #include "common.cuh"
 
@@ -699,7 +700,37 @@ static int64_t mp_index_count(const MpGeom& g) { return (int64_t)g.off[g.ntab - 
 void mark_sorted(dlrmb_tables* t, const MpGeom& g, int k0) {
     t->sorted_B = (int)g.B;
     for (int k = 0; k < g.ntab; ++k) t->h_sorted_P[k0 + k] = (int32_t)g.P[k];
+    t->sorted_jagged = -1;
     t->sorted_valid = k0 + g.ntab == t->ntab;
+}
+
+// Host-only checks (no CUDA call, so they also refuse bad arguments on a machine without a GPU).
+int check_jagged_args(const dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                      int B, const int64_t* L, int pooling, MpGeom* g) {
+    DLRMB_REQUIRE(offsets != nullptr, "offsets is null");
+    DLRMB_REQUIRE(L != nullptr, "L (per-table lookup counts) is null");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(idx_base == 0 || idx_base == 1, "idx_base must be 0 or 1 (got %d)", idx_base);
+    DLRMB_REQUIRE(pooling == 0 || pooling == 1, "pooling must be 0 (sum) or 1 (mean) (got %d)", pooling);
+    DLRMB_REQUIRE(B > 0, "B must be positive (got %d)", B);
+    DLRMB_REQUIRE(t != nullptr, "null tables handle");
+    DLRMB_REQUIRE(t->ntab <= kMpMaxTables, "jagged batches support up to %d tables (handle has %d)", kMpMaxTables,
+                  t->ntab);
+    int64_t off = 0;
+    for (int k = 0; k < t->ntab; ++k) {
+        DLRMB_REQUIRE(L[k] >= 0, "L[%d] = %lld: lookup counts must be >= 0", k, (long long)L[k]);
+        DLRMB_REQUIRE(L[k] <= t->max_lookups, "L[%d] = %lld exceeds max_lookups = %lld", k, (long long)L[k],
+                      (long long)t->max_lookups);
+        g->P[k] = (uint32_t)L[k];
+        g->off[k] = off;
+        off += L[k];
+    }
+    DLRMB_REQUIRE(values != nullptr || off == 0, "values is null");
+    DLRMB_REQUIRE(idx_bytes == 8 || off <= INT32_MAX, "%lld lookups need 8-byte offsets", (long long)off);
+    g->ntab = t->ntab;
+    g->B = 1;
+    g->nlist = 0;
+    return DLRMB_OK;
 }
 
 dlrmb_tables table_group(const dlrmb_tables& t, int k0, int n) {
@@ -793,6 +824,105 @@ int32_t dlrmb_check_indices_mp(dlrmb_tables* t, const void* idx, int32_t idx_byt
     if (bt >= 0) {
         set_error("index out of range: table %lld, flat position %lld, value %lld not in [%d, %lld]",
                   bt, bp, bv, idx_base, (long long)t->h_rows[bt] - 1 + idx_base);
+        return DLRMB_EOOB;
+    }
+    return DLRMB_OK;
+}
+
+// ---- jagged (variable-length) bags -----------------------------------------------------------------------------
+static int jagged_fwd(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base, int B,
+                      const int64_t* L, int pooling, float* out, int slots, int slot0, dlrmb_stream stream, bool sort) {
+    MpGeom g;
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, pooling, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(out != nullptr, "out is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
+                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
+    GUARD(t);
+    if (sort) t->sorted_valid = false;
+    rc = launch_lookup_jagged(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, (cudaStream_t)stream);
+    if (rc || !sort) return rc;
+    return dlrmb_embedding_sort_jagged(t, values, offsets, idx_bytes, idx_base, B, L, pooling, stream);
+}
+
+int32_t dlrmb_embedding_fwd_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                   int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream, false);
+}
+
+int32_t dlrmb_embedding_fwd_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                        int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                        int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream, true);
+}
+
+int32_t dlrmb_embedding_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                    int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, dlrmb_stream stream) {
+    MpGeom g;
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, pooling, &g);
+    if (rc) return rc;
+    GUARD(t);
+    t->sorted_valid = false;
+    const int half = sort_mp_final_half(t, g);
+    rc = launch_sort_mp(t, values, idx_bytes, idx_base, g, 0, half, (cudaStream_t)stream);
+    if (rc) return rc;
+    rc = launch_jagged_bags(t, offsets, idx_bytes, g, B, pooling, half, (cudaStream_t)stream);
+    if (rc) return rc;
+    mark_sorted(t, g, 0);
+    t->sorted_jagged = pooling;
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_check_indices_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t on_host) {
+    MpGeom g;
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, 0, &g);
+    if (rc) return rc;
+    GUARD(t);
+    const int64_t noff = (int64_t)t->ntab * B + 1;
+    const int64_t nval = g.off[t->ntab - 1] + g.P[t->ntab - 1];
+    // the offsets on the host, widened to int64
+    std::vector<char> raw;
+    const void* src = offsets;
+    if (!on_host) {
+        DLRMB_CUDA(cudaDeviceSynchronize());
+        raw.resize((size_t)noff * idx_bytes);
+        DLRMB_CUDA(cudaMemcpy(raw.data(), offsets, raw.size(), cudaMemcpyDeviceToHost));
+        src = raw.data();
+    }
+    std::vector<int64_t> ho((size_t)noff);
+    for (int64_t i = 0; i < noff; ++i)
+        ho[i] = idx_bytes == 4 ? (int64_t)static_cast<const uint32_t*>(src)[i] : static_cast<const int64_t*>(src)[i];
+    DLRMB_REQUIRE(ho[0] == 0, "offsets[0] = %lld: the first offset must be 0", (long long)ho[0]);
+    for (int64_t i = 0; i + 1 < noff; ++i)
+        DLRMB_REQUIRE(ho[i] <= ho[i + 1], "offsets decrease at table %lld, bag %lld: offsets[%lld] = %lld > offsets[%lld] = %lld",
+                      (long long)(i / B), (long long)(i % B), (long long)i, (long long)ho[i], (long long)(i + 1),
+                      (long long)ho[i + 1]);
+    for (int k = 0; k < t->ntab; ++k) {
+        const int64_t n = ho[(int64_t)(k + 1) * B] - ho[(int64_t)k * B];
+        DLRMB_REQUIRE(n == (int64_t)g.P[k], "table %d: offsets give %lld lookups, L[%d] = %lld", k, (long long)n, k,
+                      (long long)g.P[k]);
+    }
+    const void* d_val = values;
+    if (on_host && nval > 0) {
+        rc = grow(&t->stage_idx, &t->stage_idx_bytes, (size_t)nval * idx_bytes);
+        if (rc) return rc;
+        DLRMB_CUDA(cudaMemcpyAsync(t->stage_idx, values, (size_t)nval * idx_bytes, cudaMemcpyHostToDevice, t->own_stream));
+        d_val = t->stage_idx;
+    }
+    long long bt = -1, bp = -1, bv = 0;
+    if (nval > 0) {
+        rc = launch_check_indices_mp(t, d_val, idx_bytes, idx_base, g, t->own_stream, &bt, &bp, &bv);
+        if (rc) return rc;
+    }
+    if (bt >= 0) {
+        // the bag of the offender: the last bag of table bt that starts at or before it
+        const int64_t x = g.off[bt] + bp;
+        int64_t b = 0;
+        while (b + 1 < B && ho[bt * B + b + 1] <= x) ++b;
+        set_error("index out of range: table %lld, bag %lld, position %lld of the table's values, value %lld not in [%d, %lld]",
+                  bt, (long long)b, bp, bv, idx_base, (long long)t->h_rows[bt] - 1 + idx_base);
         return DLRMB_EOOB;
     }
     return DLRMB_OK;

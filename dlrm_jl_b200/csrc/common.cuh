@@ -220,7 +220,9 @@ struct dlrmb_tables {
     // state of the last sort
     bool sorted_valid = false;
     int sorted_B = 0;
-    int32_t* h_sorted_P = nullptr;            // [ntab], host: P_k of every table
+    int32_t* h_sorted_P = nullptr;            // [ntab], host: P_k of every table (L_k after a jagged sort, sorted_B = 1)
+    int sorted_jagged = -1;                   // -1: uniform or _mp sort; 0 / 1: jagged sort with sum / mean pooling,
+                                              // bag ids (and mean weights) in pos / keys [sorted_buf ^ 1]
 
     // host-entry-point staging (device side), grown on demand
     void* stage_idx = nullptr;  size_t stage_idx_bytes = 0;
@@ -279,6 +281,18 @@ void mark_sorted(dlrmb_tables* t, const MpGeom& g, int k0);
 dlrmb_tables table_group(const dlrmb_tables& t, int k0, int n);
 // gather CTAs per table of an `_mp` lookup (fills g.pre); returns the total
 int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift);
+// Jagged (variable-length) bags, the `_jagged` entry points.  The sort geometry is the `_mp` one with B = 1,
+// P[k] = L_k and off[k] = L_0 + .. + L_{k-1}: a table's block is sorted as one bag of L_k lookups.  The lookup
+// and the position -> bag pass also read the batch's B and the offsets [ntab * B + 1] (element offsets into
+// `values`, same width as the indices).
+int check_jagged_args(const dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                      int B, const int64_t* L, int pooling, MpGeom* g);
+int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                         const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s);
+// after a jagged sort into half `half`: bag id (and, with mean pooling, weight 1/n as f32 bits) of every sorted
+// entry into pos[half ^ 1] (and keys[half ^ 1])
+int launch_jagged_bags(dlrmb_tables* t, const void* offsets, int idx_bytes, const MpGeom& g, int B, int pooling,
+                       int half, cudaStream_t s);
 // lookups of table k in the last sort
 static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) { return (int64_t)t->sorted_B * t->h_sorted_P[k]; }
 

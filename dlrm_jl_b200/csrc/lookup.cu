@@ -28,6 +28,9 @@ template <> struct Vec<4> {
     static __device__ __forceinline__ float4 add(float4 a, float4 b) {
         return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
     }
+    static __device__ __forceinline__ float4 scale(float4 a, float w) {
+        return make_float4(__fmul_rn(a.x, w), __fmul_rn(a.y, w), __fmul_rn(a.z, w), __fmul_rn(a.w, w));
+    }
 };
 template <> struct Vec<1> {
     using type = float;
@@ -37,6 +40,7 @@ template <> struct Vec<1> {
     }
     static __device__ __forceinline__ float zero() { return 0.f; }
     static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
+    static __device__ __forceinline__ float scale(float a, float w) { return __fmul_rn(a, w); }
 };
 
 // P == 1: plain gather.  U independent chains per thread.  `cta` of `nctas` CTAs of 256 threads share
@@ -75,6 +79,35 @@ __device__ __forceinline__ void lookup_gather_body(const TableDesc* __restrict__
         for (int u = 0; u < U; ++u)
             if (ok[u]) reinterpret_cast<V*>(ob + (size_t)b[u] * ostride)[c[u]] = v[u];
     }
+}
+
+// Sum of chunk c of the rows ip[0 .. n) (fp32, from +0.0f, ascending), four row loads in flight: the loop of
+// lookup_pool_body (which keeps its own copy: calling this helper there changes the VEC = 1 kernels' SASS).
+template <typename IdxT, int VEC, typename RowT>
+__device__ __forceinline__ typename Vec<VEC>::type pool_bag(const float* __restrict__ tb, const IdxT* __restrict__ ip,
+                                                            uint32_t n, int idx_base, size_t D, uint32_t c) {
+    using V = typename Vec<VEC>::type;
+    V acc = Vec<VEC>::zero();
+    uint32_t p = 0;
+    for (; p + 4 <= n; p += 4) {
+        int64_t r0 = (int64_t)__ldg(ip + p) - idx_base;
+        int64_t r1 = (int64_t)__ldg(ip + p + 1) - idx_base;
+        int64_t r2 = (int64_t)__ldg(ip + p + 2) - idx_base;
+        int64_t r3 = (int64_t)__ldg(ip + p + 3) - idx_base;
+        V v0 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r0, D, c);
+        V v1 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r1, D, c);
+        V v2 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r2, D, c);
+        V v3 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r3, D, c);
+        acc = Vec<VEC>::add(acc, v0);
+        acc = Vec<VEC>::add(acc, v1);
+        acc = Vec<VEC>::add(acc, v2);
+        acc = Vec<VEC>::add(acc, v3);
+    }
+    for (; p < n; ++p) {
+        int64_t r = (int64_t)__ldg(ip + p) - idx_base;
+        acc = Vec<VEC>::add(acc, Vec<VEC>::template ldrow<RowT>(tb, (size_t)r, D, c));
+    }
+    return acc;
 }
 
 // P > 1: gather + sum-pool, ascending p.
@@ -291,6 +324,101 @@ int launch_lookup_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int i
 #undef DLRMB_LSMP
     if (rc) return rc;
     return launch_sort_mp(t, idx, idx_bytes, idx_base, g, kFusedSortMax, half, s);
+}
+
+// ---- jagged (variable-length) bags ----------------------------------------------------------------
+// One flat grid as lookup_mp_kernel: table k owns CTAs [g.pre[k], g.pre[k+1]) (lookup_grid_jagged), a thread
+// owns one (bag, 16-byte chunk), reads the bag's two offsets and pools values[o0 .. o1) with pool_bag.  MEAN
+// scales the sum by w = fl(1 / n); an empty bag stores +0.0f in both modes.
+template <typename IdxT, int VEC, typename RowT, bool MEAN>
+__global__ void __launch_bounds__(256)
+lookup_jagged_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ values, const IdxT* __restrict__ offsets,
+                     int idx_base, const __grid_constant__ MpGeom g, uint32_t B, uint32_t C, int cshift,
+                     float* __restrict__ out, int slots, int slot0, unsigned long long* clk) {
+    using V = typename Vec<VEC>::type;
+    clock_in(clk, blockIdx.x);
+    const int k = mp_find(g.pre, g.ntab, blockIdx.x);
+    const uint32_t cta = blockIdx.x - g.pre[k], nctas = g.pre[k + 1] - g.pre[k];
+    const float* __restrict__ tb = desc[k].base;
+    const IdxT* __restrict__ ok = offsets + (size_t)k * B;
+    const uint32_t n = B * C;
+    const uint32_t step = nctas * blockDim.x;
+    const size_t D = (size_t)C * VEC;
+    float* __restrict__ ob = out + (size_t)(slot0 + k) * D;
+    const size_t ostride = (size_t)slots * D;
+    for (uint32_t t = cta * blockDim.x + threadIdx.x; t < n; t += step) {
+        const uint32_t b = cshift >= 0 ? (t >> cshift) : (t / C);
+        const uint32_t c = t - b * C;
+        const int64_t o0 = (int64_t)__ldg(ok + b), o1 = (int64_t)__ldg(ok + b + 1);
+        V acc = pool_bag<IdxT, VEC, RowT>(tb, values + o0, (uint32_t)(o1 - o0), idx_base, D, c);
+        if (MEAN && o1 > o0) acc = Vec<VEC>::scale(acc, __fdiv_rn(1.0f, (float)(o1 - o0)));
+        reinterpret_cast<V*>(ob + (size_t)b * ostride)[c] = acc;
+    }
+    clock_out(clk, blockIdx.x);
+}
+
+// CTAs per table: the lookup_grid_mp budget split in proportion to the table's gathered rows plus its output rows,
+// (L_k + B) * C, so a table of long bags is not the tail; at least one per table (its B rows are written even
+// when L_k = 0) and no more than it has work items for.
+static int64_t lookup_grid_jagged(const dlrmb_tables* t, MpGeom& g, uint32_t B, uint32_t C) {
+    int64_t sumw = 0;
+    for (int k = 0; k < g.ntab; ++k) sumw += (int64_t)g.P[k] + B;
+    const int64_t budget = (int64_t)t->sm_count * 32;
+    const int64_t most = ceil_div64((int64_t)B * C, 256);
+    int64_t total = 0;
+    for (int k = 0; k < g.ntab; ++k) {
+        int64_t c = ceil_div64(budget * ((int64_t)g.P[k] + B), sumw);
+        if (c > most) c = most;
+        if (c < 1) c = 1;
+        g.pre[k] = (uint32_t)total;
+        total += c;
+    }
+    g.pre[g.ntab] = (uint32_t)total;
+    return total;
+}
+
+template <typename IdxT, int VEC, typename RowT>
+static int launch_lookup_jagged_t(dlrmb_tables* t, const IdxT* values, const IdxT* offsets, int idx_base,
+                                  const MpGeom& g0, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+    const uint32_t C = t->D / VEC;
+    const int64_t n = (int64_t)B * C;
+    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
+    MpGeom g = g0;
+    const int64_t ctas = lookup_grid_jagged(t, g, (uint32_t)B, C);
+    int cshift = -1;
+    if ((C & (C - 1)) == 0)
+        for (cshift = 0; (1u << cshift) < C; ++cshift) {}
+    if (pooling == 1)
+        lookup_jagged_kernel<IdxT, VEC, RowT, true><<<(unsigned)ctas, 256, 0, s>>>(
+            t->d_desc, values, offsets, idx_base, g, (uint32_t)B, C, cshift, out, slots, slot0, clock_slot(CLK_LOOKUP));
+    else
+        lookup_jagged_kernel<IdxT, VEC, RowT, false><<<(unsigned)ctas, 256, 0, s>>>(
+            t->d_desc, values, offsets, idx_base, g, (uint32_t)B, C, cshift, out, slots, slot0, clock_slot(CLK_LOOKUP));
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename RowT>
+static int launch_lookup_jagged_r(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                                  const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+    const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    if (idx_bytes == 4) {
+        const uint32_t* v = static_cast<const uint32_t*>(values);
+        const uint32_t* o = static_cast<const uint32_t*>(offsets);
+        return vec4 ? launch_lookup_jagged_t<uint32_t, 4, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s)
+                    : launch_lookup_jagged_t<uint32_t, 1, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s);
+    }
+    const int64_t* v = static_cast<const int64_t*>(values);
+    const int64_t* o = static_cast<const int64_t*>(offsets);
+    return vec4 ? launch_lookup_jagged_t<int64_t, 4, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s)
+                : launch_lookup_jagged_t<int64_t, 1, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s);
+}
+
+int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                         const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+    if (t->elem_bytes == 2)
+        return launch_lookup_jagged_r<__nv_bfloat16>(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, s);
+    return launch_lookup_jagged_r<float>(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, s);
 }
 
 // ---- ScaledUniform init (src/model/model.jl:61-65): U(-1/sqrt(rows), 1/sqrt(rows)) ------------

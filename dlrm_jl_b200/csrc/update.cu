@@ -52,6 +52,9 @@ template <> struct UV<4> {
         return make_float4(__fsub_rn(x.x, __fmul_rn(lr, g.x)), __fsub_rn(x.y, __fmul_rn(lr, g.y)),
                            __fsub_rn(x.z, __fmul_rn(lr, g.z)), __fsub_rn(x.w, __fmul_rn(lr, g.w)));
     }
+    static __device__ __forceinline__ float4 scale(float4 a, float w) {
+        return make_float4(__fmul_rn(a.x, w), __fmul_rn(a.y, w), __fmul_rn(a.z, w), __fmul_rn(a.w, w));
+    }
 };
 template <> struct UV<1> {
     using type = float;
@@ -60,6 +63,7 @@ template <> struct UV<1> {
     static __device__ __forceinline__ float sgd(float x, float g, float lr) {
         return __fsub_rn(x, __fmul_rn(lr, g));
     }
+    static __device__ __forceinline__ float scale(float a, float w) { return __fmul_rn(a, w); }
 };
 
 // table-row access in the row's storage type (f32 or bf16); chunk c = floats [c*VEC, c*VEC + VEC)
@@ -307,13 +311,16 @@ __device__ __forceinline__ void fixup_runs_smem(const TableDesc* __restrict__ de
 // (INLINE path; zero between launches).
 // Chunk `cta` of table k (gm: that table's geometry).  `gid` names the chunk in the two-launch head list,
 // `ndone` is the table's chunk count (the INLINE done-counter target), `clk_cta` its stamp slot.
-template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE>
+// SCALE (jagged mean pooling): each gradient row is multiplied by its entry's weight `wts` (f32 bits, the
+// stream's layout) before it is accumulated.
+template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE, bool SCALE = false>
 __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
                                                   const uint32_t* __restrict__ pos, const float* __restrict__ dT, float lr,
                                                   float* __restrict__ partial, uint8_t* __restrict__ flags,
                                                   uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count,
                                                   const UpdateGeom& gm, int k, int cta, uint32_t gid, uint32_t ndone,
-                                                  unsigned long long* clk, unsigned clk_cta) {
+                                                  unsigned long long* clk, unsigned clk_cta,
+                                                  const uint32_t* __restrict__ wts = nullptr) {
     using V = typename UV<VEC>::type;
     constexpr int U = 4;
     clock_in(clk, clk_cta);
@@ -335,6 +342,7 @@ __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ 
 
     const uint32_t* __restrict__ ks = keys + (size_t)k * gm.cap;
     const uint32_t* __restrict__ ps = pos + (size_t)k * gm.cap;
+    const uint32_t* __restrict__ ws = SCALE ? wts + (size_t)k * gm.cap : nullptr;
     float* tb = desc[k].base;
     const float* __restrict__ gbase = dT + (size_t)(gm.slot0 + k) * D;
     const size_t gstride = (size_t)gm.slots * D;
@@ -355,6 +363,8 @@ __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ 
         const int e1 = min(gm.L, e0 + gm.tile);
         uint4 kq = __ldg(reinterpret_cast<const uint4*>(ks + e0));
         uint4 pq = __ldg(reinterpret_cast<const uint4*>(ps + e0));
+        uint4 wq;
+        if (SCALE) wq = __ldg(reinterpret_cast<const uint4*>(ws + e0));
         uint32_t kn = (e0 + U < gm.L) ? __ldg(ks + e0 + U) : 0xffffffffu;
         const uint32_t kprev = (e0 > 0) ? __ldg(ks + e0 - 1) : 0xffffffffu;
         const bool cin = e0 > 0 && kprev == kq.x;
@@ -365,9 +375,11 @@ __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ 
         for (int e = e0; e < e1; e += U) {
             const uint32_t key[U + 1] = {kq.x, kq.y, kq.z, kq.w, kn};
             const uint32_t pp[U] = {pq.x, pq.y, pq.z, pq.w};
+            const uint32_t wb[U] = {SCALE ? wq.x : 0u, SCALE ? wq.y : 0u, SCALE ? wq.z : 0u, SCALE ? wq.w : 0u};
             if (e + U < e1) {   // request the next batch's keys / positions now
                 kq = __ldg(reinterpret_cast<const uint4*>(ks + e + U));
                 pq = __ldg(reinterpret_cast<const uint4*>(ps + e + U));
+                if (SCALE) wq = __ldg(reinterpret_cast<const uint4*>(ws + e + U));
                 kn = (e + 2 * U < gm.L) ? __ldg(ks + e + 2 * U) : 0xffffffffu;
             }
             bool valid[U], is_end[U];
@@ -400,7 +412,7 @@ __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ 
                 if (!valid[u]) continue;
 #pragma unroll
                 for (int m = 0; m < NCH; ++m)
-                    if (chunk_ok[m]) acc[m] = UV<VEC>::add(acc[m], dv[u][m]);
+                    if (chunk_ok[m]) acc[m] = UV<VEC>::add(acc[m], SCALE ? UV<VEC>::scale(dv[u][m], __uint_as_float(wb[u])) : dv[u][m]);
                 if (is_end[u]) {
                     if (first) {
                         // run started in an earlier tile: hand the partial sum to its owner
@@ -632,6 +644,26 @@ update_fixup_mp_kernel(const TableDesc* __restrict__ desc, const uint32_t* __res
     clock_out(clk, blockIdx.x);
 }
 
+// ---- jagged bags: the `_mp` flat grid over a stream of bag ids (P = 1) with per-table L_k (g.P[k] = L_k, g.B = 1,
+// as the jagged sort records them); tables with L_k = 0 own no chunk, and mp_find skips them (it returns the last
+// table whose range starts at or before the CTA).  The two-launch fix-up is update_fixup_mp_kernel's: it reads no
+// position.
+template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE, bool SCALE>
+__global__ void __launch_bounds__(THREADS, (NCH <= 1) ? 3 : ((NCH <= 2) ? 2 : 1))
+update_tiles_jagged_kernel(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
+                           const uint32_t* __restrict__ bags, const uint32_t* __restrict__ wts, const float* __restrict__ dT,
+                           float lr, float* __restrict__ partial, uint8_t* __restrict__ flags,
+                           uint32_t* __restrict__ head_list, uint32_t* __restrict__ head_count, UpdateGeom gm0,
+                           const __grid_constant__ MpGeom g, unsigned long long* clk) {
+    const uint32_t lin = blockIdx.x;
+    const int k = mp_find(g.pre, g.ntab, lin);
+    UpdateGeom gm = update_geom_mp(gm0, g, k);
+    gm.P = 1;
+    update_tiles_body<VEC, NCH, THREADS, RowT, INLINE, SCALE>(desc, keys, bags, dT, lr, partial, flags, head_list, head_count,
+                                                              gm, k, (int)(lin - g.pre[k]), lin, (uint32_t)gm.chunks, clk,
+                                                              lin, wts);
+}
+
 static int lanes_per_row_log2(int C) {
     int l = 0;
     while ((1 << l) < C && l < 5) ++l;
@@ -669,7 +701,9 @@ int64_t update_tiles_cap(int ntab, int D, int64_t max_lookups, int sm_count) {
 // Consumes the last sort (B and every table's P_k).  With equal P_k the tables share one geometry and the grid
 // is two-dimensional (grid.y = table); otherwise one flat grid of sum_k chunks_k CTAs, g.pre mapping a CTA to
 // (table, chunk).  The tile is chosen from the total entry count either way, so equal P_k take the same tiles
-// and chunks on both grids, hence the same bits.
+// and chunks on both grids, hence the same bits.  A jagged sort (g.B = 1, P_k = L_k) takes the flat grid with
+// update_tiles_jagged_kernel over the bag ids (and, for mean pooling, the weights) that launch_jagged_bags wrote into
+// pos / keys [sorted_buf ^ 1]; the fix-up kernel is the same for both, it reads no position.
 template <int VEC, int NCH, typename RowT>
 static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
     constexpr int THREADS = (NCH > 4) ? 128 : 256;   // keeps the two partial arrays within 48 KB
@@ -702,7 +736,8 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
     // DLRM-sized batches: level 3 runs inside the same launch (see the header comment)
     const bool inline_fixup = total <= kUpdateInlineMaxEntries &&
                               g_opt.update_two_launches.load(std::memory_order_relaxed) == 0;
-    if (equal) {
+    const int jagged = t->sorted_jagged;   // -1: uniform or _mp sort, 0 / 1: jagged sum / mean
+    if (equal && jagged < 0) {
         gm.L = (int)maxL;
         gm.P = P[0];
         gm.tiles = (gm.L + gm.tile - 1) / gm.tile;
@@ -728,7 +763,7 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
         DLRMB_LAUNCH_CHECK();
         return DLRMB_OK;
     }
-    // mixed P_k: only the `_mp` sorts, at most kMpMaxTables tables
+    // mixed P_k or jagged: only the `_mp` and jagged sorts, at most kMpMaxTables tables
     MpGeom g;
     g.ntab = t->ntab;
     g.B = (uint32_t)t->sorted_B;
@@ -751,15 +786,32 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
     }
     g.pre[t->ntab] = (uint32_t)chunks_total;
     DLRMB_REQUIRE(chunks_total < (1ll << 31), "batch too large for one update launch");
+    if (chunks_total == 0) return DLRMB_OK;   // a jagged batch without lookups
+    const uint32_t* bags = t->pos[t->sorted_buf ^ 1];
+    const uint32_t* wts = t->keys[t->sorted_buf ^ 1];
+    auto tiles = [&](auto inl) {
+        constexpr bool INL = decltype(inl)::value;
+        const unsigned n = (unsigned)chunks_total;
+        if (jagged == 1)
+            update_tiles_jagged_kernel<VEC, NCH, THREADS, RowT, INL, true><<<n, THREADS, 0, s>>>(
+                t->d_desc, keys, bags, wts, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g,
+                clock_slot(CLK_UPDATE));
+        else if (jagged == 0)
+            update_tiles_jagged_kernel<VEC, NCH, THREADS, RowT, INL, false><<<n, THREADS, 0, s>>>(
+                t->d_desc, keys, bags, wts, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g,
+                clock_slot(CLK_UPDATE));
+        else
+            update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, INL><<<n, THREADS, 0, s>>>(
+                t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g,
+                clock_slot(CLK_UPDATE));
+    };
     if (inline_fixup) {
-        update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, true><<<(unsigned)chunks_total, THREADS, 0, s>>>(
-            t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g, clock_slot(CLK_UPDATE));
+        tiles(std::true_type{});
         DLRMB_LAUNCH_CHECK();
         return DLRMB_OK;
     }
     DLRMB_CUDA(cudaMemsetAsync(t->head_count, 0, sizeof(uint32_t), s));
-    update_tiles_mp_kernel<VEC, NCH, THREADS, RowT, false><<<(unsigned)chunks_total, THREADS, 0, s>>>(
-        t->d_desc, keys, pos, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g, clock_slot(CLK_UPDATE));
+    tiles(std::false_type{});
     DLRMB_LAUNCH_CHECK();
     unsigned fgrid = (unsigned)(chunks_total < (int64_t)t->sm_count * 8 ? chunks_total : (int64_t)t->sm_count * 8);
     update_fixup_mp_kernel<VEC, NCH, RowT><<<fgrid, 256, 0, s>>>(t->d_desc, keys, lr, t->partial, t->tile_flags,

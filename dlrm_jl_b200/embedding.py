@@ -74,6 +74,105 @@ class PackedIndices:
         return PackedIndices(self.flat.to(device, non_blocking=non_blocking).contiguous(), self.P, self.B)
 
 
+_POOLING = {"sum": 0, "mean": 1}
+
+
+@dataclass(frozen=True, eq=False)
+class JaggedIndices:
+    """Variable-length bags (the input of ``torch.nn.EmbeddingBag(input, offsets)`` and of the PyTorch DLRM's
+    ``(lS_o, lS_i)``), in TorchRec's key-major jagged layout: ``values`` holds every table's indices, table-major;
+    ``offsets`` [ntab * B + 1] (same dtype, 0-based, non-decreasing, offsets[0] = 0) makes bag b of table k
+    ``values[offsets[k*B + b] : offsets[k*B + b + 1]]``; the host tuple ``L`` holds each table's lookup count.
+    ``pooling`` is ``"sum"`` or ``"mean"`` (w = fl(1 / n) times the fp32 sum; an empty bag pools to zero).
+    ``jag[k]`` is table k's ``(values_k, offsets_k)`` with offsets_k rebased to 0."""
+    values: torch.Tensor
+    offsets: torch.Tensor
+    L: Tuple[int, ...]
+    B: int
+    pooling: str = "sum"
+
+    def __post_init__(self):
+        if self.pooling not in _POOLING:
+            raise ValueError(f"pooling must be 'sum' or 'mean', got {self.pooling!r}")
+        if self.values.dtype not in (torch.int32, torch.int64) or self.offsets.dtype != self.values.dtype:
+            raise ValueError(f"values and offsets must share one dtype, int32 or int64 (got {self.values.dtype} and "
+                             f"{self.offsets.dtype})")
+        if self.B <= 0 or self.offsets.dim() != 1 or self.offsets.numel() != len(self.L) * self.B + 1:
+            raise ValueError(f"offsets must hold ntab * B + 1 = {len(self.L) * self.B + 1} entries "
+                             f"(got {tuple(self.offsets.shape)})")
+        if any(n < 0 for n in self.L):
+            raise ValueError(f"lookup counts must be >= 0, got L = {self.L}")
+        if sum(self.L) != self.values.numel():
+            raise ValueError(f"the lookup counts sum to {sum(self.L)}, values holds {self.values.numel()}")
+
+    @classmethod
+    def from_lengths(cls, values, lengths, pooling: str = "sum") -> "JaggedIndices":
+        """``lengths[ntab][B]``: the size of every bag; ``values`` the bags' indices, table-major."""
+        v = values if isinstance(values, torch.Tensor) else torch.as_tensor(np.asarray(values))
+        v = _index_dtype(v.reshape(-1))
+        n = np.asarray(lengths.cpu() if isinstance(lengths, torch.Tensor) else lengths, dtype=np.int64)
+        if n.ndim != 2:
+            raise ValueError(f"lengths must be [ntab][B], got shape {n.shape}")
+        if (n < 0).any():
+            raise ValueError("bag lengths must be >= 0")
+        if int(n.sum()) != v.numel():
+            raise ValueError(f"the bag lengths sum to {int(n.sum())}, values holds {v.numel()}")
+        off = np.zeros(n.size + 1, dtype=np.int64)
+        np.cumsum(n.reshape(-1), out=off[1:])
+        offsets = torch.from_numpy(off).to(device=v.device, dtype=v.dtype)
+        return cls(v.contiguous(), offsets, tuple(int(x) for x in n.sum(axis=1)), int(n.shape[1]), pooling)
+
+    @classmethod
+    def from_bags(cls, bags, pooling: str = "sum", dtype: torch.dtype = torch.int64) -> "JaggedIndices":
+        """``bags[k][b]``: the indices of bag b of table k (any sequence, possibly empty)."""
+        Bs = {len(t) for t in bags}
+        if len(Bs) != 1:
+            raise ValueError(f"every table must have the same number of bags, got {[len(t) for t in bags]}")
+        lengths = [[len(bag) for bag in t] for t in bags]
+        flat = [int(i) for t in bags for bag in t for i in bag]
+        return cls.from_lengths(torch.tensor(flat, dtype=dtype), lengths, pooling)
+
+    @classmethod
+    def from_dense(cls, idx, pooling: str = "sum") -> "JaggedIndices":
+        """A fixed-width batch ([ntab][B][P] tensor or :class:`PackedIndices`) as bags of constant length."""
+        if isinstance(idx, PackedIndices):
+            return cls.from_lengths(idx.flat, [[p] * idx.B for p in idx.P], pooling)
+        t = _index_dtype(idx if isinstance(idx, torch.Tensor) else torch.as_tensor(np.asarray(idx)))
+        if t.dim() == 2:
+            t = t.unsqueeze(-1)
+        ntab, B, P = t.shape
+        return cls.from_lengths(t.reshape(-1), [[P] * B] * ntab, pooling)
+
+    def __len__(self) -> int:
+        return len(self.L)
+
+    def __getitem__(self, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        o = sum(self.L[:k])
+        return self.values[o:o + self.L[k]], self.offsets[k * self.B:(k + 1) * self.B + 1] - o
+
+    def L_array(self):
+        return (C.c_int64 * len(self.L))(*self.L)
+
+    def element_size(self) -> int:
+        return self.values.element_size()
+
+    @property
+    def pooling_code(self) -> int:
+        return _POOLING[self.pooling]
+
+    @property
+    def is_cuda(self) -> bool:
+        return self.values.is_cuda
+
+    @property
+    def device(self) -> torch.device:
+        return self.values.device
+
+    def to(self, device, non_blocking: bool = False) -> "JaggedIndices":
+        return JaggedIndices(self.values.to(device, non_blocking=non_blocking).contiguous(),
+                             self.offsets.to(device, non_blocking=non_blocking).contiguous(), self.L, self.B, self.pooling)
+
+
 def _index_dtype(t: torch.Tensor) -> torch.Tensor:
     if t.dtype in (torch.uint8, torch.int8, torch.int16):
         t = t.to(torch.int32)
@@ -104,7 +203,7 @@ def _as_index_tensor(sparse, ntab: int, device: torch.device):
     matrices given here as [B][P], or one [ntab][B] / [ntab][B][P] array) to a contiguous
     table-major device tensor [ntab][B][P] of int32 or int64.  A vector whose tables have different
     widths (the reference's load_inputs with per-table P = length / B) becomes :class:`PackedIndices`."""
-    if isinstance(sparse, PackedIndices):
+    if isinstance(sparse, (PackedIndices, JaggedIndices)):
         if len(sparse) != ntab:
             raise ValueError(f"indices must hold one array per table: {ntab} tables, got {len(sparse)}")
         return sparse.to(device, non_blocking=True)
@@ -127,7 +226,7 @@ def _as_index_tensor(sparse, ntab: int, device: torch.device):
 
 
 def _batch(idx) -> int:
-    return idx.B if isinstance(idx, PackedIndices) else idx.shape[1]
+    return idx.B if isinstance(idx, (PackedIndices, JaggedIndices)) else idx.shape[1]
 
 
 class _DevicePtrView:
@@ -228,6 +327,15 @@ class EmbeddingTables:
         sorts / dedups the indices for the sparse update of this batch (dlrmb_embedding_fwd_sort), so
         :meth:`update_sorted` can follow the backward pass without a sort launch."""
         slots = out.shape[1]
+        if isinstance(idx, JaggedIndices):   # variable-length bags
+            fn = self._lib.dlrmb_embedding_fwd_sort_jagged if sort else self._lib.dlrmb_embedding_fwd_jagged
+            assert out.is_contiguous() and out.dtype == torch.float32 and out.shape == (idx.B, slots, self.D)
+            with _prof.range("lookup"):
+                _lib.check(fn(self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.element_size(), idx_base, idx.B,
+                              idx.L_array(), idx.pooling_code, out.data_ptr(), slots, slot0, _stream_ptr(self.device)))
+            if sort:
+                self._pending_side = False
+            return
         if isinstance(idx, PackedIndices):   # per-table pooling factors
             B, P = idx.B, idx.P_array()
             fn = self._lib.dlrmb_embedding_fwd_sort_mp if sort else self._lib.dlrmb_embedding_fwd_mp
@@ -279,7 +387,12 @@ class EmbeddingTables:
     def sort(self, idx: torch.Tensor, idx_base: int = 0, side_stream: bool = False) -> None:
         """Index sort/dedup for the next update.  With ``side_stream`` it is issued on a second
         stream (it depends on the indices only) so it overlaps the forward/backward pass."""
-        if isinstance(idx, PackedIndices):
+        if isinstance(idx, JaggedIndices):
+            L, code, offs = idx.L_array(), idx.pooling_code, idx.offsets.data_ptr()
+            B, P, rec = idx.B, None, (idx.values, idx.offsets)
+            fn = lambda h, v, ib, base, B, _P, st: self._lib.dlrmb_embedding_sort_jagged(h, v, offs, ib, base, B, L, code, st)
+            idx = idx.values
+        elif isinstance(idx, PackedIndices):
             B, P, fn, rec = idx.B, idx.P_array(), self._lib.dlrmb_embedding_sort_mp, idx.flat
         else:
             (ntab, B, P), fn, rec = idx.shape, self._lib.dlrmb_embedding_sort, idx
@@ -293,7 +406,8 @@ class EmbeddingTables:
                     _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, B, P,
                                   self._side_stream.cuda_stream))
                 if not torch.cuda.is_current_stream_capturing():
-                    rec.record_stream(self._side_stream)
+                    for r in rec if isinstance(rec, tuple) else (rec,):
+                        r.record_stream(self._side_stream)
                 self._sorted_event.record(self._side_stream)
             self._pending_side = True
         else:
@@ -329,6 +443,11 @@ class EmbeddingTables:
 
     def check_indices(self, idx: torch.Tensor, idx_base: int = 0) -> None:
         on_host = 0 if idx.is_cuda else 1
+        if isinstance(idx, JaggedIndices):
+            _lib.check(self._lib.dlrmb_check_indices_jagged(
+                self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.element_size(), idx_base, idx.B, idx.L_array(),
+                on_host))
+            return
         if isinstance(idx, PackedIndices):
             _lib.check(self._lib.dlrmb_check_indices_mp(
                 self._h, idx.data_ptr(), idx.element_size(), idx_base, idx.B, idx.P_array(), on_host))
@@ -401,12 +520,14 @@ class SparseEmbeddingUpdate:
     parent: Optional[torch.Tensor] = None
     slot: int = -1
     idx_base: int = 0
+    pooling: str = "sum"        # jagged bags: ``indices`` is the table's (values_k, offsets_k)
 
 
 def sparse_updates(dT: torch.Tensor, indices: torch.Tensor, slot0: int, idx_base: int = 0) -> List[SparseEmbeddingUpdate]:
     """The lookup pullback: slice dT per table, no arithmetic (test/model/embedding_update.jl:36-40).
-    ``indices`` is the [ntab][B][P] tensor or :class:`PackedIndices`."""
-    return [SparseEmbeddingUpdate(dT[:, slot0 + k, :], indices[k], dT, slot0 + k, idx_base)
+    ``indices`` is the [ntab][B][P] tensor, :class:`PackedIndices` or :class:`JaggedIndices`."""
+    pooling = indices.pooling if isinstance(indices, JaggedIndices) else "sum"
+    return [SparseEmbeddingUpdate(dT[:, slot0 + k, :], indices[k], dT, slot0 + k, idx_base, pooling)
             for k in range(len(indices))]
 
 
@@ -414,6 +535,18 @@ def uncompress(update: SparseEmbeddingUpdate, nrows: int) -> torch.Tensor:
     """``EmbeddingTables.uncompress(update, nrows)`` (test/train/backprop.jl:156): the dense
     [nrows][D] gradient.  Debug/inspection helper (torch index_add_), not on the hot path."""
     B, D = update.delta.shape
+    if isinstance(update.indices, tuple):   # jagged bags: every lookup of bag b gets delta[b] (times 1/n for mean)
+        values, offsets = update.indices
+        n = (offsets[1:] - offsets[:-1]).to(torch.int64).to(update.delta.device)
+        delta = update.delta
+        if update.pooling == "mean":
+            w = torch.where(n > 0, 1.0 / n.clamp(min=1).to(torch.float32), torch.zeros((), dtype=torch.float32,
+                                                                                    device=delta.device))
+            delta = delta * w[:, None]
+        dense = torch.zeros((nrows, D), dtype=torch.float32, device=update.delta.device)
+        rows = values.to(torch.int64).to(update.delta.device) - update.idx_base
+        dense.index_add_(0, rows, delta.repeat_interleave(n, dim=0))
+        return dense
     idx = (update.indices.reshape(B, -1).to(torch.int64) - update.idx_base)
     P = idx.shape[1]
     dense = torch.zeros((nrows, D), dtype=torch.float32, device=update.delta.device)
@@ -442,7 +575,11 @@ def update_(opt: Descent, tables: EmbeddingTables, grads: Sequence[SparseEmbeddi
     else:  # updates built one by one (DefaultStrategy): pack into one [B][ntab][D] buffer
         dT = torch.stack([g.delta for g in grads], dim=1).contiguous()
         slot0 = 0
-    if not presorted:
+    if not presorted and isinstance(grads[0].indices, tuple):   # jagged bags
+        lengths = [(g.indices[1][1:] - g.indices[1][:-1]).cpu().numpy() for g in grads]
+        idx = JaggedIndices.from_lengths(torch.cat([g.indices[0] for g in grads]), lengths, grads[0].pooling)
+        tables.sort(idx.to(tables.device), grads[0].idx_base)
+    elif not presorted:
         idx = _as_index_tensor([g.indices.reshape(g.delta.shape[0], -1) for g in grads], tables.ntab, tables.device)
         tables.sort(idx, grads[0].idx_base)
     tables.update_sorted(dT, slot0, opt.eta)

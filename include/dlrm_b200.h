@@ -207,6 +207,42 @@ int32_t dlrmb_embedding_bwd_sgd_mp_host(dlrmb_tables* t, const void* idx, int32_
                                         int32_t B, const int32_t* P, const float* dT, int32_t slots, int32_t slot0,
                                         float lr);
 
+/* ---- jagged (variable-length) bags: the input of torch.nn.EmbeddingBag(input, offsets) and of the PyTorch DLRM's
+ * (lS_o offsets, lS_i indices), in TorchRec's key-major KeyedJaggedTensor layout.  Single GPU, every table of the
+ * handle, ntab <= dlrmb_mp_max_tables().
+ *   values   all tables' indices, one flat array, table-major; `idx_base` (0 or 1) applies to values only.
+ *   offsets  [ntab * B + 1] element offsets into values, non-decreasing, offsets[0] = 0, the same width as the
+ *            indices (idx_bytes 4 or 8): bag b of table k is values[offsets[k*B + b] .. offsets[k*B + b + 1]).
+ *   L        host [ntab], L[k] = offsets[(k+1)*B] - offsets[k*B]: table k's lookups in the batch.  0 <= L[k] <=
+ *            max_lookups (grow with dlrmb_tables_reserve); L[k] = 0 is a table with no lookup.  The launchers size
+ *            their grids and choose sort regimes from L, so a device-pointer call allocates nothing, does not
+ *            synchronise or copy from the host, and can be captured into a CUDA graph.  The kernels trust that
+ *            offsets agree with L (and that the indices are in range); dlrmb_check_indices_jagged verifies both.
+ *   pooling  0 = sum, 1 = mean, for every table of the call.
+ * Sum: out[b][slot0 + k] = sum of table_k[values[j]] over the bag, j ascending, in fp32 from +0.0f.  Mean: with n
+ * the bag's length and w = 1.0f / n rounded to fp32, out = fl(S * w) for the sum S.  An empty bag gives +0.0f in
+ * both modes and no gradient.  Update (dlrmb_embedding_update_sorted, Flux.Descent): sorted entry j of table k
+ * contributes dT[b(j)][slot0 + k], times w(b(j)) in mean mode; duplicates are summed as for the other entry points
+ * and row -= lr * sum.  When every bag of table k has P_k lookups, sum pooling gives the bits of the _mp (and
+ * uniform) entry points: pooled rows, dedup export and tables after the update.
+ * Anything else returns DLRMB_EINVAL.  dlrmb_embedding_update_sorted consumes the last sort, uniform, _mp or jagged;
+ * after a jagged sort dlrmb_sort_dedup_export(k) returns table k's L[k] entries, perm holding positions inside table
+ * k's block of values. */
+int32_t dlrmb_embedding_fwd_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                   int32_t slots, int32_t slot0, dlrmb_stream stream);
+/* training form: the lookup, then the sort for the coming update */
+int32_t dlrmb_embedding_fwd_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                        int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                        int32_t slots, int32_t slot0, dlrmb_stream stream);
+int32_t dlrmb_embedding_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                    int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, dlrmb_stream stream);
+/* DLRMB_EINVAL when offsets[0] != 0, offsets decrease or a table's total disagrees with L; DLRMB_EOOB for an index
+ * outside its table.  The message names the first offender.  values / offsets on the host when on_host != 0.
+ * Synchronises. */
+int32_t dlrmb_check_indices_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t on_host);
+
 /* ---- loss: the top MLP's final sigmoid (src/model/model.jl:87-90) fused with bce_loss and its
  * pullback (src/train/train.jl:33-41, 45-71).  logits/labels [B] device f32.  Writes the mean loss
  * (one float), d(loss)/d(logit) [B] (sensitivity 1 folded in) and, if `prob` is non-NULL, the
