@@ -8,6 +8,8 @@ bandwidth; one JSON line per mode, with the GPU name and power limit read in the
          work, so the gap is the cost of the jagged path
   var    bag lengths uniform in 1 .. 2 P_k - 1 (the same expected total) through the jagged path, against `_mp` at P_k
   mean   mean against sum pooling on the var batches
+  weighted  per-sample weights (random, f32) against the unweighted sum on the var batches, and the weight
+         gradient (dw = dT . row per entry) on its own, with its algorithmic bytes over the copy bandwidth
 
     python benchmarks/jagged.py --out profiles/r07_jagged_b200.jsonl
 """
@@ -55,6 +57,11 @@ def measure(t, batches, T, dT, a):
     return {"lookup_us": us_l, "lookup_sort_us": us_ls, "lookup_sort_update_us": us_c}
 
 
+def weight_grad_bytes(L, B, D, ntab, offsets_bytes):
+    """Rows read + indices read + dw written + one dT row read per bag + the offsets."""
+    return sum(L) * D * 4 + sum(L) * 4 + sum(L) * 4 + ntab * B * D * 4 + offsets_bytes
+
+
 def with_bw(r, nbytes, bw):
     r = dict(r)
     r["lookup_algorithmic_bytes"] = nbytes
@@ -64,7 +71,7 @@ def with_bw(r, nbytes, bw):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--mode", choices=["const", "var", "mean"], nargs="+", default=["const", "var", "mean"])
+    ap.add_argument("--mode", choices=["const", "var", "mean", "weighted"], nargs="+", default=["const", "var", "mean"])
     ap.add_argument("--hotness", default=MLPERF_HOTNESS)
     ap.add_argument("--batch", type=int, default=2048)
     ap.add_argument("--rows-cap", type=int, default=20_000_000)
@@ -92,6 +99,10 @@ def main():
     const = [JaggedIndices.from_dense(p) for p in packed]
     var_sum = jagged_batches(np.random.default_rng(99), rows, P, B, a.nb, "sum", dev)
     var_mean = [JaggedIndices(j.values, j.offsets, j.L, j.B, "mean") for j in var_sum]
+    wrng = np.random.default_rng(7)
+    var_weighted = [JaggedIndices(j.values, j.offsets, j.L, j.B, "sum",
+                                  torch.from_numpy(wrng.uniform(0.0, 2.0, j.values.numel()).astype(np.float32)).to(dev))
+                    for j in var_sum]
     ntab = len(rows)
     off_bytes = (ntab * B + 1) * 4
     L_mp = [B * p for p in P]
@@ -106,14 +117,24 @@ def main():
                 base = with_bw(measure(t, packed, T, dT, a), lookup_bytes(L_mp, B, D, ntab), bw)
                 new = with_bw(measure(t, var_sum, T, dT, a), lookup_bytes(L_var, B, D, ntab, off_bytes), bw)
                 names = ("mp", "jagged_var")
-            else:
+            elif mode == "mean":
                 base = with_bw(measure(t, var_sum, T, dT, a), lookup_bytes(L_var, B, D, ntab, off_bytes), bw)
                 new = with_bw(measure(t, var_mean, T, dT, a), lookup_bytes(L_var, B, D, ntab, off_bytes), bw)
                 names = ("jagged_var_sum", "jagged_var_mean")
+            else:
+                base = with_bw(measure(t, var_sum, T, dT, a), lookup_bytes(L_var, B, D, ntab, off_bytes), bw)
+                # the weights are read once per gathered row: 4 bytes more per lookup
+                new = with_bw(measure(t, var_weighted, T, dT, a),
+                              lookup_bytes(L_var, B, D, ntab, off_bytes + 4 * sum(L_var)), bw)
+                names = ("jagged_var_sum", "jagged_var_weighted")
             r = dict(info, mode=mode, repeat=rep, rows_cap=a.rows_cap, D=D, B=B, hotness=P,
                      lookups_per_step_mp=sum(L_mp), lookups_per_step_var_mean=sum(L_var),
                      **{names[0]: base, names[1]: new},
                      ratio={k: new[k] / base[k] for k in ("lookup_us", "lookup_sort_us", "lookup_sort_update_us")})
+            if mode == "weighted":
+                us_dw = timed(lambda i: t.weight_grad(var_weighted[i], dT, 1), a.nb, a.iters)
+                nbytes = weight_grad_bytes(L_var, B, D, ntab, off_bytes)
+                r["weight_grad"] = {"us": us_dw, "algorithmic_bytes": nbytes, "frac_copy_bw": nbytes / us_dw / 1e3 / bw}
             line = json.dumps(r)
             print(line, flush=True)
             if a.out:

@@ -116,6 +116,13 @@ SIGNATURES = {
     "dlrmb_embedding_fwd_sort_jagged": (_i32, [_vp, *_idx_jagged_args, _i32, _vp, _i32, _i32, _vp]),
     "dlrmb_embedding_sort_jagged": (_i32, [_vp, *_idx_jagged_args, _i32, _vp]),
     "dlrmb_check_indices_jagged": (_i32, [_vp, *_idx_jagged_args, _i32]),
+    # values, offsets, weights, idx_bytes, idx_base, B, L[ntab], out, slots, slot0, stream
+    "dlrmb_embedding_fwd_jagged_weighted": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i64), _vp, _i32,
+                                                   _i32, _vp]),
+    "dlrmb_embedding_fwd_sort_jagged_weighted": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i64), _vp,
+                                                        _i32, _i32, _vp]),
+    "dlrmb_embedding_sort_jagged_weighted": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i64), _vp]),
+    "dlrmb_embedding_weight_grad_jagged": (_i32, [_vp, *_idx_jagged_args, _vp, _i32, _i32, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

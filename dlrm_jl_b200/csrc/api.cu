@@ -830,48 +830,106 @@ int32_t dlrmb_check_indices_mp(dlrmb_tables* t, const void* idx, int32_t idx_byt
 }
 
 // ---- jagged (variable-length) bags -----------------------------------------------------------------------------
-static int jagged_fwd(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base, int B,
-                      const int64_t* L, int pooling, float* out, int slots, int slot0, dlrmb_stream stream, bool sort) {
+// `weighted`: the `_weighted` calls, sum pooling with per-sample `weights`; the launchers take it as pooling
+// kJaggedWeighted.  Otherwise `pooling` is the caller's (0 sum or 1 mean, checked by check_jagged_args).
+static int check_jagged_call(const dlrmb_tables* t, const void* values, const void* offsets, const float* weights,
+                             bool weighted, int idx_bytes, int idx_base, int B, const int64_t* L, int* pooling,
+                             MpGeom* g) {
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, weighted ? 0 : *pooling, g);
+    if (rc || !weighted) return rc;
+    DLRMB_REQUIRE(weights != nullptr || g->off[g->ntab - 1] + g->P[g->ntab - 1] == 0, "weights is null");
+    *pooling = kJaggedWeighted;
+    return DLRMB_OK;
+}
+
+static int jagged_sort(dlrmb_tables* t, const void* values, const void* offsets, const float* weights, bool weighted,
+                       int idx_bytes, int idx_base, int B, const int64_t* L, int pooling, dlrmb_stream stream) {
     MpGeom g;
-    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, pooling, &g);
-    if (rc) return rc;
-    DLRMB_REQUIRE(out != nullptr, "out is null");
-    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
-                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
-    GUARD(t);
-    if (sort) t->sorted_valid = false;
-    rc = launch_lookup_jagged(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, (cudaStream_t)stream);
-    if (rc || !sort) return rc;
-    return dlrmb_embedding_sort_jagged(t, values, offsets, idx_bytes, idx_base, B, L, pooling, stream);
-}
-
-int32_t dlrmb_embedding_fwd_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
-                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
-                                   int32_t slots, int32_t slot0, dlrmb_stream stream) {
-    return jagged_fwd(t, values, offsets, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream, false);
-}
-
-int32_t dlrmb_embedding_fwd_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
-                                        int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
-                                        int32_t slots, int32_t slot0, dlrmb_stream stream) {
-    return jagged_fwd(t, values, offsets, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream, true);
-}
-
-int32_t dlrmb_embedding_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
-                                    int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, dlrmb_stream stream) {
-    MpGeom g;
-    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, pooling, &g);
+    int rc = check_jagged_call(t, values, offsets, weights, weighted, idx_bytes, idx_base, B, L, &pooling, &g);
     if (rc) return rc;
     GUARD(t);
     t->sorted_valid = false;
     const int half = sort_mp_final_half(t, g);
     rc = launch_sort_mp(t, values, idx_bytes, idx_base, g, 0, half, (cudaStream_t)stream);
     if (rc) return rc;
-    rc = launch_jagged_bags(t, offsets, idx_bytes, g, B, pooling, half, (cudaStream_t)stream);
+    rc = launch_jagged_bags(t, offsets, weights, idx_bytes, g, B, pooling, half, (cudaStream_t)stream);
     if (rc) return rc;
     mark_sorted(t, g, 0);
     t->sorted_jagged = pooling;
     return DLRMB_OK;
+}
+
+static int jagged_fwd(dlrmb_tables* t, const void* values, const void* offsets, const float* weights, bool weighted,
+                      int idx_bytes, int idx_base, int B, const int64_t* L, int pooling, float* out, int slots,
+                      int slot0, dlrmb_stream stream, bool sort) {
+    MpGeom g;
+    int rc = check_jagged_call(t, values, offsets, weights, weighted, idx_bytes, idx_base, B, L, &pooling, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(out != nullptr, "out is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
+                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
+    GUARD(t);
+    if (sort) t->sorted_valid = false;
+    rc = launch_lookup_jagged(t, values, offsets, weights, idx_bytes, idx_base, g, B, pooling, out, slots, slot0,
+                              (cudaStream_t)stream);
+    if (rc || !sort) return rc;
+    return jagged_sort(t, values, offsets, weights, weighted, idx_bytes, idx_base, B, L, pooling, stream);
+}
+
+int32_t dlrmb_embedding_fwd_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                   int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                   int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, nullptr, false, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream,
+                      false);
+}
+
+int32_t dlrmb_embedding_fwd_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                        int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, float* out,
+                                        int32_t slots, int32_t slot0, dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, nullptr, false, idx_bytes, idx_base, B, L, pooling, out, slots, slot0, stream,
+                      true);
+}
+
+int32_t dlrmb_embedding_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                    int32_t idx_base, int32_t B, const int64_t* L, int32_t pooling, dlrmb_stream stream) {
+    return jagged_sort(t, values, offsets, nullptr, false, idx_bytes, idx_base, B, L, pooling, stream);
+}
+
+int32_t dlrmb_embedding_fwd_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                            const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                            const int64_t* L, float* out, int32_t slots, int32_t slot0,
+                                            dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, weights, true, idx_bytes, idx_base, B, L, 0, out, slots, slot0, stream, false);
+}
+
+int32_t dlrmb_embedding_fwd_sort_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                                 const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                                 const int64_t* L, float* out, int32_t slots, int32_t slot0,
+                                                 dlrmb_stream stream) {
+    return jagged_fwd(t, values, offsets, weights, true, idx_bytes, idx_base, B, L, 0, out, slots, slot0, stream, true);
+}
+
+int32_t dlrmb_embedding_sort_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                             const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                             const int64_t* L, dlrmb_stream stream) {
+    return jagged_sort(t, values, offsets, weights, true, idx_bytes, idx_base, B, L, 0, stream);
+}
+
+int32_t dlrmb_embedding_weight_grad_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                           int32_t idx_base, int32_t B, const int64_t* L, const float* dT, int32_t slots,
+                                           int32_t slot0, float* dw, dlrmb_stream stream) {
+    MpGeom g;
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B, L, 0, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(dw != nullptr || g.off[g.ntab - 1] + g.P[g.ntab - 1] == 0, "dw is null");
+    DLRMB_REQUIRE(dT != nullptr, "dT is null");
+    DLRMB_REQUIRE(slot0 >= 0 && slots >= slot0 + t->ntab,
+                  "slots = %d too small for slot0 = %d + %d tables", slots, slot0, t->ntab);
+    DLRMB_REQUIRE(t->D % 4 != 0 || (reinterpret_cast<uintptr_t>(dT) & 15) == 0,
+                  "dT must be 16-byte aligned when D is a multiple of 4");
+    GUARD(t);
+    return launch_weight_grad_jagged(t, values, offsets, idx_bytes, idx_base, B, dT, slots, slot0, dw,
+                                     (cudaStream_t)stream);
 }
 
 int32_t dlrmb_check_indices_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,

@@ -221,8 +221,9 @@ struct dlrmb_tables {
     bool sorted_valid = false;
     int sorted_B = 0;
     int32_t* h_sorted_P = nullptr;            // [ntab], host: P_k of every table (L_k after a jagged sort, sorted_B = 1)
-    int sorted_jagged = -1;                   // -1: uniform or _mp sort; 0 / 1: jagged sort with sum / mean pooling,
-                                              // bag ids (and mean weights) in pos / keys [sorted_buf ^ 1]
+    int sorted_jagged = -1;                   // -1: uniform or _mp sort; 0 / 1 / 2: jagged sort with sum / mean /
+                                              // per-sample-weighted sum pooling, bag ids (and the entries' weights
+                                              // in modes 1 and 2) in pos / keys [sorted_buf ^ 1]
 
     // host-entry-point staging (device side), grown on demand
     void* stage_idx = nullptr;  size_t stage_idx_bytes = 0;
@@ -287,12 +288,19 @@ int64_t lookup_grid_mp(const dlrmb_tables* t, MpGeom& g, uint32_t C, int* cshift
 // `values`, same width as the indices).
 int check_jagged_args(const dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
                       int B, const int64_t* L, int pooling, MpGeom* g);
-int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
-                         const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s);
-// after a jagged sort into half `half`: bag id (and, with mean pooling, weight 1/n as f32 bits) of every sorted
-// entry into pos[half ^ 1] (and keys[half ^ 1])
-int launch_jagged_bags(dlrmb_tables* t, const void* offsets, int idx_bytes, const MpGeom& g, int B, int pooling,
-                       int half, cudaStream_t s);
+// `pooling` of the launchers below: 0 sum, 1 mean, or kJaggedWeighted for sum pooling with per-sample weights
+// (`weights`, one f32 per entry of values; null otherwise).
+constexpr int kJaggedWeighted = 2;
+int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, const float* weights, int idx_bytes,
+                         int idx_base, const MpGeom& g, int B, int pooling, float* out, int slots, int slot0,
+                         cudaStream_t s);
+// after a jagged sort into half `half`: bag id (and, with mean pooling, weight 1/n as f32 bits; with per-sample
+// weights, the entry's weight) of every sorted entry into pos[half ^ 1] (and keys[half ^ 1])
+int launch_jagged_bags(dlrmb_tables* t, const void* offsets, const float* weights, int idx_bytes, const MpGeom& g,
+                       int B, int pooling, int half, cudaStream_t s);
+// dw[j] = dT[b(j)][slot0 + k] . table_k[values[j]] for every entry of the batch (order: lookup.cu, the header)
+int launch_weight_grad_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                              int B, const float* dT, int slots, int slot0, float* dw, cudaStream_t s);
 // lookups of table k in the last sort
 static inline int64_t sorted_lookups(const dlrmb_tables* t, int k) { return (int64_t)t->sorted_B * t->h_sorted_P[k]; }
 

@@ -83,9 +83,11 @@ __device__ __forceinline__ void lookup_gather_body(const TableDesc* __restrict__
 
 // Sum of chunk c of the rows ip[0 .. n) (fp32, from +0.0f, ascending), four row loads in flight: the loop of
 // lookup_pool_body (which keeps its own copy: calling this helper there changes the VEC = 1 kernels' SASS).
-template <typename IdxT, int VEC, typename RowT>
+// WEIGHTED multiplies row p by wp[p] before it is added: acc = fl(acc + fl(w * row)), never contracted.
+template <typename IdxT, int VEC, typename RowT, bool WEIGHTED = false>
 __device__ __forceinline__ typename Vec<VEC>::type pool_bag(const float* __restrict__ tb, const IdxT* __restrict__ ip,
-                                                            uint32_t n, int idx_base, size_t D, uint32_t c) {
+                                                            uint32_t n, int idx_base, size_t D, uint32_t c,
+                                                            const float* __restrict__ wp = nullptr) {
     using V = typename Vec<VEC>::type;
     V acc = Vec<VEC>::zero();
     uint32_t p = 0;
@@ -98,6 +100,12 @@ __device__ __forceinline__ typename Vec<VEC>::type pool_bag(const float* __restr
         V v1 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r1, D, c);
         V v2 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r2, D, c);
         V v3 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r3, D, c);
+        if (WEIGHTED) {
+            v0 = Vec<VEC>::scale(v0, __ldg(wp + p));
+            v1 = Vec<VEC>::scale(v1, __ldg(wp + p + 1));
+            v2 = Vec<VEC>::scale(v2, __ldg(wp + p + 2));
+            v3 = Vec<VEC>::scale(v3, __ldg(wp + p + 3));
+        }
         acc = Vec<VEC>::add(acc, v0);
         acc = Vec<VEC>::add(acc, v1);
         acc = Vec<VEC>::add(acc, v2);
@@ -105,7 +113,9 @@ __device__ __forceinline__ typename Vec<VEC>::type pool_bag(const float* __restr
     }
     for (; p < n; ++p) {
         int64_t r = (int64_t)__ldg(ip + p) - idx_base;
-        acc = Vec<VEC>::add(acc, Vec<VEC>::template ldrow<RowT>(tb, (size_t)r, D, c));
+        V v = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r, D, c);
+        if (WEIGHTED) v = Vec<VEC>::scale(v, __ldg(wp + p));
+        acc = Vec<VEC>::add(acc, v);
     }
     return acc;
 }
@@ -357,6 +367,36 @@ lookup_jagged_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict_
     clock_out(clk, blockIdx.x);
 }
 
+// Per-sample weights (the `_weighted` entry points, sum pooling only): lookup_jagged_kernel's grid and thread
+// mapping, with row j of a bag scaled by weights[j] before it is added (pool_bag<WEIGHTED>).  The lanes of one bag
+// read the same weight, so a weight costs one L1 broadcast per gathered row.
+template <typename IdxT, int VEC, typename RowT>
+__global__ void __launch_bounds__(256)
+lookup_jagged_weighted_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ values,
+                              const IdxT* __restrict__ offsets, const float* __restrict__ weights, int idx_base,
+                              const __grid_constant__ MpGeom g, uint32_t B, uint32_t C, int cshift,
+                              float* __restrict__ out, int slots, int slot0, unsigned long long* clk) {
+    using V = typename Vec<VEC>::type;
+    clock_in(clk, blockIdx.x);
+    const int k = mp_find(g.pre, g.ntab, blockIdx.x);
+    const uint32_t cta = blockIdx.x - g.pre[k], nctas = g.pre[k + 1] - g.pre[k];
+    const float* __restrict__ tb = desc[k].base;
+    const IdxT* __restrict__ ok = offsets + (size_t)k * B;
+    const uint32_t n = B * C;
+    const uint32_t step = nctas * blockDim.x;
+    const size_t D = (size_t)C * VEC;
+    float* __restrict__ ob = out + (size_t)(slot0 + k) * D;
+    const size_t ostride = (size_t)slots * D;
+    for (uint32_t t = cta * blockDim.x + threadIdx.x; t < n; t += step) {
+        const uint32_t b = cshift >= 0 ? (t >> cshift) : (t / C);
+        const uint32_t c = t - b * C;
+        const int64_t o0 = (int64_t)__ldg(ok + b), o1 = (int64_t)__ldg(ok + b + 1);
+        reinterpret_cast<V*>(ob + (size_t)b * ostride)[c] =
+            pool_bag<IdxT, VEC, RowT, true>(tb, values + o0, (uint32_t)(o1 - o0), idx_base, D, c, weights + o0);
+    }
+    clock_out(clk, blockIdx.x);
+}
+
 // CTAs per table: the lookup_grid_mp budget split in proportion to the table's gathered rows plus its output rows,
 // (L_k + B) * C, so a table of long bags is not the tail; at least one per table (its B rows are written even
 // when L_k = 0) and no more than it has work items for.
@@ -378,8 +418,9 @@ static int64_t lookup_grid_jagged(const dlrmb_tables* t, MpGeom& g, uint32_t B, 
 }
 
 template <typename IdxT, int VEC, typename RowT>
-static int launch_lookup_jagged_t(dlrmb_tables* t, const IdxT* values, const IdxT* offsets, int idx_base,
-                                  const MpGeom& g0, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+static int launch_lookup_jagged_t(dlrmb_tables* t, const IdxT* values, const IdxT* offsets, const float* weights,
+                                  int idx_base, const MpGeom& g0, int B, int pooling, float* out, int slots, int slot0,
+                                  cudaStream_t s) {
     const uint32_t C = t->D / VEC;
     const int64_t n = (int64_t)B * C;
     DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
@@ -388,7 +429,11 @@ static int launch_lookup_jagged_t(dlrmb_tables* t, const IdxT* values, const Idx
     int cshift = -1;
     if ((C & (C - 1)) == 0)
         for (cshift = 0; (1u << cshift) < C; ++cshift) {}
-    if (pooling == 1)
+    if (pooling == kJaggedWeighted)
+        lookup_jagged_weighted_kernel<IdxT, VEC, RowT><<<(unsigned)ctas, 256, 0, s>>>(
+            t->d_desc, values, offsets, weights, idx_base, g, (uint32_t)B, C, cshift, out, slots, slot0,
+            clock_slot(CLK_LOOKUP));
+    else if (pooling == 1)
         lookup_jagged_kernel<IdxT, VEC, RowT, true><<<(unsigned)ctas, 256, 0, s>>>(
             t->d_desc, values, offsets, idx_base, g, (uint32_t)B, C, cshift, out, slots, slot0, clock_slot(CLK_LOOKUP));
     else
@@ -399,26 +444,156 @@ static int launch_lookup_jagged_t(dlrmb_tables* t, const IdxT* values, const Idx
 }
 
 template <typename RowT>
-static int launch_lookup_jagged_r(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
-                                  const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+static int launch_lookup_jagged_r(dlrmb_tables* t, const void* values, const void* offsets, const float* w,
+                                  int idx_bytes, int idx_base, const MpGeom& g, int B, int pooling, float* out, int slots,
+                                  int slot0, cudaStream_t s) {
     const bool vec4 = (t->D % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
     if (idx_bytes == 4) {
         const uint32_t* v = static_cast<const uint32_t*>(values);
         const uint32_t* o = static_cast<const uint32_t*>(offsets);
-        return vec4 ? launch_lookup_jagged_t<uint32_t, 4, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s)
-                    : launch_lookup_jagged_t<uint32_t, 1, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s);
+        return vec4 ? launch_lookup_jagged_t<uint32_t, 4, RowT>(t, v, o, w, idx_base, g, B, pooling, out, slots, slot0, s)
+                    : launch_lookup_jagged_t<uint32_t, 1, RowT>(t, v, o, w, idx_base, g, B, pooling, out, slots, slot0, s);
     }
     const int64_t* v = static_cast<const int64_t*>(values);
     const int64_t* o = static_cast<const int64_t*>(offsets);
-    return vec4 ? launch_lookup_jagged_t<int64_t, 4, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s)
-                : launch_lookup_jagged_t<int64_t, 1, RowT>(t, v, o, idx_base, g, B, pooling, out, slots, slot0, s);
+    return vec4 ? launch_lookup_jagged_t<int64_t, 4, RowT>(t, v, o, w, idx_base, g, B, pooling, out, slots, slot0, s)
+                : launch_lookup_jagged_t<int64_t, 1, RowT>(t, v, o, w, idx_base, g, B, pooling, out, slots, slot0, s);
 }
 
-int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
-                         const MpGeom& g, int B, int pooling, float* out, int slots, int slot0, cudaStream_t s) {
+int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, const float* weights, int idx_bytes,
+                         int idx_base, const MpGeom& g, int B, int pooling, float* out, int slots, int slot0,
+                         cudaStream_t s) {
     if (t->elem_bytes == 2)
-        return launch_lookup_jagged_r<__nv_bfloat16>(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, s);
-    return launch_lookup_jagged_r<float>(t, values, offsets, idx_bytes, idx_base, g, B, pooling, out, slots, slot0, s);
+        return launch_lookup_jagged_r<__nv_bfloat16>(t, values, offsets, weights, idx_bytes, idx_base, g, B, pooling, out,
+                                                     slots, slot0, s);
+    return launch_lookup_jagged_r<float>(t, values, offsets, weights, idx_bytes, idx_base, g, B, pooling, out, slots,
+                                         slot0, s);
+}
+
+// ---- gradient of the pooled rows with respect to the per-sample weights ---------------------------------------
+// dw[j] = sum_d dT[b(j)][slot0 + k][d] * table_k[values[j]][d] for every entry j of every bag, in the order the
+// header states: a group of G lanes (G = min(32, C rounded up to a power of two), C chunks of VEC floats) owns one
+// bag; lane l adds the products of its chunks c = l, l + G, .. in ascending d, acc = fl(acc + fl(g * r)) from
+// +0.0f; then the G partials meet in a butterfly, p_l = fl(p_l + p_(l xor s)) for s = G/2 .. 1 (IEEE addition
+// commutes, so every lane holds the same bits), and lane 0 stores dw[j].  Four entries are in flight per group;
+// the bag's dT row is re-read from L1 for each of them.  A flat grid of ntab * B groups; an empty bag stores
+// nothing.
+template <int VEC> struct Dot;
+template <> struct Dot<4> {
+    static __device__ __forceinline__ float acc(float a, float4 g, float4 r) {
+        a = __fadd_rn(a, __fmul_rn(g.x, r.x));
+        a = __fadd_rn(a, __fmul_rn(g.y, r.y));
+        a = __fadd_rn(a, __fmul_rn(g.z, r.z));
+        return __fadd_rn(a, __fmul_rn(g.w, r.w));
+    }
+    static __device__ __forceinline__ float4 ld(const float* p, uint32_t c) {
+        return __ldg(reinterpret_cast<const float4*>(p) + c);
+    }
+};
+template <> struct Dot<1> {
+    static __device__ __forceinline__ float acc(float a, float g, float r) { return __fadd_rn(a, __fmul_rn(g, r)); }
+    static __device__ __forceinline__ float ld(const float* p, uint32_t c) { return __ldg(p + c); }
+};
+
+template <typename IdxT, int VEC, typename RowT>
+__global__ void __launch_bounds__(256)
+weight_grad_jagged_kernel(const TableDesc* __restrict__ desc, const IdxT* __restrict__ values,
+                          const IdxT* __restrict__ offsets, int idx_base, uint32_t ntab, uint32_t B, uint32_t C,
+                          int glog2, const float* __restrict__ dT, int slots, int slot0, float* __restrict__ dw) {
+    using V = typename Vec<VEC>::type;
+    const uint32_t G = 1u << glog2;
+    const uint32_t lane = threadIdx.x & (G - 1);
+    const uint64_t grp = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> glog2;
+    if (grp >= (uint64_t)ntab * B) return;   // whole groups only: G divides 32
+    // the group's lanes, for the shuffles (groups of one warp may walk bags of different lengths)
+    const unsigned mask = G == 32 ? 0xffffffffu : (((1u << G) - 1) << ((threadIdx.x & 31) & ~(G - 1)));
+    const uint32_t k = (uint32_t)grp / B, b = (uint32_t)grp - k * B;   // ntab * B < 2^32 (the launcher checks)
+    const float* __restrict__ tb = desc[k].base;
+    const size_t D = (size_t)C * VEC;
+    const float* __restrict__ gr = dT + ((size_t)b * slots + slot0 + k) * D;
+    const int64_t o0 = (int64_t)__ldg(offsets + (size_t)k * B + b), o1 = (int64_t)__ldg(offsets + (size_t)k * B + b + 1);
+    const IdxT* __restrict__ ip = values + o0;
+    float* __restrict__ wo = dw + o0;
+    const uint32_t n = (uint32_t)(o1 - o0);
+    uint32_t p = 0;
+    for (; p + 4 <= n; p += 4) {
+        const int64_t r0 = (int64_t)__ldg(ip + p) - idx_base;
+        const int64_t r1 = (int64_t)__ldg(ip + p + 1) - idx_base;
+        const int64_t r2 = (int64_t)__ldg(ip + p + 2) - idx_base;
+        const int64_t r3 = (int64_t)__ldg(ip + p + 3) - idx_base;
+        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+        for (uint32_t c = lane; c < C; c += G) {
+            const V gv = Dot<VEC>::ld(gr, c);
+            const V v0 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r0, D, c);
+            const V v1 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r1, D, c);
+            const V v2 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r2, D, c);
+            const V v3 = Vec<VEC>::template ldrow<RowT>(tb, (size_t)r3, D, c);
+            a0 = Dot<VEC>::acc(a0, gv, v0);
+            a1 = Dot<VEC>::acc(a1, gv, v1);
+            a2 = Dot<VEC>::acc(a2, gv, v2);
+            a3 = Dot<VEC>::acc(a3, gv, v3);
+        }
+        for (uint32_t s = G >> 1; s > 0; s >>= 1) {
+            a0 = __fadd_rn(a0, __shfl_xor_sync(mask, a0, s, G));
+            a1 = __fadd_rn(a1, __shfl_xor_sync(mask, a1, s, G));
+            a2 = __fadd_rn(a2, __shfl_xor_sync(mask, a2, s, G));
+            a3 = __fadd_rn(a3, __shfl_xor_sync(mask, a3, s, G));
+        }
+        if (lane == 0) {
+            wo[p] = a0;
+            wo[p + 1] = a1;
+            wo[p + 2] = a2;
+            wo[p + 3] = a3;
+        }
+    }
+    for (; p < n; ++p) {
+        const int64_t r = (int64_t)__ldg(ip + p) - idx_base;
+        float a = 0.f;
+        for (uint32_t c = lane; c < C; c += G)
+            a = Dot<VEC>::acc(a, Dot<VEC>::ld(gr, c), Vec<VEC>::template ldrow<RowT>(tb, (size_t)r, D, c));
+        for (uint32_t s = G >> 1; s > 0; s >>= 1) a = __fadd_rn(a, __shfl_xor_sync(mask, a, s, G));
+        if (lane == 0) wo[p] = a;
+    }
+}
+
+template <typename IdxT, int VEC, typename RowT>
+static int launch_weight_grad_jagged_t(dlrmb_tables* t, const IdxT* values, const IdxT* offsets, int idx_base, int B,
+                                       const float* dT, int slots, int slot0, float* dw, cudaStream_t s) {
+    const uint32_t C = t->D / VEC;
+    int glog2 = 0;
+    while ((1u << glog2) < C && glog2 < 5) ++glog2;
+    const int64_t groups = (int64_t)t->ntab * B;
+    DLRMB_REQUIRE(groups <= (int64_t)UINT32_MAX, "batch too large for one weight-gradient launch");
+    const int64_t ctas = ceil_div64(groups << glog2, 256);
+    weight_grad_jagged_kernel<IdxT, VEC, RowT><<<(unsigned)ctas, 256, 0, s>>>(
+        t->d_desc, values, offsets, idx_base, (uint32_t)t->ntab, (uint32_t)B, C, glog2, dT, slots, slot0, dw);
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename RowT>
+static int launch_weight_grad_jagged_r(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes,
+                                       int idx_base, int B, const float* dT, int slots, int slot0, float* dw,
+                                       cudaStream_t s) {
+    const bool vec4 = t->D % 4 == 0;   // the caller checked dT's alignment
+    if (idx_bytes == 4) {
+        const uint32_t* v = static_cast<const uint32_t*>(values);
+        const uint32_t* o = static_cast<const uint32_t*>(offsets);
+        return vec4 ? launch_weight_grad_jagged_t<uint32_t, 4, RowT>(t, v, o, idx_base, B, dT, slots, slot0, dw, s)
+                    : launch_weight_grad_jagged_t<uint32_t, 1, RowT>(t, v, o, idx_base, B, dT, slots, slot0, dw, s);
+    }
+    const int64_t* v = static_cast<const int64_t*>(values);
+    const int64_t* o = static_cast<const int64_t*>(offsets);
+    return vec4 ? launch_weight_grad_jagged_t<int64_t, 4, RowT>(t, v, o, idx_base, B, dT, slots, slot0, dw, s)
+                : launch_weight_grad_jagged_t<int64_t, 1, RowT>(t, v, o, idx_base, B, dT, slots, slot0, dw, s);
+}
+
+int launch_weight_grad_jagged(dlrmb_tables* t, const void* values, const void* offsets, int idx_bytes, int idx_base,
+                              int B, const float* dT, int slots, int slot0, float* dw, cudaStream_t s) {
+    if (t->elem_bytes == 2)
+        return launch_weight_grad_jagged_r<__nv_bfloat16>(t, values, offsets, idx_bytes, idx_base, B, dT, slots, slot0,
+                                                          dw, s);
+    return launch_weight_grad_jagged_r<float>(t, values, offsets, idx_bytes, idx_base, B, dT, slots, slot0, dw, s);
 }
 
 // ---- ScaledUniform init (src/model/model.jl:61-65): U(-1/sqrt(rows), 1/sqrt(rows)) ------------

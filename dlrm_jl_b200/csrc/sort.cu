@@ -374,8 +374,20 @@ int launch_sort_mp(dlrmb_tables* t, const void* idx, int idx_bytes, int idx_base
 // (element g.off[k] of `values`); the bag of x = g.off[k] + pos is the largest b with offsets[k*B + b] <= x,
 // found by binary search over the table's B offsets (L1-resident: B * 4 or 8 bytes).  Written in sorted order
 // so that the update reads a bag id where it reads a position, four per 16-byte load.  MEAN also writes the
-// bag's weight fl(1 / n) as f32 bits.  Table k owns CTAs [g.pre[k], g.pre[k+1]) (none when L_k = 0).
+// bag's weight fl(1 / n) as f32 bits; WEIGHTED writes the entry's own weight, weights[x], in its place.  Table k
+// owns CTAs [g.pre[k], g.pre[k+1]) (none when L_k = 0).
 // ---------------------------------------------------------------------------------------------
+template <typename IdxT>
+__device__ __forceinline__ uint32_t jagged_bag_of(const IdxT* __restrict__ ok, uint32_t B, int64_t x) {
+    uint32_t lo = 0, hi = B - 1;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi + 1) >> 1;
+        if ((int64_t)__ldg(ok + mid) <= x) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
 template <typename IdxT, bool MEAN>
 __global__ void __launch_bounds__(256)
 jagged_bags_kernel(const IdxT* __restrict__ offsets, uint32_t B, const __grid_constant__ MpGeom g,
@@ -387,20 +399,34 @@ jagged_bags_kernel(const IdxT* __restrict__ offsets, uint32_t B, const __grid_co
     const uint32_t step = (g.pre[k + 1] - g.pre[k]) * blockDim.x;
     for (uint32_t i = (blockIdx.x - g.pre[k]) * blockDim.x + threadIdx.x; i < L; i += step) {
         const int64_t x = g.off[k] + (int64_t)pos[o + i];
-        uint32_t lo = 0, hi = B - 1;
-        while (lo < hi) {
-            const uint32_t mid = (lo + hi + 1) >> 1;
-            if ((int64_t)__ldg(ok + mid) <= x) lo = mid;
-            else hi = mid - 1;
-        }
+        const uint32_t lo = jagged_bag_of(ok, B, x);
         bags[o + i] = lo;
         if (MEAN) wts[o + i] = __float_as_uint(__fdiv_rn(1.0f, (float)((int64_t)__ldg(ok + lo + 1) - (int64_t)__ldg(ok + lo))));
     }
 }
 
+// WEIGHTED: the same pass, the weight gathered from the entry's position in `values`
 template <typename IdxT>
-static int launch_jagged_bags_t(dlrmb_tables* t, const IdxT* offsets, const MpGeom& g0, int B, int pooling, int half,
-                                cudaStream_t s) {
+__global__ void __launch_bounds__(256)
+jagged_bags_weighted_kernel(const IdxT* __restrict__ offsets, const float* __restrict__ weights, uint32_t B,
+                            const __grid_constant__ MpGeom g, const uint32_t* __restrict__ pos,
+                            uint32_t* __restrict__ bags, uint32_t* __restrict__ wts, int64_t cap) {
+    const int k = mp_find(g.pre, g.ntab, blockIdx.x);
+    const uint32_t L = g.P[k];
+    const IdxT* __restrict__ ok = offsets + (size_t)k * B;
+    const size_t o = (size_t)k * cap;
+    const uint32_t step = (g.pre[k + 1] - g.pre[k]) * blockDim.x;
+    for (uint32_t i = (blockIdx.x - g.pre[k]) * blockDim.x + threadIdx.x; i < L; i += step) {
+        const int64_t x = g.off[k] + (int64_t)pos[o + i];
+        const uint32_t lo = jagged_bag_of(ok, B, x);
+        bags[o + i] = lo;
+        wts[o + i] = __float_as_uint(__ldg(weights + x));
+    }
+}
+
+template <typename IdxT>
+static int launch_jagged_bags_t(dlrmb_tables* t, const IdxT* offsets, const float* weights, const MpGeom& g0, int B,
+                                int pooling, int half, cudaStream_t s) {
     MpGeom g = g0;
     int64_t total = 0;
     for (int k = 0; k < g.ntab; ++k) {
@@ -412,7 +438,10 @@ static int launch_jagged_bags_t(dlrmb_tables* t, const IdxT* offsets, const MpGe
     const uint32_t* pos = t->pos[half];
     uint32_t* bags = t->pos[half ^ 1];
     uint32_t* wts = t->keys[half ^ 1];
-    if (pooling == 1)
+    if (pooling == kJaggedWeighted)
+        jagged_bags_weighted_kernel<IdxT><<<(unsigned)total, 256, 0, s>>>(offsets, weights, (uint32_t)B, g, pos, bags,
+                                                                          wts, t->cap);
+    else if (pooling == 1)
         jagged_bags_kernel<IdxT, true><<<(unsigned)total, 256, 0, s>>>(offsets, (uint32_t)B, g, pos, bags, wts, t->cap);
     else
         jagged_bags_kernel<IdxT, false><<<(unsigned)total, 256, 0, s>>>(offsets, (uint32_t)B, g, pos, bags, wts, t->cap);
@@ -420,10 +449,11 @@ static int launch_jagged_bags_t(dlrmb_tables* t, const IdxT* offsets, const MpGe
     return DLRMB_OK;
 }
 
-int launch_jagged_bags(dlrmb_tables* t, const void* offsets, int idx_bytes, const MpGeom& g, int B, int pooling,
-                       int half, cudaStream_t s) {
-    if (idx_bytes == 4) return launch_jagged_bags_t<uint32_t>(t, static_cast<const uint32_t*>(offsets), g, B, pooling, half, s);
-    return launch_jagged_bags_t<int64_t>(t, static_cast<const int64_t*>(offsets), g, B, pooling, half, s);
+int launch_jagged_bags(dlrmb_tables* t, const void* offsets, const float* weights, int idx_bytes, const MpGeom& g,
+                       int B, int pooling, int half, cudaStream_t s) {
+    if (idx_bytes == 4)
+        return launch_jagged_bags_t<uint32_t>(t, static_cast<const uint32_t*>(offsets), weights, g, B, pooling, half, s);
+    return launch_jagged_bags_t<int64_t>(t, static_cast<const int64_t*>(offsets), weights, g, B, pooling, half, s);
 }
 
 // ---------------------------------------------------------------------------------------------

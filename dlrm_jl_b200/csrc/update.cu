@@ -311,7 +311,7 @@ __device__ __forceinline__ void fixup_runs_smem(const TableDesc* __restrict__ de
 // (INLINE path; zero between launches).
 // Chunk `cta` of table k (gm: that table's geometry).  `gid` names the chunk in the two-launch head list,
 // `ndone` is the table's chunk count (the INLINE done-counter target), `clk_cta` its stamp slot.
-// SCALE (jagged mean pooling): each gradient row is multiplied by its entry's weight `wts` (f32 bits, the
+// SCALE (jagged mean pooling or per-sample weights): each gradient row is multiplied by its entry's weight `wts` (f32 bits, the
 // stream's layout) before it is accumulated.
 template <int VEC, int NCH, int THREADS, typename RowT, bool INLINE, bool SCALE = false>
 __device__ __forceinline__ void update_tiles_body(const TableDesc* __restrict__ desc, const uint32_t* __restrict__ keys,
@@ -702,7 +702,7 @@ int64_t update_tiles_cap(int ntab, int D, int64_t max_lookups, int sm_count) {
 // is two-dimensional (grid.y = table); otherwise one flat grid of sum_k chunks_k CTAs, g.pre mapping a CTA to
 // (table, chunk).  The tile is chosen from the total entry count either way, so equal P_k take the same tiles
 // and chunks on both grids, hence the same bits.  A jagged sort (g.B = 1, P_k = L_k) takes the flat grid with
-// update_tiles_jagged_kernel over the bag ids (and, for mean pooling, the weights) that launch_jagged_bags wrote into
+// update_tiles_jagged_kernel over the bag ids (and, for mean or weighted pooling, the weights) that launch_jagged_bags wrote into
 // pos / keys [sorted_buf ^ 1]; the fix-up kernel is the same for both, it reads no position.
 template <int VEC, int NCH, typename RowT>
 static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot0, float lr, cudaStream_t s) {
@@ -736,7 +736,7 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
     // DLRM-sized batches: level 3 runs inside the same launch (see the header comment)
     const bool inline_fixup = total <= kUpdateInlineMaxEntries &&
                               g_opt.update_two_launches.load(std::memory_order_relaxed) == 0;
-    const int jagged = t->sorted_jagged;   // -1: uniform or _mp sort, 0 / 1: jagged sum / mean
+    const int jagged = t->sorted_jagged;   // -1: uniform or _mp sort, 0 / 1 / 2: jagged sum / mean / weighted sum
     if (equal && jagged < 0) {
         gm.L = (int)maxL;
         gm.P = P[0];
@@ -792,7 +792,7 @@ static int launch_update_t(dlrmb_tables* t, const float* dT, int slots, int slot
     auto tiles = [&](auto inl) {
         constexpr bool INL = decltype(inl)::value;
         const unsigned n = (unsigned)chunks_total;
-        if (jagged == 1)
+        if (jagged >= 1)   // mean or per-sample weights: one weight per sorted entry
             update_tiles_jagged_kernel<VEC, NCH, THREADS, RowT, INL, true><<<n, THREADS, 0, s>>>(
                 t->d_desc, keys, bags, wts, dT, lr, t->partial, t->tile_flags, t->head_list, t->head_count, gm, g,
                 clock_slot(CLK_UPDATE));

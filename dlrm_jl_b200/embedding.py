@@ -84,16 +84,31 @@ class JaggedIndices:
     ``offsets`` [ntab * B + 1] (same dtype, 0-based, non-decreasing, offsets[0] = 0) makes bag b of table k
     ``values[offsets[k*B + b] : offsets[k*B + b + 1]]``; the host tuple ``L`` holds each table's lookup count.
     ``pooling`` is ``"sum"`` or ``"mean"`` (w = fl(1 / n) times the fp32 sum; an empty bag pools to zero).
-    ``jag[k]`` is table k's ``(values_k, offsets_k)`` with offsets_k rebased to 0."""
+    ``weights`` (optional, float32, one per entry of ``values``, same device) are per-sample weights, the
+    ``per_sample_weights`` of ``EmbeddingBag`` in mode ``"sum"``: a bag pools sum_j fl(w_j * row_j); they go with
+    sum pooling only.  ``jag[k]`` is table k's ``(values_k, offsets_k)`` with offsets_k rebased to 0, and
+    ``(values_k, offsets_k, weights_k)`` for a weighted batch."""
     values: torch.Tensor
     offsets: torch.Tensor
     L: Tuple[int, ...]
     B: int
     pooling: str = "sum"
+    weights: Optional[torch.Tensor] = None
 
     def __post_init__(self):
         if self.pooling not in _POOLING:
             raise ValueError(f"pooling must be 'sum' or 'mean', got {self.pooling!r}")
+        if self.weights is not None:
+            w = self.weights
+            if self.pooling != "sum":
+                raise ValueError(f"per-sample weights go with pooling='sum' only, got pooling={self.pooling!r}")
+            if w.dtype != torch.float32:
+                raise ValueError(f"weights must be float32, got {w.dtype}")
+            if w.dim() != 1 or w.numel() != self.values.numel():
+                raise ValueError(f"weights must hold one float per value: {self.values.numel()} values, "
+                                 f"weights of shape {tuple(w.shape)}")
+            if w.device != self.values.device:
+                raise ValueError(f"weights on {w.device}, values on {self.values.device}")
         if self.values.dtype not in (torch.int32, torch.int64) or self.offsets.dtype != self.values.dtype:
             raise ValueError(f"values and offsets must share one dtype, int32 or int64 (got {self.values.dtype} and "
                              f"{self.offsets.dtype})")
@@ -106,8 +121,9 @@ class JaggedIndices:
             raise ValueError(f"the lookup counts sum to {sum(self.L)}, values holds {self.values.numel()}")
 
     @classmethod
-    def from_lengths(cls, values, lengths, pooling: str = "sum") -> "JaggedIndices":
-        """``lengths[ntab][B]``: the size of every bag; ``values`` the bags' indices, table-major."""
+    def from_lengths(cls, values, lengths, pooling: str = "sum", weights=None) -> "JaggedIndices":
+        """``lengths[ntab][B]``: the size of every bag; ``values`` the bags' indices, table-major; ``weights`` their
+        per-sample weights in the same order (a float32 tensor, or any array, converted to float32)."""
         v = values if isinstance(values, torch.Tensor) else torch.as_tensor(np.asarray(values))
         v = _index_dtype(v.reshape(-1))
         n = np.asarray(lengths.cpu() if isinstance(lengths, torch.Tensor) else lengths, dtype=np.int64)
@@ -120,35 +136,46 @@ class JaggedIndices:
         off = np.zeros(n.size + 1, dtype=np.int64)
         np.cumsum(n.reshape(-1), out=off[1:])
         offsets = torch.from_numpy(off).to(device=v.device, dtype=v.dtype)
-        return cls(v.contiguous(), offsets, tuple(int(x) for x in n.sum(axis=1)), int(n.shape[1]), pooling)
+        if weights is not None:
+            if not isinstance(weights, torch.Tensor):
+                weights = torch.from_numpy(np.asarray(weights, dtype=np.float32))
+            weights = weights.reshape(-1).to(v.device).contiguous()
+        return cls(v.contiguous(), offsets, tuple(int(x) for x in n.sum(axis=1)), int(n.shape[1]), pooling, weights)
 
     @classmethod
-    def from_bags(cls, bags, pooling: str = "sum", dtype: torch.dtype = torch.int64) -> "JaggedIndices":
-        """``bags[k][b]``: the indices of bag b of table k (any sequence, possibly empty)."""
+    def from_bags(cls, bags, pooling: str = "sum", dtype: torch.dtype = torch.int64, weights=None) -> "JaggedIndices":
+        """``bags[k][b]``: the indices of bag b of table k (any sequence, possibly empty); ``weights[k][b]`` their
+        per-sample weights, bag for bag."""
         Bs = {len(t) for t in bags}
         if len(Bs) != 1:
             raise ValueError(f"every table must have the same number of bags, got {[len(t) for t in bags]}")
         lengths = [[len(bag) for bag in t] for t in bags]
         flat = [int(i) for t in bags for bag in t for i in bag]
-        return cls.from_lengths(torch.tensor(flat, dtype=dtype), lengths, pooling)
+        if weights is not None:
+            if [[len(w) for w in t] for t in weights] != lengths:
+                raise ValueError("weights must hold one weight per index, bag for bag")
+            weights = np.array([float(x) for t in weights for w in t for x in w], dtype=np.float32)
+        return cls.from_lengths(torch.tensor(flat, dtype=dtype), lengths, pooling, weights)
 
     @classmethod
-    def from_dense(cls, idx, pooling: str = "sum") -> "JaggedIndices":
-        """A fixed-width batch ([ntab][B][P] tensor or :class:`PackedIndices`) as bags of constant length."""
+    def from_dense(cls, idx, pooling: str = "sum", weights=None) -> "JaggedIndices":
+        """A fixed-width batch ([ntab][B][P] tensor or :class:`PackedIndices`) as bags of constant length;
+        ``weights`` in the same shape (the flat layout of :class:`PackedIndices`)."""
         if isinstance(idx, PackedIndices):
-            return cls.from_lengths(idx.flat, [[p] * idx.B for p in idx.P], pooling)
+            return cls.from_lengths(idx.flat, [[p] * idx.B for p in idx.P], pooling, weights)
         t = _index_dtype(idx if isinstance(idx, torch.Tensor) else torch.as_tensor(np.asarray(idx)))
         if t.dim() == 2:
             t = t.unsqueeze(-1)
         ntab, B, P = t.shape
-        return cls.from_lengths(t.reshape(-1), [[P] * B] * ntab, pooling)
+        return cls.from_lengths(t.reshape(-1), [[P] * B] * ntab, pooling, weights)
 
     def __len__(self) -> int:
         return len(self.L)
 
-    def __getitem__(self, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    def __getitem__(self, k: int) -> Tuple[torch.Tensor, ...]:
         o = sum(self.L[:k])
-        return self.values[o:o + self.L[k]], self.offsets[k * self.B:(k + 1) * self.B + 1] - o
+        vo = (self.values[o:o + self.L[k]], self.offsets[k * self.B:(k + 1) * self.B + 1] - o)
+        return vo if self.weights is None else vo + (self.weights[o:o + self.L[k]],)
 
     def L_array(self):
         return (C.c_int64 * len(self.L))(*self.L)
@@ -169,8 +196,10 @@ class JaggedIndices:
         return self.values.device
 
     def to(self, device, non_blocking: bool = False) -> "JaggedIndices":
+        w = None if self.weights is None else self.weights.to(device, non_blocking=non_blocking).contiguous()
         return JaggedIndices(self.values.to(device, non_blocking=non_blocking).contiguous(),
-                             self.offsets.to(device, non_blocking=non_blocking).contiguous(), self.L, self.B, self.pooling)
+                             self.offsets.to(device, non_blocking=non_blocking).contiguous(), self.L, self.B, self.pooling,
+                             w)
 
 
 def _index_dtype(t: torch.Tensor) -> torch.Tensor:
@@ -328,11 +357,19 @@ class EmbeddingTables:
         :meth:`update_sorted` can follow the backward pass without a sort launch."""
         slots = out.shape[1]
         if isinstance(idx, JaggedIndices):   # variable-length bags
-            fn = self._lib.dlrmb_embedding_fwd_sort_jagged if sort else self._lib.dlrmb_embedding_fwd_jagged
             assert out.is_contiguous() and out.dtype == torch.float32 and out.shape == (idx.B, slots, self.D)
             with _prof.range("lookup"):
-                _lib.check(fn(self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.element_size(), idx_base, idx.B,
-                              idx.L_array(), idx.pooling_code, out.data_ptr(), slots, slot0, _stream_ptr(self.device)))
+                if idx.weights is not None:
+                    fn = (self._lib.dlrmb_embedding_fwd_sort_jagged_weighted if sort
+                          else self._lib.dlrmb_embedding_fwd_jagged_weighted)
+                    _lib.check(fn(self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.weights.data_ptr(),
+                                  idx.element_size(), idx_base, idx.B, idx.L_array(), out.data_ptr(), slots, slot0,
+                                  _stream_ptr(self.device)))
+                else:
+                    fn = self._lib.dlrmb_embedding_fwd_sort_jagged if sort else self._lib.dlrmb_embedding_fwd_jagged
+                    _lib.check(fn(self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.element_size(), idx_base,
+                                  idx.B, idx.L_array(), idx.pooling_code, out.data_ptr(), slots, slot0,
+                                  _stream_ptr(self.device)))
             if sort:
                 self._pending_side = False
             return
@@ -390,7 +427,13 @@ class EmbeddingTables:
         if isinstance(idx, JaggedIndices):
             L, code, offs = idx.L_array(), idx.pooling_code, idx.offsets.data_ptr()
             B, P, rec = idx.B, None, (idx.values, idx.offsets)
-            fn = lambda h, v, ib, base, B, _P, st: self._lib.dlrmb_embedding_sort_jagged(h, v, offs, ib, base, B, L, code, st)
+            if idx.weights is not None:
+                w, rec = idx.weights.data_ptr(), rec + (idx.weights,)
+                fn = lambda h, v, ib, base, B, _P, st: self._lib.dlrmb_embedding_sort_jagged_weighted(
+                    h, v, offs, w, ib, base, B, L, st)
+            else:
+                fn = lambda h, v, ib, base, B, _P, st: self._lib.dlrmb_embedding_sort_jagged(
+                    h, v, offs, ib, base, B, L, code, st)
             idx = idx.values
         elif isinstance(idx, PackedIndices):
             B, P, fn, rec = idx.B, idx.P_array(), self._lib.dlrmb_embedding_sort_mp, idx.flat
@@ -424,6 +467,22 @@ class EmbeddingTables:
         with _prof.range("update"):
             _lib.check(self._lib.dlrmb_embedding_update_sorted(
                 self._h, dT.data_ptr(), slots, slot0, float(lr), _stream_ptr(self.device)))
+
+    def weight_grad(self, idx: JaggedIndices, dT: torch.Tensor, slot0: int, idx_base: int = 0) -> torch.Tensor:
+        """Gradient of the pooled rows with respect to per-sample weights (``per_sample_weights.grad``): a float32
+        tensor of sum(L) values, dw[j] = dT[b(j), slot0 + k] . table_k[values[j]], in the order of ``idx.values``
+        (zero-length bags contribute nothing).  It reads the rows as they are: call it before
+        :meth:`update_sorted` of the same batch.  ``idx`` need not carry weights."""
+        if not isinstance(idx, JaggedIndices):
+            raise TypeError(f"weight_grad takes JaggedIndices, got {type(idx).__name__}")
+        B, slots, D = dT.shape
+        assert dT.is_contiguous() and dT.dtype == torch.float32 and D == self.D and B == idx.B
+        dw = torch.empty(idx.values.numel(), dtype=torch.float32, device=self.device)
+        with _prof.range("weight_grad"):
+            _lib.check(self._lib.dlrmb_embedding_weight_grad_jagged(
+                self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), idx.element_size(), idx_base, idx.B,
+                idx.L_array(), dT.data_ptr(), slots, slot0, dw.data_ptr(), _stream_ptr(self.device)))
+        return dw
 
     def bwd_sgd(self, idx: torch.Tensor, dT: torch.Tensor, slot0: int, lr: float, idx_base: int = 0) -> None:
         self.sort(idx, idx_base)
@@ -520,7 +579,7 @@ class SparseEmbeddingUpdate:
     parent: Optional[torch.Tensor] = None
     slot: int = -1
     idx_base: int = 0
-    pooling: str = "sum"        # jagged bags: ``indices`` is the table's (values_k, offsets_k)
+    pooling: str = "sum"        # jagged bags: ``indices`` is the table's (values_k, offsets_k[, weights_k])
 
 
 def sparse_updates(dT: torch.Tensor, indices: torch.Tensor, slot0: int, idx_base: int = 0) -> List[SparseEmbeddingUpdate]:
@@ -535,8 +594,8 @@ def uncompress(update: SparseEmbeddingUpdate, nrows: int) -> torch.Tensor:
     """``EmbeddingTables.uncompress(update, nrows)`` (test/train/backprop.jl:156): the dense
     [nrows][D] gradient.  Debug/inspection helper (torch index_add_), not on the hot path."""
     B, D = update.delta.shape
-    if isinstance(update.indices, tuple):   # jagged bags: every lookup of bag b gets delta[b] (times 1/n for mean)
-        values, offsets = update.indices
+    if isinstance(update.indices, tuple):   # jagged bags: every lookup of bag b gets delta[b] (times 1/n for mean,
+        values, offsets = update.indices[:2]  # times its own weight for per-sample weights)
         n = (offsets[1:] - offsets[:-1]).to(torch.int64).to(update.delta.device)
         delta = update.delta
         if update.pooling == "mean":
@@ -545,7 +604,10 @@ def uncompress(update: SparseEmbeddingUpdate, nrows: int) -> torch.Tensor:
             delta = delta * w[:, None]
         dense = torch.zeros((nrows, D), dtype=torch.float32, device=update.delta.device)
         rows = values.to(torch.int64).to(update.delta.device) - update.idx_base
-        dense.index_add_(0, rows, delta.repeat_interleave(n, dim=0))
+        contrib = delta.repeat_interleave(n, dim=0)
+        if len(update.indices) == 3:
+            contrib = contrib * update.indices[2].to(update.delta.device)[:, None]
+        dense.index_add_(0, rows, contrib)
         return dense
     idx = (update.indices.reshape(B, -1).to(torch.int64) - update.idx_base)
     P = idx.shape[1]
@@ -577,7 +639,8 @@ def update_(opt: Descent, tables: EmbeddingTables, grads: Sequence[SparseEmbeddi
         slot0 = 0
     if not presorted and isinstance(grads[0].indices, tuple):   # jagged bags
         lengths = [(g.indices[1][1:] - g.indices[1][:-1]).cpu().numpy() for g in grads]
-        idx = JaggedIndices.from_lengths(torch.cat([g.indices[0] for g in grads]), lengths, grads[0].pooling)
+        w = torch.cat([g.indices[2] for g in grads]) if len(grads[0].indices) == 3 else None
+        idx = JaggedIndices.from_lengths(torch.cat([g.indices[0] for g in grads]), lengths, grads[0].pooling, w)
         tables.sort(idx.to(tables.device), grads[0].idx_base)
     elif not presorted:
         idx = _as_index_tensor([g.indices.reshape(g.delta.shape[0], -1) for g in grads], tables.ntab, tables.device)

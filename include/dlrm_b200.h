@@ -243,6 +243,45 @@ int32_t dlrmb_embedding_sort_jagged(dlrmb_tables* t, const void* values, const v
 int32_t dlrmb_check_indices_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
                                    int32_t idx_base, int32_t B, const int64_t* L, int32_t on_host);
 
+/* ---- weighted jagged bags: torch.nn.EmbeddingBag(input, offsets, per_sample_weights=w) in mode 'sum', TorchRec's
+ * weighted KeyedJaggedTensor.  The jagged layout and rules above, plus
+ *   weights  device f32 [sum(L)], one weight per entry of values, in the same order, whatever the table storage.
+ *            Null only when the batch has no lookup.  Weights go with sum pooling only (these calls take no pooling
+ *            argument), as torch refuses per_sample_weights outside mode 'sum'.
+ * Forward: the pooled row of a bag starts at +0.0f; for j ascending over the bag, acc = fl(acc + fl(w_j * row_j)),
+ * the product and the sum rounded separately (never a fused multiply-add).  An empty bag gives +0.0f.  With every
+ * w_j = 1.0f the pooled rows are those of the unweighted sum, bit for bit.
+ * Update (dlrmb_embedding_update_sorted after the weighted sort, Flux.Descent): sorted entry j of table k contributes
+ * fl(dT[b(j)][slot0 + k] * w_j); the contributions of one row are added in ascending position, then
+ * row -= fl(lr * sum).  With every w_j = 1.0f the tables after the update are those of the unweighted sum.  The
+ * update and dlrmb_sort_dedup_export consume a weighted sort like any other; a later sort of any kind replaces it.
+ * dlrmb_check_indices_jagged checks a weighted batch as it is (it does not read the weights). */
+int32_t dlrmb_embedding_fwd_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                            const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                            const int64_t* L, float* out, int32_t slots, int32_t slot0,
+                                            dlrmb_stream stream);
+/* training form: the lookup, then the weighted sort for the coming update */
+int32_t dlrmb_embedding_fwd_sort_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                                 const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                                 const int64_t* L, float* out, int32_t slots, int32_t slot0,
+                                                 dlrmb_stream stream);
+int32_t dlrmb_embedding_sort_jagged_weighted(dlrmb_tables* t, const void* values, const void* offsets,
+                                             const float* weights, int32_t idx_bytes, int32_t idx_base, int32_t B,
+                                             const int64_t* L, dlrmb_stream stream);
+/* Gradient of the pooled rows with respect to the weights (per_sample_weights.grad):
+ *   dw[j] = sum over d of dT[b][slot0 + k][d] * table_k[values[j]][d]   for entry j of bag b of table k,
+ * dw device f32 [sum(L)] in the order of values (null only when the batch has no lookup), dT [B][slots][D] as for the
+ * update (16-byte aligned when D % 4 == 0).  The rows are read as they are now, so call it before
+ * dlrmb_embedding_update_sorted of the same batch to get the gradient of the forward's rows.  A bag with no entries
+ * writes nothing.  Order of the sum, fixed by D alone: with V = 4 if D % 4 == 0 else 1, C = D / V chunks of V
+ * floats and G = min(32, C rounded up to a power of two), partial l (0 <= l < G) adds the products of chunks
+ * c = l, l + G, l + 2G, .. in ascending d, p_l = fl(p_l + fl(dT[d] * row[d])) from +0.0f; then for s = G/2, G/4,
+ * .., 1: p_l = fl(p_l + p_(l xor s)) for every l; dw[j] = p_0.  Bit-identical from call to call.  It does not
+ * read the weights.  Allocates nothing, does not synchronise, can be captured into a CUDA graph. */
+int32_t dlrmb_embedding_weight_grad_jagged(dlrmb_tables* t, const void* values, const void* offsets, int32_t idx_bytes,
+                                           int32_t idx_base, int32_t B, const int64_t* L, const float* dT, int32_t slots,
+                                           int32_t slot0, float* dw, dlrmb_stream stream);
+
 /* ---- loss: the top MLP's final sigmoid (src/model/model.jl:87-90) fused with bce_loss and its
  * pullback (src/train/train.jl:33-41, 45-71).  logits/labels [B] device f32.  Writes the mean loss
  * (one float), d(loss)/d(logit) [B] (sensitivity 1 folded in) and, if `prob` is non-NULL, the
