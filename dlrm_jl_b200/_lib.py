@@ -78,6 +78,16 @@ SIGNATURES = {
     "dlrmb_indices_scatter_p2p_mp": (_i32, [_i32, _vp, _i32, _i32, _i32, C.POINTER(_i32), _vp, _i32, _vp]),
     "dlrmb_indices_scatter_p2p_mp_list": (_i32, [_i32, _vp, _i32, _i32, _i32, C.POINTER(_i32), _i32, C.POINTER(_i32),
                                                  _vp, _i32, _vp]),
+    # values, offsets, weights, idx_bytes, ntab, B_local, owner[ntab], L_all[world][ntab], world, rank, peer_values,
+    # peer_offsets, peer_weights, cap_values[world], stream
+    "dlrmb_indices_scatter_p2p_jagged": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i32), C.POINTER(_i64),
+                                                _i32, _i32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp),
+                                                C.POINTER(_i64), _vp]),
+    # values, offsets, weights, idx_bytes, idx_base, B_global, L[ntab], pooling, peer_T, world, B_local, slots, stream
+    "dlrmb_embedding_fwd_p2p_jagged": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i64), _i32, C.POINTER(_vp),
+                                              _i32, _i32, _i32, _vp]),
+    "dlrmb_embedding_fwd_p2p_sort_jagged": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, C.POINTER(_i64), _i32,
+                                                   C.POINTER(_vp), _i32, _i32, _i32, _vp]),
     "dlrmb_interaction_has_warp_path": (_i32, [_i32, _i32]),
     "dlrmb_dense_fwd_bias_act": (_i32, [_i32, _vp, _vp, _i32, _i32, _i32, _vp]),
     "dlrmb_dense_bwd_scratch_floats": (_i64, [_i32]),

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 LIB_DIR = os.path.join(os.path.dirname(HERE), "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libdlrm_b200.so")
 SOURCES = ["api.cu", "lookup.cu", "interact.cu", "interact_warp.cu", "sort.cu", "update.cu", "loss.cu", "dense.cu", "p2p.cu", "loader.cu", "comm.cu"]
-HEADERS = [os.path.join(HERE, "common.cuh"), os.path.join(HERE, "sort_small.cuh"), os.path.join(ROOT, "include", "dlrm_b200.h")]
+HEADERS = [os.path.join(HERE, "common.cuh"), os.path.join(HERE, "sort_small.cuh"), os.path.join(HERE, "pool_bag.cuh"), os.path.join(ROOT, "include", "dlrm_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

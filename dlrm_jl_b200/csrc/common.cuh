@@ -294,6 +294,8 @@ constexpr int kJaggedWeighted = 2;
 int launch_lookup_jagged(dlrmb_tables* t, const void* values, const void* offsets, const float* weights, int idx_bytes,
                          int idx_base, const MpGeom& g, int B, int pooling, float* out, int slots, int slot0,
                          cudaStream_t s);
+// CTAs per table of a jagged lookup over B bags per table (fills g.pre from g.P = L); returns the total
+int64_t lookup_grid_jagged(const dlrmb_tables* t, MpGeom& g, uint32_t B, uint32_t C);
 // after a jagged sort into half `half`: bag id (and, with mean pooling, weight 1/n as f32 bits; with per-sample
 // weights, the entry's weight) of every sorted entry into pos[half ^ 1] (and keys[half ^ 1])
 int launch_jagged_bags(dlrmb_tables* t, const void* offsets, const float* weights, int idx_bytes, const MpGeom& g,

@@ -7,8 +7,10 @@
 //
 // New functionality (DLRM.jl is single-process); BASELINE.json north_star / SURVEY.md section 8(e).
 #include "common.cuh"
+#include "pool_bag.cuh"
 #include "sort_small.cuh"
 
+#include <algorithm>
 #include <vector>
 
 struct dlrmb_xbuf {
@@ -198,6 +200,88 @@ static int launch_p2p_mp_i(dlrmb_tables* t, const IdxT* idx, int idx_base, const
                            : launch_p2p_mp_t<IdxT, 4, RowT, 16>(t, idx, idx_base, gs, peers, B_local, slots, half, s);
     if (rc) return rc;
     return launch_sort_mp(t, idx, (int)sizeof(IdxT), idx_base, g, kFusedSortMax, half, s);
+}
+
+
+// Jagged bags (variable length, dlrmb_embedding_fwd_p2p_jagged): the grid and thread mapping of lookup_jagged_kernel
+// (lookup_grid_jagged, one thread per (bag, 16-byte chunk)) and its pool_bag call, so the pooled rows are those of
+// dlrmb_embedding_fwd_jagged / _jagged_weighted bit for bit; the epilogue of lookup_p2p_mp_cta stores bag b of table k
+// at peers.p[b / B_local] + (b % B_local) * ostride + dstoff[k].  MODE: 0 sum, 1 mean (times fl(1 / n)),
+// kJaggedWeighted (row j scaled by weights[j] before it is added).  An empty bag stores +0.0f.
+template <typename IdxT, int VEC, typename RowT, int MODE>
+__global__ void __launch_bounds__(256)
+lookup_p2p_jagged_kernel(const TableDesc* __restrict__ desc, const int32_t* __restrict__ dstoff,
+                         const IdxT* __restrict__ values, const IdxT* __restrict__ offsets,
+                         const float* __restrict__ weights, int idx_base, const __grid_constant__ MpGeom g, uint32_t B,
+                         uint32_t C, int cshift, uint32_t B_local, const __grid_constant__ PeerPtrs peers,
+                         long long ostride, unsigned long long* clk) {
+    using V = typename Vec<VEC>::type;
+    clock_in(clk, blockIdx.x);
+    const int k = mp_find(g.pre, g.ntab, blockIdx.x);
+    const uint32_t cta = blockIdx.x - g.pre[k], nctas = g.pre[k + 1] - g.pre[k];
+    const float* __restrict__ tb = desc[k].base;
+    const IdxT* __restrict__ ok = offsets + (size_t)k * B;
+    const uint32_t n = B * C;
+    const uint32_t step = nctas * blockDim.x;
+    const size_t D = (size_t)C * VEC;
+    const size_t slot_off = (size_t)dstoff[k];
+    for (uint32_t t = cta * blockDim.x + threadIdx.x; t < n; t += step) {
+        const uint32_t b = cshift >= 0 ? (t >> cshift) : (t / C);
+        const uint32_t c = t - b * C;
+        const int64_t o0 = (int64_t)__ldg(ok + b), o1 = (int64_t)__ldg(ok + b + 1);
+        V acc;
+        if constexpr (MODE == kJaggedWeighted) {
+            acc = pool_bag<IdxT, VEC, RowT, true>(tb, values + o0, (uint32_t)(o1 - o0), idx_base, D, c, weights + o0);
+        } else {
+            acc = pool_bag<IdxT, VEC, RowT>(tb, values + o0, (uint32_t)(o1 - o0), idx_base, D, c);
+            if (MODE == 1 && o1 > o0) acc = Vec<VEC>::scale(acc, __fdiv_rn(1.0f, (float)(o1 - o0)));
+        }
+        const uint32_t h = b / B_local;
+        const uint32_t bl = b - h * B_local;
+        reinterpret_cast<V*>(peers.p[h] + (size_t)bl * ostride + slot_off)[c] = acc;
+    }
+    clock_out(clk, blockIdx.x);
+}
+
+template <typename IdxT, int VEC, typename RowT>
+static int launch_p2p_jagged_t(dlrmb_tables* t, const IdxT* values, const IdxT* offsets, const float* weights,
+                               int idx_base, const MpGeom& g0, int B, int mode, const PeerPtrs& peers, int B_local,
+                               int slots, cudaStream_t s) {
+    const uint32_t C = t->D / VEC;
+    const int64_t n = (int64_t)B * C;
+    DLRMB_REQUIRE(n < (1ll << 30), "B * D too large for one lookup launch (%lld chunks)", (long long)n);
+    MpGeom g = g0;
+    const int64_t ctas = lookup_grid_jagged(t, g, (uint32_t)B, C);
+    int cshift = -1;
+    if ((C & (C - 1)) == 0)
+        for (cshift = 0; (1u << cshift) < C; ++cshift) {}
+    const long long ostride = (long long)slots * t->dest_D;
+#define DLRMB_P2P_JAGGED(MODE)                                                                                      \
+    lookup_p2p_jagged_kernel<IdxT, VEC, RowT, MODE><<<(unsigned)ctas, 256, 0, s>>>(                                 \
+        t->d_desc, t->d_slotmap, values, offsets, weights, idx_base, g, (uint32_t)B, C, cshift, (uint32_t)B_local, \
+        peers, ostride, clock_slot(CLK_LOOKUP))
+    if (mode == kJaggedWeighted) DLRMB_P2P_JAGGED(kJaggedWeighted);
+    else if (mode == 1) DLRMB_P2P_JAGGED(1);
+    else DLRMB_P2P_JAGGED(0);
+#undef DLRMB_P2P_JAGGED
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+template <typename RowT>
+static int launch_p2p_jagged_r(dlrmb_tables* t, const void* values, const void* offsets, const float* w, int idx_bytes,
+                               int idx_base, const MpGeom& g, int B, int mode, const PeerPtrs& peers, int B_local,
+                               int slots, bool vec4, cudaStream_t s) {
+    if (idx_bytes == 4) {
+        const uint32_t* v = static_cast<const uint32_t*>(values);
+        const uint32_t* o = static_cast<const uint32_t*>(offsets);
+        return vec4 ? launch_p2p_jagged_t<uint32_t, 4, RowT>(t, v, o, w, idx_base, g, B, mode, peers, B_local, slots, s)
+                    : launch_p2p_jagged_t<uint32_t, 1, RowT>(t, v, o, w, idx_base, g, B, mode, peers, B_local, slots, s);
+    }
+    const int64_t* v = static_cast<const int64_t*>(values);
+    const int64_t* o = static_cast<const int64_t*>(offsets);
+    return vec4 ? launch_p2p_jagged_t<int64_t, 4, RowT>(t, v, o, w, idx_base, g, B, mode, peers, B_local, slots, s)
+                : launch_p2p_jagged_t<int64_t, 1, RowT>(t, v, o, w, idx_base, g, B, mode, peers, B_local, slots, s);
 }
 
 }  // namespace dlrmb
@@ -418,6 +502,65 @@ int32_t dlrmb_embedding_fwd_p2p_sort_mp(dlrmb_tables* t, const void* idx, int32_
                                      stream);
 }
 
+// The jagged owner batch at B_global (dlrmb_indices_scatter_p2p_jagged / exchange_indices_jagged fill it): checked as
+// dlrmb_embedding_fwd_jagged (weights: pooling 0 only) plus the p2p arguments, then the fused lookup; the training
+// form follows it with the jagged sort of the same batch (dlrmb_embedding_sort_jagged / _weighted).
+static int32_t embedding_fwd_p2p_jagged_impl(dlrmb_tables* t, const void* values, const void* offsets,
+                                             const float* weights, int32_t idx_bytes, int32_t idx_base,
+                                             int32_t B_global, const int64_t* L, int32_t pooling, float* const* peer_T,
+                                             int32_t world, int32_t B_local, int32_t slots, bool with_sort,
+                                             dlrmb_stream stream) {
+    DLRMB_REQUIRE(t != nullptr && peer_T != nullptr, "null argument");
+    DLRMB_REQUIRE(weights == nullptr || pooling == 0,
+                  "per-sample weights go with pooling = 0 (sum) only (got pooling = %d)", pooling);
+    MpGeom g;
+    int rc = check_jagged_args(t, values, offsets, idx_bytes, idx_base, B_global, L, pooling, &g);
+    if (rc) return rc;
+    DLRMB_REQUIRE(world >= 1 && world <= kMaxPeers, "world must be in 1..%d (got %d)", kMaxPeers, world);
+    DLRMB_REQUIRE(B_local > 0 && (int64_t)B_global == (int64_t)B_local * world,
+                  "B_global (%d) must equal B_local (%d) * world (%d)", B_global, B_local, world);
+    if (!t->d_slotmap) {
+        set_error("dlrmb_embedding_fwd_p2p_jagged needs dlrmb_tables_set_slot_map first");
+        return DLRMB_ESTATE;
+    }
+    DLRMB_REQUIRE(slots > t->slotmap_max, "slots = %d does not cover the slot map (largest slot %d)", slots,
+                  t->slotmap_max);
+    DeviceGuard guard(t->device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", t->device);
+    PeerPtrs peers;
+    bool vec4;
+    rc = peer_ptrs(t, peer_T, world, &peers, &vec4);
+    if (rc) return rc;
+    const int mode = weights ? kJaggedWeighted : pooling;
+    cudaStream_t s = (cudaStream_t)stream;
+    rc = t->elem_bytes == 2
+             ? launch_p2p_jagged_r<__nv_bfloat16>(t, values, offsets, weights, idx_bytes, idx_base, g, B_global, mode,
+                                                  peers, B_local, slots, vec4, s)
+             : launch_p2p_jagged_r<float>(t, values, offsets, weights, idx_bytes, idx_base, g, B_global, mode, peers,
+                                          B_local, slots, vec4, s);
+    if (rc || !with_sort) return rc;
+    return weights ? dlrmb_embedding_sort_jagged_weighted(t, values, offsets, weights, idx_bytes, idx_base, B_global, L,
+                                                          stream)
+                   : dlrmb_embedding_sort_jagged(t, values, offsets, idx_bytes, idx_base, B_global, L, pooling, stream);
+}
+
+int32_t dlrmb_embedding_fwd_p2p_jagged(dlrmb_tables* t, const void* values, const void* offsets, const float* weights,
+                                       int32_t idx_bytes, int32_t idx_base, int32_t B_global, const int64_t* L,
+                                       int32_t pooling, float* const* peer_T, int32_t world, int32_t B_local,
+                                       int32_t slots, dlrmb_stream stream) {
+    return embedding_fwd_p2p_jagged_impl(t, values, offsets, weights, idx_bytes, idx_base, B_global, L, pooling, peer_T,
+                                         world, B_local, slots, false, stream);
+}
+
+int32_t dlrmb_embedding_fwd_p2p_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets,
+                                            const float* weights, int32_t idx_bytes, int32_t idx_base,
+                                            int32_t B_global, const int64_t* L, int32_t pooling, float* const* peer_T,
+                                            int32_t world, int32_t B_local, int32_t slots, dlrmb_stream stream) {
+    if (t) t->sorted_valid = false;
+    return embedding_fwd_p2p_jagged_impl(t, values, offsets, weights, idx_bytes, idx_base, B_global, L, pooling, peer_T,
+                                         world, B_local, slots, true, stream);
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------
@@ -533,6 +676,66 @@ indices_scatter_list_kernel(const IdxT* __restrict__ idx_local, const IdxDest* _
     const IdxT* src = idx_local + g.src_off[k];
     IdxT* dst = static_cast<IdxT*>(dests[blockIdx.y].base) + (size_t)rank * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = src[i];
+}
+
+// Jagged bags: this rank's batch (values / weights table-major, offsets [ntab * B_local + 1]) into the owners' jagged
+// batches over the global batch (dlrmb_indices_scatter_p2p_jagged).  Block row y = table k: this rank's n[k] entries of
+// k go to element dst_off[k] of its owner's values (and weights), its B_local offsets, rebased by dst_off[k] -
+// src_off[k], to entries bag0[k] + rank * B_local .. of the owner's offsets; the last rank also writes the closing
+// entry bag0[k] + B_global = end of k's block.  The geometry goes by value.
+struct IdxScatterJaggedGeom {
+    int B_local;
+    int B_global;
+    int rank;
+    int last;                                // rank == world - 1
+    void* values[kMaxPeers];                 // owners' buffers (peer mappings)
+    void* offsets[kMaxPeers];
+    float* weights[kMaxPeers];
+    int64_t src_off[kMpMaxTables];           // table k's first entry in this rank's values
+    int64_t dst_off[kMpMaxTables];           // where this rank's entries of table k land in the owner's values
+    int64_t close[kMpMaxTables];             // end of table k's block in the owner's values
+    uint32_t n[kMpMaxTables];                // this rank's lookups of table k
+    uint32_t bag0[kMpMaxTables];             // j * B_global: table k's first bag in the owner's offsets
+    uint8_t owner[kMpMaxTables];
+};
+
+// dst[0 .. n) = src[0 .. n) by the grid's threads `tid` of `nth`: 16-byte copies after a scalar head when source and
+// destination share their offset inside 16 bytes, one element at a time otherwise
+template <typename T>
+__device__ __forceinline__ void copy_elems(T* __restrict__ dst, const T* __restrict__ src, int64_t n, uint32_t tid,
+                                           uint32_t nth) {
+    constexpr int E = 16 / sizeof(T);
+    const uintptr_t sa = reinterpret_cast<uintptr_t>(src) & 15, da = reinterpret_cast<uintptr_t>(dst) & 15;
+    int64_t head = n;
+    if (sa == da) {
+        head = (int64_t)(((16 - sa) & 15) / sizeof(T));
+        if (head > n) head = n;
+    }
+    for (int64_t i = tid; i < head; i += nth) dst[i] = src[i];
+    if (head == n) return;
+    const int64_t nv = (n - head) / E;
+    const int4* __restrict__ s4 = reinterpret_cast<const int4*>(src + head);
+    int4* __restrict__ d4 = reinterpret_cast<int4*>(dst + head);
+    for (int64_t i = tid; i < nv; i += nth) d4[i] = __ldg(s4 + i);
+    for (int64_t i = head + nv * E + tid; i < n; i += nth) dst[i] = src[i];
+}
+
+template <typename IdxT>
+__global__ void __launch_bounds__(256)
+indices_scatter_jagged_kernel(const IdxT* __restrict__ values, const IdxT* __restrict__ offsets,
+                              const float* __restrict__ weights, const __grid_constant__ IdxScatterJaggedGeom g) {
+    const int k = blockIdx.y;
+    const int o = g.owner[k];
+    const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
+    copy_elems(static_cast<IdxT*>(g.values[o]) + g.dst_off[k], values + g.src_off[k], (int64_t)g.n[k], tid, nth);
+    if (weights != nullptr)
+        copy_elems(g.weights[o] + g.dst_off[k], weights + g.src_off[k], (int64_t)g.n[k], tid, nth);
+    IdxT* __restrict__ od = static_cast<IdxT*>(g.offsets[o]) + g.bag0[k];
+    const IdxT* __restrict__ os = offsets + (size_t)k * g.B_local;
+    const int64_t delta = g.dst_off[k] - g.src_off[k];
+    for (uint32_t i = tid; i < (uint32_t)g.B_local; i += nth)
+        od[(size_t)g.rank * g.B_local + i] = (IdxT)((int64_t)os[i] + delta);
+    if (g.last && tid == 0) od[g.B_global] = (IdxT)g.close[k];
 }
 
 }  // namespace dlrmb
@@ -651,6 +854,90 @@ int32_t dlrmb_indices_scatter_p2p_mp_list(int32_t device, const void* idx_local,
         indices_scatter_list_kernel<uint32_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)idx_local, d, g, rank);
     else
         indices_scatter_list_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>((const int64_t*)idx_local, d, g, rank);
+    DLRMB_LAUNCH_CHECK();
+    return DLRMB_OK;
+}
+
+int32_t dlrmb_indices_scatter_p2p_jagged(int32_t device, const void* values, const void* offsets, const float* weights,
+                                         int32_t idx_bytes, int32_t ntab, int32_t B_local, const int32_t* owner,
+                                         const int64_t* L_all, int32_t world, int32_t rank, void* const* peer_values,
+                                         void* const* peer_offsets, float* const* peer_weights,
+                                         const int64_t* cap_values, dlrmb_stream stream) {
+    DLRMB_REQUIRE(offsets && owner && L_all && peer_values && peer_offsets && cap_values, "null argument");
+    DLRMB_REQUIRE(idx_bytes == 4 || idx_bytes == 8, "idx_bytes must be 4 or 8 (got %d)", idx_bytes);
+    DLRMB_REQUIRE(ntab > 0 && ntab <= kMpMaxTables, "ntab must be in 1..%d (got %d)", kMpMaxTables, ntab);
+    DLRMB_REQUIRE(world >= 1 && world <= kMaxPeers && rank >= 0 && rank < world, "bad world / rank (%d, %d)", world,
+                  rank);
+    DLRMB_REQUIRE(B_local > 0, "B_local must be positive (got %d)", B_local);
+    DLRMB_REQUIRE((weights == nullptr) == (peer_weights == nullptr),
+                  "weights and peer_weights must be both null or both set");
+    const int64_t Bg = (int64_t)B_local * world;
+    const int64_t lim = idx_bytes == 4 ? INT32_MAX : INT64_MAX;
+    IdxScatterJaggedGeom g;
+    g.B_local = B_local;
+    g.B_global = (int)Bg;
+    g.rank = rank;
+    g.last = rank == world - 1;
+    int64_t tables[kMaxPeers] = {0}, total[kMaxPeers] = {0};     // per owner: tables owned, entries of its batch
+    for (int k = 0; k < ntab; ++k) {
+        DLRMB_REQUIRE(owner[k] >= 0 && owner[k] < world, "owner[%d] = %d is not a rank (world %d)", k, owner[k], world);
+        for (int h = 0; h < world; ++h)
+            DLRMB_REQUIRE(L_all[(size_t)h * ntab + k] >= 0, "L_all[%d][%d] = %lld: lookup counts must be >= 0", h, k,
+                          (long long)L_all[(size_t)h * ntab + k]);
+    }
+    int64_t src = 0, mine = 0;
+    for (int k = 0; k < ntab; ++k) {           // ascending k = ascending j inside every owner
+        const int o = owner[k];
+        int64_t before = 0, sum = 0;
+        for (int h = 0; h < world; ++h) {
+            const int64_t n = L_all[(size_t)h * ntab + k];
+            if (h < rank) before += n;
+            sum += n;
+        }
+        const int64_t n = L_all[(size_t)rank * ntab + k];
+        DLRMB_REQUIRE(n < (1ll << 32), "L_all[%d][%d] too large", rank, k);
+        g.owner[k] = (uint8_t)o;
+        g.src_off[k] = src;
+        g.n[k] = (uint32_t)n;
+        g.dst_off[k] = total[o] + before;
+        g.bag0[k] = (uint32_t)(tables[o] * Bg);
+        total[o] += sum;
+        g.close[k] = total[o];
+        tables[o] += 1;
+        src += n;
+        mine += n;
+        DLRMB_REQUIRE(tables[o] * Bg < INT32_MAX, "owner %d: %lld tables of %lld bags overflow the offsets", o,
+                      (long long)tables[o], (long long)Bg);
+    }
+    DLRMB_REQUIRE(values != nullptr || mine == 0, "values is null");
+    for (int o = 0; o < world; ++o) {
+        g.values[o] = g.offsets[o] = nullptr;
+        g.weights[o] = nullptr;
+        if (tables[o] == 0) continue;
+        DLRMB_REQUIRE(total[o] <= cap_values[o], "owner %d receives %lld entries, its buffer holds cap_values[%d] = %lld",
+                      o, (long long)total[o], o, (long long)cap_values[o]);
+        DLRMB_REQUIRE(total[o] <= lim, "owner %d receives %lld entries: 4-byte offsets reach 2^31", o,
+                      (long long)total[o]);
+        DLRMB_REQUIRE(peer_values[o] != nullptr && peer_offsets[o] != nullptr, "owner %d's buffers are null", o);
+        DLRMB_REQUIRE(peer_weights == nullptr || peer_weights[o] != nullptr, "peer_weights[%d] is null", o);
+        g.values[o] = peer_values[o];
+        g.offsets[o] = peer_offsets[o];
+        g.weights[o] = peer_weights ? peer_weights[o] : nullptr;
+    }
+    DeviceGuard guard(device);
+    DLRMB_REQUIRE(guard.ok, "cudaSetDevice(%d) failed", device);
+    int64_t most = B_local;                   // work items of the largest table: offsets, or 16-byte value copies
+    for (int k = 0; k < ntab; ++k) most = std::max(most, (int64_t)g.n[k] * idx_bytes / 16);
+    int bx = (int)((most + 255) / 256);
+    if (bx > 64) bx = 64;
+    dim3 grid((unsigned)bx, (unsigned)ntab);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (idx_bytes == 4)
+        indices_scatter_jagged_kernel<uint32_t><<<grid, 256, 0, s>>>((const uint32_t*)values, (const uint32_t*)offsets,
+                                                                     weights, g);
+    else
+        indices_scatter_jagged_kernel<int64_t><<<grid, 256, 0, s>>>((const int64_t*)values, (const int64_t*)offsets,
+                                                                    weights, g);
     DLRMB_LAUNCH_CHECK();
     return DLRMB_OK;
 }

@@ -406,15 +406,25 @@ class EmbeddingTables:
         the owning rank's interaction buffer (NVLink peer stores): lookup + forward exchange fused.
         ``sort=True`` also sorts / dedups the indices for this batch's sparse update in the same launch
         (dlrmb_embedding_fwd_p2p_sort).  ``idx`` may be :class:`PackedIndices` at B_global (per-table
-        pooling factors, dlrmb_embedding_fwd_p2p_mp / _sort_mp)."""
+        pooling factors, dlrmb_embedding_fwd_p2p_mp / _sort_mp) or :class:`JaggedIndices` at B_global (the owner batch
+        of variable-length bags, sum, mean or weighted; dlrmb_embedding_fwd_p2p_jagged / _sort_jagged)."""
+        world = len(peer_ptrs)
+        arr = (C.c_void_p * world)(*[int(p) for p in peer_ptrs])
+        if isinstance(idx, JaggedIndices):
+            fn = self._lib.dlrmb_embedding_fwd_p2p_sort_jagged if sort else self._lib.dlrmb_embedding_fwd_p2p_jagged
+            w = None if idx.weights is None else idx.weights.data_ptr() or None
+            with _prof.range("lookup"):
+                _lib.check(fn(self._h, idx.values.data_ptr(), idx.offsets.data_ptr(), w, idx.element_size(), idx_base,
+                              idx.B, idx.L_array(), idx.pooling_code, arr, world, B_local, slots, _stream_ptr(self.device)))
+            if sort:
+                self._pending_side = False
+            return
         if isinstance(idx, PackedIndices):
             Bg, P = idx.B, idx.P_array()
             fn = self._lib.dlrmb_embedding_fwd_p2p_sort_mp if sort else self._lib.dlrmb_embedding_fwd_p2p_mp
         else:
             ntab, Bg, P = idx.shape
             fn = self._lib.dlrmb_embedding_fwd_p2p_sort if sort else self._lib.dlrmb_embedding_fwd_p2p
-        world = len(peer_ptrs)
-        arr = (C.c_void_p * world)(*[int(p) for p in peer_ptrs])
         with _prof.range("lookup"):
             _lib.check(fn(self._h, idx.data_ptr(), idx.element_size(), idx_base, Bg, P, arr, world, B_local, slots,
                           _stream_ptr(self.device)))

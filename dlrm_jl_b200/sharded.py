@@ -251,6 +251,85 @@ def exchange_indices_mp(packed, sh: TableSharding, rank: int, group=None):
     return PackedIndices(owned.contiguous(), tuple(P[k] for k in mine), Bl * W)
 
 
+def gloo_group(group=None):
+    """``group`` when it runs on gloo, else a new gloo group over every rank of the job.  The per-step lookup counts of
+    jagged batches travel over it, so the host never waits on the device.  ``dist.new_group`` must be entered by every
+    rank of the default group, which the ranks of a proper subgroup cannot arrange among themselves: a non-gloo
+    ``group`` must span the whole job (pass a gloo group otherwise)."""
+    if dist.get_backend(group) == "gloo":
+        return group
+    if group is not None and dist.get_world_size(group) != dist.get_world_size():
+        raise ValueError(f"the lookup counts of jagged batches travel over a gloo group, and group (backend "
+                         f"{dist.get_backend(group)}, {dist.get_world_size(group)} of {dist.get_world_size()} ranks) is "
+                         "neither gloo nor the whole job: pass count_group, a gloo group over the same ranks")
+    return dist.new_group(backend="gloo")
+
+
+def exchange_jagged_counts(jag_local, group=None) -> np.ndarray:
+    """Every rank's lookup counts of this step: [world][ntab] int64, row h = rank h's ``L``.  ``jag_local`` is this
+    rank's :class:`~dlrm_jl_b200.embedding.JaggedIndices`; ``group`` a gloo (CPU) group.  The jagged kernels size
+    their grids from host counts, so an owner needs the counts of its tables summed over the ranks and a sender the
+    counts of the ranks before it.  Every rank raises ValueError when the ranks disagree on B_local, the pooling or
+    whether the batch is weighted."""
+    W = dist.get_world_size(group)
+    mine = torch.tensor(list(jag_local.L) + [jag_local.B, jag_local.pooling_code, int(jag_local.weights is not None)],
+                        dtype=torch.int64)
+    got = [torch.empty_like(mine) for _ in range(W)]
+    dist.all_gather(got, mine, group=group)
+    a = torch.stack(got).numpy()
+    if (a[:, -3:] != a[0, -3:]).any():
+        desc = [f"rank {h}: B_local {r[-3]}, pooling {'mean' if r[-2] else 'sum'}, {'weighted' if r[-1] else 'unweighted'}"
+                for h, r in enumerate(a)]
+        raise ValueError("the ranks' jagged batches disagree on B_local, pooling or weighting: " + "; ".join(desc))
+    return a[:, :-3].copy()
+
+
+def exchange_indices_jagged(jag_local, counts: np.ndarray, sh: TableSharding, rank: int, group=None):
+    """Jagged bags: ``jag_local`` (:class:`~dlrm_jl_b200.embedding.JaggedIndices` of this rank's B_local bags per
+    table, every table) -> this rank's tables in the owner layout, a JaggedIndices at B_global = world * B_local of the
+    owned tables in ascending id: table j's entries after those of the owned tables before it, rank h's entries inside
+    them after those of the ranks before h, in their own order; bag j * B_global + h * B_local + b is rank h's bag b;
+    weights beside their values.  ``counts`` is :func:`exchange_jagged_counts`'s [world][ntab].  Values, bag lengths
+    and weights travel with three all-to-alls; the owner rebuilds its offsets by a cumulative sum.  The owner's jagged
+    lookup, sort and update read the result as is."""
+    from .embedding import JaggedIndices
+    W = sh.world
+    if W == 1:
+        return jag_local
+    Bl, L = jag_local.B, jag_local.L
+    counts = np.asarray(counts, dtype=np.int64)
+    mine = sh.local[rank]
+    t = len(mine)
+    dev = jag_local.values.device
+    starts = np.concatenate([[0], np.cumsum(L)]).tolist()
+    order = [k for r in range(W) for k in sh.local[r]]                                  # grouped by owner
+    lengths = (jag_local.offsets[1:] - jag_local.offsets[:-1]).view(len(L), Bl)
+    in_splits = [int(sum(L[k] for k in sh.local[r])) for r in range(W)]
+    out_splits = [int(counts[h, mine].sum()) for h in range(W)]
+
+    def values_a2a(flat):
+        send = torch.cat([flat[starts[k]:starts[k + 1]] for k in order]) if order else flat[:0]
+        recv = torch.empty((sum(out_splits),), dtype=flat.dtype, device=dev)
+        _a2a(recv, send.contiguous(), out_splits, in_splits, group)
+        # [h][j][entries] -> [j][h][entries]
+        parts, base = [], np.concatenate([[0], np.cumsum(out_splits)]).tolist()
+        inner = np.concatenate([np.zeros((W, 1), np.int64), np.cumsum(counts[:, mine], axis=1)], axis=1)
+        for j in range(t):
+            parts.extend(recv[base[h] + inner[h, j]:base[h] + inner[h, j + 1]] for h in range(W))
+        return torch.cat(parts) if parts else recv[:0]
+
+    values = values_a2a(jag_local.values)
+    weights = None if jag_local.weights is None else values_a2a(jag_local.weights)
+    send_n = lengths.index_select(0, sh.owner_order(dev)).reshape(-1).contiguous()
+    recv_n = torch.empty((W * t * Bl,), dtype=lengths.dtype, device=dev)
+    _a2a(recv_n, send_n, [t * Bl] * W, [len(sh.local[r]) * Bl for r in range(W)], group)
+    n_own = recv_n.view(W, t, Bl).permute(1, 0, 2).reshape(-1)
+    offsets = torch.zeros((t * W * Bl + 1,), dtype=jag_local.offsets.dtype, device=dev)
+    offsets[1:] = torch.cumsum(n_own, 0).to(offsets.dtype)
+    L_own = tuple(int(counts[:, k].sum()) for k in mine)
+    return JaggedIndices(values.contiguous(), offsets, L_own, Bl * W, jag_local.pooling, weights)
+
+
 def exchange_pooled(pooled: torch.Tensor, T: torch.Tensor, sh: TableSharding, rank: int, group=None) -> None:
     """pooled [B_global][t_mine][D] (owner side) -> T[:, 1 + k, :] for every table k, on the rank
     that owns the samples.  T is [B_local][1 + ntab][D]; slot 0 is left for x."""
@@ -418,6 +497,7 @@ class PeerExchange:
         self._ibuf = None
         self.idx_owned = None
         self._idx_dests = None
+        self._jag = None
         if barrier is None and flag_barrier:
             # ordering without NCCL: a flag array per rank, mapped by every peer (dlrmb_peer_barrier)
             self._fbuf, _own, self.peer_flag_ptrs = self._share(int(self.lib.dlrmb_peer_barrier_flag_bytes()))
@@ -511,6 +591,79 @@ class PeerExchange:
         self._idx_geom = (len(sharding.rows), B_local, P, idx_bytes)
         self._idx_P = (C.c_int32 * len(P))(*P)
 
+    def enable_jagged_index_exchange(self, sharding: "TableSharding", B_local: int, cap: Sequence[int],
+                                     idx_bytes: int = 4, weighted: bool = False) -> None:
+        """Index exchange of jagged batches by peer stores (:meth:`scatter_jagged`).  ``cap[k]`` is the most lookups of
+        table k in one rank's local batch.  Every rank allocates, and maps on every peer, the buffers of its owner
+        batch: values of world * (sum of cap over its tables) entries, offsets of t * B_global + 1 entries (t tables,
+        the width of the indices) and, with ``weighted``, one f32 weight per value."""
+        import ctypes as C
+
+        from .embedding import _DevicePtrView
+        if sharding.split:
+            raise ValueError("jagged batches support table-wise plans only (a column-wise plan splits a table)")
+        ntab, W = len(sharding.rows), self.world
+        cap = tuple(int(c) for c in cap)
+        if len(cap) != ntab or min(cap) < 0:
+            raise ValueError(f"cap must hold one lookup count >= 0 per table ({ntab} tables), got {list(cap)}")
+        Bg = B_local * W
+        cap_own = [W * sum(cap[k] for k in sharding.local[o]) for o in range(W)]
+        n_val, n_off = cap_own[self.rank], len(sharding.local[self.rank]) * Bg + 1
+        ts = "<i4" if idx_bytes == 4 else "<i8"
+        _h, own_v, peer_v = self._share(max(1, n_val) * idx_bytes)
+        _h, own_o, peer_o = self._share(n_off * idx_bytes)
+        self._jag_values = torch.as_tensor(_DevicePtrView(own_v, (max(1, n_val),), self, ts), device=self.device)
+        self._jag_offsets = torch.as_tensor(_DevicePtrView(own_o, (n_off,), self, ts), device=self.device)
+        self._jag_weights, peer_w = None, None
+        if weighted:
+            _h, own_w, peer_w = self._share(max(1, n_val) * 4)
+            self._jag_weights = torch.as_tensor(_DevicePtrView(own_w, (max(1, n_val),), self), device=self.device)
+            peer_w = (C.c_void_p * W)(*peer_w)
+        self._jag = {"ntab": ntab, "B_local": B_local, "idx_bytes": idx_bytes, "cap": np.array(cap, dtype=np.int64),
+                     "mine": list(sharding.local[self.rank]), "owner": (C.c_int32 * ntab)(*sharding.owner),
+                     "peer_values": (C.c_void_p * W)(*peer_v), "peer_offsets": (C.c_void_p * W)(*peer_o),
+                     "peer_weights": peer_w, "cap_values": (C.c_int64 * W)(*cap_own),
+                     "empty": torch.zeros(4, dtype=torch.float32, device=self.device)}
+
+    def scatter_jagged(self, jag_local, counts: np.ndarray):
+        """This rank's :class:`~dlrm_jl_b200.embedding.JaggedIndices` -> the owners' buffers (peer stores, one launch)
+        + barrier; returns this rank's owner batch, the layout of :func:`exchange_indices_jagged`, as a JaggedIndices
+        view of its buffers.  ``counts``: :func:`exchange_jagged_counts`.  A batch over ``cap`` on any rank raises
+        ValueError on every rank, before any launch."""
+        import ctypes as C
+
+        from . import _lib, _prof
+        from .embedding import JaggedIndices
+        j = self._jag
+        counts = np.asarray(counts, dtype=np.int64)
+        if jag_local.B != j["B_local"] or jag_local.element_size() != j["idx_bytes"] or len(jag_local) != j["ntab"]:
+            raise ValueError(f"a jagged batch of {len(jag_local)} tables, B = {jag_local.B} and {jag_local.element_size()}-"
+                             f"byte indices, the exchange was set up for {j['ntab']} tables, B_local = {j['B_local']} "
+                             f"and {j['idx_bytes']}-byte indices")
+        if (jag_local.weights is not None) != (j["peer_weights"] is not None):
+            raise ValueError("the batch's per-sample weights do not match the exchange (enable_jagged_index_exchange("
+                             "weighted=...))")
+        over = np.argwhere(counts > j["cap"][None, :])
+        if len(over):
+            h, k = (int(x) for x in over[0])
+            raise ValueError(f"rank {h} has {int(counts[h, k])} lookups of table {k}, more than cap[{k}] = "
+                             f"{int(j['cap'][k])}")
+        W, ntab = self.world, j["ntab"]
+        L_all = (C.c_int64 * (W * ntab))(*counts.reshape(-1).tolist())
+        w = None
+        if jag_local.weights is not None:
+            w = jag_local.weights.data_ptr() or j["empty"].data_ptr()
+        with _prof.range("indices_scatter"):
+            _lib.check(self.lib.dlrmb_indices_scatter_p2p_jagged(
+                self.device.index or 0, jag_local.values.data_ptr() or None, jag_local.offsets.data_ptr(), w,
+                j["idx_bytes"], ntab, j["B_local"], j["owner"], L_all, W, self.rank, j["peer_values"],
+                j["peer_offsets"], j["peer_weights"], j["cap_values"], int(torch.cuda.current_stream(self.device).cuda_stream)))
+        self.barrier(0)
+        L_own = tuple(int(counts[:, k].sum()) for k in j["mine"])
+        n = sum(L_own)
+        return JaggedIndices(self._jag_values[:n], self._jag_offsets, L_own, j["B_local"] * W, jag_local.pooling,
+                             None if self._jag_weights is None else self._jag_weights[:n])
+
     def enable_small_allreduce(self, n: int) -> None:
         """Exchange buffer [2][world][n] floats for `allreduce_small` (dlrmb_peer_allreduce_f32)."""
         import ctypes as C
@@ -575,6 +728,7 @@ class PeerExchange:
                 if r != self.rank and q:
                     self.lib.dlrmb_xbuf_close(dev, q)
         self.T = self.G = self.idx_owned = None
+        self._jag = self._jag_values = self._jag_offsets = self._jag_weights = None
         for h in [self._xbuf] + self._owned:
             if h is not None:
                 self.lib.dlrmb_xbuf_destroy(h)
@@ -758,7 +912,8 @@ class ShardedEmbedding:
 
     def __init__(self, rows: Sequence[int], D: int, rank: int, world: int, lookup_fn: Callable,
                  update_fn: Callable, group=None, sort_fn: Optional[Callable] = None, idx_base: int = 0,
-                 lookup_sorts: bool = False, P: Optional[Sequence[int]] = None, max_col_shards: int = 1):
+                 lookup_sorts: bool = False, P: Optional[Sequence[int]] = None, max_col_shards: int = 1,
+                 jagged_cap: Optional[Sequence[int]] = None, count_group=None):
         """``idx_base``: 1 for reference-format (1-based) ids, 0 for PyTorch-style ids; it is handed to
         every kernel that reads the indices.  ``lookup_sorts``: `lookup_fn` also prepares the sort /
         dedup of the step's update (the fused launch), so `sort_async` has nothing left to do.
@@ -767,13 +922,27 @@ class ShardedEmbedding:
         (or anything ``_as_index_tensor`` turns into one) and the owners receive theirs in the owner layout
         of :func:`exchange_indices_mp`.  Without it every table has the same P and mixed widths are refused.
         ``max_col_shards``: split hot tables by columns into up to that many slices (a power of two, D divisible into
-        slices of a multiple of 4 columns); see :meth:`TableSharding.build`."""
+        slices of a multiple of 4 columns); see :meth:`TableSharding.build`.
+        ``jagged_cap``: the handle takes :class:`~dlrm_jl_b200.embedding.JaggedIndices` (variable-length bags, sum,
+        mean or weighted pooling), ``jagged_cap[k]`` being the most lookups of table k in one rank's local batch.  ``P``
+        then only weighs the tables in the plan: pass each table's expected bag length (at least 1), for instance the
+        MLPerf hotness list.  Every step starts with a host all-gather of the ranks' lookup counts
+        (:func:`exchange_jagged_counts`) over ``count_group`` if given, else over ``group`` when it runs on gloo, else
+        over a gloo group made here across the whole job (:func:`gloo_group`; a non-gloo proper subgroup needs
+        ``count_group``).  Column-wise plans of jagged tables are not supported."""
         self.P = None if P is None else tuple(int(p) for p in P)
+        self.jagged_cap = None if jagged_cap is None else tuple(int(c) for c in jagged_cap)
+        if self.jagged_cap is not None and len(self.jagged_cap) != len(rows):
+            raise ValueError(f"jagged_cap must hold one lookup count per table ({len(rows)} tables), got "
+                             f"{list(self.jagged_cap)}")
         if int(max_col_shards) == 1:
             self.sharding = TableSharding.build(rows, world, self.P)
         else:
             self.sharding = TableSharding.build(rows, world, self.P, D=D, max_col_shards=max_col_shards)
         self.split = self.sharding.split
+        if self.split and self.jagged_cap is not None:
+            raise ValueError("jagged_cap: jagged batches support table-wise plans only, and this column-wise plan "
+                             f"(max_col_shards = {max_col_shards}) splits a table")
         self.groups = self.sharding.groups(rank)
         self.rank, self.world, self.group = rank, world, group
         self.idx_base = int(idx_base)
@@ -789,6 +958,9 @@ class ShardedEmbedding:
         self.peer: Optional[PeerExchange] = None
         self.scatter_plan = None
         self._auto_update = None
+        self._count_group = None
+        if self.jagged_cap is not None and world > 1:
+            self._count_group = count_group if count_group is not None else gloo_group(group)
 
     # ---- column-wise plans: one handle / index block / gradient per width group -------------------------
     def _forward_cw(self, idx_local, Bl: int) -> torch.Tensor:
@@ -888,7 +1060,12 @@ class ShardedEmbedding:
     def _fuse_sort(self, idx_owned) -> bool:
         """Whether every owned table's sort fits the lookup launch (B_global * P_k <= FUSED_SORT_MAX); otherwise
         the large sorts go to the side stream (`sort_async`), off the critical path."""
-        from .embedding import PackedIndices
+        from .embedding import JaggedIndices, PackedIndices
+        if isinstance(idx_owned, JaggedIndices):
+            # no jagged sort rides inside the lookup launch.  With the fused backward the sort goes to the side stream
+            # and finish_backward joins it before barrier(2); without it the _sort_ form sorts on this stream ahead of
+            # barrier(1), so no peer's next index scatter can overwrite the owner batch while the sort reads it
+            return self.scatter_plan is None
         if isinstance(idx_owned, PackedIndices):
             return max(idx_owned.P) * idx_owned.B <= self.tables.FUSED_SORT_MAX
         return idx_owned.shape[1] * idx_owned.shape[2] <= self.tables.FUSED_SORT_MAX
@@ -896,7 +1073,11 @@ class ShardedEmbedding:
     def _indices(self, idx_local):
         """A handle with one P refuses mixed widths; one with per-table P takes PackedIndices or anything
         `_as_index_tensor` normalises (the reference's mixed list, or a [ntab][B][P] tensor when every P_k
-        is equal) and checks the widths against its P."""
+        is equal) and checks the widths against its P.  A handle created with ``jagged_cap`` takes JaggedIndices
+        only, every other handle refuses them."""
+        from .embedding import JaggedIndices
+        if isinstance(idx_local, JaggedIndices) or self.jagged_cap is not None:
+            return self._jagged_indices(idx_local)
         if self.P is None:
             _require_uniform_pooling(idx_local)
             if self.split:       # column-wise plans exchange through the per-table-P machinery
@@ -920,9 +1101,32 @@ class ShardedEmbedding:
             raise ValueError(f"batch widths {list(idx.P)} differ from the handle's P {list(self.P)}")
         return idx
 
+    def _jagged_indices(self, idx_local):
+        from .embedding import JaggedIndices
+        if self.jagged_cap is None:
+            raise ValueError("jagged batches need a handle created with jagged_cap (the most lookups of each table in "
+                             "one rank's batch)")
+        if not isinstance(idx_local, JaggedIndices):
+            raise ValueError(f"a handle created with jagged_cap takes JaggedIndices, got {type(idx_local).__name__}")
+        if len(idx_local) != self.ntab:
+            raise ValueError(f"indices must hold one table per table of the handle: {self.ntab} tables, got "
+                             f"{len(idx_local)}")
+        over = [k for k in range(self.ntab) if idx_local.L[k] > self.jagged_cap[k]]
+        if over:
+            k = over[0]
+            raise ValueError(f"table {k} has {idx_local.L[k]} lookups, more than jagged_cap[{k}] = {self.jagged_cap[k]}")
+        tables = getattr(self, "tables", None)
+        return idx_local if tables is None else idx_local.to(tables.device, non_blocking=True)
+
     def _exchange_indices(self, idx_local: torch.Tensor) -> torch.Tensor:
         """Index columns to the tables' owners: peer stores + flag barrier when the index buffers are
-        mapped (`enable_index_exchange`), NCCL all-to-all otherwise."""
+        mapped (`enable_index_exchange`), NCCL all-to-all otherwise.  Jagged batches first gather every rank's
+        lookup counts on the host."""
+        if self.jagged_cap is not None:
+            counts = exchange_jagged_counts(idx_local, self._count_group)
+            if self.peer is not None and self.peer._jag is not None:
+                return self.peer.scatter_jagged(idx_local, counts)
+            return exchange_indices_jagged(idx_local, counts, self.sharding, self.rank, self.group)
         if self.split:
             if self.peer is not None and self.peer._idx_dests is not None:
                 return self.peer.scatter_indices(idx_local)
@@ -952,12 +1156,15 @@ class ShardedEmbedding:
         self.owned_grad = self.peer.G
 
     def enable_peer_exchange(self, B_local: int, barrier: Optional[Callable] = None, flag_barrier: bool = True,
-                             P: Optional[Union[int, Sequence[int]]] = None, idx_bytes: int = 4) -> None:
+                             P: Optional[Union[int, Sequence[int]]] = None, idx_bytes: int = 4,
+                             weighted: bool = False) -> None:
         """Switch the forward exchange to the fused lookup + NVLink peer-store kernel.  Safe with
         one buffer per rank when every step also runs the backward exchange (a barrier all ranks
         reach only after they have finished reading T).  With ``P`` (lookups per sample, or the handle's
         per-table pooling factors) given, the index exchange also goes over peer stores instead of an NCCL
-        all-to-all."""
+        all-to-all; for a handle created with ``jagged_cap`` that is the jagged exchange
+        (:meth:`PeerExchange.enable_jagged_index_exchange`), ``weighted`` saying whether its batches carry per-sample
+        weights."""
         if self.P is not None and P is not None and tuple(int(p) for p in P) != self.P:
             raise ValueError(f"P {list(P)} differs from the handle's per-table P {list(self.P)}")
         if self.world == 1:
@@ -970,27 +1177,38 @@ class ShardedEmbedding:
             self.tables.set_slot_map([1 + k for k in self.local_ids] or [1])
         self.peer = PeerExchange(B_local, self.ntab, self.D, self.rank, self.world, self.tables.device,
                                  self.group, barrier, flag_barrier)
-        if P is not None:
+        if P is not None and self.jagged_cap is not None:
+            self.peer.enable_jagged_index_exchange(self.sharding, B_local, self.jagged_cap, idx_bytes, weighted)
+        elif P is not None:
             self.peer.enable_index_exchange(self.sharding, B_local, P, idx_bytes)
 
     @classmethod
     def create(cls, rows: Sequence[int], D: int, B_local: int, P: Union[int, Sequence[int]], rank: int, world: int,
                device, group=None, seed: int = 51234, idx_base: int = 0, dtype=None,
-               max_col_shards: int = 1) -> "ShardedEmbedding":
+               max_col_shards: int = 1, jagged_cap: Optional[Sequence[int]] = None,
+               count_group=None) -> "ShardedEmbedding":
         """``P``: lookups per sample of every table, or a sequence of one pooling factor per table (mixed
         multi-hot; the plan then weighs each table by its P_k, see :class:`TableSharding`).  ``max_col_shards``:
-        split hot tables by columns (one EmbeddingTables per width group of this rank)."""
+        split hot tables by columns (one EmbeddingTables per width group of this rank).  ``jagged_cap``: the handle
+        takes JaggedIndices (see :class:`ShardedEmbedding`); ``P`` are then the plan's weights, each table's expected
+        bag length, and the tables are sized for world * max(jagged_cap[k]) lookups of an owned table."""
         from .embedding import EmbeddingTables
         Pseq = None if isinstance(P, (int, np.integer)) else tuple(int(p) for p in P)
         if int(max_col_shards) != 1:
             sh = TableSharding.build(rows, world, Pseq, D=D, max_col_shards=max_col_shards)
+            if sh.split and jagged_cap is not None:
+                raise ValueError("jagged_cap: jagged batches support table-wise plans only, and this column-wise plan "
+                                 f"(max_col_shards = {max_col_shards}) splits a table")
             if sh.split:
                 return cls._create_cw(rows, D, B_local, P, Pseq, rank, world, device, group, seed, idx_base, dtype,
                                       max_col_shards)
         sh = TableSharding.build(rows, world, Pseq)
         mine = sh.local[rank]
         kw = {} if dtype is None else {"dtype": dtype}
-        max_lookups = B_local * world * (P if Pseq is None else max([Pseq[k] for k in mine] or [1]))
+        if jagged_cap is not None:
+            max_lookups = world * max([int(jagged_cap[k]) for k in mine] or [1])
+        else:
+            max_lookups = B_local * world * (P if Pseq is None else max([Pseq[k] for k in mine] or [1]))
         tables = EmbeddingTables([rows[k] for k in mine] or [1], D, max_lookups, device, **kw)
         tables.init_uniform(seed + 7919 * rank)
         fused_sort = world == 1      # single GPU: the sort rides in the lookup launch
@@ -1000,7 +1218,7 @@ class ShardedEmbedding:
                      tables.update_sorted(g, slot0, lr) if presorted else tables.bwd_sgd(idx, g, slot0, lr, idx_base)),
                  group=group,
                  sort_fn=lambda idx: tables.sort(idx, idx_base, side_stream=True),
-                 idx_base=idx_base, lookup_sorts=fused_sort, P=Pseq)
+                 idx_base=idx_base, lookup_sorts=fused_sort, P=Pseq, jagged_cap=jagged_cap, count_group=count_group)
         se.tables = tables
         return se
 

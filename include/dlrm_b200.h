@@ -361,6 +361,25 @@ int32_t dlrmb_embedding_fwd_p2p_sort_mp(dlrmb_tables* t, const void* idx, int32_
                                         int32_t B_global, const int32_t* P, float* const* peer_T, int32_t world,
                                         int32_t B_local, int32_t slots, dlrmb_stream stream);
 
+/* Jagged bags (variable length, the layout of dlrmb_embedding_fwd_jagged): `values` / `offsets` / `weights` are the
+ * owner's jagged batch of its tables at B = B_global (dlrmb_indices_scatter_p2p_jagged below fills it: bag
+ * j * B_global + h * B_local + b is rank h's bag b of the owner's table j) and `L` its host [ntab] lookup counts.  The
+ * pooled rows are bit-identical to dlrmb_embedding_fwd_jagged's (pooling 0 sum, 1 mean) or, with `weights` non-null,
+ * to dlrmb_embedding_fwd_jagged_weighted's (then pooling must be 0).  They land as for dlrmb_embedding_fwd_p2p_mp.
+ * Arguments are checked as for dlrmb_embedding_fwd_jagged and the p2p entry points (L[k] <= max_lookups, B_global =
+ * B_local * world; DLRMB_ESTATE without a slot map).  The _sort_ form then sorts the batch for the coming
+ * dlrmb_embedding_update_sorted as dlrmb_embedding_sort_jagged / _weighted do (dlrmb_sort_dedup_export works after
+ * it).  No allocation, synchronisation or host copy: graph-capturable.  The weights' gradient of a sharded batch
+ * (dlrmb_embedding_weight_grad_jagged returned to the samples' ranks) is not provided. */
+int32_t dlrmb_embedding_fwd_p2p_jagged(dlrmb_tables* t, const void* values, const void* offsets, const float* weights,
+                                       int32_t idx_bytes, int32_t idx_base, int32_t B_global, const int64_t* L,
+                                       int32_t pooling, float* const* peer_T, int32_t world, int32_t B_local,
+                                       int32_t slots, dlrmb_stream stream);
+int32_t dlrmb_embedding_fwd_p2p_sort_jagged(dlrmb_tables* t, const void* values, const void* offsets,
+                                            const float* weights, int32_t idx_bytes, int32_t idx_base,
+                                            int32_t B_global, const int64_t* L, int32_t pooling, float* const* peer_T,
+                                            int32_t world, int32_t B_local, int32_t slots, dlrmb_stream stream);
+
 /* Ordering point of the fused exchanges without NCCL: a flag barrier over IPC-mapped memory, one tiny
  * kernel per call.  Every rank allocates a zero-initialised dlrmb_xbuf of dlrmb_peer_barrier_flag_bytes()
  * (its flag array, mapped by all peers) and a zero-initialised private device buffer of
@@ -406,6 +425,25 @@ int32_t dlrmb_indices_scatter_p2p_mp(int32_t device, const void* idx_local, int3
 int32_t dlrmb_indices_scatter_p2p_mp_list(int32_t device, const void* idx_local, int32_t idx_bytes, int32_t ntab,
                                           int32_t B_local, const int32_t* P, int32_t ndest, const int32_t* dest_table,
                                           const void* const* dests_dev, int32_t rank, dlrmb_stream stream);
+
+/* Jagged bags: this rank's jagged batch of B_local bags per table (values, offsets [ntab * B_local + 1] of width
+ * idx_bytes, and per-sample `weights` or null) goes into the owners' jagged batches over the global batch.  Host
+ * arrays: owner[ntab] (the plan), L_all[world][ntab] (every rank's lookup counts of this step), cap_values[world]
+ * (entries each owner's values buffer holds) and peer_values / peer_offsets / peer_weights[world] (device pointers of
+ * the owners' mapped buffers; peer_weights null exactly when weights is null).  For owner o with tables j = 0..t-1
+ * in ascending global id k_j, L_own[j] = sum over h of L_all[h][k_j]: table j's block of values starts at
+ * L_own[0] + .. + L_own[j-1], rank h's entries inside it after those of ranks h' < h, in their own order; offsets has
+ * t * B_global + 1 entries, bag j * B_global + h * B_local + b being rank h's bag b of k_j, rebased; weights sit in the
+ * positions of their values.  One launch stores this rank's values (and weights) and B_local offsets of every table;
+ * rank world - 1 also writes each table's closing entry (j + 1) * B_global.  DLRMB_EINVAL, before any launch, when an
+ * owner's total exceeds cap_values[o], a 4-byte total reaches 2^31, or weights and peer_weights disagree.  Follow with
+ * dlrmb_peer_barrier.  No allocation; graph-capturable.  (NCCL exchanges of jagged batches and column-wise splits of
+ * jagged tables are not provided: dlrmb_comm_a2a_indices* and the _list scatter stay fixed-width.) */
+int32_t dlrmb_indices_scatter_p2p_jagged(int32_t device, const void* values, const void* offsets, const float* weights,
+                                         int32_t idx_bytes, int32_t ntab, int32_t B_local, const int32_t* owner,
+                                         const int64_t* L_all, int32_t world, int32_t rank, void* const* peer_values,
+                                         void* const* peer_offsets, float* const* peer_weights,
+                                         const int64_t* cap_values, dlrmb_stream stream);
 
 /* Interaction backward fused with the gradient exchange: as dlrmb_interaction_bwd, but the gradient
  * row of feature slot f >= 1 of local sample b is stored at
